@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo's CUDA path (one rank per GPU)
   python bench.py --impl reference ...                         # the reference's qpOASES CPU path (oracle/_ref)
+  python bench.py ... --dump-outputs DIR                       # + the last timed step's result records as DIR/*.npy
 
 A "step" is one tick of MPCSolver::solve (formulation C: vertical QP + x QP + y QP = 3 QP solves per instance)
 over one batch of synthetic instances: BASELINE.json configs[1], 1,024 independent trot instances, N = 100,
@@ -207,6 +208,28 @@ def spread(xs):
     return {"n": len(xs), "median": statistics.median(xs), "min": xs[0], "max": xs[-1]}
 
 
+DUMP_MAX_BYTES = 64_000_000
+NPY_HEADER_BYTES = 256          # an upper bound of np.save's header for these arrays (version 1.0 writes 128)
+
+
+def dump_records(d, rec):
+    """The result records of the timed path's last step (FORMC_OUT: what a caller of ismpc_formc_solve_batch receives),
+    one float64 array per field as d/<field>.npy, nested fields joined by '_' (next_com_pos, ...).  `instance.npy` holds
+    each row's index in the batch: where the files would exceed DUMP_MAX_BYTES in all, headers included, a fixed seeded
+    sample of the instances is written."""
+    fields = [("next_" + f, rec["next"][f]) for f in rec["next"].dtype.names]
+    fields += [(f, rec[f]) for f in rec.dtype.names if f != "next"]
+    per_row = 8 * (1 + sum(int(np.prod(a.shape[1:], dtype=np.int64)) for _, a in fields))
+    max_rows = (DUMP_MAX_BYTES - NPY_HEADER_BYTES * (len(fields) + 1)) // per_row
+    idx = np.arange(len(rec))
+    if len(rec) > max_rows:
+        idx = np.sort(np.random.default_rng(0).choice(len(rec), max_rows, replace=False))
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "instance.npy"), idx.astype(np.float64))
+    for name, a in fields:
+        np.save(os.path.join(d, name + ".npy"), np.ascontiguousarray(a[idx], dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -219,8 +242,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-form-a", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the horizon sweep and the dense-seam leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result records of the last timed step as DIR/<field>.npy (float64), for comparing builds")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the CUDA path (--impl b200)")
         return run_reference(args)
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -592,8 +619,14 @@ def main():
     clk = clocks.stop() if clocks else None
 
     # ---- final gather of the result records (the only collective on this path) -----------------------------
+    # the arms timed after the headline write the same output slots with other builds: replay the headline graph once, so
+    # that the records are those of the timed path's last step
+    (gt if use_thr else gp if use_pdl else g).replay()
+    torch.cuda.synchronize()
     last = np.frombuffer(slots[(W + K - 1) % n_slots]["out"].cpu().numpy().tobytes(), dtype=abi.FORMC_OUT)
     full = sharding.gather_records(last.copy(), n * world, device=dev) if world > 1 else last
+    if rank == 0 and args.dump_outputs:
+        dump_records(args.dump_outputs, full)
 
     line = None
     if rank == 0:

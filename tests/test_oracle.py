@@ -9,7 +9,8 @@ from oracle import oracle as O
 from quadruped_gait_generation_ismpc_b200 import abi, plans, synth
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
-needs_ref = pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref (reference qpOASES) not built")
+needs_ref = pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built: it is the reference's qpOASES 3.2, compiled "
+                                                        "from the reference's sources, which this repository does not contain")
 
 
 def _probe_problem():
@@ -52,8 +53,7 @@ def test_known_answer_probe(kind):
     np.testing.assert_allclose(r["x"], u, atol=1e-9)
 
 
-@needs_ref
-def test_port_solver_matches_qpoases_on_random_qps():
+def _random_qps():
     rng = np.random.default_rng(0)
     n, nV, nC = 40, 12, 20
     M = rng.normal(size=(n, nV, nV))
@@ -64,6 +64,37 @@ def test_port_solver_matches_qpoases_on_random_qps():
     lb = ax - rng.uniform(0.0, 1.0, size=(n, nC)); ub = ax + rng.uniform(0.0, 1.0, size=(n, nC))
     lb[:, :2] = ub[:, :2] = ax[:, :2]            # two equality rows
     lb[:, 2:5] = -1e20                           # some one-sided rows
+    return H, g, A, lb, ub
+
+
+def test_port_solver_certifies_its_optimum_on_random_qps():
+    """The QPs of the qpOASES comparison below, checked without qpOASES: H > 0, so the minimiser is unique, and a point
+    with multipliers that satisfy the KKT conditions (stationarity H x + g = A' y in qpOASES' sign convention, feasibility,
+    y >= 0 on rows held at the lower bound and y <= 0 at the upper one, y = 0 off the working set) is that minimiser.
+    With independent active rows and every multiplier away from zero the working set is unique too, so x and the strongly
+    active rows are what any exact solver -- qpOASES included -- returns."""
+    H, g, A, lb, ub = _random_qps()
+    p = O.qp_batch(H, g, A, lb, ub, solver=O.SOLVER_PORT, kind="port")
+    assert (p["ret"] == 0).all()
+    x, y, ws = p["x"], p["y"], p["ws"]
+    stat = np.einsum("nij,nj->ni", H, x) + g - np.einsum("nci,nc->ni", A, y)
+    assert np.abs(stat).max() < 1e-10 * max(1.0, np.abs(g).max())
+    ax = np.einsum("nij,nj->ni", A, x)
+    assert (ax - lb).min() > -1e-10 and (ub - ax).min() > -1e-10
+    eq = lb == ub
+    lo, up = (ws == -1) & ~eq, ws == 1
+    assert (ws[eq] != 0).all() and (y[ws == 0] == 0).all()
+    assert np.abs(ax - lb)[lo | eq].max() < 1e-10 and np.abs(ub - ax)[up].max() < 1e-10
+    assert (y[lo] > 1e-7).all() and (y[up] < -1e-7).all()           # strictly complementary: no weak row
+    for i in range(len(H)):
+        act = A[i][ws[i] != 0]
+        assert np.linalg.matrix_rank(act) == len(act)
+    assert lo.any() and up.any()                                     # not vacuous: rows held at both bounds
+
+
+@needs_ref
+def test_port_solver_matches_qpoases_on_random_qps():
+    H, g, A, lb, ub = _random_qps()
     r = O.qp_batch(H, g, A, lb, ub, solver=O.SOLVER_QPOASES, kind="ref")
     p = O.qp_batch(H, g, A, lb, ub, solver=O.SOLVER_PORT, kind="ref")
     assert (r["ret"] == 0).all() and (p["ret"] == 0).all()
@@ -236,7 +267,7 @@ def _riccati_vertical(model, state, walk, inst, plan, i):
 
 def test_vertical_qp_is_an_lq_tracking_problem():
     """The identity the warp kernels build on: the Riccati solution of the LQ problem IS the minimiser of the condensed
-    vertical QP that the oracle solves with qpOASES (instances without an active row of 0 <= S f <= fz_max)."""
+    vertical QP that the oracle solves (instances without an active row of 0 <= S f <= fz_max)."""
     model = abi.formc_model()
     state, walk, inst, plan = synth.formc_batch(48, seed=3, running_frac=0.7, vary_height=True)
     rng = np.random.default_rng(0)
@@ -245,7 +276,9 @@ def test_vertical_qp_is_an_lq_tracking_problem():
     N = 100
     checked = 0
     for i in range(len(state)):
-        if o["ret"][i][0] != 0 or o["nwsr"][i][0] != 0 or (o["out"]["status"][i] & abi.ST_WINDOW):
+        # the final working set, not the iteration count: the portable solver counts every equality row it adds as an
+        # iteration, qpOASES starts with them in its working set
+        if o["ret"][i][0] != 0 or o["active"][i][:N].any() or (o["out"]["status"][i] & abi.ST_WINDOW):
             continue
         f = _riccati_vertical(model, state, walk, inst, plan, i)
         ref = o["primal"][i][:N]
