@@ -453,6 +453,22 @@ int ismpc_qp_solve_batch(ismpc_handle* h, int n, int nV, int nC,
                          double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
                          int mem, void* stream);
 
+/* ismpc_qp_solve_batch hot-started from a guessed working set (qpOASES' init(..., guessedBounds, guessedConstraints)):
+ * ws_guess: n x nC int8 in the ws_opt convention, -1 lower active / +1 upper active / 0 inactive (any negative value
+ * reads as -1, any positive as +1); it lives where mem says and may be the same buffer as ws_opt, so that a loop can
+ * feed each call's working set into the next call in place.  ws_guess = NULL is ismpc_qp_solve_batch.
+ * A guess is never trusted: entries of equality rows (always active), entries on an infinite side (|bound| >= 1e20),
+ * and guessed rows linearly dependent on those already installed or beyond nV independent rows are ignored (the row
+ * starts free); guessed rows whose multiplier comes out with the wrong sign are dropped again.  The results are those
+ * of the cold call to rounding for any guess: the same primal, strongly active set, duals and status bits.
+ * iters_opt counts the working-set changes made after the guess is installed: guessed rows dropped for a wrong-signed
+ * multiplier plus the adds and drops of the active-set loop, so the exact optimal working set as the guess gives 0. */
+int ismpc_qp_solve_batch_ws(ismpc_handle* h, int n, int nV, int nC,
+                            const double* H, const double* g, const double* A,
+                            const double* lbA, const double* ubA, const int8_t* ws_guess,
+                            double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
+                            int mem, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

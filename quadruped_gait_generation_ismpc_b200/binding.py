@@ -21,7 +21,7 @@ EXPORTS = ["ismpc_version", "ismpc_error_string", "ismpc_create", "ismpc_destroy
            "ismpc_plan_generate", "ismpc_kf_init", "ismpc_kf_filter_batch", "ismpc_formc_set_plan",
            "ismpc_handle_stream", "ismpc_wait", "ismpc_host_alloc", "ismpc_host_free", "ismpc_formc_rollout_ex",
            "ismpc_forma_rollout_ex2", "ismpc_kf_filter_batch_f64", "ismpc_formc_set_instances",
-           "ismpc_formc_solve_batch_packed"]
+           "ismpc_formc_solve_batch_packed", "ismpc_qp_solve_batch_ws"]
 
 _lib = None
 
@@ -90,6 +90,7 @@ def lib():
     L.ismpc_kf_filter_batch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
     L.ismpc_kf_filter_batch_f64.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
     L.ismpc_qp_solve_batch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 10 + [C.c_int, C.c_void_p]
+    L.ismpc_qp_solve_batch_ws.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 11 + [C.c_int, C.c_void_p]
     L.ismpc_handle_stream.restype = C.c_void_p
     L.ismpc_handle_stream.argtypes = [C.c_void_p]
     L.ismpc_wait.argtypes = [C.c_void_p, C.c_void_p]
@@ -402,14 +403,22 @@ class Handle:
         self._check(rc, "ismpc_forma_rollout")
 
     def qp_solve_batch_raw(self, n, nV, nC, H, g, A, lbA, ubA, x, y=None, ws=None, status=None, iters=None,
-                           mem=abi.MEM_DEVICE, stream=None):
-        rc = self._L.ismpc_qp_solve_batch(self._h, n, nV, nC, _ptr(H), _ptr(g), _ptr(A), _ptr(lbA), _ptr(ubA), _ptr(x),
-                                          _ptr(y), _ptr(ws), _ptr(status), _ptr(iters), mem,
-                                          C.c_void_p(stream) if stream else None)
-        self._check(rc, "ismpc_qp_solve_batch")
+                           mem=abi.MEM_DEVICE, stream=None, ws_guess=None):
+        """ws_guess (a pointer, may equal ws): hot start from that working set (ismpc_qp_solve_batch_ws)."""
+        st = C.c_void_p(stream) if stream else None
+        if ws_guess is None:
+            rc = self._L.ismpc_qp_solve_batch(self._h, n, nV, nC, _ptr(H), _ptr(g), _ptr(A), _ptr(lbA), _ptr(ubA), _ptr(x),
+                                              _ptr(y), _ptr(ws), _ptr(status), _ptr(iters), mem, st)
+            self._check(rc, "ismpc_qp_solve_batch")
+            return
+        rc = self._L.ismpc_qp_solve_batch_ws(self._h, n, nV, nC, _ptr(H), _ptr(g), _ptr(A), _ptr(lbA), _ptr(ubA),
+                                             _ptr(ws_guess), _ptr(x), _ptr(y), _ptr(ws), _ptr(status), _ptr(iters), mem, st)
+        self._check(rc, "ismpc_qp_solve_batch_ws")
 
     # ---- generic dense QP (solveQP seam) ----------------------------------------------------------
-    def qp_solve_batch(self, H, g, A, lbA, ubA):
+    def qp_solve_batch(self, H, g, A, lbA, ubA, ws_guess=None):
+        """ws_guess (n x nC int8, <0 lower / >0 upper / 0 free, e.g. the "ws" of an earlier call): hot start from that
+        working set; the results are those of the cold call to rounding, "iters" counts the changes made after it."""
         H = np.ascontiguousarray(H, dtype=np.float64); g = np.ascontiguousarray(g, dtype=np.float64)
         A = np.ascontiguousarray(A, dtype=np.float64)
         lbA = np.ascontiguousarray(lbA, dtype=np.float64); ubA = np.ascontiguousarray(ubA, dtype=np.float64)
@@ -417,9 +426,18 @@ class Handle:
         nC = A.shape[1]
         x = np.zeros((n, nV)); y = np.zeros((n, nC)); ws = np.zeros((n, nC), dtype=np.int8)
         status = np.zeros(n, dtype=np.int32); iters = np.zeros(n, dtype=np.int32)
-        rc = self._L.ismpc_qp_solve_batch(self._h, n, nV, nC, _ptr(H), _ptr(g), _ptr(A), _ptr(lbA), _ptr(ubA),
-                                          _ptr(x), _ptr(y), _ptr(ws), _ptr(status), _ptr(iters), abi.MEM_HOST, None)
-        self._check(rc, "ismpc_qp_solve_batch")
+        if ws_guess is None:
+            rc = self._L.ismpc_qp_solve_batch(self._h, n, nV, nC, _ptr(H), _ptr(g), _ptr(A), _ptr(lbA), _ptr(ubA),
+                                              _ptr(x), _ptr(y), _ptr(ws), _ptr(status), _ptr(iters), abi.MEM_HOST, None)
+            self._check(rc, "ismpc_qp_solve_batch")
+            return dict(x=x, y=y, ws=ws, status=status, iters=iters)
+        guess = np.ascontiguousarray(ws_guess, dtype=np.int8)
+        if guess.shape != (n, nC):
+            raise ValueError("ws_guess must be %d x %d, got %s" % (n, nC, guess.shape))
+        rc = self._L.ismpc_qp_solve_batch_ws(self._h, n, nV, nC, _ptr(H), _ptr(g), _ptr(A), _ptr(lbA), _ptr(ubA),
+                                             _ptr(guess), _ptr(x), _ptr(y), _ptr(ws), _ptr(status), _ptr(iters),
+                                             abi.MEM_HOST, None)
+        self._check(rc, "ismpc_qp_solve_batch_ws")
         return dict(x=x, y=y, ws=ws, status=status, iters=iters)
 
 

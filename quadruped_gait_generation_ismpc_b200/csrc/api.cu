@@ -969,21 +969,23 @@ extern "C" int ismpc_kf_filter_batch_f64(ismpc_handle* h, int n, int n_steps, co
 // ---------------------------------------------------------------------------------------------------
 // Generic dense QP (solveQP seam)
 // ---------------------------------------------------------------------------------------------------
-extern "C" int ismpc_qp_solve_batch(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* g,
-                                    const double* A, const double* lbA, const double* ubA, double* x, double* y_opt,
-                                    int8_t* ws_opt, int32_t* status, int32_t* iters_opt, int mem, void* stream)
+extern "C" int ismpc_qp_solve_batch_ws(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* g,
+                                       const double* A, const double* lbA, const double* ubA, const int8_t* ws_guess,
+                                       double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
+                                       int mem, void* stream)
 {
     if (!h) return ISMPC_ERR_ARG;
     if (n < 0 || n > h->max_batch || nV < 1 || nV > ISMPC_MAX_N || nC < 0 || nC > 2 * ISMPC_MAX_N + 8 || !H || !g ||
         (nC > 0 && (!A || !lbA || !ubA)) || !x || !status)
         return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
+    if (nC == 0) ws_guess = nullptr;           // nothing to guess
     CK(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
     if (h->q_work.ensure(qp_dense_work_doubles(n, nV, nC) * sizeof(double))) return ISMPC_ERR_ALLOC;
     if (mem == ISMPC_MEM_DEVICE) {
-        int rc = qp_dense_launch(n, nV, nC, H, g, A, lbA, ubA, x, y_opt, (signed char*)ws_opt, status, iters_opt,
-                                 (double*)h->q_work.p, h->opt_dense_dmma, st);
+        int rc = qp_dense_launch(n, nV, nC, H, g, A, lbA, ubA, (const signed char*)ws_guess, x, y_opt, (signed char*)ws_opt,
+                                 status, iters_opt, (double*)h->q_work.p, h->opt_dense_dmma, st);
         h->launches += 1;
         if (rc) return fail_cuda(h, (cudaError_t)rc, "qp_dense_launch");
         return ISMPC_OK;
@@ -1004,7 +1006,10 @@ extern "C" int ismpc_qp_solve_batch(ismpc_handle* h, int n, int nV, int nC, cons
         CK(cudaMemcpyAsync(dlb, lbA, szb * sizeof(double), cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(dub, ubA, szb * sizeof(double), cudaMemcpyHostToDevice, st));
     }
-    int rc = qp_dense_launch(n, nV, nC, dH, dg, dA, dlb, dub, dx, dy, dws, dst, dit, (double*)h->q_work.p, h->opt_dense_dmma, st);
+    // the guess is staged where the working set comes out: each problem's warp reads its row before it writes it
+    if (ws_guess) CK(cudaMemcpyAsync(dws, ws_guess, szb, cudaMemcpyHostToDevice, st));
+    int rc = qp_dense_launch(n, nV, nC, dH, dg, dA, dlb, dub, ws_guess ? dws : nullptr, dx, dy, dws, dst, dit,
+                             (double*)h->q_work.p, h->opt_dense_dmma, st);
     h->launches += 1;
     if (rc) return fail_cuda(h, (cudaError_t)rc, "qp_dense_launch");
     CK(cudaMemcpyAsync(x, dx, szg * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -1014,6 +1019,13 @@ extern "C" int ismpc_qp_solve_batch(ismpc_handle* h, int n, int nV, int nC, cons
     if (iters_opt) CK(cudaMemcpyAsync(iters_opt, dit, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return ISMPC_OK;
+}
+
+extern "C" int ismpc_qp_solve_batch(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* g,
+                                    const double* A, const double* lbA, const double* ubA, double* x, double* y_opt,
+                                    int8_t* ws_opt, int32_t* status, int32_t* iters_opt, int mem, void* stream)
+{
+    return ismpc_qp_solve_batch_ws(h, n, nV, nC, H, g, A, lbA, ubA, nullptr, x, y_opt, ws_opt, status, iters_opt, mem, stream);
 }
 
 // ---------------------------------------------------------------------------------------------------

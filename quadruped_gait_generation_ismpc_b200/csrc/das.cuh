@@ -31,6 +31,10 @@
 //                   double* z)          z = H^-1 (sgp*a_idp - sum_k wsg_k r_k a_{wid_k})  (shared memory out)
 //   int    nvar()
 //   void   on_step(double t)            called after x += t*z (policies that maintain row values incrementally)
+// and, for the warm start (das_warm_install) only:
+//   double rv0(int i)                   a_i' x0, x0 = -H^-1 g the unconstrained minimiser
+//   void   combine(const int* wid, const signed char* wsg, const double* mu, int q, double* x)
+//                                       x = x0 + sum_k mu_k wsg_k H^-1 a_{wid_k}, and the row values that go with it
 #pragma once
 #include "common.cuh"
 
@@ -296,6 +300,101 @@ __device__ int das_solve(P& prob, DasWork& w, double* x, double* rv, double* z, 
 done:
     *iters_out = iters;
     return rc;
+}
+
+// Append (p, sgp) factor only, unless it is dependent on the entries in W.  Returns whether it was appended.
+template <class P>
+__device__ bool das_factor_append(const P& prob, DasWork& w, int p, int sgp)
+{
+    const double spp = das_schur_col(prob, w, p, sgp);
+    const double zn = spp - das_apply_J(w);
+    if (!(zn > 1e-13 * spp)) return false;
+    das_apply_Jt(w);
+    das_append(w, p, sgp, zn, 0.0);
+    if (lane_id() == 0) w.state[p] = (signed char)(sgp > 0 ? -1 : +1);
+    __syncwarp();
+    return true;
+}
+
+// Warm start (the role of qpOASES' init with guessed bounds / constraints): on entry W holds the equalities and x is the
+// minimiser over them.  The guessed inequality entries are installed in row order, FACTOR ONLY -- Schur column, J update,
+// append; a row dependent on those installed, or beyond nvar rows, is skipped -- without moving x per row (a step per row
+// reads q rows of the step tables, the cost of one cold iteration).  Then, with S = N'H^-1 N over W,
+//     mu = S^-1 (beta_W - N_W' x0) = J'J (beta_W - N_W' x0)     (the minimiser over W with its rows held active),
+// and while an inequality entry has mu_k < -tau the most negative one is dropped (a Givens downdate of J, O(q^2)) and mu
+// recomputed.  Only then is x recombined, once: x = x0 + sum_k mu_k n_k through the tables.  On return x is stationary
+// for (W, mu) with mu >= 0 on the inequality entries -- the invariant das_solve starts from.
+// guess(i) (called by the lane that owns row i): the normal sign of row i's usable guess, +1 lower / -1 upper, or 0 for
+// none (the caller filters equality rows and infinite sides).  Returns the number of guessed entries dropped (each is one
+// working-set change).
+template <class P, class Guess>
+__device__ int das_warm_install(P& prob, DasWork& w, double* x, const Guess& guess)
+{
+    const int lane = lane_id();
+    const int m = prob.m();
+    const int n = prob.nvar();
+    const int q0 = w.q;
+    for (int base = 0; base < m; base += 32) {
+        const int i = base + lane;
+        int sg = 0;
+        if (i < m) sg = guess(i);
+        unsigned cand = __ballot_sync(ISMPC_FULL_MASK, sg != 0);
+        while (cand) {
+            const int b = __ffs(cand) - 1;
+            cand &= cand - 1;
+            const int p = base + b;
+            const int sgp = __shfl_sync(ISMPC_FULL_MASK, sg, b);
+            if (w.q >= n || w.q >= w.qmax) break;
+            das_factor_append(prob, w, p, sgp);
+        }
+    }
+    if (w.q == q0) return 0;                    // nothing installed: x is the equality minimiser, as in the cold path
+    int drops = 0;
+    bool fresh = true;                          // no downdate of J since its rows were last appended
+    for (;;) {
+        for (int k = lane; k < w.q; k += 32) {
+            const int id = w.wid[k], sg = w.wsg[k];
+            w.y[k] = (double)sg * ((sg > 0 ? prob.lo(id) : prob.hi(id)) - prob.rv0(id));
+        }
+        __syncwarp();
+        das_apply_J(w);
+        das_apply_Jt(w);                         // w.r = mu
+        double big = 0.0;
+        for (int k = lane; k < w.q; k += 32) big = fmax(big, fabs(w.r[k]));
+        const double tau = 1e-12 * (1.0 + warp_max(big));
+        double worst = -tau; int l = 0x7fffffff;
+        for (int k = w.neq + lane; k < w.q; k += 32)
+            if (w.r[k] < worst) { worst = w.r[k]; l = k; }
+        warp_argmin(worst, l);
+        if (l == 0x7fffffff) {
+            if (fresh) break;
+            // Refactor the survivors before trusting their signs: a hostile guess can fill W up to nvar rows, where S is
+            // nearly singular, and the Givens downdates from there leave J too inaccurate for the multipliers (seen as a
+            // wrong-signed row kept active, 4e-7 off the minimiser on the nV = 206 shape guessed all-lower).
+            const int q1 = w.q;
+            w.q = w.neq;
+            for (int k = w.neq; k < q1; ++k) {
+                const int id = w.wid[k], sg = w.wsg[k];
+                __syncwarp();
+                if (!das_factor_append(prob, w, id, sg)) {
+                    if (lane == 0) w.state[id] = 0;
+                    __syncwarp();
+                    ++drops;
+                }
+            }
+            fresh = true;
+            continue;
+        }
+        if (lane == 0) w.state[w.wid[l]] = 0;
+        __syncwarp();
+        das_drop(w, l);
+        ++drops;
+        fresh = false;
+    }
+    for (int k = lane; k < w.q; k += 32) w.mu[k] = k < w.neq ? w.r[k] : fmax(w.r[k], 0.0);
+    __syncwarp();
+    prob.combine(w.wid, w.wsg, w.mu, w.q, x);
+    return drops;
 }
 
 }  // namespace ismpc

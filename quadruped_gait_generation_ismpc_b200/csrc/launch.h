@@ -55,8 +55,8 @@ int feet_export_launch(int n, const ismpc_feet_model_t& m, const ismpc_feet_inst
                        cudaStream_t st);
 
 int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, const double* A, const double* lbA,
-                    const double* ubA, double* x, double* y, signed char* ws, int32_t* status, int32_t* iters,
-                    double* work, int use_dmma, cudaStream_t st);
+                    const double* ubA, const signed char* ws_guess, double* x, double* y, signed char* ws,
+                    int32_t* status, int32_t* iters, double* work, int use_dmma, cudaStream_t st);
 size_t qp_dense_work_doubles(int n, int nV, int nC);
 
 }  // namespace ismpc

@@ -7,6 +7,8 @@
 // every Schur-complement entry, step direction and row-value update of the active-set loop is a coalesced
 // table lookup.  One warp per QP; the first R rows of the packed inverse factor of the working-set Schur
 // complement (das.cuh) live in shared memory, the rest in the problem's global workspace slice.
+#include <type_traits>
+
 #include "common.cuh"
 #include "das.cuh"
 #include "launch.h"
@@ -34,7 +36,9 @@ __host__ __device__ inline DenseLayout dense_layout(int nV, int nC)
     return l;
 }
 
-size_t qp_dense_work_doubles(int n, int nV, int nC) { return dense_layout(nV, nC).total * (size_t)n + 16; }
+// n problem slices, then (warm start only) n x nC doubles of A x0, kept while rv moves; outside the slices so that the
+// cold path's layout does not depend on it
+size_t qp_dense_work_doubles(int n, int nV, int nC) { return (dense_layout(nV, nC).total + nC) * (size_t)n + 16; }
 
 // ---- set-up kernels (batched over problems with blockIdx.z / blockIdx.y) --------------------------------
 __global__ void dense_copy_H(int nV, const double* H, double* work, size_t stride, size_t offL)
@@ -251,12 +255,36 @@ struct DenseProb {
     }
 };
 
+// The warm start's additions (das_warm_install): x0 and A x0, kept while x and rv move.
+struct DenseWarmProb : DenseProb {
+    const double *x0, *rv0_;
+    __device__ double rv0(int i) const { return rv0_[i]; }
+    __device__ void combine(const int* wid, const signed char* wsg, const double* mu, int q, double* x) const
+    {
+        const int lane = lane_id();
+        for (int i = lane; i < nV; i += 32) {
+            double acc = x0[i];
+            for (int k = 0; k < q; ++k) acc += (double)wsg[k] * mu[k] * D[(size_t)wid[k] * nV + i];
+            x[i] = acc;
+        }
+        for (int i = lane; i < nC; i += 32) {
+            double acc = rv0_[i];
+            for (int k = 0; k < q; ++k) acc += (double)wsg[k] * mu[k] * S[(size_t)wid[k] * nC + i];
+            rv[i] = acc;
+        }
+        __syncwarp();
+    }
+};
+
 constexpr int DENSE_R = 64;      // rows of the inverse factor kept in shared memory (16.6 KB per warp)
 constexpr int DENSE_WARPS = 4;   // QPs per CTA
 
+// WARM = false: the cold solve (ismpc_qp_solve_batch).  WARM = true: the same, started from the guessed working set
+// ws_guess (n x nC, <0 lower / >0 upper / 0 free; may alias ws) through das_warm_install after the equalities.
+template <bool WARM>
 __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const double* ubA, double* work,
                                  size_t stride, DenseLayout l, int R, double* x, double* y, signed char* ws,
-                                 int32_t* status, int32_t* iters)
+                                 int32_t* status, int32_t* iters, const signed char* ws_guess)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int p = blockIdx.x * DENSE_WARPS + warp_id();
@@ -279,7 +307,14 @@ __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const
     if (st == 0 && nC > 0) {
         for (int i = lane; i < nC; i += 32) dw.state[i] = 0;
         __syncwarp();
-        DenseProb pb{nV, nC, w + l.D, w + l.S, lb, ub, w + l.rv, w + l.az};
+        const DenseProb pb0{nV, nC, w + l.D, w + l.S, lb, ub, w + l.rv, w + l.az};
+        std::conditional_t<WARM, DenseWarmProb, DenseProb> pb{pb0};
+        if constexpr (WARM) {
+            double* rv0 = work + (size_t)n * stride + (size_t)p * nC;
+            pb.x0 = w + l.x0; pb.rv0_ = rv0;
+            for (int i = lane; i < nC; i += 32) rv0[i] = pb.rv[i];
+            __syncwarp();
+        }
         // equalities first, in row order; never dropped (enableEqualities, qpOASES/Options.cpp:191-218)
         for (int c = 0; c < nC; ++c) {
             const double lo = lb[c], hi = ub[c];
@@ -295,7 +330,20 @@ __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const
             }
         }
         dw.neq = dw.q;
+        int drops = 0;
+        if constexpr (WARM) {
+            const signed char* gp = ws_guess + (size_t)p * nC;
+            drops = das_warm_install(pb, dw, xp, [&](int i) {
+                const int gs = gp[i];
+                if (gs == 0) return 0;
+                const double lo = lb[i], hi = ub[i];
+                if (fabs(hi - lo) <= 1e-12 * fmax(1.0, fabs(lo))) return 0;          // equality rows: always active
+                if (fabs(gs < 0 ? lo : hi) >= 1e20) return 0;                         // infinite side (qpOASES INFTY)
+                return gs < 0 ? +1 : -1;
+            });
+        }
         int rc = das_solve(pb, dw, xp, pb.rv, w + l.z, 20 * (nV + nC) + 50, &it);
+        it += drops;
         if (rc != 0) st |= ISMPC_ST_QP_FAIL;
         if (y) for (int i = lane; i < nC; i += 32) y[(size_t)p * nC + i] = 0.0;
         if (ws) for (int i = lane; i < nC; i += 32) ws[(size_t)p * nC + i] = dw.state[i];
@@ -324,8 +372,8 @@ void dense_hinv_launch(int n, int nV, double* work, size_t stride, size_t offLin
 }
 
 int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, const double* A, const double* lbA,
-                    const double* ubA, double* x, double* y, signed char* ws, int32_t* status, int32_t* iters,
-                    double* work, int use_dmma, cudaStream_t st)
+                    const double* ubA, const signed char* ws_guess, double* x, double* y, signed char* ws,
+                    int32_t* status, int32_t* iters, double* work, int use_dmma, cudaStream_t st)
 {
     const DenseLayout l = dense_layout(nV, nC);
     const size_t stride = l.total;
@@ -345,9 +393,10 @@ int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, con
     dense_x0_rv<<<n, 128, 0, st>>>(nV, nC, g, A, work, stride, l, x);
     const int R = l.qmax < DENSE_R ? l.qmax : DENSE_R;
     const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
-    cudaFuncSetAttribute(dense_das_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
-    dense_das_kernel<<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
-        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters);
+    auto kern = ws_guess ? dense_das_kernel<true> : dense_das_kernel<false>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
+    kern<<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
+        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess);
     return (int)cudaGetLastError();
 }
 

@@ -198,3 +198,26 @@ def dense_qp_batch(shape, n, seed=SEED0 ^ 21):
         lb[p, :2] = ub[p, :2] = r0[:2]
         g[p] = np.concatenate([np.zeros(C), -Qf * plan[:, 0], np.zeros(C), -Qf * plan[:, 1]])
     return H, g, A, lb, ub
+
+
+def dense_qp_sequence(shape, n, T, seed=SEED0 ^ 23):
+    """T consecutive ticks of the dense_qp_batch workload, drifting a little per tick, as an MPC or IK loop would feed
+    ismpc_qp_solve_batch: tick 0 is dense_qp_batch(shape, n); from tick to tick the unconstrained minimiser -H^-1 g moves
+    by a random step and the constraint set is translated by a random step dv (lbA += A dv, ubA += A dv; infinite sides
+    stay infinite, equality rows stay equalities).  Every tick stays feasible by construction: translating the feasible
+    set of tick 0 keeps it non-empty.  Steps are 2 mm (the variables are positions in metres and velocities in m/s).
+    Returns H (n, nV, nV) and A (n, nC, nV), shared by all ticks, and g (T, n, nV), lbA / ubA (T, n, nC)."""
+    H, g0, A, lb0, ub0 = dense_qp_batch(shape, n)
+    rng = np.random.default_rng(seed)
+    nV, nC = H.shape[1], A.shape[1]
+    g = np.empty((T, n, nV)); lb = np.empty((T, n, nC)); ub = np.empty((T, n, nC))
+    dx = np.zeros((n, nV)); dv = np.zeros((n, nV))
+    for t in range(T):
+        if t:
+            dx += 2e-3 * rng.standard_normal((n, nV))
+            dv += 2e-3 * rng.standard_normal((n, nV))
+        g[t] = g0 - np.einsum("nij,nj->ni", H, dx)
+        adv = np.einsum("nij,nj->ni", A, dv)
+        lb[t] = np.where(np.abs(lb0) >= 1e20, lb0, lb0 + adv)
+        ub[t] = np.where(np.abs(ub0) >= 1e20, ub0, ub0 + adv)
+    return H, g, A, lb, ub
