@@ -211,6 +211,9 @@ void ismpc_host_free(void* p);
  *   "host_zero_copy":     ismpc_formc_solve_batch_packed with host buffers: 1 (default; ISMPC_HOST_ZERO_COPY sets the default at
  *                         creation) = the kernel reads / writes pinned host buffers itself, 0 = staging buffers and copies.
  *   "dense_dmma":         ismpc_qp_solve_batch: 1 = condensing GEMMs on the FP64 tensor cores (DMMA, default), 0 = CUDA cores.
+ *   "dense_resident_gemm": ismpc_qp_hotstart_batch against a single shared set: 1 (default) = the unconstrained minimisers
+ *                         x0 = -H^-1 g and A x0 of the whole batch as one FP64 tensor-core product (the same answers to
+ *                         rounding), 0 = the per-problem mat-vecs of ismpc_qp_solve_batch (the same bytes).
  * See DESIGN.md section 4. */
 int ismpc_set_option(ismpc_handle* h, const char* name, int value);
 
@@ -466,6 +469,31 @@ int ismpc_qp_solve_batch(ismpc_handle* h, int n, int nV, int nC,
 int ismpc_qp_solve_batch_ws(ismpc_handle* h, int n, int nV, int nC,
                             const double* H, const double* g, const double* A,
                             const double* lbA, const double* ubA, const int8_t* ws_guess,
+                            double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
+                            int mem, void* stream);
+
+/* Resident matrices for the dense seam (qpOASES' QProblem::init keeps H and A, and QProblem::hotstart re-solves with new
+ * g, lbA, ubA against the factorisation it has).  n_mat matrix sets of one shape: H n_mat x nV x nV, A n_mat x nC x nV
+ * (row-major).  n_mat = 1: one set shared by every problem of the later calls; n_mat > 1: sets picked per problem;
+ * n_mat = 0 forgets them.  The call copies H and A to memory owned by the handle, builds the factor and the condensing
+ * tables on the device (the set-up ismpc_qp_solve_batch repeats on every call) and synchronises; mem = ISMPC_MEM_HOST or
+ * ISMPC_MEM_DEVICE says where H and A live.  mat_status_opt (nullable, n_mat int32, host memory): ISMPC_ST_QP_FAIL for a set
+ * whose H is not positive definite, 0 otherwise; the problems of such a set fail.  Setting again replaces the sets (any
+ * shape).  Like ismpc_formc_set_instances: call while no work of this handle is in flight.  Cold calls of the seam on the
+ * same handle, of any shape, and the form-C / form-A calls leave the resident sets alone. */
+int ismpc_qp_set_matrices(ismpc_handle* h, int n_mat, int nV, int nC, const double* H, const double* A,
+                          int32_t* mat_status_opt, int mem);
+
+/* ismpc_qp_solve_batch_ws against the resident sets: only g (n x nV), lbA / ubA (n x nC) and the optional guess move.
+ * mat_index_opt (nullable, n int32, where mem says): the set of problem p; NULL = set p (n_mat > 1, which needs
+ * n <= n_mat) or set 0 (n_mat = 1).  An index outside [0, n_mat) flags that problem ISMPC_ST_QP_FAIL with iters 0 and
+ * leaves its rows of x, y_opt and ws_opt as they were; the other problems are unaffected.
+ * ws_guess: as in ismpc_qp_solve_batch_ws (NULL = cold start; may alias ws_opt).  Results and iters as that call: with
+ * the same H and A, per problem, the bytes of ismpc_qp_solve_batch_ws; with a single shared set and "dense_resident_gemm"
+ * = 1 (default) the same answers to rounding (x0 from a tensor-core product, see ismpc_set_option).
+ * ISMPC_ERR_MODEL when no sets are resident. */
+int ismpc_qp_hotstart_batch(ismpc_handle* h, int n, const int32_t* mat_index_opt,
+                            const double* g, const double* lbA, const double* ubA, const int8_t* ws_guess,
                             double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
                             int mem, void* stream);
 

@@ -21,7 +21,8 @@ EXPORTS = ["ismpc_version", "ismpc_error_string", "ismpc_create", "ismpc_destroy
            "ismpc_plan_generate", "ismpc_kf_init", "ismpc_kf_filter_batch", "ismpc_formc_set_plan",
            "ismpc_handle_stream", "ismpc_wait", "ismpc_host_alloc", "ismpc_host_free", "ismpc_formc_rollout_ex",
            "ismpc_forma_rollout_ex2", "ismpc_kf_filter_batch_f64", "ismpc_formc_set_instances",
-           "ismpc_formc_solve_batch_packed", "ismpc_qp_solve_batch_ws"]
+           "ismpc_formc_solve_batch_packed", "ismpc_qp_solve_batch_ws", "ismpc_qp_set_matrices",
+           "ismpc_qp_hotstart_batch"]
 
 _lib = None
 
@@ -91,6 +92,8 @@ def lib():
     L.ismpc_kf_filter_batch_f64.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
     L.ismpc_qp_solve_batch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 10 + [C.c_int, C.c_void_p]
     L.ismpc_qp_solve_batch_ws.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 11 + [C.c_int, C.c_void_p]
+    L.ismpc_qp_set_matrices.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 3 + [C.c_int]
+    L.ismpc_qp_hotstart_batch.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 10 + [C.c_int, C.c_void_p]
     L.ismpc_handle_stream.restype = C.c_void_p
     L.ismpc_handle_stream.argtypes = [C.c_void_p]
     L.ismpc_wait.argtypes = [C.c_void_p, C.c_void_p]
@@ -439,6 +442,54 @@ class Handle:
                                              abi.MEM_HOST, None)
         self._check(rc, "ismpc_qp_solve_batch_ws")
         return dict(x=x, y=y, ws=ws, status=status, iters=iters)
+
+    # ---- resident matrices of the dense seam (factor once, solve many right-hand sides) -----------------------
+    def qp_set_matrices(self, H, A):
+        """H (n_mat, nV, nV) and A (n_mat, nC, nV), or one set as (nV, nV) / (nC, nV), resident in the handle
+        (ismpc_qp_set_matrices); H=None forgets them.  Returns the n_mat factor statuses (ISMPC_ST_QP_FAIL: H not
+        positive definite)."""
+        if H is None:
+            self._check(self._L.ismpc_qp_set_matrices(self._h, 0, 0, 0, None, None, None, abi.MEM_HOST),
+                        "ismpc_qp_set_matrices")
+            return np.zeros(0, dtype=np.int32)
+        H = np.ascontiguousarray(H, dtype=np.float64); A = np.ascontiguousarray(A, dtype=np.float64)
+        if H.ndim == 2:
+            H, A = H[None], A[None]
+        n_mat, nV, nC = H.shape[0], H.shape[1], A.shape[1]
+        if H.shape != (n_mat, nV, nV) or A.shape != (n_mat, nC, nV):
+            raise ValueError("H must be n_mat x nV x nV and A n_mat x nC x nV, got %s and %s" % (H.shape, A.shape))
+        mat_status = np.zeros(n_mat, dtype=np.int32)
+        self._check(self._L.ismpc_qp_set_matrices(self._h, n_mat, nV, nC, _ptr(H), _ptr(A), _ptr(mat_status),
+                                                  abi.MEM_HOST), "ismpc_qp_set_matrices")
+        return mat_status
+
+    def qp_hotstart_batch(self, g, lbA, ubA, ws_guess=None, mat_index=None):
+        """ismpc_qp_hotstart_batch: n problems against the resident sets, problem p on set mat_index[p] (None: set p, or
+        set 0 when one set is resident).  ws_guess as in qp_solve_batch.  Returns the dict of qp_solve_batch."""
+        g = np.ascontiguousarray(g, dtype=np.float64)
+        lbA = np.ascontiguousarray(lbA, dtype=np.float64); ubA = np.ascontiguousarray(ubA, dtype=np.float64)
+        n, nV = g.shape
+        nC = lbA.shape[1]
+        x = np.zeros((n, nV)); y = np.zeros((n, nC)); ws = np.zeros((n, nC), dtype=np.int8)
+        status = np.zeros(n, dtype=np.int32); iters = np.zeros(n, dtype=np.int32)
+        guess = None if ws_guess is None else np.ascontiguousarray(ws_guess, dtype=np.int8)
+        if guess is not None and guess.shape != (n, nC):
+            raise ValueError("ws_guess must be %d x %d, got %s" % (n, nC, guess.shape))
+        idx = None if mat_index is None else np.ascontiguousarray(mat_index, dtype=np.int32)
+        if idx is not None and idx.shape != (n,):
+            raise ValueError("mat_index must have %d entries, got %s" % (n, idx.shape))
+        rc = self._L.ismpc_qp_hotstart_batch(self._h, n, _ptr(idx), _ptr(g), _ptr(lbA), _ptr(ubA), _ptr(guess), _ptr(x),
+                                             _ptr(y), _ptr(ws), _ptr(status), _ptr(iters), abi.MEM_HOST, None)
+        self._check(rc, "ismpc_qp_hotstart_batch")
+        return dict(x=x, y=y, ws=ws, status=status, iters=iters)
+
+    def qp_hotstart_batch_raw(self, n, g, lbA, ubA, x, y=None, ws=None, status=None, iters=None, mat_index=None,
+                              ws_guess=None, mem=abi.MEM_DEVICE, stream=None):
+        """Raw ismpc_qp_hotstart_batch: every array is a numpy array (host) or an integer address (device)."""
+        rc = self._L.ismpc_qp_hotstart_batch(self._h, n, _ptr(mat_index), _ptr(g), _ptr(lbA), _ptr(ubA), _ptr(ws_guess),
+                                             _ptr(x), _ptr(y), _ptr(ws), _ptr(status), _ptr(iters), mem,
+                                             C.c_void_p(stream) if stream else None)
+        self._check(rc, "ismpc_qp_hotstart_batch")
 
 
 # ---- all GPUs of one box behind one C ABI (include/ismpc_b200_multigpu.h, lib/libismpc_b200_mg.so) --------------------

@@ -61,6 +61,10 @@ struct ismpc_handle {
     DevBuf s_in;                   // [state | walk | inst] of one form-C tick call
     DevBuf s_ainst, s_aout, s_timing, a_Lwork, a_queue;
     DevBuf q_in, q_out, q_work;
+    // dense seam, resident matrix family (ismpc_qp_set_matrices): tables, factor status, workspace of its calls
+    DevBuf r_tab, r_stat, r_work;
+    int r_nmat = 0, r_nV = 0, r_nC = 0;    // resident sets and their shape, 0 = none
+    int opt_dense_resident_gemm = 1;       // a single shared set: x0 | A x0 of a call as one tensor-core product
     DevBuf s_pred, f_inst, f_plan, f_out, s_trace;
     cudaStream_t own_stream = nullptr;     // ismpc_handle_stream: created on first use, destroyed with the handle
 };
@@ -119,7 +123,7 @@ extern "C" int ismpc_destroy(ismpc_handle* h)
     cudaSetDevice(h->device);
     DevBuf* all[] = {&h->c_tables, &h->c_work, &h->c_info, &h->c_ptab, &h->c_ric_none, &h->c_ric_gait, &h->c_law_none, &h->c_law_gait, &h->c_ws, &h->c_plan, &h->c_inst, &h->s_tick, &h->s_state, &h->s_walk, &h->s_cinst, &h->s_cout, &h->s_in,
                      &h->s_plan, &h->s_primal, &h->s_active, &h->s_push, &h->s_traj, &h->s_status,
-                     &h->s_ainst, &h->s_aout, &h->s_timing, &h->a_Lwork, &h->a_queue, &h->q_in, &h->q_out, &h->q_work, &h->s_pred, &h->f_inst, &h->f_plan, &h->f_out, &h->s_trace};
+                     &h->s_ainst, &h->s_aout, &h->s_timing, &h->a_Lwork, &h->a_queue, &h->q_in, &h->q_out, &h->q_work, &h->r_tab, &h->r_stat, &h->r_work, &h->s_pred, &h->f_inst, &h->f_plan, &h->f_out, &h->s_trace};
     for (DevBuf* b : all) b->release();
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
@@ -208,6 +212,7 @@ extern "C" int ismpc_set_option(ismpc_handle* h, const char* name, int value)
     if (strcmp(name, "formc_pdl") == 0) { h->opt_formc_pdl = value != 0; return ISMPC_OK; }
     if (strcmp(name, "host_zero_copy") == 0) { h->opt_host_zero_copy = value != 0; return ISMPC_OK; }
     if (strcmp(name, "dense_dmma") == 0) { h->opt_dense_dmma = value != 0; return ISMPC_OK; }
+    if (strcmp(name, "dense_resident_gemm") == 0) { h->opt_dense_resident_gemm = value != 0; return ISMPC_OK; }
     if (strcmp(name, "formc_kernel") == 0) {
         if (value < 0 || value > 2) return ISMPC_ERR_ARG;
         h->opt_formc_kernel = value;
@@ -1026,6 +1031,101 @@ extern "C" int ismpc_qp_solve_batch(ismpc_handle* h, int n, int nV, int nC, cons
                                     int8_t* ws_opt, int32_t* status, int32_t* iters_opt, int mem, void* stream)
 {
     return ismpc_qp_solve_batch_ws(h, n, nV, nC, H, g, A, lbA, ubA, nullptr, x, y_opt, ws_opt, status, iters_opt, mem, stream);
+}
+
+// The resident matrix family: H and A set once (factor, [Hinv; D], S built on the device), then many (g, lbA, ubA)
+// batches against them.  Tables in r_tab, factor status in r_stat, the calls' workspace in r_work: nothing of the
+// per-call seam (q_work) is shared, so cold calls of any shape leave the sets alone.
+extern "C" int ismpc_qp_set_matrices(ismpc_handle* h, int n_mat, int nV, int nC, const double* H, const double* A,
+                                     int32_t* mat_status_opt, int mem)
+{
+    if (!h) return ISMPC_ERR_ARG;
+    if (n_mat < 0 || n_mat > h->max_batch || n_mat > 65535 || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
+        return ISMPC_ERR_ARG;
+    if (n_mat == 0) { h->r_nmat = 0; return ISMPC_OK; }
+    if (nV < 1 || nV > ISMPC_MAX_N || nC < 0 || nC > 2 * ISMPC_MAX_N + 8 || !H || (nC > 0 && !A)) return ISMPC_ERR_ARG;
+    CK(cudaSetDevice(h->device));
+    h->r_nmat = 0;                             // until the new sets are built
+    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
+    if (h->r_tab.ensure(qp_sets_table_doubles(n_mat, nV, nC) * sizeof(double)) ||
+        h->r_stat.ensure((size_t)n_mat * sizeof(int32_t)) ||
+        h->r_work.ensure(qp_sets_work_doubles(0, n_mat, nV, nC) * sizeof(double)))
+        return ISMPC_ERR_ALLOC;
+    const cudaMemcpyKind kind = mem == ISMPC_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+    double* tab = (double*)h->r_tab.p;
+    double* Ares = tab + (size_t)n_mat * (vv + cv + (size_t)nC * nC);
+    CK(cudaMemcpy(h->r_work.p, H, (size_t)n_mat * vv * sizeof(double), kind));        // the factor's scratch (Lh)
+    if (nC > 0) CK(cudaMemcpy(Ares, A, (size_t)n_mat * cv * sizeof(double), kind));
+    int rc = qp_sets_build(n_mat, nV, nC, tab, (int32_t*)h->r_stat.p, (double*)h->r_work.p, h->opt_dense_dmma, 0);
+    h->launches += 1;
+    if (rc) return fail_cuda(h, (cudaError_t)rc, "qp_sets_build");
+    CK(cudaDeviceSynchronize());
+    if (mat_status_opt) CK(cudaMemcpy(mat_status_opt, h->r_stat.p, (size_t)n_mat * sizeof(int32_t), cudaMemcpyDeviceToHost));
+    h->r_nmat = n_mat; h->r_nV = nV; h->r_nC = nC;
+    return ISMPC_OK;
+}
+
+extern "C" int ismpc_qp_hotstart_batch(ismpc_handle* h, int n, const int32_t* mat_index_opt, const double* g,
+                                       const double* lbA, const double* ubA, const int8_t* ws_guess, double* x,
+                                       double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt, int mem,
+                                       void* stream)
+{
+    if (!h) return ISMPC_ERR_ARG;
+    if (n < 0 || n > h->max_batch || !g || !x || !status || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
+        return ISMPC_ERR_ARG;
+    if (h->r_nmat == 0) return ISMPC_ERR_MODEL;
+    const int nV = h->r_nV, nC = h->r_nC, n_mat = h->r_nmat;
+    if ((nC > 0 && (!lbA || !ubA)) || (!mat_index_opt && n_mat > 1 && n > n_mat)) return ISMPC_ERR_ARG;
+    if (n == 0) return ISMPC_OK;
+    if (nC == 0) ws_guess = nullptr;
+    CK(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (h->r_work.ensure(qp_sets_work_doubles(n, n_mat, nV, nC) * sizeof(double))) return ISMPC_ERR_ALLOC;
+    const double* tab = (const double*)h->r_tab.p;
+    const int32_t* fstat = (const int32_t*)h->r_stat.p;
+    double* work = (double*)h->r_work.p;
+    if (mem == ISMPC_MEM_DEVICE) {
+        int rc = qp_sets_launch(n, nV, nC, n_mat, tab, fstat, mat_index_opt, g, lbA, ubA, (const signed char*)ws_guess, x,
+                                y_opt, (signed char*)ws_opt, status, iters_opt, work, h->opt_dense_resident_gemm,
+                                h->opt_dense_dmma, st);
+        h->launches += 1;
+        if (rc) return fail_cuda(h, (cudaError_t)rc, "qp_sets_launch");
+        return ISMPC_OK;
+    }
+    const size_t szg = (size_t)n * nV, szb = (size_t)n * nC;
+    const size_t in_b = (szg + 2 * szb) * sizeof(double) + (size_t)n * sizeof(int32_t) + szb;
+    const size_t out_b = (szg + szb) * sizeof(double) + szb + 2 * (size_t)n * sizeof(int32_t) + 64;
+    if (h->q_in.ensure(in_b) || h->q_out.ensure(out_b)) return ISMPC_ERR_ALLOC;
+    double* dg = (double*)h->q_in.p; double* dlb = dg + szg; double* dub = dlb + szb;
+    int32_t* didx = (int32_t*)(dub + szb);
+    signed char* dgs = (signed char*)(didx + n);
+    double* dx = (double*)h->q_out.p; double* dy = dx + szg;
+    int32_t* dst = (int32_t*)(dy + szb); int32_t* dit = dst + n;
+    signed char* dws = (signed char*)(dit + n);
+    CK(cudaMemcpyAsync(dg, g, szg * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (nC > 0) {
+        CK(cudaMemcpyAsync(dlb, lbA, szb * sizeof(double), cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(dub, ubA, szb * sizeof(double), cudaMemcpyHostToDevice, st));
+    }
+    if (mat_index_opt) CK(cudaMemcpyAsync(didx, mat_index_opt, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    // the outputs are staged with the caller's bytes, so that a problem the call does not touch (set index out of range)
+    // keeps them, as with device buffers
+    if (ws_guess) CK(cudaMemcpyAsync(dgs, ws_guess, szb, cudaMemcpyHostToDevice, st));
+    if (ws_opt && nC > 0) CK(cudaMemcpyAsync(dws, ws_opt, szb, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(dx, x, szg * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (y_opt && nC > 0) CK(cudaMemcpyAsync(dy, y_opt, szb * sizeof(double), cudaMemcpyHostToDevice, st));
+    int rc = qp_sets_launch(n, nV, nC, n_mat, tab, fstat, mat_index_opt ? didx : nullptr, dg, dlb, dub,
+                            ws_guess ? dgs : nullptr, dx, dy, dws, dst, dit, work, h->opt_dense_resident_gemm,
+                            h->opt_dense_dmma, st);
+    h->launches += 1;
+    if (rc) return fail_cuda(h, (cudaError_t)rc, "qp_sets_launch");
+    CK(cudaMemcpyAsync(x, dx, szg * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (y_opt && nC > 0) CK(cudaMemcpyAsync(y_opt, dy, szb * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (ws_opt && nC > 0) CK(cudaMemcpyAsync(ws_opt, dws, szb, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(status, dst, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (iters_opt) CK(cudaMemcpyAsync(iters_opt, dit, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return ISMPC_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------

@@ -20,15 +20,17 @@ struct DenseLayout {          // offsets (in doubles) inside one problem's works
     int qmax;
 };
 
-__host__ __device__ inline DenseLayout dense_layout(int nV, int nC)
+// tables = false: the slice of the resident path (qp_resident_launch), the vectors only -- the tables belong to the resident
+// set, x0 and A x0 to the n x (nV + nC) block its x0 step writes
+__host__ __device__ inline DenseLayout dense_layout(int nV, int nC, bool tables = true)
 {
     DenseLayout l;
-    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV, cc = (size_t)nC * nC;
+    const size_t vv = tables ? (size_t)nV * nV : 0, cv = tables ? (size_t)nC * nV : 0, cc = tables ? (size_t)nC * nC : 0;
     l.qmax = (nV + 1 < nC ? nV + 1 : nC); if (l.qmax < 1) l.qmax = 1;
     size_t o = 0;
     l.Lh = o; o += vv; l.Linv = o; o += vv; l.Hinv = o; o += vv;
     l.D = o; o += cv; l.S = o; o += cc;
-    l.x0 = o; o += nV; l.rv = o; o += nC; l.az = o; o += nC; l.z = o; o += nV;
+    l.x0 = o; o += tables ? nV : 0; l.rv = o; o += tables ? nC : 0; l.az = o; o += nC; l.z = o; o += nV;
     l.Lw = o; o += (size_t)l.qmax * (l.qmax + 1) / 2;
     l.mu = o; o += l.qmax; l.r = o; o += l.qmax; l.y = o; o += l.qmax;
     l.ints = o; o += (size_t)(l.qmax * sizeof(int) + l.qmax + nC + 15) / 8 + 2;
@@ -97,7 +99,8 @@ __global__ void dense_tri_inverse(int N, double* work, size_t stride, size_t off
 // Element (r, k) of X sits at X[r * sxr + k * sxk] (likewise Y), which covers the row-major operands and the transposed
 // read of Linv.  CTA = 4 warps, 64 x 64 tile of C, each warp 32 x 32 = 4 x 4 DMMA tiles (32 accumulators per thread);
 // K in chunks of 16 through shared memory, rows padded to 20 doubles so that the 8 x 4 / 4 x 8 fragment loads of a
-// half-warp fall into 16 distinct 8-byte banks.
+// half-warp fall into 16 distinct 8-byte banks.  C is stored as alpha times the sum: the set-up products pass 1 (exact),
+// the resident path's x0 step (qp_resident_launch) passes -1.
 constexpr int DG_T = 64, DG_KC = 16, DG_LD = 20;
 
 __device__ __forceinline__ void dmma_m8n8k4(double& d0, double& d1, double a, double b)
@@ -108,7 +111,7 @@ __device__ __forceinline__ void dmma_m8n8k4(double& d0, double& d1, double a, do
 
 __global__ void __launch_bounds__(128)
 dense_gemm_nt(int M, int Nc, int K, const double* Xb, size_t sx, int sxr, int sxk, const double* Yb, size_t sy, int syr, int syk,
-              double* Cb, size_t sc)
+              double* Cb, size_t sc, double alpha)
 {
     __shared__ double xs[DG_T * DG_LD], ys[DG_T * DG_LD];
     const double* X = Xb + (size_t)blockIdx.z * sx;
@@ -156,8 +159,8 @@ dense_gemm_nt(int M, int Nc, int K, const double* Xb, size_t sx, int sxr, int sx
         for (int j = 0; j < 4; ++j) {
             const int r = row0 + wr + 8 * i + g, c = col0 + wc + 8 * j + 2 * t4;
             if (r < M) {
-                if (c < Nc) C[(size_t)r * Nc + c] = acc[i][j][0];
-                if (c + 1 < Nc) C[(size_t)r * Nc + c + 1] = acc[i][j][1];
+                if (c < Nc) C[(size_t)r * Nc + c] = alpha * acc[i][j][0];
+                if (c + 1 < Nc) C[(size_t)r * Nc + c + 1] = alpha * acc[i][j][1];
             }
         }
 }
@@ -166,7 +169,7 @@ dense_gemm_nt(int M, int Nc, int K, const double* Xb, size_t sx, int sxr, int sx
 // (ismpc_set_option "dense_dmma" = 0) and for the record of what DMMA buys (3.8 ms -> 1.6 ms per product of the
 // nV = 206 / nC = 208 shape over 1,024 problems).
 __global__ void dense_gemm_nt_cc(int M, int Nc, int K, const double* Xb, size_t sx, int sxr, int sxk, const double* Yb, size_t sy,
-                                 int syr, int syk, double* Cb, size_t sc)
+                                 int syr, int syk, double* Cb, size_t sc, double alpha)
 {
     __shared__ double xs[16][17], ys[16][17];
     const double* X = Xb + (size_t)blockIdx.z * sx;
@@ -185,16 +188,17 @@ __global__ void dense_gemm_nt_cc(int M, int Nc, int K, const double* Xb, size_t 
         for (int kk = 0; kk < 16; ++kk) acc += xs[ty][kk] * ys[tx][kk];
         __syncthreads();
     }
-    if (row < M && col < Nc) C[(size_t)row * Nc + col] = acc;
+    if (row < M && col < Nc) C[(size_t)row * Nc + col] = alpha * acc;
 }
 
 static void dense_gemm_launch(int use_dmma, int n, int M, int Nc, int K, const double* X, size_t sx, int sxr, int sxk,
-                              const double* Y, size_t sy, int syr, int syk, double* C, size_t sc, cudaStream_t st)
+                              const double* Y, size_t sy, int syr, int syk, double* C, size_t sc, cudaStream_t st,
+                              double alpha = 1.0)
 {
     if (use_dmma)
-        dense_gemm_nt<<<dim3((Nc + DG_T - 1) / DG_T, (M + DG_T - 1) / DG_T, n), 128, 0, st>>>(M, Nc, K, X, sx, sxr, sxk, Y, sy, syr, syk, C, sc);
+        dense_gemm_nt<<<dim3((Nc + DG_T - 1) / DG_T, (M + DG_T - 1) / DG_T, n), 128, 0, st>>>(M, Nc, K, X, sx, sxr, sxk, Y, sy, syr, syk, C, sc, alpha);
     else
-        dense_gemm_nt_cc<<<dim3((Nc + 15) / 16, (M + 15) / 16, n), dim3(16, 16), 0, st>>>(M, Nc, K, X, sx, sxr, sxk, Y, sy, syr, syk, C, sc);
+        dense_gemm_nt_cc<<<dim3((Nc + 15) / 16, (M + 15) / 16, n), dim3(16, 16), 0, st>>>(M, Nc, K, X, sx, sxr, sxk, Y, sy, syr, syk, C, sc, alpha);
 }
 
 // x0 = -Hinv g ; rv0 = A x0 ; one CTA per problem
@@ -217,6 +221,45 @@ __global__ void dense_x0_rv(int nV, int nC, const double* g, const double* A, do
         double s = 0.0;
         for (int j = 0; j < nV; ++j) s += Ap[(size_t)c * nV + j] * w[l.x0 + j];
         w[l.rv + c] = s;
+    }
+}
+
+// ---- the resident matrix family (ismpc_qp_set_matrices / ismpc_qp_hotstart_batch) --------------------------
+// n_mat sets of one shape, built once by the set-up kernels above: per set [Hinv; D] as one (nV + nC) x nV row-major
+// block (HD, stride nV^2 + nC nV), S (stride nC^2), a copy of A (stride nC nV) and the factor status.  Problem p of a call
+// solves against set idx[p] (idx = NULL: set p, or set 0 when n_mat = 1).
+struct DenseSets {
+    const double *HD, *S, *A;
+    const int32_t* fstat;       // n_mat: dense_cholesky's status of each set
+    const int32_t* idx;         // n, or NULL
+    int n_mat;
+    double* xr;                 // n x (nV + nC): x0 | A x0 of each problem (written by the x0 step, rv moves in place)
+    __host__ __device__ int set_of(int p) const { return idx ? idx[p] : (n_mat == 1 ? 0 : p); }
+};
+
+// x0 = -Hinv g ; rv0 = A x0 from the problem's set, one CTA per problem: the loops of dense_x0_rv in the same order, so
+// that x0 and A x0 (and with them every later decision) are bit-identical to the seam's.  A problem whose index is out of
+// range is skipped here and flagged by dense_das_kernel.
+__global__ void dense_x0_rv_sets(int n, int nV, int nC, const double* g, DenseSets sets)
+{
+    const size_t p = blockIdx.x;
+    const int m = sets.set_of((int)p);
+    if (m < 0 || m >= sets.n_mat) return;
+    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
+    const double* Hinv = sets.HD + (size_t)m * (vv + cv);
+    const double* gp = g + p * nV;
+    double* x0 = sets.xr + p * (nV + nC);
+    for (int i = threadIdx.x; i < nV; i += blockDim.x) {
+        double s = 0.0;
+        for (int j = 0; j < nV; ++j) s += Hinv[(size_t)j * nV + i] * gp[j];
+        x0[i] = -s;
+    }
+    __syncthreads();
+    const double* Ap = sets.A + (size_t)m * cv;
+    for (int c = threadIdx.x; c < nC; c += blockDim.x) {
+        double s = 0.0;
+        for (int j = 0; j < nV; ++j) s += Ap[(size_t)c * nV + j] * x0[j];
+        x0[nV + c] = s;
     }
 }
 
@@ -281,10 +324,14 @@ constexpr int DENSE_WARPS = 4;   // QPs per CTA
 
 // WARM = false: the cold solve (ismpc_qp_solve_batch).  WARM = true: the same, started from the guessed working set
 // ws_guess (n x nC, <0 lower / >0 upper / 0 free; may alias ws) through das_warm_install after the equalities.
-template <bool WARM>
+// SETS = false: the tables (D, S) and x0 / A x0 sit in the problem's workspace slice, status[p] holds the factor status
+// (the seam).  SETS = true: they come from the problem's resident set and sets.xr, the slice (dense_layout(.., false))
+// holds the vectors only, and the status starts from the set's; a problem whose set index is out of range is flagged and
+// nothing else of it is written.  The algorithm is the same, so the same inputs give the same bytes.
+template <bool WARM, bool SETS>
 __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const double* ubA, double* work,
                                  size_t stride, DenseLayout l, int R, double* x, double* y, signed char* ws,
-                                 int32_t* status, int32_t* iters, const signed char* ws_guess)
+                                 int32_t* status, int32_t* iters, const signed char* ws_guess, DenseSets sets)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int p = blockIdx.x * DENSE_WARPS + warp_id();
@@ -302,16 +349,36 @@ __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const
     const double* lb = lbA + (size_t)p * nC;
     const double* ub = ubA + (size_t)p * nC;
     double* xp = x + (size_t)p * nV;
-    int st = status[p];
+    const double* D = w + l.D;
+    const double* S = w + l.S;
+    double* x0 = w + l.x0;
+    int st;
+    if constexpr (SETS) {
+        const int m = sets.set_of(p);
+        if (m < 0 || m >= sets.n_mat) {
+            if (lane == 0) { status[p] = ISMPC_ST_QP_FAIL; if (iters) iters[p] = 0; }
+            return;
+        }
+        const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
+        D = sets.HD + (size_t)m * (vv + cv) + vv;
+        S = sets.S + (size_t)m * nC * nC;
+        x0 = sets.xr + (size_t)p * (nV + nC);
+        for (int i = lane; i < nV; i += 32) xp[i] = x0[i];
+        __syncwarp();
+        st = sets.fstat[m];
+    } else {
+        st = status[p];
+    }
+    double* rv = SETS ? x0 + nV : w + l.rv;
     int it = 0;
     if (st == 0 && nC > 0) {
         for (int i = lane; i < nC; i += 32) dw.state[i] = 0;
         __syncwarp();
-        const DenseProb pb0{nV, nC, w + l.D, w + l.S, lb, ub, w + l.rv, w + l.az};
+        const DenseProb pb0{nV, nC, D, S, lb, ub, rv, w + l.az};
         std::conditional_t<WARM, DenseWarmProb, DenseProb> pb{pb0};
         if constexpr (WARM) {
             double* rv0 = work + (size_t)n * stride + (size_t)p * nC;
-            pb.x0 = w + l.x0; pb.rv0_ = rv0;
+            pb.x0 = x0; pb.rv0_ = rv0;
             for (int i = lane; i < nC; i += 32) rv0[i] = pb.rv[i];
             __syncwarp();
         }
@@ -393,10 +460,73 @@ int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, con
     dense_x0_rv<<<n, 128, 0, st>>>(nV, nC, g, A, work, stride, l, x);
     const int R = l.qmax < DENSE_R ? l.qmax : DENSE_R;
     const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
-    auto kern = ws_guess ? dense_das_kernel<true> : dense_das_kernel<false>;
+    auto kern = ws_guess ? dense_das_kernel<true, false> : dense_das_kernel<false, false>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
     kern<<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
-        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess);
+        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess, DenseSets{});
+    return (int)cudaGetLastError();
+}
+
+// ---- resident matrix family ------------------------------------------------------------------------------
+size_t qp_sets_table_doubles(int n_mat, int nV, int nC)
+{
+    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV, cc = (size_t)nC * nC;
+    return (size_t)n_mat * (vv + cv + cc + cv);
+}
+
+// set-up: 2 n_mat nV^2 (Lh | Linv, scratch); per call: n slices of vectors, x0 | A x0 (n x (nV + nC)), A x0 kept for the
+// warm start (n x nC)
+size_t qp_sets_work_doubles(int n, int n_mat, int nV, int nC)
+{
+    const size_t setup = 2 * (size_t)n_mat * nV * nV;
+    const size_t call = (dense_layout(nV, nC, false).total + nV + 2 * (size_t)nC) * n;
+    return (setup > call ? setup : call) + 16;
+}
+
+// [Hinv; D], S and the factor status of n_mat sets, with the seam's set-up kernels and products: H (n_mat x nV x nV,
+// device) is already copied into the Lh scratch (work, stride nV^2), A into the set's copy.
+int qp_sets_build(int n_mat, int nV, int nC, double* tab, int32_t* fstat, double* work, int use_dmma, cudaStream_t st)
+{
+    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV, cc = (size_t)nC * nC;
+    double* HD = tab;
+    double* S = HD + (size_t)n_mat * (vv + cv);
+    const double* A = S + (size_t)n_mat * cc;
+    const size_t offLinv = (size_t)n_mat * vv;
+    dense_cholesky<<<n_mat, 256, 0, st>>>(nV, work, vv, 0, fstat);
+    dense_tri_inverse<<<dim3((nV + 63) / 64, n_mat), 64, 0, st>>>(nV, work, vv, 0, offLinv);
+    dense_gemm_launch(use_dmma, n_mat, nV, nV, nV, work + offLinv, vv, 1, nV, work + offLinv, vv, 1, nV, HD, vv + cv, st);
+    if (nC > 0) {
+        dense_gemm_launch(use_dmma, n_mat, nC, nV, nV, A, cv, nV, 1, HD, vv + cv, nV, 1, HD + vv, vv + cv, st);
+        dense_gemm_launch(use_dmma, n_mat, nC, nC, nV, A, cv, nV, 1, HD + vv, vv + cv, nV, 1, S, cc, st);
+    }
+    return (int)cudaGetLastError();
+}
+
+// One call against the resident sets: the x0 step, then dense_das_kernel<WARM, true>.  A single shared set (n_mat = 1,
+// use_gemm) takes x0 | A x0 for the whole batch from one tensor-core product, [X0 | R0] (n x (nV + nC)) = -G [Hinv; D]';
+// otherwise the per-problem mat-vecs of the seam.
+int qp_sets_launch(int n, int nV, int nC, int n_mat, const double* tab, const int32_t* fstat, const int32_t* idx,
+                   const double* g, const double* lbA, const double* ubA, const signed char* ws_guess, double* x,
+                   double* y, signed char* ws, int32_t* status, int32_t* iters, double* work, int use_gemm, int use_dmma,
+                   cudaStream_t st)
+{
+    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV, cc = (size_t)nC * nC;
+    const DenseLayout l = dense_layout(nV, nC, false);
+    const size_t stride = l.total;
+    DenseSets sets;
+    sets.HD = tab; sets.S = tab + (size_t)n_mat * (vv + cv); sets.A = sets.S + (size_t)n_mat * cc;
+    sets.fstat = fstat; sets.idx = idx; sets.n_mat = n_mat;
+    sets.xr = work + (size_t)n * (stride + nC);
+    if (n_mat == 1 && use_gemm)
+        dense_gemm_launch(use_dmma, 1, n, nV + nC, nV, g, 0, nV, 1, sets.HD, 0, nV, 1, sets.xr, 0, st, -1.0);
+    else
+        dense_x0_rv_sets<<<n, 128, 0, st>>>(n, nV, nC, g, sets);
+    const int R = l.qmax < DENSE_R ? l.qmax : DENSE_R;
+    const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
+    auto kern = ws_guess ? dense_das_kernel<true, true> : dense_das_kernel<false, true>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
+    kern<<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
+        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess, sets);
     return (int)cudaGetLastError();
 }
 

@@ -161,43 +161,61 @@ def dense_qp_batch(shape, n, seed=SEED0 ^ 21):
         lb = np.concatenate([(u0 @ a)[:, None], mid - 0.045], axis=1)
         ub = np.concatenate([(u0 @ a)[:, None], mid + 0.045], axis=1)
         return H, -mid, A, lb, ub
-    C, F, dt, step, ds, Qf = 100, 3, 0.01, 50, 20, 1e7
-    eta = np.sqrt(9.8 / 0.56)
+    C, F, step = _FORMA_STACKED["C"], _FORMA_STACKED["F"], _FORMA_STACKED["step"]
+    nV = 2 * (C + F); nC = nV + 2
+    H = np.zeros((n, nV, nV)); g = np.zeros((n, nV)); A = np.zeros((n, nC, nV)); lb = np.zeros((n, nC)); ub = np.zeros((n, nC))
+    for p in range(n):
+        H[p], A[p] = _forma_stacked_matrices(int(rng.integers(0, step)))
+        g[p], lb[p], ub[p] = _forma_stacked_vectors(rng, A[p])
+    return H, g, A, lb, ub
+
+
+_FORMA_STACKED = dict(C=100, F=3, dt=0.01, step=50, ds=20, Qf=1e7, height=0.56)
+
+
+def _forma_stacked_matrices(j0):
+    """H and A of the "forma_stacked" shape with the next footstep switch j0 ticks into the current step."""
+    C, F, dt, step, ds, Qf = (_FORMA_STACKED[k] for k in ("C", "F", "dt", "step", "ds", "Qf"))
+    eta = np.sqrt(9.8 / _FORMA_STACKED["height"])
     nv1 = C + F; nV = 2 * nv1; nC = nV + 2
     lam = np.exp(-eta * dt)
     stab = (1.0 / eta) * (1.0 - lam) / (1.0 - lam ** C) * np.exp(-eta * dt * np.arange(C)) - dt * np.exp(-eta * dt * C)
     P = dt * np.tril(np.ones((C, C)))
-    H = np.zeros((n, nV, nV)); g = np.zeros((n, nV)); A = np.zeros((n, nC, nV)); lb = np.zeros((n, nC)); ub = np.zeros((n, nC))
     hd = np.concatenate([np.ones(C), Qf * np.ones(F), np.ones(C), Qf * np.ones(F)])
     D = np.eye(F) - np.eye(F, k=-1)
-    for p in range(n):
-        j0 = int(rng.integers(0, step))
-        T = np.arange(1, F + 2) * step - j0                       # ticks until the next F+1 footstep switches
-        mp = np.zeros((C, F + 1))
-        for i in range(1, C + 1):
-            pf = int((T <= i).sum())
-            pf = min(pf, F)
-            rem = (T[pf] - i) if pf <= F else ds + 1
-            if rem > ds or pf == F:
-                mp[i - 1, pf] = 1.0
-            else:
-                mp[i - 1, pf] = rem / ds; mp[i - 1, pf + 1] = 1.0 - rem / ds
-        H[p][np.arange(nV), np.arange(nV)] = hd
-        for ax in range(2):
-            o = ax * nv1
-            A[p, ax, o:o + C] = stab
-            A[p, 2 + ax * C: 2 + (ax + 1) * C, o:o + C] = P
-            A[p, 2 + ax * C: 2 + (ax + 1) * C, o + C:o + nv1] = -mp[:, 1:]
-            A[p, 2 + 2 * C + ax * F: 2 + 2 * C + (ax + 1) * F, o + C:o + nv1] = D
-        stepl = rng.uniform(0.05, 0.15) * np.array([np.cos(0.3), np.sin(0.3)])
-        plan = np.arange(1, F + 1)[:, None] * stepl[None, :]
-        v0 = np.concatenate([rng.normal(0, 0.2, C), plan[:, 0] + rng.normal(0, 0.01, F),
-                             rng.normal(0, 0.2, C), plan[:, 1] + rng.normal(0, 0.01, F)])
-        r0 = A[p] @ v0
-        lb[p] = r0 - rng.uniform(0.0, 0.02, nC); ub[p] = r0 + rng.uniform(0.0, 0.02, nC)
-        lb[p, :2] = ub[p, :2] = r0[:2]
-        g[p] = np.concatenate([np.zeros(C), -Qf * plan[:, 0], np.zeros(C), -Qf * plan[:, 1]])
-    return H, g, A, lb, ub
+    T = np.arange(1, F + 2) * step - j0                       # ticks until the next F+1 footstep switches
+    mp = np.zeros((C, F + 1))
+    for i in range(1, C + 1):
+        pf = int((T <= i).sum())
+        pf = min(pf, F)
+        rem = (T[pf] - i) if pf <= F else ds + 1
+        if rem > ds or pf == F:
+            mp[i - 1, pf] = 1.0
+        else:
+            mp[i - 1, pf] = rem / ds; mp[i - 1, pf + 1] = 1.0 - rem / ds
+    H = np.diag(hd); A = np.zeros((nC, nV))
+    for ax in range(2):
+        o = ax * nv1
+        A[ax, o:o + C] = stab
+        A[2 + ax * C: 2 + (ax + 1) * C, o:o + C] = P
+        A[2 + ax * C: 2 + (ax + 1) * C, o + C:o + nv1] = -mp[:, 1:]
+        A[2 + 2 * C + ax * F: 2 + 2 * C + (ax + 1) * F, o + C:o + nv1] = D
+    return H, A
+
+
+def _forma_stacked_vectors(rng, A):
+    """g, lbA, ubA of one "forma_stacked" problem: bounds laid around A v0 for a reference point v0 near a straight plan."""
+    C, F, Qf = _FORMA_STACKED["C"], _FORMA_STACKED["F"], _FORMA_STACKED["Qf"]
+    nC = A.shape[0]
+    stepl = rng.uniform(0.05, 0.15) * np.array([np.cos(0.3), np.sin(0.3)])
+    plan = np.arange(1, F + 1)[:, None] * stepl[None, :]
+    v0 = np.concatenate([rng.normal(0, 0.2, C), plan[:, 0] + rng.normal(0, 0.01, F),
+                         rng.normal(0, 0.2, C), plan[:, 1] + rng.normal(0, 0.01, F)])
+    r0 = A @ v0
+    lb = r0 - rng.uniform(0.0, 0.02, nC); ub = r0 + rng.uniform(0.0, 0.02, nC)
+    lb[:2] = ub[:2] = r0[:2]
+    g = np.concatenate([np.zeros(C), -Qf * plan[:, 0], np.zeros(C), -Qf * plan[:, 1]])
+    return g, lb, ub
 
 
 def dense_qp_sequence(shape, n, T, seed=SEED0 ^ 23):
@@ -221,3 +239,65 @@ def dense_qp_sequence(shape, n, T, seed=SEED0 ^ 23):
         lb[t] = np.where(np.abs(lb0) >= 1e20, lb0, lb0 + adv)
         ub[t] = np.where(np.abs(ub0) >= 1e20, ub0, ub0 + adv)
     return H, g, A, lb, ub
+
+
+def _drift(H, A, idx, g0, lb0, ub0, T, rng):
+    """T ticks of dense_qp_sequence's drift on per-problem vectors; problem p's matrices are H[idx[p]], A[idx[p]]."""
+    n, nV = g0.shape
+    nC = lb0.shape[1]
+    g = np.empty((T, n, nV)); lb = np.empty((T, n, nC)); ub = np.empty((T, n, nC))
+    dx = np.zeros((n, nV)); dv = np.zeros((n, nV))
+    for t in range(T):
+        if t:
+            dx += 2e-3 * rng.standard_normal((n, nV))
+            dv += 2e-3 * rng.standard_normal((n, nV))
+        adv = np.empty((n, nC))
+        for k in range(H.shape[0]):                       # per set, without expanding H and A to n copies
+            sel = idx == k
+            g[t][sel] = g0[sel] - dx[sel] @ H[k].T
+            adv[sel] = dv[sel] @ A[k].T
+        lb[t] = np.where(np.abs(lb0) >= 1e20, lb0, lb0 + adv)
+        ub[t] = np.where(np.abs(ub0) >= 1e20, ub0, ub0 + adv)
+    return g, lb, ub
+
+
+def dense_qp_family(shape, n, n_mat=1, T=1, seed=SEED0 ^ 29):
+    """A family of dense QPs for the resident sets of the seam (ismpc_qp_set_matrices / ismpc_qp_hotstart_batch): n_mat
+    matrix sets (H, A) of one shape, n problems of which problem p uses set p % n_mat, and T drifting ticks of per-problem
+    vectors (the drift of dense_qp_sequence).  The shape of a condensed linear MPC: the matrices are built once, every
+    tick moves g and the bounds.
+    "formc_horizontal": the dense_qp_batch shape (nV = 100, nC = 101); set k has CoM height 0.69 m for k = 0, otherwise
+        drawn from U[0.55, 0.8], which changes the stability row a.
+    "forma_stacked": the dense_qp_batch shape (nV = 206, nC = 208); every problem of set k is at the same footstep phase j0
+        (drawn per set), which fixes the ZMP rows.
+    Every problem is feasible at every tick (its bounds are laid around A v0, then translated).
+    Returns H (n_mat, nV, nV), A (n_mat, nC, nV), mat_index (n,) int32, g (T, n, nV), lbA / ubA (T, n, nC)."""
+    rng = np.random.default_rng(seed)
+    idx = (np.arange(n) % n_mat).astype(np.int32)
+    if shape == "formc_horizontal":
+        N, dt = 100, 0.01
+        hs = np.concatenate([[0.69], rng.uniform(0.55, 0.8, n_mat - 1)])
+        Hs = np.broadcast_to(np.eye(N), (n_mat, N, N)).copy()
+        As = np.zeros((n_mat, N + 1, N)); As[:, 1:, :] = np.eye(N)
+        for k, h in enumerate(hs):
+            eta = np.sqrt(9.81 / h)
+            As[k, 0] = -np.exp(eta * dt * (N - 1 - np.arange(N))) * (np.exp(eta * dt) - 1.0)
+        a = As[idx, 0]
+        L = rng.uniform(0.05, 0.25, (n, 1)); k0 = rng.integers(0, 45, (n, 1))
+        t = k0 + np.arange(N)[None, :]
+        si, ri = t // 45, t % 45
+        mid = L * (si + np.where(ri < 35, 0.0, (ri - 35) / 10.0))
+        sgn = rng.choice([-1.0, 1.0], (n, 1)); width = rng.integers(18, 40, (n, 1))
+        u0 = mid + 0.045 * sgn * (np.arange(N)[None, :] < width) * rng.uniform(0.8, 1.0, (n, N))
+        ua = np.einsum("ni,ni->n", u0, a)[:, None]
+        lb0 = np.concatenate([ua, mid - 0.045], axis=1); ub0 = np.concatenate([ua, mid + 0.045], axis=1)
+        g0 = -mid
+    elif shape == "forma_stacked":
+        mats = [_forma_stacked_matrices(int(j0)) for j0 in rng.integers(0, _FORMA_STACKED["step"], n_mat)]
+        Hs = np.array([m[0] for m in mats]); As = np.array([m[1] for m in mats])
+        vec = [_forma_stacked_vectors(rng, As[idx[p]]) for p in range(n)]
+        g0 = np.array([v[0] for v in vec]); lb0 = np.array([v[1] for v in vec]); ub0 = np.array([v[2] for v in vec])
+    else:
+        raise ValueError("unknown shape %r" % shape)
+    g, lb, ub = _drift(Hs, As, idx, g0, lb0, ub0, T, rng)
+    return Hs, As, idx, g, lb, ub
