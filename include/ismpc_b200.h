@@ -22,7 +22,7 @@
  * void* (NULL = default stream).  With ISMPC_MEM_DEVICE every data pointer is a device pointer, the
  * call only enqueues work on `stream` and returns; with ISMPC_MEM_HOST every data pointer is a host
  * pointer (pinned for best speed), the call copies in, launches, copies out and synchronises the
- * stream before returning; ISMPC_MEM_HOST_ASYNC (ismpc_formc_solve_batch, ismpc_forma_solve_batch and the ismpc_forma_rollout calls) is the same without the final
+ * stream before returning; ISMPC_MEM_HOST_ASYNC (ismpc_formc_solve_batch, ismpc_forma_solve_batch[_ws] and the ismpc_forma_rollout calls) is the same without the final
  * synchronisation: the call returns as soon as the copies and the kernel are enqueued, the host buffers must be
  * pinned and stay untouched, and the handle must not be used again, until the caller has synchronised `stream` --
  * two handles on two streams give a double-buffered pipeline.  The caller owns all buffers; the handle owns only its workspace.
@@ -195,7 +195,8 @@ void ismpc_host_free(void* p);
  *                         registers, 16 = one warp per instance held to 128 registers (16 resident warps per SM).
  *   "forma_pdas":         1 = structured primal-dual active set with the dual active set as fallback (default), 0 = dual
  *                         active set only.   "forma_warm": 1 = rollouts start each tick from the previous working set
- *                         (default), 0 = every tick cold.   "forma_R", "forma_warps_per_cta": shared-memory rows of
+ *                         (default), 0 = every tick cold; rollouts only (a single tick starts from the set handed to
+ *                         ismpc_forma_solve_batch_ws, or cold without one).   "forma_R", "forma_warps_per_cta": shared-memory rows of
  *                         the fallback's factor and warps per CTA of the form-A kernels (0 = default).
  *                         "forma_reg": 1 = the working-set iteration keeps its rows in registers where the shape allows
  *                         (C <= 128, F <= 3; default), 0 = shared-memory walk.
@@ -322,6 +323,29 @@ int ismpc_forma_solve_batch(ismpc_handle* h, int n, const ismpc_forma_inst_t* in
                             const double* fs_plan, int plan_rows,
                             ismpc_forma_out_t* out, double* primal_opt, int8_t* active_opt,
                             int mem, void* stream);
+
+/* ismpc_forma_solve_batch hot-started from a guessed working set -- for a caller that drives the tick itself (a robot or
+ * simulator supplying the measured state, a serving loop) and so holds last tick's working set in active_opt.
+ * ws_guess (nullable): n x 2(C+F) int8 in the layout of active_opt, -1 lower / +1 upper / 0 free (any other value is
+ *           read as free).  NULL = the cold tick (ismpc_forma_solve_batch forwards here with NULL).  It may be the same
+ *           buffer as active_opt in every memory mode, so a closed loop passes one buffer in place on every call.
+ * ws_shift: 0 = the guess is for these records' rows as given; 1 = the guess is the working set these instances had on
+ *           the PREVIOUS tick (the active_opt of the call that produced these records): it is shifted by one tick as the
+ *           rollouts do, ZMP row i taking row i+1, and the kinematic rows are cleared on the first tick after a footstep
+ *           switch (the record has fs_counter >= 2 and j == fs_timing[timing_first + fs_counter - 1]).  Other values:
+ *           ISMPC_ERR_ARG.
+ * The guess only decides where the working-set iteration starts: the minimiser of each strictly convex QP is unique,
+ * and a guess that stalls the iteration is dropped for the empty set (then the dual active set, as in the cold tick),
+ * so results are the cold tick's to rounding for ANY guess; ISMPC_ST_GI_FALLBACK may differ (informational).  out.iters
+ * keeps its meaning, the iterations of both axes: 2 per instance when the guess is the optimal working set.
+ * Records outside the tables are flagged and skipped as in the cold tick; their guess and active rows are neither read
+ * nor written. */
+int ismpc_forma_solve_batch_ws(ismpc_handle* h, int n, const ismpc_forma_inst_t* inst,
+                               const int32_t* fs_timing, int timing_len,
+                               const double* fs_plan, int plan_rows,
+                               const int8_t* ws_guess, int ws_shift,
+                               ismpc_forma_out_t* out, double* primal_opt, int8_t* active_opt,
+                               int mem, void* stream);
 
 /* Closed loop of the MATLAB scripts (bang.m:99-563, QP-1 loop): n_ticks ticks on the device with the
  * footstep switch, plan shift and centerline rebuild (bang.m:529-563).  inst is advanced in place;

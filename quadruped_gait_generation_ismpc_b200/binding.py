@@ -22,7 +22,7 @@ EXPORTS = ["ismpc_version", "ismpc_error_string", "ismpc_create", "ismpc_destroy
            "ismpc_handle_stream", "ismpc_wait", "ismpc_host_alloc", "ismpc_host_free", "ismpc_formc_rollout_ex",
            "ismpc_forma_rollout_ex2", "ismpc_kf_filter_batch_f64", "ismpc_formc_set_instances",
            "ismpc_formc_solve_batch_packed", "ismpc_qp_solve_batch_ws", "ismpc_qp_set_matrices",
-           "ismpc_qp_hotstart_batch"]
+           "ismpc_qp_hotstart_batch", "ismpc_forma_solve_batch_ws"]
 
 _lib = None
 
@@ -80,6 +80,7 @@ def lib():
     L.ismpc_forma_rollout_ex2.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 5 + [C.c_int, C.c_void_p]
     L.ismpc_forma_set_model.argtypes = [C.c_void_p, C.c_void_p]
     L.ismpc_forma_solve_batch.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
+    L.ismpc_forma_solve_batch_ws.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
     L.ismpc_forma_rollout.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
     L.ismpc_forma_rollout_ex.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [C.c_int, C.c_void_p]
     L.ismpc_feet_place_rollout.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
@@ -291,7 +292,10 @@ class Handle:
         self._check(self._L.ismpc_forma_set_model(self._h, _ptr(model)), "ismpc_forma_set_model")
         self.forma = model.copy()
 
-    def forma_solve_batch(self, inst, fs_timing, fs_plan, want_primal=True, want_active=True):
+    def forma_solve_batch(self, inst, fs_timing, fs_plan, want_primal=True, want_active=True, ws_guess=None, ws_shift=0):
+        """ws_guess (n x 2(C+F) int8 in the layout of "active", e.g. the "active" of an earlier call): hot start from that
+        working set (ismpc_forma_solve_batch_ws); ws_shift=1 when it is the previous tick's set of these instances.  The
+        results are the cold tick's to rounding."""
         n = len(inst)
         nV = 2 * (int(self.forma["C"][0]) + int(self.forma["F"][0]))
         fs_timing = np.ascontiguousarray(fs_timing, dtype=np.int32)
@@ -299,17 +303,33 @@ class Handle:
         out = np.zeros(n, dtype=abi.FORMA_OUT)
         primal = np.zeros((n, nV)) if want_primal else None
         active = np.zeros((n, nV), dtype=np.int8) if want_active else None
-        rc = self._L.ismpc_forma_solve_batch(self._h, n, _ptr(inst), _ptr(fs_timing), len(fs_timing), _ptr(fs_plan),
-                                             fs_plan.shape[0], _ptr(out), _ptr(primal), _ptr(active), abi.MEM_HOST, None)
-        self._check(rc, "ismpc_forma_solve_batch")
+        if ws_guess is None:
+            rc = self._L.ismpc_forma_solve_batch(self._h, n, _ptr(inst), _ptr(fs_timing), len(fs_timing), _ptr(fs_plan),
+                                                 fs_plan.shape[0], _ptr(out), _ptr(primal), _ptr(active), abi.MEM_HOST, None)
+            self._check(rc, "ismpc_forma_solve_batch")
+            return dict(out=out, primal=primal, active=active)
+        guess = np.ascontiguousarray(ws_guess, dtype=np.int8)
+        if guess.shape != (n, nV):
+            raise ValueError("ws_guess must be %d x %d, got %s" % (n, nV, guess.shape))
+        rc = self._L.ismpc_forma_solve_batch_ws(self._h, n, _ptr(inst), _ptr(fs_timing), len(fs_timing), _ptr(fs_plan),
+                                                fs_plan.shape[0], _ptr(guess), ws_shift, _ptr(out), _ptr(primal),
+                                                _ptr(active), abi.MEM_HOST, None)
+        self._check(rc, "ismpc_forma_solve_batch_ws")
         return dict(out=out, primal=primal, active=active)
 
     def forma_solve_batch_raw(self, n, inst, fs_timing, timing_len, fs_plan, plan_rows, out, primal=None, active=None,
-                              mem=abi.MEM_DEVICE, stream=None):
-        rc = self._L.ismpc_forma_solve_batch(self._h, n, _ptr(inst), _ptr(fs_timing), timing_len, _ptr(fs_plan),
-                                             plan_rows, _ptr(out), _ptr(primal), _ptr(active), mem,
-                                             C.c_void_p(stream) if stream else None)
-        self._check(rc, "ismpc_forma_solve_batch")
+                              mem=abi.MEM_DEVICE, stream=None, ws_guess=None, ws_shift=0):
+        """ws_guess (a pointer, may equal active): hot start from that working set (ismpc_forma_solve_batch_ws)."""
+        st = C.c_void_p(stream) if stream else None
+        if ws_guess is None:
+            rc = self._L.ismpc_forma_solve_batch(self._h, n, _ptr(inst), _ptr(fs_timing), timing_len, _ptr(fs_plan),
+                                                 plan_rows, _ptr(out), _ptr(primal), _ptr(active), mem, st)
+            self._check(rc, "ismpc_forma_solve_batch")
+            return
+        rc = self._L.ismpc_forma_solve_batch_ws(self._h, n, _ptr(inst), _ptr(fs_timing), timing_len, _ptr(fs_plan),
+                                                plan_rows, _ptr(ws_guess), ws_shift, _ptr(out), _ptr(primal), _ptr(active),
+                                                mem, st)
+        self._check(rc, "ismpc_forma_solve_batch_ws")
 
     def forma_rollout(self, inst, fs_timing, fs_plan, n_ticks, push=None, want_traj=True):
         n = len(inst)

@@ -60,6 +60,7 @@ struct ismpc_handle {
     DevBuf s_state, s_walk, s_cinst, s_cout, s_plan, s_primal, s_active, s_push, s_traj, s_status;
     DevBuf s_in;                   // [state | walk | inst] of one form-C tick call
     DevBuf s_ainst, s_aout, s_timing, a_Lwork, a_queue;
+    DevBuf s_aguess;               // working-set guess of a host-memory form-A tick (its own buffer: it may alias active_opt)
     DevBuf q_in, q_out, q_work;
     // dense seam, resident matrix family (ismpc_qp_set_matrices): tables, factor status, workspace of its calls
     DevBuf r_tab, r_stat, r_work;
@@ -123,7 +124,7 @@ extern "C" int ismpc_destroy(ismpc_handle* h)
     cudaSetDevice(h->device);
     DevBuf* all[] = {&h->c_tables, &h->c_work, &h->c_info, &h->c_ptab, &h->c_ric_none, &h->c_ric_gait, &h->c_law_none, &h->c_law_gait, &h->c_ws, &h->c_plan, &h->c_inst, &h->s_tick, &h->s_state, &h->s_walk, &h->s_cinst, &h->s_cout, &h->s_in,
                      &h->s_plan, &h->s_primal, &h->s_active, &h->s_push, &h->s_traj, &h->s_status,
-                     &h->s_ainst, &h->s_aout, &h->s_timing, &h->a_Lwork, &h->a_queue, &h->q_in, &h->q_out, &h->q_work, &h->r_tab, &h->r_stat, &h->r_work, &h->s_pred, &h->f_inst, &h->f_plan, &h->f_out, &h->s_trace};
+                     &h->s_ainst, &h->s_aout, &h->s_timing, &h->a_Lwork, &h->a_queue, &h->q_in, &h->q_out, &h->q_work, &h->r_tab, &h->r_stat, &h->r_work, &h->s_pred, &h->f_inst, &h->f_plan, &h->f_out, &h->s_trace, &h->s_aguess};
     for (DevBuf* b : all) b->release();
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
@@ -641,7 +642,8 @@ extern "C" int ismpc_forma_set_model(ismpc_handle* h, const ismpc_forma_model_t*
 static int forma_common(ismpc_handle* h, int n, int n_ticks, bool rollout, ismpc_forma_inst_t* inst,
                         const int32_t* fs_timing, int timing_len, double* fs_plan, int plan_rows,
                         const ismpc_push_t* push, ismpc_forma_out_t* out, double* primal_opt, int8_t* active_opt,
-                        double* traj_opt, double* pred_opt, int32_t* status_opt, int32_t* trace_opt, int mem, void* stream)
+                        double* traj_opt, double* pred_opt, int32_t* status_opt, int32_t* trace_opt, int mem, void* stream,
+                        const int8_t* ws_guess = nullptr, int ws_shift = 0)
 {
     if (!h) return ISMPC_ERR_ARG;
     if (!h->forma_ready) return ISMPC_ERR_MODEL;
@@ -655,7 +657,7 @@ static int forma_common(ismpc_handle* h, int n, int n_ticks, bool rollout, ismpc
     FormAArgs a;
     a.n = n; a.model = h->am; a.timing_len = timing_len; a.plan_rows = plan_rows; a.sm_count = h->sm_count;
     FormALaunchPlan lp;
-    forma_plan(h->am, h->sm_count, 2LL * n, h->a_tune, &lp, &h->a_occ);
+    forma_plan(h->am, h->sm_count, 2LL * n, h->a_tune, &lp, &h->a_occ, !rollout && ws_guess);
     if (h->a_Lwork.ensure((lp.spill_doubles + 2) * sizeof(double))) return ISMPC_ERR_ALLOC;
     if (!h->a_queue.p) {
         // work-queue head + exit counter of the form-A kernels: zeroed once, every launch leaves them at zero (forma_queue_exit)
@@ -669,7 +671,7 @@ static int forma_common(ismpc_handle* h, int n, int n_ticks, bool rollout, ismpc
         a.inst = inst; a.fs_timing = fs_timing; a.fs_plan = fs_plan; a.out = out; a.primal = primal_opt;
         a.active = (signed char*)active_opt;
         int rc = rollout ? forma_rollout_launch(a, lp, inst, fs_plan, push, n_ticks, traj_opt, pred_opt, status_opt, trace_opt, st)
-                         : forma_tick_launch(a, lp, st);
+                         : forma_tick_launch(a, lp, (const signed char*)ws_guess, ws_shift, st);
         h->launches += rollout ? 2 : 1;
         if (rc) return fail_cuda(h, (cudaError_t)rc, "forma launch");
         return ISMPC_OK;
@@ -681,6 +683,7 @@ static int forma_common(ismpc_handle* h, int n, int n_ticks, bool rollout, ismpc
         return ISMPC_ERR_ALLOC;
     if (primal_opt && h->s_primal.ensure(mb * nV * sizeof(double))) return ISMPC_ERR_ALLOC;
     if (active_opt && h->s_active.ensure(mb * nV)) return ISMPC_ERR_ALLOC;
+    if (ws_guess && h->s_aguess.ensure(mb * nV)) return ISMPC_ERR_ALLOC;
     if (push && h->s_push.ensure(mb * sizeof(ismpc_push_t))) return ISMPC_ERR_ALLOC;
     if (traj_opt && h->s_traj.ensure((size_t)n * n_ticks * 6 * sizeof(double))) return ISMPC_ERR_ALLOC;
     if (pred_opt && h->s_pred.ensure((size_t)n * n_ticks * 2 * sizeof(double))) return ISMPC_ERR_ALLOC;
@@ -690,6 +693,7 @@ static int forma_common(ismpc_handle* h, int n, int n_ticks, bool rollout, ismpc
     CK(cudaMemcpyAsync(h->s_timing.p, fs_timing, (size_t)timing_len * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(h->s_plan.p, fs_plan, (size_t)plan_rows * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
     if (push) CK(cudaMemcpyAsync(h->s_push.p, push, n * sizeof(ismpc_push_t), cudaMemcpyHostToDevice, st));
+    if (ws_guess) CK(cudaMemcpyAsync(h->s_aguess.p, ws_guess, (size_t)n * nV, cudaMemcpyHostToDevice, st));
     a.inst = (const ismpc_forma_inst_t*)h->s_ainst.p; a.fs_timing = (const int32_t*)h->s_timing.p;
     a.fs_plan = (const double*)h->s_plan.p; a.out = (ismpc_forma_out_t*)h->s_aout.p;
     a.primal = primal_opt ? (double*)h->s_primal.p : nullptr;
@@ -702,7 +706,7 @@ static int forma_common(ismpc_handle* h, int n, int n_ticks, bool rollout, ismpc
                                   status_opt ? (int32_t*)h->s_status.p : nullptr,
                                   trace_opt ? (int32_t*)h->s_trace.p : nullptr, st);
     else
-        rc = forma_tick_launch(a, lp, st);
+        rc = forma_tick_launch(a, lp, ws_guess ? (const signed char*)h->s_aguess.p : nullptr, ws_shift, st);
     h->launches += rollout ? 2 : 1;
     if (rc) return fail_cuda(h, (cudaError_t)rc, "forma launch");
     if (rollout) {
@@ -721,13 +725,23 @@ static int forma_common(ismpc_handle* h, int n, int n_ticks, bool rollout, ismpc
     return ISMPC_OK;
 }
 
+extern "C" int ismpc_forma_solve_batch_ws(ismpc_handle* h, int n, const ismpc_forma_inst_t* inst,
+                                          const int32_t* fs_timing, int timing_len, const double* fs_plan, int plan_rows,
+                                          const int8_t* ws_guess, int ws_shift, ismpc_forma_out_t* out, double* primal_opt,
+                                          int8_t* active_opt, int mem, void* stream)
+{
+    if (ws_shift != 0 && ws_shift != 1) return ISMPC_ERR_ARG;
+    return forma_common(h, n, 1, false, const_cast<ismpc_forma_inst_t*>(inst), fs_timing, timing_len,
+                        const_cast<double*>(fs_plan), plan_rows, nullptr, out, primal_opt, active_opt, nullptr,
+                        nullptr, nullptr, nullptr, mem, stream, ws_guess, ws_shift);
+}
+
 extern "C" int ismpc_forma_solve_batch(ismpc_handle* h, int n, const ismpc_forma_inst_t* inst, const int32_t* fs_timing,
                                        int timing_len, const double* fs_plan, int plan_rows, ismpc_forma_out_t* out,
                                        double* primal_opt, int8_t* active_opt, int mem, void* stream)
 {
-    return forma_common(h, n, 1, false, const_cast<ismpc_forma_inst_t*>(inst), fs_timing, timing_len,
-                        const_cast<double*>(fs_plan), plan_rows, nullptr, out, primal_opt, active_opt, nullptr,
-                        nullptr, nullptr, nullptr, mem, stream);
+    return ismpc_forma_solve_batch_ws(h, n, inst, fs_timing, timing_len, fs_plan, plan_rows, nullptr, 0, out, primal_opt,
+                                      active_opt, mem, stream);
 }
 
 extern "C" int ismpc_forma_rollout(ismpc_handle* h, int n, int n_ticks, ismpc_forma_inst_t* inst,

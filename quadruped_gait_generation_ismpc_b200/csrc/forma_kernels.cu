@@ -55,8 +55,12 @@ __device__ __forceinline__ bool forma_inst_in_range(const ismpc_forma_inst_t& in
     return ft[1] > ft[0];
 }
 
-template <int FT, bool HOT>
-__global__ void __maxnreg__(HOT ? FORMA_MAX_REGS : 255) forma_tick_kernel(FormAArgs a)
+// GUESS: every (instance, axis) item starts from a working-set guess instead of the empty set.  ws_guess holds n x 2(C+F)
+// int8 in the layout of `active` ([ZMP_x(C) | ZMP_y(C) | kin_x(F) | kin_y(F)]; -1 lower, +1 upper, anything else free)
+// and may be the same buffer as a.active: an item reads only its own rows, and all of them before it writes any.
+// ws_shift = 1: the guess is the set of the previous tick, shifted here by one tick as the rollout does.
+template <int FT, bool HOT, bool GUESS>
+__global__ void __maxnreg__(HOT ? FORMA_MAX_REGS : 255) forma_tick_kernel(FormAArgs a, const signed char* ws_guess, int ws_shift)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int warp = warp_id(), lane = lane_id();
@@ -84,9 +88,27 @@ __global__ void __maxnreg__(HOT ? FORMA_MAX_REGS : 255) forma_tick_kernel(FormAA
         const double* plan = a.fs_plan + (size_t)in.plan_first_row * 2;
         const int32_t* ft = a.fs_timing + in.timing_first;
         double s3[3] = {in.st[axis * 3 + 0], in.st[axis * 3 + 1], in.st[axis * 3 + 2]};
+        if constexpr (GUESS) {
+            const signed char* g = ws_guess + (size_t)inst * 2 * n;
+            for (int i = lane; i < C; i += 32) {
+                const signed char v = g[axis * C + i];
+                sm.das.state[i] = (v == 1 || v == -1) ? v : (signed char)0;
+            }
+            for (int f = lane; f < F; f += 32) {
+                const signed char v = g[2 * C + axis * F + f];
+                sm.das.state[C + f] = (v == 1 || v == -1) ? v : (signed char)0;
+            }
+            __syncwarp();          // (every lane's reads of the guess rows are done: the item may write `active` later)
+            if (ws_shift) {
+                // first tick after a footstep switch -- the rollout's switch test (forma_rollout_kernel), one tick back:
+                // it moved fs_counter from k to k+1 when j+1 reached ft[k], so this record has j == ft[fs_counter-1]
+                const bool switched = in.fs_counter >= 2 && in.fs_counter <= in.n_timing && in.j == ft[in.fs_counter - 1];
+                forma_shift_working_set(sm.das.state, C, F, switched);
+            }
+        }
         int iters; double kkt;
         int status = forma_tick_axis<FT, HOT>(sm, a.model, in, s3, in.cur_fs[axis], in.fs_store[axis], in.j, in.fs_counter,
-                                         in.cl_first_ramp, plan, ft, axis, 0, a.use_pdas, rg, &iters, &kkt);
+                                         in.cl_first_ramp, plan, ft, axis, GUESS ? 1 : 0, a.use_pdas, rg, &iters, &kkt);
         DasTimer tme; tme.start();
         const double eta = sqrt(a.model.g_eta / in.height);
         const double zd0 = sm.x[0];
@@ -221,11 +243,22 @@ __global__ void forma_rollout_fold(int n, int n_ticks, ismpc_forma_inst_t* inst_
     io->j = j; io->fs_counter = fsc; io->cl_first_ramp = first_ramp;
 }
 
+using FormATickKernel = void (*)(FormAArgs, const signed char*, int);
+
+// build of the tick kernel (FormALaunchPlan::kernel), cold or started from a guessed working set
+static FormATickKernel forma_tick_kernel_for(int kernel, bool guess)
+{
+    if (guess) return kernel == 0 ? forma_tick_kernel<3, true, true> : kernel == 1 ? forma_tick_kernel<3, false, true>
+                                                                     : forma_tick_kernel<ISMPC_MAX_FSTEPS, false, true>;
+    return kernel == 0 ? forma_tick_kernel<3, true, false> : kernel == 1 ? forma_tick_kernel<3, false, false>
+                                                         : forma_tick_kernel<ISMPC_MAX_FSTEPS, false, false>;
+}
+
 // Shared-memory / residency plan for a model: R rows of the inverse factor in shared memory, the rest spilled.
 // occ (in/out, may be null): cache of the occupancy query for this (kernel, CTA size, shared memory) -- the caller keeps it
-// with its handle, the query costs microseconds.
+// with its handle, the query costs microseconds.  guess: the occupancy is that of the tick kernel's GUESS build.
 void forma_plan(const ismpc_forma_model_t& m, int sm_count, long long items, const FormATuning& tune, FormALaunchPlan* p,
-                FormAOccCache* occ)
+                FormAOccCache* occ, bool guess)
 {
     const int C = m.C, F = m.F, q = C + F + 1;
     const size_t lim = 227 * 1024;
@@ -249,23 +282,16 @@ void forma_plan(const ismpc_forma_model_t& m, int sm_count, long long items, con
     // 2 = <ISMPC_MAX_FSTEPS, cold>
     p->kernel = (F <= 3 && C <= 128 && tune.reg) ? 0 : (F <= 3 ? 1 : 2);
     int per_sm = 0;
-    if (occ && occ->per_sm > 0 && occ->F3 == p->kernel && occ->wpc == wpc && occ->smem == p->smem) per_sm = occ->per_sm;
+    if (occ && occ->per_sm > 0 && occ->F3 == p->kernel && occ->guess == (int)guess && occ->wpc == wpc && occ->smem == p->smem)
+        per_sm = occ->per_sm;
     if (per_sm <= 0) {
         // what the GPU really keeps resident (registers and shared memory), asked of the runtime
         int b = 0;
-        cudaError_t e;
-        if (p->kernel == 0) {
-            cudaFuncSetAttribute(forma_tick_kernel<3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
-            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, forma_tick_kernel<3, true>, 32 * wpc, p->smem);
-        } else if (p->kernel == 1) {
-            cudaFuncSetAttribute(forma_tick_kernel<3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
-            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, forma_tick_kernel<3, false>, 32 * wpc, p->smem);
-        } else {
-            cudaFuncSetAttribute(forma_tick_kernel<ISMPC_MAX_FSTEPS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
-            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, forma_tick_kernel<ISMPC_MAX_FSTEPS, false>, 32 * wpc, p->smem);
-        }
+        const FormATickKernel kern = forma_tick_kernel_for(p->kernel, guess);
+        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
+        const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kern, 32 * wpc, p->smem);
         per_sm = (e == cudaSuccess && b > 0) ? b : 1;
-        if (occ) { occ->per_sm = per_sm; occ->F3 = p->kernel; occ->wpc = wpc; occ->smem = p->smem; }
+        if (occ) { occ->per_sm = per_sm; occ->F3 = p->kernel; occ->guess = (int)guess; occ->wpc = wpc; occ->smem = p->smem; }
     }
     long long ctas = (items + wpc - 1) / wpc;
     long long resident = (long long)per_sm * sm_count;
@@ -276,16 +302,18 @@ void forma_plan(const ismpc_forma_model_t& m, int sm_count, long long items, con
     p->warm_start = tune.warm;
 }
 
-int forma_tick_launch(const FormAArgs& a_in, const FormALaunchPlan& p, cudaStream_t st)
+// ws_guess (nullable): n x 2(C+F) working-set guess, may alias a.active; ws_shift: 1 = shift it by one tick first
+int forma_tick_launch(const FormAArgs& a_in, const FormALaunchPlan& p, const signed char* ws_guess, int ws_shift,
+                      cudaStream_t st)
 {
     FormAArgs a = a_in;
     a.R = p.R; a.warps_per_cta = p.warps_per_cta; a.use_pdas = p.use_pdas; a.warm_start = 0;
-    auto kern = p.kernel == 0 ? forma_tick_kernel<3, true> : p.kernel == 1 ? forma_tick_kernel<3, false> : forma_tick_kernel<ISMPC_MAX_FSTEPS, false>;
+    const FormATickKernel kern = forma_tick_kernel_for(p.kernel, ws_guess != nullptr);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
     if (e != cudaSuccess) return (int)e;
     // (the work-queue head needs no reset: the previous launch on this handle left it at zero, forma_queue_exit)
     cudaMemsetAsync(a.out, 0, (size_t)a.n * sizeof(ismpc_forma_out_t), st);
-    kern<<<p.grid, 32 * p.warps_per_cta, p.smem, st>>>(a);
+    kern<<<p.grid, 32 * p.warps_per_cta, p.smem, st>>>(a, ws_guess, ws_shift);
     return (int)cudaGetLastError();
 }
 

@@ -34,10 +34,10 @@ int formc_rollout_warp_launch(const FormCWarpArgs& a, ismpc_state_t* state_io, i
 struct FormALaunchPlan { int R, warps_per_cta, grid, use_pdas, warm_start, kernel; size_t smem, spill_doubles; };
 // tuning of the form-A kernels (ismpc_set_option "forma_*"): 0 = default for R and warps_per_cta
 struct FormATuning { int R = 0, warps_per_cta = 0, pdas = 1, warm = 1, reg = 1; };
-struct FormAOccCache { int per_sm = 0, F3 = -1 /* build of the kernels the entry belongs to */, wpc = 0; size_t smem = 0; };
+struct FormAOccCache { int per_sm = 0, F3 = -1 /* build of the kernels the entry belongs to */, guess = 0, wpc = 0; size_t smem = 0; };
 void forma_plan(const ismpc_forma_model_t& m, int sm_count, long long items, const FormATuning& tune, FormALaunchPlan* p,
-                FormAOccCache* occ);
-int forma_tick_launch(const FormAArgs& a, const FormALaunchPlan& p, cudaStream_t st);
+                FormAOccCache* occ, bool guess);
+int forma_tick_launch(const FormAArgs& a, const FormALaunchPlan& p, const signed char* ws_guess, int ws_shift, cudaStream_t st);
 int forma_rollout_launch(const FormAArgs& a, const FormALaunchPlan& p, ismpc_forma_inst_t* inst_io,
                          double* fs_plan_io, const ismpc_push_t* push, int n_ticks, double* traj, double* pred,
                          int32_t* status, int32_t* trace, cudaStream_t st);

@@ -3,6 +3,7 @@
 formc_batch  -- config 2: independent trot instances for MPCSolver::solve (formulation C)
 forma_batch  -- configs 2/3: trot / walk instances for the canonical ISMPC (formulation A) at the
                 start-of-gait state (tick j = 1); mid-gait states are produced by rolling these forward
+forma_next_records -- the next tick's formulation-A records from a tick's results (a caller-driven closed loop)
 """
 import numpy as np
 
@@ -117,6 +118,37 @@ def forma_batch(n, seed=SEED0 ^ 3, gait="trot", C=100, step=50, ds=20, sim_ticks
         inst["timing_first"][i], inst["n_timing"][i] = first[s]
         inst["plan_first_row"][i] = i * N_gait; inst["n_fs"][i] = N_gait
     return inst, fs_timing, fs_plan
+
+
+def forma_next_records(inst, fs_timing, fs_plan, out, F=3):
+    """The records of the next tick after a formulation-A tick (ismpc_forma_solve_batch[_ws]) returned `out` for `inst`:
+    one step of the closed loop, on the host, as forma_rollout_kernel / forma_rollout_fold take it on the device.  The
+    state comes from out["st"]; where the timing table says the step ends (j + 1 >= ft[fs_counter]), fs_counter advances,
+    the predicted footstep out["pred_fs"] (x at [0], y at [F]; F = the model's footstep count) becomes cur_fs / fs_store,
+    the instance's plan rows are shifted to it and cl_first_ramp drops (bang.m:529-556); j advances.  Records outside
+    the tables (which the tick flags and skips) stay as they are.  Returns (inst, fs_plan), new arrays; a push is the
+    caller's to add to "st" before the next call."""
+    ft = np.asarray(fs_timing)
+    nxt = inst.copy()
+    plan = np.array(fs_plan, dtype=np.float64)
+    for i in range(len(inst)):
+        r = inst[i]
+        tf, nt, pf, nf = int(r["timing_first"]), int(r["n_timing"]), int(r["plan_first_row"]), int(r["n_fs"])
+        fsc, j = int(r["fs_counter"]), int(r["j"])
+        if not (pf >= 0 and nf >= 2 and pf + nf <= plan.shape[0] and tf >= 0 and nt >= 2 and tf + nt <= len(ft)
+                and fsc >= 1 and j >= 1 and r["ds"] >= 1 and ft[tf + 1] > ft[tf]):
+            continue                                            # forma_inst_in_range: the tick did not touch it
+        nxt["st"][i] = out["st"][i]
+        if fsc + 1 <= nt and j + 1 >= ft[tf + fsc]:
+            fsc += 1
+            pred = np.array([out["pred_fs"][i][0], out["pred_fs"][i][F]])
+            nxt["cur_fs"][i] = pred; nxt["fs_store"][i] = pred
+            if 2 <= fsc <= nf:
+                plan[pf:pf + nf] += pred - plan[pf + fsc - 1]
+                nxt["cl_first_ramp"][i] = 0
+            nxt["fs_counter"][i] = fsc
+        nxt["j"][i] = j + 1
+    return nxt, plan
 
 
 def push_batch(n, seed=SEED0 ^ 5, formc=False):
