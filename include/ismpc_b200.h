@@ -22,7 +22,7 @@
  * void* (NULL = default stream).  With ISMPC_MEM_DEVICE every data pointer is a device pointer, the
  * call only enqueues work on `stream` and returns; with ISMPC_MEM_HOST every data pointer is a host
  * pointer (pinned for best speed), the call copies in, launches, copies out and synchronises the
- * stream before returning; ISMPC_MEM_HOST_ASYNC (ismpc_formc_solve_batch, ismpc_forma_solve_batch[_ws] and the ismpc_forma_rollout calls) is the same without the final
+ * stream before returning; ISMPC_MEM_HOST_ASYNC (ismpc_formc_solve_batch[_packed], ismpc_forma_solve_batch[_ws] and the ismpc_forma_rollout calls) is the same without the final
  * synchronisation: the call returns as soon as the copies and the kernel are enqueued, the host buffers must be
  * pinned and stay untouched, and the handle must not be used again, until the caller has synchronised `stream` --
  * two handles on two streams give a double-buffered pipeline.  The caller owns all buffers; the handle owns only its workspace.

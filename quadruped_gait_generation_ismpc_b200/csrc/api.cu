@@ -15,6 +15,10 @@ using namespace ismpc;
 struct DevBuf {
     void* p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() { if (p) cudaFree(p); }
     int ensure(size_t bytes)
     {
         if (bytes <= cap) return 0;
@@ -24,8 +28,12 @@ struct DevBuf {
         cap = bytes;
         return 0;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
 };
+
+// Host-memory calls stage their buffers in ismpc_handle::stage, taken in the order the call asks for them: a loop of one
+// call keeps each buffer in one role, so a buffer grows once.  The form-A tick and rollouts stage the most (12 arguments;
+// NULL ones keep their place).
+constexpr int STAGE_SLOTS = 12;
 
 struct ismpc_handle {
     int device = 0;
@@ -47,8 +55,7 @@ struct ismpc_handle {
     DevBuf c_ric_none, c_ric_gait, c_law_none, c_law_gait, c_ws, c_plan, c_inst;
     int inst_res_n = 0;            // instance records resident in c_inst (ismpc_formc_set_instances), 0 = none
     int opt_host_zero_copy = 1;    // packed host-memory ticks: the kernel reads / writes the caller's pinned buffers itself
-    DevBuf s_tick;                 // staging of the packed tick records when they cannot be read in place
-    int plan_res_rows = 0;         // rows of the resident footstep-plan table (ismpc_formc_set_plan), 0 = none   // Riccati tables (warp kernels) and the per-warp workspace of their general path
+    int plan_res_rows = 0;         // rows of the resident footstep-plan table (ismpc_formc_set_plan), 0 = none
     int gait_S = 0, gait_F = 0;            // prepared gait (projector tables in c_ptab), 0 = none
     int ric_S = 0, ric_F = 0;              // prepared gait of the Riccati tables (c_ric_gait), 0 = none
     // form A
@@ -56,17 +63,13 @@ struct ismpc_handle {
     ismpc_forma_model_t am{};
     FormAOccCache a_occ;           // occupancy of the form-A kernels for the current shape (queried once)
     FormATuning a_tune;            // ismpc_set_option("forma_*"); the ISMPC_FORMA_* environment variables set the defaults at creation
-    // staging (host-memory calls)
-    DevBuf s_state, s_walk, s_cinst, s_cout, s_plan, s_primal, s_active, s_push, s_traj, s_status;
-    DevBuf s_in;                   // [state | walk | inst] of one form-C tick call
-    DevBuf s_ainst, s_aout, s_timing, a_Lwork, a_queue;
-    DevBuf s_aguess;               // working-set guess of a host-memory form-A tick (its own buffer: it may alias active_opt)
-    DevBuf q_in, q_out, q_work;
+    DevBuf a_Lwork, a_queue;
+    DevBuf q_work;                         // dense seam: workspace of its calls
     // dense seam, resident matrix family (ismpc_qp_set_matrices): tables, factor status, workspace of its calls
     DevBuf r_tab, r_stat, r_work;
     int r_nmat = 0, r_nV = 0, r_nC = 0;    // resident sets and their shape, 0 = none
     int opt_dense_resident_gemm = 1;       // a single shared set: x0 | A x0 of a call as one tensor-core product
-    DevBuf s_pred, f_inst, f_plan, f_out, s_trace;
+    DevBuf stage[STAGE_SLOTS];             // staging of host-memory calls (Staged)
     cudaStream_t own_stream = nullptr;     // ismpc_handle_stream: created on first use, destroyed with the handle
 };
 
@@ -122,12 +125,8 @@ extern "C" int ismpc_destroy(ismpc_handle* h)
 {
     if (!h) return ISMPC_ERR_ARG;
     cudaSetDevice(h->device);
-    DevBuf* all[] = {&h->c_tables, &h->c_work, &h->c_info, &h->c_ptab, &h->c_ric_none, &h->c_ric_gait, &h->c_law_none, &h->c_law_gait, &h->c_ws, &h->c_plan, &h->c_inst, &h->s_tick, &h->s_state, &h->s_walk, &h->s_cinst, &h->s_cout, &h->s_in,
-                     &h->s_plan, &h->s_primal, &h->s_active, &h->s_push, &h->s_traj, &h->s_status,
-                     &h->s_ainst, &h->s_aout, &h->s_timing, &h->a_Lwork, &h->a_queue, &h->q_in, &h->q_out, &h->q_work, &h->r_tab, &h->r_stat, &h->r_work, &h->s_pred, &h->f_inst, &h->f_plan, &h->f_out, &h->s_trace, &h->s_aguess};
-    for (DevBuf* b : all) b->release();
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
-    delete h;
+    delete h;                      // the DevBufs free their device memory
     return ISMPC_OK;
 }
 
@@ -225,6 +224,90 @@ extern "C" int ismpc_set_option(ismpc_handle* h, const char* name, int value)
 extern "C" const char* ismpc_last_cuda_error(const ismpc_handle* h) { return h ? h->err : ""; }
 extern "C" int64_t ismpc_kernel_launches(const ismpc_handle* h) { return h ? h->launches : 0; }
 
+// Device address of a host buffer the kernels may touch in place: pinned (cudaHostAlloc / cudaHostRegister), 128-byte
+// aligned, at most ZC_MAX_BYTES (larger transfers are the copy engines' business); nullptr otherwise.
+static void* zero_copy_address(const void* p, size_t bytes)
+{
+    constexpr size_t ZC_MAX_BYTES = 8u << 20;
+    if (!p || ((uintptr_t)p & 127u) != 0 || bytes > ZC_MAX_BYTES) return nullptr;
+    if (host_range_known(p, bytes)) return const_cast<void*>(p);
+    cudaPointerAttributes pa;
+    if (cudaPointerGetAttributes(&pa, p) != cudaSuccess) { (void)cudaGetLastError(); return nullptr; }
+    return (pa.type == cudaMemoryTypeHost && pa.devicePointer) ? pa.devicePointer : nullptr;
+}
+
+// The buffers of one call that takes data.  ISMPC_MEM_DEVICE passes every pointer through.  The host modes stage each
+// buffer in the handle's next staging slot, copy inputs in at once and queue outputs to be copied back by finish(),
+// which also synchronises the stream for ISMPC_MEM_HOST.  A NULL pointer stays NULL in every mode.  `reserve` (in
+// elements) sizes a staging buffer beyond this call: per-instance arrays reserve max_batch rows, so a batch that grows
+// does not reallocate in the middle of a loop.  The first failure is kept in err; the call returns it before the launch.
+struct Staged {
+    ismpc_handle* h;
+    cudaStream_t st;
+    int mem;
+    bool host = false;             // a host mode the call accepts
+    int err = ISMPC_OK;
+    int slot = 0, n_back = 0;
+    struct CopyBack { void* dst; const void* src; size_t bytes; } back[STAGE_SLOTS];
+
+    Staged(ismpc_handle* h_, int mem_, void* stream, bool async_ok) : h(h_), st((cudaStream_t)stream), mem(mem_)
+    {
+        host = mem == ISMPC_MEM_HOST || (async_ok && mem == ISMPC_MEM_HOST_ASYNC);
+        if (!host && mem != ISMPC_MEM_DEVICE) err = ISMPC_ERR_ARG;
+    }
+    template <class T> T* in(T* p, size_t count, size_t reserve = 0) { return stage(p, count, reserve, true, false); }
+    template <class T> T* out(T* p, size_t count, size_t reserve = 0) { return stage(p, count, reserve, false, true); }
+    template <class T> T* inout(T* p, size_t count, size_t reserve = 0) { return stage(p, count, reserve, true, true); }
+    // the packed tick: a pinned host buffer the kernel can address is read / written in place (option host_zero_copy)
+    template <class T> T* in_place_or_in(T* p, size_t count, size_t reserve)
+    {
+        if (T* d = in_place(p, count)) return d;
+        return in(p, count, reserve);
+    }
+    template <class T> T* in_place_or_out(T* p, size_t count, size_t reserve)
+    {
+        if (T* d = in_place(p, count)) return d;
+        return out(p, count, reserve);
+    }
+    // After the launch (`launches` kernels counted, `rc` its result): queue the copies back, then synchronise for
+    // ISMPC_MEM_HOST.
+    int finish(int rc, const char* what, int launches = 1)
+    {
+        h->launches += launches;
+        if (rc) return fail_cuda(h, (cudaError_t)rc, what);
+        for (int i = 0; i < n_back; ++i) {
+            const cudaError_t e = cudaMemcpyAsync(back[i].dst, back[i].src, back[i].bytes, cudaMemcpyDeviceToHost, st);
+            if (e != cudaSuccess) return fail_cuda(h, e, "cudaMemcpyAsync (device to host)");
+        }
+        if (mem == ISMPC_MEM_HOST) CK(cudaStreamSynchronize(st));
+        return ISMPC_OK;
+    }
+
+  private:
+    template <class T> T* stage(T* p, size_t count, size_t reserve, bool copy_in, bool copy_back)
+    {
+        if (!host) return p;
+        if (slot >= STAGE_SLOTS) { if (!err) err = ISMPC_ERR_ALLOC; return nullptr; }
+        DevBuf& b = h->stage[slot++];
+        if (!p || err) return nullptr;
+        const size_t bytes = count * sizeof(T);
+        if (b.ensure((count > reserve ? count : reserve) * sizeof(T))) { err = ISMPC_ERR_ALLOC; return nullptr; }
+        if (copy_in && bytes) {
+            const cudaError_t e = cudaMemcpyAsync(b.p, p, bytes, cudaMemcpyHostToDevice, st);
+            if (e != cudaSuccess) { err = fail_cuda(h, e, "cudaMemcpyAsync (host to device)"); return nullptr; }
+        }
+        if (copy_back && bytes) back[n_back++] = {const_cast<void*>((const void*)p), b.p, bytes};
+        return (T*)b.p;
+    }
+    template <class T> T* in_place(T* p, size_t count)
+    {
+        if (!host || !h->opt_host_zero_copy) return nullptr;
+        T* d = (T*)zero_copy_address(p, count * sizeof(T));
+        if (d) ++slot;
+        return d;
+    }
+};
+
 // ---------------------------------------------------------------------------------------------------
 // Formulation C
 // ---------------------------------------------------------------------------------------------------
@@ -272,14 +355,37 @@ static int formc_cluster_size(const ismpc_handle* h, int n)
     return 1;
 }
 
-static void formc_fill_args(ismpc_handle* h, FormCArgs& a, int n)
+// A form-C call with inst == NULL / plan_xyzt == NULL reads the instances / plan made resident by
+// ismpc_formc_set_instances / ismpc_formc_set_plan.  Resolves the call's plan rows; false when the call cannot run.
+static bool formc_resident_ok(const ismpc_handle* h, int n, const ismpc_formc_inst_t* inst, const double* plan_xyzt,
+                              int& plan_rows)
+{
+    if (!plan_xyzt) plan_rows = h->plan_res_rows;
+    return (inst || n <= h->inst_res_n) && plan_rows > 0;
+}
+
+// Host buffers can be read here: a host-memory call with instances prepares the gait of inst[0] if none is prepared.
+static int formc_auto_gait(ismpc_handle* h, const ismpc_formc_inst_t* inst, bool host)
+{
+    if (!host || !inst || !h->formc_ready || h->ric_S + h->ric_F != 0) return ISMPC_OK;
+    const int S = inst[0].S, F = inst[0].F_ds;
+    return (S >= 0 && F >= 0 && S + F > 0) ? ismpc_formc_prepare_gait(h, S, F) : ISMPC_OK;
+}
+
+// Tables and defaults of a form-C launch: no outputs, the resident instances and plan (callers that pass their own
+// replace them).
+static void formc_fill_args(ismpc_handle* h, FormCArgs& a, int n, int plan_rows)
 {
     const size_t NN = (size_t)h->cm.N * h->cm.N;
     const double* T = (const double*)h->c_tables.p;
-    a.n = n; a.model = h->cm; a.tick = nullptr;
+    a.n = n; a.model = h->cm;
     a.T.Hinv = T; a.T.G = T + NN; a.T.M = T + 2 * NN;
     a.T.P = (h->gait_S + h->gait_F > 0) ? (const double*)h->c_ptab.p : nullptr;
     a.T.gS = h->gait_S; a.T.gF = h->gait_F;
+    a.state = nullptr; a.walk = nullptr; a.tick = nullptr;
+    a.inst = (const ismpc_formc_inst_t*)h->c_inst.p;
+    a.plan = (const double*)h->c_plan.p; a.plan_rows = plan_rows;
+    a.out = nullptr; a.primal = nullptr; a.active = nullptr;
 }
 
 // Warp-per-instance kernels cover N <= 512; the CTA/cluster kernels stay for the cluster latency mode and on request.
@@ -385,66 +491,34 @@ extern "C" int ismpc_formc_solve_batch(ismpc_handle* h, int n, const ismpc_state
 {
     if (!h) return ISMPC_ERR_ARG;
     if (!h->formc_ready) return ISMPC_ERR_MODEL;
-    const bool plan_res = plan_xyzt == nullptr;
-    if (plan_res) plan_rows = h->plan_res_rows;
-    const bool inst_res = inst == nullptr;
-    if (n < 0 || n > h->max_batch || !state || !walk || (inst_res && n > h->inst_res_n) || !out || plan_rows <= 0)
+    if (n < 0 || n > h->max_batch || !state || !walk || !out || !formc_resident_ok(h, n, inst, plan_xyzt, plan_rows))
         return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    const int N = h->cm.N;
+    Staged s(h, mem, stream, true);
+    if (int rc = formc_auto_gait(h, inst, s.host)) return rc;
+    const size_t mb = (size_t)h->max_batch, N3 = 3 * (size_t)h->cm.N;
     FormCArgs a;
-    formc_fill_args(h, a, n);
-    if (mem == ISMPC_MEM_DEVICE) {
-        a.state = state; a.walk = walk; a.inst = inst_res ? (const ismpc_formc_inst_t*)h->c_inst.p : inst; a.plan = plan_res ? (const double*)h->c_plan.p : plan_xyzt; a.plan_rows = plan_rows;
-        a.out = out; a.primal = primal_opt; a.active = (signed char*)active_opt;
-        int rc = formc_launch_tick(h, a, n, st);
-        h->launches += 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "formc_tick_launch");
-        return ISMPC_OK;
-    }
-    if (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_HOST_ASYNC) return ISMPC_ERR_ARG;
-    if (!inst_res && h->ric_S + h->ric_F == 0 && inst[0].S + inst[0].F_ds > 0 && inst[0].S >= 0 && inst[0].F_ds >= 0) {
-        int prc = ismpc_formc_prepare_gait(h, inst[0].S, inst[0].F_ds);      // host buffers: the gait can be read here
-        if (prc != ISMPC_OK) return prc;
-        formc_fill_args(h, a, n);
-    }
-    const size_t mb = (size_t)h->max_batch;
-    // one staging buffer laid out [state n | walk n | inst n]: when the caller's three arrays lie back to back in one
-    // (pinned) allocation the tick's inputs move in ONE copy instead of three (each small copy costs ~2 us of API and
-    // DMA set-up, about a quarter of the kernel)
+    formc_fill_args(h, a, n, plan_rows);
+    // when the caller's three arrays lie back to back in one (pinned) allocation the tick's inputs move in ONE copy
+    // instead of three (each small copy costs ~2 us of API and DMA set-up, about a quarter of the kernel)
     const size_t b_state = (size_t)n * sizeof(ismpc_state_t), b_walk = (size_t)n * sizeof(ismpc_walk_t),
-                 b_inst = inst_res ? 0 : (size_t)n * sizeof(ismpc_formc_inst_t);
-    if (h->s_in.ensure(mb * (sizeof(ismpc_state_t) + sizeof(ismpc_walk_t) + sizeof(ismpc_formc_inst_t))) ||
-        h->s_cout.ensure(mb * sizeof(ismpc_formc_out_t)) ||
-        (!plan_res && h->s_plan.ensure((size_t)plan_rows * 4 * sizeof(double))))
-        return ISMPC_ERR_ALLOC;
-    if (primal_opt && h->s_primal.ensure(mb * 3 * N * sizeof(double))) return ISMPC_ERR_ALLOC;
-    if (active_opt && h->s_active.ensure(mb * 3 * N)) return ISMPC_ERR_ALLOC;
-    char* d_in = (char*)h->s_in.p;
-    if ((const char*)walk == (const char*)state + b_state && (inst_res || (const char*)inst == (const char*)walk + b_walk)) {
-        CK(cudaMemcpyAsync(d_in, state, b_state + b_walk + b_inst, cudaMemcpyHostToDevice, st));
+                 b_inst = inst ? (size_t)n * sizeof(ismpc_formc_inst_t) : 0;
+    if ((const char*)walk == (const char*)state + b_state && (!inst || (const char*)inst == (const char*)walk + b_walk)) {
+        const char* in = s.in((const char*)state, b_state + b_walk + b_inst,
+                              mb * (sizeof(ismpc_state_t) + sizeof(ismpc_walk_t) + sizeof(ismpc_formc_inst_t)));
+        a.state = (const ismpc_state_t*)in; a.walk = (const ismpc_walk_t*)(in + b_state);
+        if (inst) a.inst = (const ismpc_formc_inst_t*)(in + b_state + b_walk);
     } else {
-        CK(cudaMemcpyAsync(d_in, state, b_state, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d_in + b_state, walk, b_walk, cudaMemcpyHostToDevice, st));
-        if (!inst_res) CK(cudaMemcpyAsync(d_in + b_state + b_walk, inst, b_inst, cudaMemcpyHostToDevice, st));
+        a.state = s.in(state, n, mb); a.walk = s.in(walk, n, mb);
+        if (const ismpc_formc_inst_t* p = s.in(inst, n, mb)) a.inst = p;
     }
-    if (!plan_res) CK(cudaMemcpyAsync(h->s_plan.p, plan_xyzt, (size_t)plan_rows * 4 * sizeof(double), cudaMemcpyHostToDevice, st));
-    a.state = (const ismpc_state_t*)d_in; a.walk = (const ismpc_walk_t*)(d_in + b_state);
-    a.inst = inst_res ? (const ismpc_formc_inst_t*)h->c_inst.p : (const ismpc_formc_inst_t*)(d_in + b_state + b_walk); a.plan = plan_res ? (const double*)h->c_plan.p : (const double*)h->s_plan.p;
-    a.plan_rows = plan_rows;
-    a.out = (ismpc_formc_out_t*)h->s_cout.p;
-    a.primal = primal_opt ? (double*)h->s_primal.p : nullptr;
-    a.active = active_opt ? (signed char*)h->s_active.p : nullptr;
-    int rc = formc_launch_tick(h, a, n, st);
-    h->launches += 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "formc_tick_launch");
-    CK(cudaMemcpyAsync(out, h->s_cout.p, n * sizeof(ismpc_formc_out_t), cudaMemcpyDeviceToHost, st));
-    if (primal_opt) CK(cudaMemcpyAsync(primal_opt, h->s_primal.p, (size_t)n * 3 * N * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (active_opt) CK(cudaMemcpyAsync(active_opt, h->s_active.p, (size_t)n * 3 * N, cudaMemcpyDeviceToHost, st));
-    if (mem == ISMPC_MEM_HOST) CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    if (const double* p = s.in(plan_xyzt, (size_t)plan_rows * 4)) a.plan = p;
+    a.out = s.out(out, n, mb);
+    a.primal = s.out(primal_opt, n * N3, mb * N3);
+    a.active = (signed char*)s.out(active_opt, n * N3, mb * N3);
+    if (s.err) return s.err;
+    return s.finish(formc_launch_tick(h, a, n, s.st), "formc_tick_launch");
 }
 
 extern "C" int ismpc_formc_set_instances(ismpc_handle* h, const ismpc_formc_inst_t* inst, int n, int mem)
@@ -452,28 +526,12 @@ extern "C" int ismpc_formc_set_instances(ismpc_handle* h, const ismpc_formc_inst
     if (!h || n < 0 || n > h->max_batch || (n > 0 && !inst) || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE)) return ISMPC_ERR_ARG;
     if (n == 0) { h->inst_res_n = 0; return ISMPC_OK; }
     CK(cudaSetDevice(h->device));
-    if (mem == ISMPC_MEM_HOST && h->formc_ready && h->ric_S + h->ric_F == 0 && inst[0].S + inst[0].F_ds > 0 && inst[0].S >= 0 &&
-        inst[0].F_ds >= 0) {
-        int prc = ismpc_formc_prepare_gait(h, inst[0].S, inst[0].F_ds);
-        if (prc != ISMPC_OK) return prc;
-    }
+    if (int rc = formc_auto_gait(h, inst, mem == ISMPC_MEM_HOST)) return rc;
     if (h->c_inst.ensure((size_t)h->max_batch * sizeof(ismpc_formc_inst_t))) return ISMPC_ERR_ALLOC;
     CK(cudaMemcpy(h->c_inst.p, inst, (size_t)n * sizeof(ismpc_formc_inst_t),
                   mem == ISMPC_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice));
     h->inst_res_n = n;
     return ISMPC_OK;
-}
-
-// Device address of a host buffer the kernels may touch in place: pinned (cudaHostAlloc / cudaHostRegister), 128-byte
-// aligned, at most ZC_MAX_BYTES (larger transfers are the copy engines' business); nullptr otherwise.
-static void* zero_copy_address(const void* p, size_t bytes)
-{
-    constexpr size_t ZC_MAX_BYTES = 8u << 20;
-    if (!p || ((uintptr_t)p & 127u) != 0 || bytes > ZC_MAX_BYTES) return nullptr;
-    if (host_range_known(p, bytes)) return const_cast<void*>(p);
-    cudaPointerAttributes pa;
-    if (cudaPointerGetAttributes(&pa, p) != cudaSuccess) { (void)cudaGetLastError(); return nullptr; }
-    return (pa.type == cudaMemoryTypeHost && pa.devicePointer) ? pa.devicePointer : nullptr;
 }
 
 extern "C" int ismpc_formc_solve_batch_packed(ismpc_handle* h, int n, const ismpc_formc_tick_t* tick,
@@ -483,73 +541,26 @@ extern "C" int ismpc_formc_solve_batch_packed(ismpc_handle* h, int n, const ismp
 {
     if (!h) return ISMPC_ERR_ARG;
     if (!h->formc_ready) return ISMPC_ERR_MODEL;
-    const bool plan_res = plan_xyzt == nullptr, inst_res = inst == nullptr;
-    if (plan_res) plan_rows = h->plan_res_rows;
-    if (n < 0 || n > h->max_batch || !tick || ((uintptr_t)tick & 15u) != 0 || (inst_res && n > h->inst_res_n) || !out ||
-        plan_rows <= 0 || !formc_use_warp(h))
+    if (n < 0 || n > h->max_batch || !tick || ((uintptr_t)tick & 15u) != 0 || !out ||
+        !formc_resident_ok(h, n, inst, plan_xyzt, plan_rows) || !formc_use_warp(h))
         return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    const int N = h->cm.N;
+    Staged s(h, mem, stream, true);
+    if (int rc = formc_auto_gait(h, inst, s.host)) return rc;
+    const size_t mb = (size_t)h->max_batch, N3 = 3 * (size_t)h->cm.N;
     FormCArgs a;
-    formc_fill_args(h, a, n);
-    a.state = nullptr; a.walk = nullptr; a.plan_rows = plan_rows;
-    if (mem == ISMPC_MEM_DEVICE) {
-        a.tick = tick; a.inst = inst_res ? (const ismpc_formc_inst_t*)h->c_inst.p : inst;
-        a.plan = plan_res ? (const double*)h->c_plan.p : plan_xyzt;
-        a.out = out; a.primal = primal_opt; a.active = (signed char*)active_opt;
-        int rc = formc_launch_tick(h, a, n, st);
-        h->launches += 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "formc_tick_launch");
-        return ISMPC_OK;
-    }
-    if (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_HOST_ASYNC) return ISMPC_ERR_ARG;
-    if (!inst_res && h->ric_S + h->ric_F == 0 && inst[0].S + inst[0].F_ds > 0 && inst[0].S >= 0 && inst[0].F_ds >= 0) {
-        int prc = ismpc_formc_prepare_gait(h, inst[0].S, inst[0].F_ds);
-        if (prc != ISMPC_OK) return prc;
-        formc_fill_args(h, a, n);
-        a.state = nullptr; a.walk = nullptr; a.plan_rows = plan_rows;
-    }
-    const size_t mb = (size_t)h->max_batch;
-    const size_t b_tick = (size_t)n * sizeof(ismpc_formc_tick_t), b_out = (size_t)n * sizeof(ismpc_formc_out_t);
+    formc_fill_args(h, a, n, plan_rows);
     // in place where the buffers allow it (see the header): one 128-byte PCIe read and one posted 128-byte write per
     // instance, issued by the instance's own CTA, instead of two DMA copies around the kernel
-    const ismpc_formc_tick_t* tick_dev = h->opt_host_zero_copy ? (const ismpc_formc_tick_t*)zero_copy_address(tick, b_tick) : nullptr;
-    ismpc_formc_out_t* out_dev = h->opt_host_zero_copy ? (ismpc_formc_out_t*)zero_copy_address(out, b_out) : nullptr;
-    if (!tick_dev) {
-        if (h->s_tick.ensure(mb * sizeof(ismpc_formc_tick_t))) return ISMPC_ERR_ALLOC;
-        CK(cudaMemcpyAsync(h->s_tick.p, tick, b_tick, cudaMemcpyHostToDevice, st));
-        tick_dev = (const ismpc_formc_tick_t*)h->s_tick.p;
-    }
-    if (!out_dev) {
-        if (h->s_cout.ensure(mb * sizeof(ismpc_formc_out_t))) return ISMPC_ERR_ALLOC;
-        out_dev = (ismpc_formc_out_t*)h->s_cout.p;
-    }
-    if (!inst_res) {
-        if (h->s_cinst.ensure(mb * sizeof(ismpc_formc_inst_t))) return ISMPC_ERR_ALLOC;
-        CK(cudaMemcpyAsync(h->s_cinst.p, inst, (size_t)n * sizeof(ismpc_formc_inst_t), cudaMemcpyHostToDevice, st));
-    }
-    if (!plan_res) {
-        if (h->s_plan.ensure((size_t)plan_rows * 4 * sizeof(double))) return ISMPC_ERR_ALLOC;
-        CK(cudaMemcpyAsync(h->s_plan.p, plan_xyzt, (size_t)plan_rows * 4 * sizeof(double), cudaMemcpyHostToDevice, st));
-    }
-    if (primal_opt && h->s_primal.ensure(mb * 3 * N * sizeof(double))) return ISMPC_ERR_ALLOC;
-    if (active_opt && h->s_active.ensure(mb * 3 * N)) return ISMPC_ERR_ALLOC;
-    a.tick = tick_dev;
-    a.inst = inst_res ? (const ismpc_formc_inst_t*)h->c_inst.p : (const ismpc_formc_inst_t*)h->s_cinst.p;
-    a.plan = plan_res ? (const double*)h->c_plan.p : (const double*)h->s_plan.p;
-    a.out = out_dev;
-    a.primal = primal_opt ? (double*)h->s_primal.p : nullptr;
-    a.active = active_opt ? (signed char*)h->s_active.p : nullptr;
-    int rc = formc_launch_tick(h, a, n, st);
-    h->launches += 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "formc_tick_launch");
-    if ((void*)out_dev == h->s_cout.p) CK(cudaMemcpyAsync(out, h->s_cout.p, b_out, cudaMemcpyDeviceToHost, st));
-    if (primal_opt) CK(cudaMemcpyAsync(primal_opt, h->s_primal.p, (size_t)n * 3 * N * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (active_opt) CK(cudaMemcpyAsync(active_opt, h->s_active.p, (size_t)n * 3 * N, cudaMemcpyDeviceToHost, st));
-    if (mem == ISMPC_MEM_HOST) CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    a.tick = s.in_place_or_in(tick, n, mb);
+    if (const ismpc_formc_inst_t* p = s.in(inst, n, mb)) a.inst = p;
+    if (const double* p = s.in(plan_xyzt, (size_t)plan_rows * 4)) a.plan = p;
+    a.out = s.in_place_or_out(out, n, mb);
+    a.primal = s.out(primal_opt, n * N3, mb * N3);
+    a.active = (signed char*)s.out(active_opt, n * N3, mb * N3);
+    if (s.err) return s.err;
+    return s.finish(formc_launch_tick(h, a, n, s.st), "formc_tick_launch");
 }
 
 extern "C" int ismpc_formc_rollout(ismpc_handle* h, int n, int n_ticks, ismpc_state_t* state, ismpc_walk_t* walk,
@@ -568,61 +579,27 @@ extern "C" int ismpc_formc_rollout_ex(ismpc_handle* h, int n, int n_ticks, ismpc
 {
     if (!h) return ISMPC_ERR_ARG;
     if (!h->formc_ready) return ISMPC_ERR_MODEL;
-    const bool plan_res = plan_xyzt == nullptr;
-    if (plan_res) plan_rows = h->plan_res_rows;
-    const bool inst_res = inst == nullptr;      // the per-instance constants given to ismpc_formc_set_instances
-    if (n < 0 || n > h->max_batch || n_ticks < 0 || !state || !walk || (inst_res && n > h->inst_res_n) || plan_rows <= 0)
+    if (n < 0 || n > h->max_batch || n_ticks < 0 || !state || !walk || !formc_resident_ok(h, n, inst, plan_xyzt, plan_rows))
         return ISMPC_ERR_ARG;
     if (n == 0 || n_ticks == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
+    Staged s(h, mem, stream, false);
+    if (int rc = formc_auto_gait(h, inst, s.host)) return rc;
+    const size_t mb = (size_t)h->max_batch, nt = (size_t)n * n_ticks;
     FormCArgs a;
-    formc_fill_args(h, a, n);
-    a.out = nullptr; a.primal = nullptr; a.active = nullptr; a.plan_rows = plan_rows;
-    if (mem == ISMPC_MEM_DEVICE) {
-        a.state = state; a.walk = walk; a.inst = inst_res ? (const ismpc_formc_inst_t*)h->c_inst.p : inst;
-        a.plan = plan_res ? (const double*)h->c_plan.p : plan_xyzt;
-        int rc = formc_launch_rollout(h, a, n, state, walk, push, n_ticks, traj_opt, status_opt, status_trace_opt, st);
-        h->launches += 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "formc_rollout_launch");
-        return ISMPC_OK;
-    }
-    if (mem != ISMPC_MEM_HOST) return ISMPC_ERR_ARG;
-    if (!inst_res && h->ric_S + h->ric_F == 0 && inst[0].S + inst[0].F_ds > 0 && inst[0].S >= 0 && inst[0].F_ds >= 0) {
-        int prc = ismpc_formc_prepare_gait(h, inst[0].S, inst[0].F_ds);
-        if (prc != ISMPC_OK) return prc;
-        formc_fill_args(h, a, n);
-    }
-    const size_t mb = (size_t)h->max_batch;
-    if (h->s_state.ensure(mb * sizeof(ismpc_state_t)) || h->s_walk.ensure(mb * sizeof(ismpc_walk_t)) ||
-        h->s_cinst.ensure(mb * sizeof(ismpc_formc_inst_t)) ||
-        (!plan_res && h->s_plan.ensure((size_t)plan_rows * 4 * sizeof(double))))
-        return ISMPC_ERR_ALLOC;
-    if (push && h->s_push.ensure(mb * sizeof(ismpc_push_t))) return ISMPC_ERR_ALLOC;
-    if (traj_opt && h->s_traj.ensure((size_t)n * n_ticks * 6 * sizeof(double))) return ISMPC_ERR_ALLOC;
-    if (status_opt && h->s_status.ensure(mb * sizeof(int32_t))) return ISMPC_ERR_ALLOC;
-    if (status_trace_opt && h->s_trace.ensure((size_t)n * n_ticks * sizeof(int32_t))) return ISMPC_ERR_ALLOC;
-    CK(cudaMemcpyAsync(h->s_state.p, state, n * sizeof(ismpc_state_t), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->s_walk.p, walk, n * sizeof(ismpc_walk_t), cudaMemcpyHostToDevice, st));
-    if (!inst_res) CK(cudaMemcpyAsync(h->s_cinst.p, inst, n * sizeof(ismpc_formc_inst_t), cudaMemcpyHostToDevice, st));
-    if (!plan_res) CK(cudaMemcpyAsync(h->s_plan.p, plan_xyzt, (size_t)plan_rows * 4 * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (push) CK(cudaMemcpyAsync(h->s_push.p, push, n * sizeof(ismpc_push_t), cudaMemcpyHostToDevice, st));
-    a.state = (const ismpc_state_t*)h->s_state.p; a.walk = (const ismpc_walk_t*)h->s_walk.p;
-    a.inst = inst_res ? (const ismpc_formc_inst_t*)h->c_inst.p : (const ismpc_formc_inst_t*)h->s_cinst.p; a.plan = plan_res ? (const double*)h->c_plan.p : (const double*)h->s_plan.p;
-    int rc = formc_launch_rollout(h, a, n, (ismpc_state_t*)h->s_state.p, (ismpc_walk_t*)h->s_walk.p,
-                                  push ? (const ismpc_push_t*)h->s_push.p : nullptr, n_ticks,
-                                  traj_opt ? (double*)h->s_traj.p : nullptr,
-                                  status_opt ? (int32_t*)h->s_status.p : nullptr,
-                                  status_trace_opt ? (int32_t*)h->s_trace.p : nullptr, st);
-    h->launches += 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "formc_rollout_launch");
-    if (status_trace_opt) CK(cudaMemcpyAsync(status_trace_opt, h->s_trace.p, (size_t)n * n_ticks * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(state, h->s_state.p, n * sizeof(ismpc_state_t), cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(walk, h->s_walk.p, n * sizeof(ismpc_walk_t), cudaMemcpyDeviceToHost, st));
-    if (traj_opt) CK(cudaMemcpyAsync(traj_opt, h->s_traj.p, (size_t)n * n_ticks * 6 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (status_opt) CK(cudaMemcpyAsync(status_opt, h->s_status.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    formc_fill_args(h, a, n, plan_rows);
+    ismpc_state_t* state_io = s.inout(state, n, mb);
+    ismpc_walk_t* walk_io = s.inout(walk, n, mb);
+    a.state = state_io; a.walk = walk_io;
+    if (const ismpc_formc_inst_t* p = s.in(inst, n, mb)) a.inst = p;
+    if (const double* p = s.in(plan_xyzt, (size_t)plan_rows * 4)) a.plan = p;
+    const ismpc_push_t* push_d = s.in(push, n, mb);
+    double* traj = s.out(traj_opt, nt * 6);
+    int32_t* status = s.out(status_opt, n, mb);
+    int32_t* trace = s.out(status_trace_opt, nt);
+    if (s.err) return s.err;
+    return s.finish(formc_launch_rollout(h, a, n, state_io, walk_io, push_d, n_ticks, traj, status, trace, s.st),
+                    "formc_rollout_launch");
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -652,7 +629,6 @@ static int forma_common(ismpc_handle* h, int n, int n_ticks, bool rollout, ismpc
     if (!rollout && !out) return ISMPC_ERR_ARG;
     if (n == 0 || (rollout && n_ticks <= 0)) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
     const int nV = 2 * (h->am.C + h->am.F);
     FormAArgs a;
     a.n = n; a.model = h->am; a.timing_len = timing_len; a.plan_rows = plan_rows; a.sm_count = h->sm_count;
@@ -667,62 +643,26 @@ static int forma_common(ismpc_handle* h, int n, int n_ticks, bool rollout, ismpc
     a.Jspill = lp.spill_doubles ? (double*)h->a_Lwork.p : nullptr;
     a.queue = (int*)h->a_queue.p;
     a.R = lp.R; a.warps_per_cta = lp.warps_per_cta;
-    if (mem == ISMPC_MEM_DEVICE) {
-        a.inst = inst; a.fs_timing = fs_timing; a.fs_plan = fs_plan; a.out = out; a.primal = primal_opt;
-        a.active = (signed char*)active_opt;
-        int rc = rollout ? forma_rollout_launch(a, lp, inst, fs_plan, push, n_ticks, traj_opt, pred_opt, status_opt, trace_opt, st)
-                         : forma_tick_launch(a, lp, (const signed char*)ws_guess, ws_shift, st);
-        h->launches += rollout ? 2 : 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "forma launch");
-        return ISMPC_OK;
-    }
-    if (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_HOST_ASYNC) return ISMPC_ERR_ARG;
-    const size_t mb = (size_t)h->max_batch;
-    if (h->s_ainst.ensure(mb * sizeof(ismpc_forma_inst_t)) || h->s_aout.ensure(mb * sizeof(ismpc_forma_out_t)) ||
-        h->s_timing.ensure((size_t)timing_len * sizeof(int32_t)) || h->s_plan.ensure((size_t)plan_rows * 2 * sizeof(double)))
-        return ISMPC_ERR_ALLOC;
-    if (primal_opt && h->s_primal.ensure(mb * nV * sizeof(double))) return ISMPC_ERR_ALLOC;
-    if (active_opt && h->s_active.ensure(mb * nV)) return ISMPC_ERR_ALLOC;
-    if (ws_guess && h->s_aguess.ensure(mb * nV)) return ISMPC_ERR_ALLOC;
-    if (push && h->s_push.ensure(mb * sizeof(ismpc_push_t))) return ISMPC_ERR_ALLOC;
-    if (traj_opt && h->s_traj.ensure((size_t)n * n_ticks * 6 * sizeof(double))) return ISMPC_ERR_ALLOC;
-    if (pred_opt && h->s_pred.ensure((size_t)n * n_ticks * 2 * sizeof(double))) return ISMPC_ERR_ALLOC;
-    if (status_opt && h->s_status.ensure(mb * sizeof(int32_t))) return ISMPC_ERR_ALLOC;
-    if (trace_opt && h->s_trace.ensure((size_t)n * n_ticks * 2 * sizeof(int32_t))) return ISMPC_ERR_ALLOC;
-    CK(cudaMemcpyAsync(h->s_ainst.p, inst, n * sizeof(ismpc_forma_inst_t), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->s_timing.p, fs_timing, (size_t)timing_len * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->s_plan.p, fs_plan, (size_t)plan_rows * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (push) CK(cudaMemcpyAsync(h->s_push.p, push, n * sizeof(ismpc_push_t), cudaMemcpyHostToDevice, st));
-    if (ws_guess) CK(cudaMemcpyAsync(h->s_aguess.p, ws_guess, (size_t)n * nV, cudaMemcpyHostToDevice, st));
-    a.inst = (const ismpc_forma_inst_t*)h->s_ainst.p; a.fs_timing = (const int32_t*)h->s_timing.p;
-    a.fs_plan = (const double*)h->s_plan.p; a.out = (ismpc_forma_out_t*)h->s_aout.p;
-    a.primal = primal_opt ? (double*)h->s_primal.p : nullptr;
-    a.active = active_opt ? (signed char*)h->s_active.p : nullptr;
-    int rc;
-    if (rollout)
-        rc = forma_rollout_launch(a, lp, (ismpc_forma_inst_t*)h->s_ainst.p, (double*)h->s_plan.p,
-                                  push ? (const ismpc_push_t*)h->s_push.p : nullptr, n_ticks,
-                                  traj_opt ? (double*)h->s_traj.p : nullptr, pred_opt ? (double*)h->s_pred.p : nullptr,
-                                  status_opt ? (int32_t*)h->s_status.p : nullptr,
-                                  trace_opt ? (int32_t*)h->s_trace.p : nullptr, st);
-    else
-        rc = forma_tick_launch(a, lp, ws_guess ? (const signed char*)h->s_aguess.p : nullptr, ws_shift, st);
-    h->launches += rollout ? 2 : 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "forma launch");
-    if (rollout) {
-        CK(cudaMemcpyAsync(inst, h->s_ainst.p, n * sizeof(ismpc_forma_inst_t), cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(fs_plan, h->s_plan.p, (size_t)plan_rows * 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-        if (traj_opt) CK(cudaMemcpyAsync(traj_opt, h->s_traj.p, (size_t)n * n_ticks * 6 * sizeof(double), cudaMemcpyDeviceToHost, st));
-        if (pred_opt) CK(cudaMemcpyAsync(pred_opt, h->s_pred.p, (size_t)n * n_ticks * 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-        if (status_opt) CK(cudaMemcpyAsync(status_opt, h->s_status.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        if (trace_opt) CK(cudaMemcpyAsync(trace_opt, h->s_trace.p, (size_t)n * n_ticks * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    } else {
-        CK(cudaMemcpyAsync(out, h->s_aout.p, n * sizeof(ismpc_forma_out_t), cudaMemcpyDeviceToHost, st));
-        if (primal_opt) CK(cudaMemcpyAsync(primal_opt, h->s_primal.p, (size_t)n * nV * sizeof(double), cudaMemcpyDeviceToHost, st));
-        if (active_opt) CK(cudaMemcpyAsync(active_opt, h->s_active.p, (size_t)n * nV, cudaMemcpyDeviceToHost, st));
-    }
-    if (mem == ISMPC_MEM_HOST) CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    Staged s(h, mem, stream, true);
+    const size_t mb = (size_t)h->max_batch, nt = (size_t)n * n_ticks;
+    // a rollout advances the instances and the plan in place
+    ismpc_forma_inst_t* inst_io = rollout ? s.inout(inst, n, mb) : s.in(inst, n, mb);
+    double* plan_io = rollout ? s.inout(fs_plan, (size_t)plan_rows * 2) : s.in(fs_plan, (size_t)plan_rows * 2);
+    a.inst = inst_io; a.fs_plan = plan_io;
+    a.fs_timing = s.in(fs_timing, timing_len);
+    const int8_t* guess = s.in(ws_guess, (size_t)n * nV, mb * nV);    // a buffer of its own: the guess may alias active_opt
+    a.out = s.out(out, n, mb);
+    a.primal = s.out(primal_opt, (size_t)n * nV, mb * nV);
+    a.active = (signed char*)s.out(active_opt, (size_t)n * nV, mb * nV);
+    const ismpc_push_t* push_d = s.in(push, n, mb);
+    double* traj = s.out(traj_opt, nt * 6);
+    double* pred = s.out(pred_opt, nt * 2);
+    int32_t* status = s.out(status_opt, n, mb);
+    int32_t* trace = s.out(trace_opt, nt * 2);
+    if (s.err) return s.err;
+    const int rc = rollout ? forma_rollout_launch(a, lp, inst_io, plan_io, push_d, n_ticks, traj, pred, status, trace, s.st)
+                           : forma_tick_launch(a, lp, (const signed char*)guess, ws_shift, s.st);
+    return s.finish(rc, "forma launch", rollout ? 2 : 1);
 }
 
 extern "C" int ismpc_forma_solve_batch_ws(ismpc_handle* h, int n, const ismpc_forma_inst_t* inst,
@@ -791,28 +731,14 @@ extern "C" int ismpc_feet_place_rollout(ismpc_handle* h, int n, int n_ticks, con
         return ISMPC_ERR_ARG;
     if (n == 0 || n_ticks == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    if (mem == ISMPC_MEM_DEVICE) {
-        int rc = feet_place_launch(n, n_ticks, *model, inst, fs_timing, timing_len, pred_traj, foot_plan, foot_plan_rows, st);
-        h->launches += 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "feet_place_launch");
-        return ISMPC_OK;
-    }
-    if (mem != ISMPC_MEM_HOST) return ISMPC_ERR_ARG;
-    const size_t bi = (size_t)n * sizeof(ismpc_feet_inst_t), bt = (size_t)timing_len * sizeof(int32_t);
-    const size_t bp = (size_t)n * n_ticks * 2 * sizeof(double), bf = (size_t)foot_plan_rows * 8 * sizeof(double);
-    if (h->f_inst.ensure(bi) || h->s_timing.ensure(bt) || h->s_pred.ensure(bp) || h->f_plan.ensure(bf)) return ISMPC_ERR_ALLOC;
-    CK(cudaMemcpyAsync(h->f_inst.p, inst, bi, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->s_timing.p, fs_timing, bt, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->s_pred.p, pred_traj, bp, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->f_plan.p, foot_plan, bf, cudaMemcpyHostToDevice, st));
-    int rc = feet_place_launch(n, n_ticks, *model, (const ismpc_feet_inst_t*)h->f_inst.p, (const int32_t*)h->s_timing.p,
-                               timing_len, (const double*)h->s_pred.p, (double*)h->f_plan.p, foot_plan_rows, st);
-    h->launches += 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "feet_place_launch");
-    CK(cudaMemcpyAsync(foot_plan, h->f_plan.p, bf, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    Staged s(h, mem, stream, false);
+    const ismpc_feet_inst_t* inst_d = s.in(inst, n);
+    const int32_t* timing_d = s.in(fs_timing, timing_len);
+    const double* pred_d = s.in(pred_traj, (size_t)n * n_ticks * 2);
+    double* plan_io = s.inout(foot_plan, (size_t)foot_plan_rows * 8);
+    if (s.err) return s.err;
+    return s.finish(feet_place_launch(n, n_ticks, *model, inst_d, timing_d, timing_len, pred_d, plan_io, foot_plan_rows, s.st),
+                    "feet_place_launch");
 }
 
 extern "C" int ismpc_feet_export(ismpc_handle* h, int n, const ismpc_feet_model_t* model, const ismpc_feet_inst_t* inst,
@@ -826,31 +752,14 @@ extern "C" int ismpc_feet_export(ismpc_handle* h, int n, const ismpc_feet_model_
         return ISMPC_ERR_ARG;
     if (n == 0 || n_steps == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    if (mem == ISMPC_MEM_DEVICE) {
-        int rc = feet_export_launch(n, *model, inst, foot_plan, foot_plan_rows, n_steps, fixed, swing, fl, fr, rl, rr, st);
-        h->launches += 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "feet_export_launch");
-        return ISMPC_OK;
-    }
-    if (mem != ISMPC_MEM_HOST) return ISMPC_ERR_ARG;
-    const size_t bi = (size_t)n * sizeof(ismpc_feet_inst_t), bf = (size_t)foot_plan_rows * 8 * sizeof(double);
-    const size_t bo = (size_t)n * n_steps * (fixed + swing) * 3 * sizeof(double);
-    if (h->f_inst.ensure(bi) || h->f_plan.ensure(bf) || h->f_out.ensure(4 * bo)) return ISMPC_ERR_ALLOC;
-    CK(cudaMemcpyAsync(h->f_inst.p, inst, bi, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->f_plan.p, foot_plan, bf, cudaMemcpyHostToDevice, st));
-    double* o = (double*)h->f_out.p;
-    const size_t od = bo / sizeof(double);
-    int rc = feet_export_launch(n, *model, (const ismpc_feet_inst_t*)h->f_inst.p, (const double*)h->f_plan.p,
-                                foot_plan_rows, n_steps, fixed, swing, o, o + od, o + 2 * od, o + 3 * od, st);
-    h->launches += 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "feet_export_launch");
-    CK(cudaMemcpyAsync(fl, o, bo, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(fr, o + od, bo, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(rl, o + 2 * od, bo, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(rr, o + 3 * od, bo, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    Staged s(h, mem, stream, false);
+    const size_t od = (size_t)n * n_steps * (fixed + swing) * 3;
+    const ismpc_feet_inst_t* inst_d = s.in(inst, n);
+    const double* plan_d = s.in(foot_plan, (size_t)foot_plan_rows * 8);
+    double* fl_d = s.out(fl, od); double* fr_d = s.out(fr, od); double* rl_d = s.out(rl, od); double* rr_d = s.out(rr, od);
+    if (s.err) return s.err;
+    return s.finish(feet_export_launch(n, *model, inst_d, plan_d, foot_plan_rows, n_steps, fixed, swing, fl_d, fr_d, rl_d, rr_d, s.st),
+                    "feet_export_launch");
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -884,25 +793,13 @@ extern "C" int ismpc_plan_generate(ismpc_handle* h, int n, const ismpc_plan_mode
     if (n < 0 || n > h->max_batch || !req || !foot_plan || !center) return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
+    Staged s(h, mem, stream, false);
     const int rows = ismpc_plan_rows(model);
-    if (mem == ISMPC_MEM_DEVICE) {
-        int rc = plan_generate_launch(n, *model, req, foot_plan, center, rows, st);
-        h->launches += 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "plan_generate_launch");
-        return ISMPC_OK;
-    }
-    if (mem != ISMPC_MEM_HOST) return ISMPC_ERR_ARG;
-    const size_t br = (size_t)n * sizeof(ismpc_plan_req_t), bf = (size_t)n * rows * 8 * sizeof(double), bc = bf / 4;
-    if (h->f_inst.ensure(br) || h->f_plan.ensure(bf) || h->f_out.ensure(bc)) return ISMPC_ERR_ALLOC;
-    CK(cudaMemcpyAsync(h->f_inst.p, req, br, cudaMemcpyHostToDevice, st));
-    int rc = plan_generate_launch(n, *model, (const ismpc_plan_req_t*)h->f_inst.p, (double*)h->f_plan.p, (double*)h->f_out.p, rows, st);
-    h->launches += 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "plan_generate_launch");
-    CK(cudaMemcpyAsync(foot_plan, h->f_plan.p, bf, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(center, h->f_out.p, bc, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    const ismpc_plan_req_t* req_d = s.in(req, n);
+    double* plan_d = s.out(foot_plan, (size_t)n * rows * 8);
+    double* center_d = s.out(center, (size_t)n * rows * 2);
+    if (s.err) return s.err;
+    return s.finish(plan_generate_launch(n, *model, req_d, plan_d, center_d, rows, s.st), "plan_generate_launch");
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -930,27 +827,12 @@ extern "C" int ismpc_kf_filter_batch(ismpc_handle* h, int n, int n_steps, const 
     if (!(model->sampling_time > 0.0f) || !(model->mass > 0.0f)) return ISMPC_ERR_MODEL;
     if (n == 0 || n_steps == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    if (mem == ISMPC_MEM_DEVICE) {
-        int rc = kf_filter_launch(n, n_steps, *model, state, samples, zmp_opt, st);
-        h->launches += 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "kf_filter_launch");
-        return ISMPC_OK;
-    }
-    if (mem != ISMPC_MEM_HOST) return ISMPC_ERR_ARG;
-    const size_t bs = (size_t)n * sizeof(ismpc_kf_state_t), bu = (size_t)n * n_steps * sizeof(ismpc_kf_sample_t);
-    const size_t bz = (size_t)n * n_steps * 2 * sizeof(float);
-    if (h->f_inst.ensure(bs) || h->f_plan.ensure(bu) || (zmp_opt && h->f_out.ensure(bz))) return ISMPC_ERR_ALLOC;
-    CK(cudaMemcpyAsync(h->f_inst.p, state, bs, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->f_plan.p, samples, bu, cudaMemcpyHostToDevice, st));
-    int rc = kf_filter_launch(n, n_steps, *model, (ismpc_kf_state_t*)h->f_inst.p, (const ismpc_kf_sample_t*)h->f_plan.p,
-                              zmp_opt ? (float*)h->f_out.p : nullptr, st);
-    h->launches += 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "kf_filter_launch");
-    CK(cudaMemcpyAsync(state, h->f_inst.p, bs, cudaMemcpyDeviceToHost, st));
-    if (zmp_opt) CK(cudaMemcpyAsync(zmp_opt, h->f_out.p, bz, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    Staged s(h, mem, stream, false);
+    ismpc_kf_state_t* state_io = s.inout(state, n);
+    const ismpc_kf_sample_t* samples_d = s.in(samples, (size_t)n * n_steps);
+    float* zmp = s.out(zmp_opt, (size_t)n * n_steps * 2);
+    if (s.err) return s.err;
+    return s.finish(kf_filter_launch(n, n_steps, *model, state_io, samples_d, zmp, s.st), "kf_filter_launch");
 }
 
 extern "C" int ismpc_kf_filter_batch_f64(ismpc_handle* h, int n, int n_steps, const ismpc_kf_model_t* model,
@@ -962,27 +844,12 @@ extern "C" int ismpc_kf_filter_batch_f64(ismpc_handle* h, int n, int n_steps, co
     if (!(model->sampling_time > 0.0f) || !(model->mass > 0.0f)) return ISMPC_ERR_MODEL;
     if (n == 0 || n_steps == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    if (mem == ISMPC_MEM_DEVICE) {
-        int rc = kf_filter64_launch(n, n_steps, *model, state, samples, zmp_opt, joseph != 0, st);
-        h->launches += 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "kf_filter64_launch");
-        return ISMPC_OK;
-    }
-    if (mem != ISMPC_MEM_HOST) return ISMPC_ERR_ARG;
-    const size_t bs = (size_t)n * sizeof(ismpc_kf_state64_t), bu = (size_t)n * n_steps * sizeof(ismpc_kf_sample_t);
-    const size_t bz = (size_t)n * n_steps * 2 * sizeof(double);
-    if (h->f_inst.ensure(bs) || h->f_plan.ensure(bu) || (zmp_opt && h->f_out.ensure(bz))) return ISMPC_ERR_ALLOC;
-    CK(cudaMemcpyAsync(h->f_inst.p, state, bs, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->f_plan.p, samples, bu, cudaMemcpyHostToDevice, st));
-    int rc = kf_filter64_launch(n, n_steps, *model, (ismpc_kf_state64_t*)h->f_inst.p, (const ismpc_kf_sample_t*)h->f_plan.p,
-                                zmp_opt ? (double*)h->f_out.p : nullptr, joseph != 0, st);
-    h->launches += 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "kf_filter64_launch");
-    CK(cudaMemcpyAsync(state, h->f_inst.p, bs, cudaMemcpyDeviceToHost, st));
-    if (zmp_opt) CK(cudaMemcpyAsync(zmp_opt, h->f_out.p, bz, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    Staged s(h, mem, stream, false);
+    ismpc_kf_state64_t* state_io = s.inout(state, n);
+    const ismpc_kf_sample_t* samples_d = s.in(samples, (size_t)n * n_steps);
+    double* zmp = s.out(zmp_opt, (size_t)n * n_steps * 2);
+    if (s.err) return s.err;
+    return s.finish(kf_filter64_launch(n, n_steps, *model, state_io, samples_d, zmp, joseph != 0, s.st), "kf_filter64_launch");
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1000,44 +867,26 @@ extern "C" int ismpc_qp_solve_batch_ws(ismpc_handle* h, int n, int nV, int nC, c
     if (n == 0) return ISMPC_OK;
     if (nC == 0) ws_guess = nullptr;           // nothing to guess
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
     if (h->q_work.ensure(qp_dense_work_doubles(n, nV, nC) * sizeof(double))) return ISMPC_ERR_ALLOC;
-    if (mem == ISMPC_MEM_DEVICE) {
-        int rc = qp_dense_launch(n, nV, nC, H, g, A, lbA, ubA, (const signed char*)ws_guess, x, y_opt, (signed char*)ws_opt,
-                                 status, iters_opt, (double*)h->q_work.p, h->opt_dense_dmma, st);
-        h->launches += 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "qp_dense_launch");
-        return ISMPC_OK;
-    }
-    if (mem != ISMPC_MEM_HOST) return ISMPC_ERR_ARG;
-    const size_t szH = (size_t)n * nV * nV, szg = (size_t)n * nV, szA = (size_t)n * nC * nV, szb = (size_t)n * nC;
-    const size_t in_d = szH + szg + szA + 2 * szb;
-    const size_t out_b = (szg + szb) * sizeof(double) + szb + 2 * (size_t)n * sizeof(int32_t) + 64;
-    if (h->q_in.ensure(in_d * sizeof(double)) || h->q_out.ensure(out_b)) return ISMPC_ERR_ALLOC;
-    double* dH = (double*)h->q_in.p; double* dg = dH + szH; double* dA = dg + szg; double* dlb = dA + szA; double* dub = dlb + szb;
-    double* dx = (double*)h->q_out.p; double* dy = dx + szg;
-    int32_t* dst = (int32_t*)(dy + szb); int32_t* dit = dst + n;
-    signed char* dws = (signed char*)(dit + n);
-    CK(cudaMemcpyAsync(dH, H, szH * sizeof(double), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(dg, g, szg * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (nC > 0) {
-        CK(cudaMemcpyAsync(dA, A, szA * sizeof(double), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(dlb, lbA, szb * sizeof(double), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(dub, ubA, szb * sizeof(double), cudaMemcpyHostToDevice, st));
-    }
-    // the guess is staged where the working set comes out: each problem's warp reads its row before it writes it
-    if (ws_guess) CK(cudaMemcpyAsync(dws, ws_guess, szb, cudaMemcpyHostToDevice, st));
-    int rc = qp_dense_launch(n, nV, nC, dH, dg, dA, dlb, dub, ws_guess ? dws : nullptr, dx, dy, dws, dst, dit,
-                             (double*)h->q_work.p, h->opt_dense_dmma, st);
-    h->launches += 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "qp_dense_launch");
-    CK(cudaMemcpyAsync(x, dx, szg * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (y_opt && nC > 0) CK(cudaMemcpyAsync(y_opt, dy, szb * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (ws_opt && nC > 0) CK(cudaMemcpyAsync(ws_opt, dws, szb, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(status, dst, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    if (iters_opt) CK(cudaMemcpyAsync(iters_opt, dit, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    Staged s(h, mem, stream, false);
+    const size_t szg = (size_t)n * nV, szb = (size_t)n * nC;
+    // both dense-seam calls stage their outputs first and in one order, so that they share the output staging: the
+    // rows a failed problem leaves unwritten come back as the previous dense-seam call left them
+    double* dx = s.out(x, szg);
+    double* dy = s.out(y_opt, szb);
+    int8_t* dws = s.out(ws_opt, szb);
+    int32_t* dst = s.out(status, n);
+    int32_t* dit = s.out(iters_opt, n);
+    const double* dH = s.in(H, szg * nV);
+    const double* dg = s.in(g, szg);
+    const double* dA = s.in(A, szb * nV);
+    const double* dlb = s.in(lbA, szb);
+    const double* dub = s.in(ubA, szb);
+    const int8_t* dgs = s.in(ws_guess, szb);       // a buffer of its own: the guess may alias ws_opt
+    if (s.err) return s.err;
+    return s.finish(qp_dense_launch(n, nV, nC, dH, dg, dA, dlb, dub, (const signed char*)dgs, dx, dy, (signed char*)dws, dst,
+                                    dit, (double*)h->q_work.p, h->opt_dense_dmma, s.st),
+                    "qp_dense_launch");
 }
 
 extern "C" int ismpc_qp_solve_batch(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* g,
@@ -1093,53 +942,26 @@ extern "C" int ismpc_qp_hotstart_batch(ismpc_handle* h, int n, const int32_t* ma
     if (n == 0) return ISMPC_OK;
     if (nC == 0) ws_guess = nullptr;
     CK(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
     if (h->r_work.ensure(qp_sets_work_doubles(n, n_mat, nV, nC) * sizeof(double))) return ISMPC_ERR_ALLOC;
-    const double* tab = (const double*)h->r_tab.p;
-    const int32_t* fstat = (const int32_t*)h->r_stat.p;
-    double* work = (double*)h->r_work.p;
-    if (mem == ISMPC_MEM_DEVICE) {
-        int rc = qp_sets_launch(n, nV, nC, n_mat, tab, fstat, mat_index_opt, g, lbA, ubA, (const signed char*)ws_guess, x,
-                                y_opt, (signed char*)ws_opt, status, iters_opt, work, h->opt_dense_resident_gemm,
-                                h->opt_dense_dmma, st);
-        h->launches += 1;
-        if (rc) return fail_cuda(h, (cudaError_t)rc, "qp_sets_launch");
-        return ISMPC_OK;
-    }
+    Staged s(h, mem, stream, false);
     const size_t szg = (size_t)n * nV, szb = (size_t)n * nC;
-    const size_t in_b = (szg + 2 * szb) * sizeof(double) + (size_t)n * sizeof(int32_t) + szb;
-    const size_t out_b = (szg + szb) * sizeof(double) + szb + 2 * (size_t)n * sizeof(int32_t) + 64;
-    if (h->q_in.ensure(in_b) || h->q_out.ensure(out_b)) return ISMPC_ERR_ALLOC;
-    double* dg = (double*)h->q_in.p; double* dlb = dg + szg; double* dub = dlb + szb;
-    int32_t* didx = (int32_t*)(dub + szb);
-    signed char* dgs = (signed char*)(didx + n);
-    double* dx = (double*)h->q_out.p; double* dy = dx + szg;
-    int32_t* dst = (int32_t*)(dy + szb); int32_t* dit = dst + n;
-    signed char* dws = (signed char*)(dit + n);
-    CK(cudaMemcpyAsync(dg, g, szg * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (nC > 0) {
-        CK(cudaMemcpyAsync(dlb, lbA, szb * sizeof(double), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(dub, ubA, szb * sizeof(double), cudaMemcpyHostToDevice, st));
-    }
-    if (mat_index_opt) CK(cudaMemcpyAsync(didx, mat_index_opt, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    // the outputs are staged with the caller's bytes, so that a problem the call does not touch (set index out of range)
-    // keeps them, as with device buffers
-    if (ws_guess) CK(cudaMemcpyAsync(dgs, ws_guess, szb, cudaMemcpyHostToDevice, st));
-    if (ws_opt && nC > 0) CK(cudaMemcpyAsync(dws, ws_opt, szb, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(dx, x, szg * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (y_opt && nC > 0) CK(cudaMemcpyAsync(dy, y_opt, szb * sizeof(double), cudaMemcpyHostToDevice, st));
-    int rc = qp_sets_launch(n, nV, nC, n_mat, tab, fstat, mat_index_opt ? didx : nullptr, dg, dlb, dub,
-                            ws_guess ? dgs : nullptr, dx, dy, dws, dst, dit, work, h->opt_dense_resident_gemm,
-                            h->opt_dense_dmma, st);
-    h->launches += 1;
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "qp_sets_launch");
-    CK(cudaMemcpyAsync(x, dx, szg * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (y_opt && nC > 0) CK(cudaMemcpyAsync(y_opt, dy, szb * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (ws_opt && nC > 0) CK(cudaMemcpyAsync(ws_opt, dws, szb, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(status, dst, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    if (iters_opt) CK(cudaMemcpyAsync(iters_opt, dit, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return ISMPC_OK;
+    // outputs first, as in ismpc_qp_solve_batch_ws; x, y and ws are staged with the caller's bytes, so that a problem
+    // the call does not touch (set index out of range) keeps them, as with device buffers
+    double* dx = s.inout(x, szg);
+    double* dy = s.inout(y_opt, szb);
+    int8_t* dws = s.inout(ws_opt, szb);
+    int32_t* dst = s.out(status, n);
+    int32_t* dit = s.out(iters_opt, n);
+    const double* dg = s.in(g, szg);
+    const double* dlb = s.in(lbA, szb);
+    const double* dub = s.in(ubA, szb);
+    const int32_t* didx = s.in(mat_index_opt, n);
+    const int8_t* dgs = s.in(ws_guess, szb);
+    if (s.err) return s.err;
+    return s.finish(qp_sets_launch(n, nV, nC, n_mat, (const double*)h->r_tab.p, (const int32_t*)h->r_stat.p, didx, dg, dlb,
+                                   dub, (const signed char*)dgs, dx, dy, (signed char*)dws, dst, dit,
+                                   (double*)h->r_work.p, h->opt_dense_resident_gemm, h->opt_dense_dmma, s.st),
+                    "qp_sets_launch");
 }
 
 // ---------------------------------------------------------------------------------------------------

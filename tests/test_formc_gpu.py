@@ -2,7 +2,7 @@
 import numpy as np
 import pytest
 
-from quadruped_gait_generation_ismpc_b200 import abi, synth
+from quadruped_gait_generation_ismpc_b200 import abi, binding, synth
 from oracle import oracle as O
 from parity import PRIMAL_TOL, primal_rel_err, active_set_mismatch
 
@@ -359,6 +359,31 @@ def test_packed_tick_records_and_resident_instances(handle, variant):
         handle.formc_solve_batch_packed_raw(n, t_dev.data_ptr(), None, None, 0, o_dev.data_ptr(), mem=abi.MEM_DEVICE)
         torch.cuda.synchronize()
         assert o_dev.cpu().numpy().tobytes() == a["out"].tobytes()
+        # ISMPC_MEM_HOST_ASYNC on ismpc_host_alloc buffers (records in place, or staged with zero copy off; primal and
+        # active staged), finished by ismpc_wait
+        N3 = a["primal"].shape[1]
+        pins = [binding.PinnedBuffer(n * 128, fill=tick), binding.PinnedBuffer(n * abi.FORMC_OUT.itemsize),
+                binding.PinnedBuffer(n * N3 * 8), binding.PinnedBuffer(n * N3)]
+        st = handle.stream()
+        try:
+            for zc in (1, 0):
+                handle.set_option("host_zero_copy", zc)
+                for b in pins[1:]:
+                    b.array[:] = 0
+                l0 = handle.kernel_launches
+                handle.formc_solve_batch_packed_raw(n, pins[0].ptr, None, None, 0, pins[1].ptr, pins[2].ptr, pins[3].ptr,
+                                                    mem=abi.MEM_HOST_ASYNC, stream=st)
+                handle.wait(st)
+                assert handle.kernel_launches == l0 + 1
+                assert pins[1].array.tobytes() == a["out"].tobytes(), "host async, host_zero_copy = %d" % zc
+                assert pins[2].array.tobytes() == a["primal"].tobytes() and pins[3].array.tobytes() == a["active"].tobytes()
+        finally:
+            handle.set_option("host_zero_copy", 1)
+            for b in pins:
+                b.close()
+        # an unknown memory mode is refused
+        assert handle._L.ismpc_formc_solve_batch_packed(handle._h, n, tick.ctypes.data, None, None, 0, o_pin.data_ptr(),
+                                                        None, None, 7, None) == -1
         # more instances than the resident constants cover, or constants forgotten: refused
         handle.formc_set_instances(inst[:50])
         with pytest.raises(Exception):

@@ -69,6 +69,14 @@ def test_indexed_sets(handle):
     assert (rb["x"][~keep] == 0).all() and (rb["ws"][~keep] == 0).all() and (rb["iters"][~keep] == 0).all()
     for k in KEYS:
         assert rb[k][keep].tobytes() == c[k][keep].tobytes(), k
+    # host memory: the problems the call does not touch keep the caller's x, y and ws rows
+    x = np.full_like(c["x"], 7.5); y = np.full_like(c["y"], -2.5); ws = np.full_like(c["ws"], 3)
+    st, it = np.zeros(48, np.int32), np.zeros(48, np.int32)
+    handle.qp_hotstart_batch_raw(48, g, lb, ub, x, y, ws, st, it, mat_index=bad, mem=abi.MEM_HOST)
+    assert (x[~keep] == 7.5).all() and (y[~keep] == -2.5).all() and (ws[~keep] == 3).all()
+    assert (st[~keep] == abi.ST_QP_FAIL).all()
+    for k, v in (("x", x), ("y", y), ("ws", ws), ("status", st), ("iters", it)):
+        assert v[keep].tobytes() == c[k][keep].tobytes(), k
 
 
 def _vertical_family(n, mpc_iter=7, seed=6):

@@ -247,6 +247,20 @@ def test_plumbing(handle):
         wd = device_call(alias)
         for k in wd:
             assert wd[k].tobytes() == wh[k].tobytes(), (alias, k)
+    # host memory: the guess in the working-set output itself; each optional output NULL
+    ho = {k: np.zeros_like(v) for k, v in wh.items()}
+    ho["ws"][:] = guess
+    handle.qp_solve_batch_raw(n, nV, nC, *arrs, ho["x"], ho["y"], ho["ws"], ho["status"], ho["iters"], mem=abi.MEM_HOST,
+                              ws_guess=ho["ws"])
+    for k in ho:
+        assert ho[k].tobytes() == wh[k].tobytes(), ("host alias", k)
+    for drop in ("y", "ws", "iters"):
+        ho = {k: np.zeros_like(v) for k, v in wh.items()}
+        ho[drop] = None
+        handle.qp_solve_batch_raw(n, nV, nC, *arrs, ho["x"], ho["y"], ho["ws"], ho["status"], ho["iters"],
+                                  mem=abi.MEM_HOST, ws_guess=guess)
+        for k in ho:
+            assert ho[k] is None or ho[k].tobytes() == wh[k].tobytes(), ("host, %s NULL" % drop, k)
     assert np.array_equal(dgs.cpu().numpy(), guess)       # a separate guess buffer is only read
     handle.set_option("dense_dmma", 0)
     try:
