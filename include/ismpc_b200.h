@@ -185,11 +185,8 @@ int ismpc_wait(ismpc_handle* h, void* stream);
 void* ismpc_host_alloc(size_t bytes);
 void ismpc_host_free(void* p);
 
-/* Tuning knobs that do not change results beyond rounding (every kernel family is an exact solver of the same
- * strictly convex QPs; tests/test_formc_gpu.py holds them to 1e-9 of each other).
- *   "formc_kernel":       0 = automatic (the warp-per-instance kernels), 1 = CTA / cluster per instance, 2 = warp.
- *   "formc_cluster_size": CTAs per instance of the CTA-per-instance family (1 = CTA-per-QP, 2/4/8 = thread-block-
- *                         cluster-per-QP); setting it selects that family, 0 returns to automatic.
+/* Tuning knobs that do not change results beyond rounding (every build of the warp family is an exact solver of the
+ * same strictly convex QPs; tests/test_formc_gpu.py holds them to 1e-12 of each other).
  *   "formc_variant":      build of the warp family: 0 = by batch size, 2 = two warps per instance (latency build, the
  *                         choice while every instance has a resident CTA), 1 = one warp per instance with unlimited
  *                         registers, 16 = one warp per instance held to 128 registers (16 resident warps per SM).
@@ -228,10 +225,9 @@ int ismpc_formc_set_model(ismpc_handle* h, const ismpc_formc_model_t* model);
 
 /* Optional, after ismpc_formc_set_model: declares the step timing (S single-support, F_ds double-support samples;
  * parameters.cpp:43-44) most instances use, so that the flight-phase equalities of stage 1 (MPCSolver.cpp:223-243)
- * are folded into precomputed tables per mpcIter (Riccati gains and the explicit feedback law for the warp kernels,
- * one projector per mpcIter for the CTA kernels).  Results do not change; instances with another (S, F_ds) take the
- * generic path (the recursion is run in-kernel).  Calls with host buffers do this by themselves from the first
- * instance. */
+ * are folded into precomputed tables per mpcIter (Riccati gains and the explicit feedback law).  Results do not
+ * change; instances with another (S, F_ds) take the generic path (the recursion is run in-kernel).  Calls with host
+ * buffers do this by themselves from the first instance. */
 int ismpc_formc_prepare_gait(ismpc_handle* h, int S, int F_ds);
 
 /* Optional: hands the footstep plans to the handle once, as the reference's constructor receives them
@@ -280,8 +276,7 @@ int ismpc_formc_set_instances(ismpc_handle* h, const ismpc_formc_inst_t* inst, i
 
 /* ismpc_formc_solve_batch with the per-tick arguments packed: tick[i] = {state, walk} of instance i (128-byte records;
  * the array must be 16-byte aligned).  inst / plan_xyzt may be NULL (= the resident ones), results are bit-identical to
- * ismpc_formc_solve_batch on the same values.  Needs the warp-per-instance kernel family (N <= ISMPC_MAX_N and
- * "formc_kernel" != 1; ISMPC_ERR_ARG otherwise).
+ * ismpc_formc_solve_batch on the same values.
  * Host-memory modes, option "host_zero_copy" = 1 (default): when `tick` / `out` are pinned host memory the device can
  * address (ismpc_host_alloc, cudaHostAlloc, cudaHostRegister), 128-byte aligned and at most 8 MB, no copy engine is
  * involved: every instance's CTA reads its record with ONE 128-byte PCIe read and writes its result with one 128-byte

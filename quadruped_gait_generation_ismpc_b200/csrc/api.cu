@@ -41,22 +41,18 @@ struct ismpc_handle {
     int sm_count = 148;
     long long launches = 0;
     char err[256] = {0};
-    int opt_formc_cluster = 0;     // 0 = automatic
     int opt_formc_variant = 0;     // 0 = by batch size, 2 = two warps per instance, 1 / 16 = one warp (register budgets)
     int opt_formc_pdl = 0;         // tick launches as programmatic dependents of the previous kernel on the stream
     int opt_dense_dmma = 1;        // dense seam: condensing GEMMs on the FP64 tensor cores (DMMA); 0 = CUDA cores
-    int opt_formc_kernel = 0;      // 0 = automatic (warp-per-instance where it covers the horizon), 1 = CTA/cluster-per-instance, 2 = warp
-    int c_ctas_per_sm = 1;
     int w_res[5] = {0, 0, 0, 0, 0};   // CTAs the GPU keeps resident: tick kernel (two register budgets), rollout kernel, pair tick / rollout kernels; 0 = not queried
     // form C
     bool formc_ready = false;
     ismpc_formc_model_t cm{};
-    DevBuf c_tables, c_work, c_info, c_ptab;
+    DevBuf c_tables, c_work, c_info;
     DevBuf c_ric_none, c_ric_gait, c_law_none, c_law_gait, c_ws, c_plan, c_inst;
     int inst_res_n = 0;            // instance records resident in c_inst (ismpc_formc_set_instances), 0 = none
     int opt_host_zero_copy = 1;    // packed host-memory ticks: the kernel reads / writes the caller's pinned buffers itself
     int plan_res_rows = 0;         // rows of the resident footstep-plan table (ismpc_formc_set_plan), 0 = none
-    int gait_S = 0, gait_F = 0;            // prepared gait (projector tables in c_ptab), 0 = none
     int ric_S = 0, ric_F = 0;              // prepared gait of the Riccati tables (c_ric_gait), 0 = none
     // form A
     bool forma_ready = false;
@@ -194,11 +190,6 @@ extern "C" void ismpc_host_free(void* p)
 extern "C" int ismpc_set_option(ismpc_handle* h, const char* name, int value)
 {
     if (!h || !name) return ISMPC_ERR_ARG;
-    if (strcmp(name, "formc_cluster_size") == 0) {
-        if (value != 0 && value != 1 && value != 2 && value != 4 && value != 8) return ISMPC_ERR_ARG;
-        h->opt_formc_cluster = value;
-        return ISMPC_OK;
-    }
     if (strcmp(name, "formc_variant") == 0) {      // build of the warp kernel family used by this handle
         if (value != 0 && value != 1 && value != 2 && value != 16) return ISMPC_ERR_ARG;
         h->opt_formc_variant = value;
@@ -213,11 +204,6 @@ extern "C" int ismpc_set_option(ismpc_handle* h, const char* name, int value)
     if (strcmp(name, "host_zero_copy") == 0) { h->opt_host_zero_copy = value != 0; return ISMPC_OK; }
     if (strcmp(name, "dense_dmma") == 0) { h->opt_dense_dmma = value != 0; return ISMPC_OK; }
     if (strcmp(name, "dense_resident_gemm") == 0) { h->opt_dense_resident_gemm = value != 0; return ISMPC_OK; }
-    if (strcmp(name, "formc_kernel") == 0) {
-        if (value < 0 || value > 2) return ISMPC_ERR_ARG;
-        h->opt_formc_kernel = value;
-        return ISMPC_OK;
-    }
     return ISMPC_ERR_ARG;
 }
 
@@ -336,23 +322,9 @@ extern "C" int ismpc_formc_set_model(ismpc_handle* h, const ismpc_formc_model_t*
     if (rc) return fail_cuda(h, (cudaError_t)rc, "formc_law_launch");
     CK(cudaStreamSynchronize(0));
     h->cm = *m;
-    h->gait_S = h->gait_F = 0; h->ric_S = h->ric_F = 0; h->w_res[0] = 0;
-    h->c_ctas_per_sm = formc_cluster_ctas_per_sm(m->N);
+    h->ric_S = h->ric_F = 0; h->w_res[0] = 0;
     h->formc_ready = true;
     return ISMPC_OK;
-}
-
-// Cluster-per-QP is the latency mode (measured, profiles/r1_horizon_sweep.json): splitting the O(N^2) mat-vec
-// over 4 CTAs pays from N = 200 on, as long as all clusters of the batch are resident at once; a batch that
-// fills the GPU anyway is faster with one CTA per QP (the O(N) stages are replicated in every CTA of a cluster).
-static int formc_cluster_size(const ismpc_handle* h, int n)
-{
-    if (h->opt_formc_cluster > 0) return h->opt_formc_cluster;
-    if (h->cm.N < 200) return 1;   // (only reached when the CTA family is selected: formc_kernel = 1)
-    const long long resident = (long long)h->c_ctas_per_sm * h->sm_count;
-    if (4LL * n <= resident) return 4;
-    if (2LL * n <= resident) return 2;
-    return 1;
 }
 
 // A form-C call with inst == NULL / plan_xyzt == NULL reads the instances / plan made resident by
@@ -380,19 +352,10 @@ static void formc_fill_args(ismpc_handle* h, FormCArgs& a, int n, int plan_rows)
     const double* T = (const double*)h->c_tables.p;
     a.n = n; a.model = h->cm;
     a.T.Hinv = T; a.T.G = T + NN; a.T.M = T + 2 * NN;
-    a.T.P = (h->gait_S + h->gait_F > 0) ? (const double*)h->c_ptab.p : nullptr;
-    a.T.gS = h->gait_S; a.T.gF = h->gait_F;
     a.state = nullptr; a.walk = nullptr; a.tick = nullptr;
     a.inst = (const ismpc_formc_inst_t*)h->c_inst.p;
     a.plan = (const double*)h->c_plan.p; a.plan_rows = plan_rows;
     a.out = nullptr; a.primal = nullptr; a.active = nullptr;
-}
-
-// Warp-per-instance kernels cover N <= 512; the CTA/cluster kernels stay for the cluster latency mode and on request.
-static bool formc_use_warp(const ismpc_handle* h)
-{
-    if (h->opt_formc_kernel == 1 || h->opt_formc_cluster > 0) return false;   // an explicit cluster size asks for the CTA/cluster family
-    return formc_warp_supported(h->cm.N) != 0;
 }
 
 // Resident CTAs of the warp kernels are queried once per model (the occupancy query costs microseconds per call).
@@ -416,10 +379,9 @@ static int formc_warp_prepare(ismpc_handle* h, FormCWarpArgs& wa, const FormCArg
     return 0;
 }
 
-// One tick launch (either kernel family) on device-resident arguments.
+// One tick launch on device-resident arguments.
 static int formc_launch_tick(ismpc_handle* h, const FormCArgs& a, int n, cudaStream_t st)
 {
-    if (!formc_use_warp(h)) return formc_tick_launch(a, n, formc_cluster_size(h, n), st);
     FormCWarpArgs wa;
     int rc = formc_warp_prepare(h, wa, a, n);
     if (rc) return rc;
@@ -431,7 +393,6 @@ static int formc_launch_rollout(ismpc_handle* h, const FormCArgs& a, int n, ismp
                                 const ismpc_push_t* push, int n_ticks, double* traj, int32_t* status, int32_t* trace,
                                 cudaStream_t st)
 {
-    if (!formc_use_warp(h)) return formc_rollout_launch(a, state_io, walk_io, push, n_ticks, traj, status, trace, n, st);
     FormCWarpArgs wa;
     int rc = formc_warp_prepare(h, wa, a, n);
     if (rc) return rc;
@@ -443,10 +404,9 @@ extern "C" int ismpc_formc_prepare_gait(ismpc_handle* h, int S, int F_ds)
     if (!h) return ISMPC_ERR_ARG;
     if (!h->formc_ready) return ISMPC_ERR_MODEL;
     if (S < 0 || F_ds < 0 || S + F_ds <= 0 || S + F_ds > 4096) return ISMPC_ERR_ARG;
-    if (h->gait_S == S && h->gait_F == F_ds && h->ric_S == S && h->ric_F == F_ds) return ISMPC_OK;
+    if (h->ric_S == S && h->ric_F == F_ds) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
-    const size_t NN = (size_t)h->cm.N * h->cm.N;
-    h->gait_S = h->gait_F = 0; h->ric_S = h->ric_F = 0;
+    h->ric_S = h->ric_F = 0;
     // Riccati gain tables of the warp kernels: one pattern per mpcIter
     if (h->c_ric_gait.ensure((size_t)(S + F_ds) * h->cm.N * FORMC_RIC_W * sizeof(double))) return ISMPC_ERR_ALLOC;
     int rc = formc_riccati_launch(h->cm, S, F_ds, 0, (double*)h->c_ric_gait.p, 0, &h->launches);
@@ -456,17 +416,6 @@ extern "C" int ismpc_formc_prepare_gait(ismpc_handle* h, int S, int F_ds)
     if (rc) return fail_cuda(h, (cudaError_t)rc, "formc_law_launch");
     CK(cudaStreamSynchronize(0));
     h->ric_S = S; h->ric_F = F_ds;
-    // projector tables of the CTA/cluster kernels
-    if (h->c_ptab.ensure((size_t)(S + F_ds) * NN * sizeof(double))) return ISMPC_ERR_ALLOC;
-    CK(cudaMemset(h->c_info.p, 0, sizeof(int)));
-    rc = formc_prepare_gait_launch(h->cm.N, S, F_ds, (const double*)h->c_tables.p, (double*)h->c_ptab.p,
-                                   (int*)h->c_info.p, 0, &h->launches);
-    if (rc == -1) return ISMPC_OK;             // block too large for shared memory: stay on the generic path
-    if (rc) return fail_cuda(h, (cudaError_t)rc, "formc_prepare_gait_launch");
-    int info = 0;
-    CK(cudaMemcpy(&info, h->c_info.p, sizeof(int), cudaMemcpyDeviceToHost));
-    if (info != 0) return ISMPC_ERR_MODEL;
-    h->gait_S = S; h->gait_F = F_ds;
     return ISMPC_OK;
 }
 
@@ -542,7 +491,7 @@ extern "C" int ismpc_formc_solve_batch_packed(ismpc_handle* h, int n, const ismp
     if (!h) return ISMPC_ERR_ARG;
     if (!h->formc_ready) return ISMPC_ERR_MODEL;
     if (n < 0 || n > h->max_batch || !tick || ((uintptr_t)tick & 15u) != 0 || !out ||
-        !formc_resident_ok(h, n, inst, plan_xyzt, plan_rows) || !formc_use_warp(h))
+        !formc_resident_ok(h, n, inst, plan_xyzt, plan_rows))
         return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));

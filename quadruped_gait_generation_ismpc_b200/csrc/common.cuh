@@ -8,8 +8,8 @@
 namespace ismpc {
 
 // Debug-only cycle counters (make dbg -> lib/libismpc_b200_dbg.so; never in the product library).
-// g_phase[0..31]: form-C tick phase stamps of CTA 0; g_phase[32..63]: accumulated cycles per section of the
-// dual active-set loop over all warps (DasTimer).
+// g_phase[0..31]: accumulated cycles per phase and event counts of the form-C warp tick; g_phase[32..63]: accumulated
+// cycles per section of the dual active-set loop over all warps (DasTimer).
 #ifdef ISMPC_PHASE_TIMING
 __device__ long long g_phase[64];     // defined here: the debug build is a single translation unit (unity_dbg.cu)
 __device__ long long g_trace[3 * 8192];   // per CTA of the warp tick kernel: start / end (globaltimer ns), SM id

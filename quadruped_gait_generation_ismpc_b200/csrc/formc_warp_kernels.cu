@@ -336,9 +336,6 @@ formc_rollout_warp_kernel(FormCWarpArgs wa, ismpc_state_t* state_io, ismpc_walk_
     }
 }
 
-// The warp kernels cover every horizon the ABI accepts (N <= ISMPC_MAX_N).
-int formc_warp_supported(int N) { return N >= 2 && N <= ISMPC_MAX_N; }
-
 // Grid of the warp kernels for n instances: one 32-thread CTA per instance up to what the GPU keeps resident,
 // grid-stride beyond that (bounds the workspace of the general vertical path).
 // Builds of the tick kernel: the PAIR kernel (two warps per instance, formc_pair.cuh) is the latency build, used while

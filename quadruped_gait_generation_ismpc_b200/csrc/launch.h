@@ -12,19 +12,11 @@ struct FormCWarpArgs;
 
 int formc_setup_launch(const ismpc_formc_model_t& m, double* work, double* Hinv, double* G, double* M,
                        int* d_info, cudaStream_t st, long long* launches);
-int formc_prepare_gait_launch(int N, int S, int F, const double* Hinv, double* P, int* d_info, cudaStream_t st,
-                              long long* launches);
-int formc_cluster_ctas_per_sm(int N);
-int formc_tick_launch(const FormCArgs& a, int grid, int cluster_size, cudaStream_t st);
-int formc_rollout_launch(const FormCArgs& a, ismpc_state_t* state_io, ismpc_walk_t* walk_io,
-                         const ismpc_push_t* push, int n_ticks, double* traj, int32_t* status, int32_t* trace, int grid,
-                         cudaStream_t st);
 
 // warp-per-instance kernels (formc_warp_kernels.cu)
 int formc_riccati_launch(const ismpc_formc_model_t& m, int S, int F, int none, double* tab, cudaStream_t st,
                          long long* launches);
 int formc_law_launch(const ismpc_formc_model_t& m, int n_pat, const double* ric, double* law, cudaStream_t st, long long* launches);
-int formc_warp_supported(int N);
 int formc_warp_resident(int N, int sm_count, int res[5]);   // 0 or a cudaError_t
 int formc_tick_warp_launch(const FormCWarpArgs& a, int n, const int res[5], int variant, int pdl, int* grid_out, cudaStream_t st);
 int formc_rollout_warp_launch(const FormCWarpArgs& a, ismpc_state_t* state_io, ismpc_walk_t* walk_io,

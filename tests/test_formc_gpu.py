@@ -31,9 +31,14 @@ def _compare(handle, model, state, walk, inst, plan, nthreads=8, oracle_failures
     handle.formc_set_model(model)
     g = handle.formc_solve_batch(state, walk, inst, plan)
     o = O.formc_batch(model, state, walk, inst, plan, nthreads=nthreads)
+    ok = _check_against_oracle(model, g, o, len(state), oracle_failures)
+    return g, o, ok
+
+
+def _check_against_oracle(model, g, o, n, oracle_failures):
     N = int(model["N"][0])
     ok = (o["ret"] == 0).all(axis=1) & (o["out"]["status"] & abi.ST_WINDOW == 0)
-    assert (~ok).sum() <= oracle_failures, "oracle failures: %d of %d (expected %d)" % ((~ok).sum(), len(state), oracle_failures)
+    assert (~ok).sum() <= oracle_failures, "oracle failures: %d of %d (expected %d)" % ((~ok).sum(), n, oracle_failures)
     assert np.array_equal(g["out"]["status"] & abi.ST_WINDOW, o["out"]["status"] & abi.ST_WINDOW)
     _status_parity(g["out"]["status"], o["ret"])
     gfail = (g["out"]["status"] & (abi.ST_Z_FAIL | abi.ST_X_FAIL | abi.ST_Y_FAIL)) != 0
@@ -51,7 +56,7 @@ def _compare(handle, model, state, walk, inst, plan, nthreads=8, oracle_failures
     # the self-check is an absolute residual of a'u = b, and |a| grows like exp(eta dt N): 1e-8 up to N = 400
     kkt_tol = 1e-8 * max(1.0, float(np.exp(np.sqrt(9.81 / 0.69) * 0.01 * (N - 400))))
     assert g["out"]["kkt_res"][ok].max() < kkt_tol
-    return g, o, ok
+    return ok
 
 
 def test_reference_instance_closed_loop(handle):
@@ -137,28 +142,9 @@ def test_rollout_matches_tick_by_tick(handle):
     assert np.array_equal(r["walk"]["footstep_counter"], wk["footstep_counter"])
 
 
-@pytest.mark.parametrize("N,cs", [(100, 2), (100, 4), (200, 1), (200, 8), (400, 2)])
-def test_cluster_per_qp_identical_to_cta_per_qp(handle, N, cs):
-    """Config 4: the thread-block-cluster variant (x0 mat-vec split over the cluster, slices exchanged through
-    distributed shared memory) gives bit-identical results to one CTA per QP."""
-    n = 48
-    steps = (2 * N + 900) // 45 + 3
-    state, walk, inst, plan = synth.formc_batch(n, seed=1000 + N, N=N, n_steps=steps, z_spread=0.05)
-    handle.formc_set_model(abi.formc_model(N=N))
-    try:
-        handle.set_option("formc_cluster_size", 1 if cs != 1 else 4)
-        a = handle.formc_solve_batch(state, walk, inst, plan)
-        handle.set_option("formc_cluster_size", cs)
-        b = handle.formc_solve_batch(state, walk, inst, plan)
-    finally:
-        handle.set_option("formc_cluster_size", 0)
-    assert np.array_equal(a["primal"], b["primal"]) and np.array_equal(a["active"], b["active"])
-    assert a["out"].tobytes() == b["out"].tobytes()
-
-
 def test_prepared_gait_equals_generic_path(handle):
-    """ismpc_formc_prepare_gait folds the flight-phase equalities into a projector table: same results as the
-    closed-form equality solve of the generic path; instances with another step timing fall back to it."""
+    """ismpc_formc_prepare_gait tabulates the Riccati gains and the feedback law of every mpcIter of the gait: same results
+    as the recursion the generic path runs in the kernel; instances with another step timing fall back to it."""
     model = abi.formc_model()
     state, walk, inst, plan = synth.formc_batch(192, seed=4242, z_spread=0.04)
     # a third of the batch walks with another timing (S=30, F_ds=15: same 45-tick steps, other flight phase)
@@ -182,39 +168,33 @@ def test_prepared_gait_equals_generic_path(handle):
 
 
 @pytest.mark.parametrize("N", [50, 100, 200, 400])
-def test_warp_per_instance_equals_cta_per_instance(handle, N):
-    """The warp-per-instance tick (Riccati form of the vertical QP, register-resident) and the CTA-per-instance tick
-    (H_z^-1 tables) solve the same strictly convex QPs: same primal to 1e-9, same active sets, same status -- with the
-    prepared-gait tables, with the in-warp recursion (another step timing), and on the general vertical path."""
+def test_warp_builds_against_oracle_general_path(handle, N):
+    """Every build of the warp tick (one warp per instance with two register budgets, two warps per instance) against the
+    oracle -- with the prepared-gait tables, with the in-warp recursion (another step timing), and on the general
+    vertical path; and the builds against each other."""
     n = 96 if N <= 200 else 24
     steps = (2 * N + 900) // 45 + 3
     state, walk, inst, plan = synth.formc_batch(n, seed=31 + N, N=N, n_steps=steps, z_spread=0.06, running_frac=0.8)
     inst["S"][::4] = 30; inst["F_ds"][::4] = 15
-    handle.formc_set_model(abi.formc_model(N=N))
+    model = abi.formc_model(N=N)
+    handle.formc_set_model(model)
     handle.formc_prepare_gait(35, 10)
+    o = O.formc_batch(model, state, walk, inst, plan, nthreads=8)
+    res = []
     try:
-        handle.set_option("formc_kernel", 1)
-        a = handle.formc_solve_batch(state, walk, inst, plan)
-        handle.set_option("formc_kernel", 2)
-        res = []
-        for variant in (1, 16, 2):       # one warp per instance (two register budgets), two warps per instance
+        for variant in (1, 16, 2):
             handle.set_option("formc_variant", variant)
             res.append(handle.formc_solve_batch(state, walk, inst, plan))
     finally:
-        handle.set_option("formc_kernel", 0)
         handle.set_option("formc_variant", 0)
-    assert (a["out"]["iters"][:, 0] > 0).any(), "test is vacuous: the general vertical path never ran"
+    assert (res[0]["out"]["iters"][:, 0] > 0).any(), "test is vacuous: the general vertical path never ran"
     for b in res:
-        assert np.array_equal(a["out"]["status"], b["out"]["status"])
-        ok = (a["out"]["status"] & (abi.ST_Z_FAIL | abi.ST_X_FAIL | abi.ST_Y_FAIL)) == 0
-        assert (~ok).sum() <= {50: 3, 100: 1}.get(N, 0)      # instances qpOASES finds infeasible on these inputs
-        # H_z loses digits with the horizon (cond ~ N^4): at N = 400 the explicit H_z^-1 table is good to ~1e-8 only
+        ok = _check_against_oracle(model, b, o, n, {50: 3, 100: 1}.get(N, 0))   # instances qpOASES finds infeasible
+        # the oracle solves the dense QP in H_z, which loses digits with the horizon (cond ~ N^4)
         tol = 1e-9 if N <= 200 else 1e-7
-        assert primal_rel_err(b["primal"][ok].reshape(-1, 3, N), a["primal"][ok].reshape(-1, 3, N)).max() <= tol
-        assert np.array_equal(a["active"][ok], b["active"][ok])
-        assert np.abs(a["out"]["next"]["com_pos"][ok] - b["out"]["next"]["com_pos"][ok]).max() <= 1e-10
-        assert np.abs(a["out"]["next"]["com_vel"][ok] - b["out"]["next"]["com_vel"][ok]).max() <= 1e-9
-        assert b["out"]["kkt_res"][ok].max() < 1e-8
+        assert primal_rel_err(b["primal"][ok].reshape(-1, 3, N), o["primal"][ok].reshape(-1, 3, N)).max() <= tol
+        assert np.abs(b["out"]["next"]["com_pos"][ok] - o["out"]["next"]["com_pos"][ok]).max() <= 1e-10
+        assert np.abs(b["out"]["next"]["com_vel"][ok] - o["out"]["next"]["com_vel"][ok]).max() <= 1e-9
     # the builds of the warp family run the same arithmetic
     for b in res[1:]:
         assert np.array_equal(res[0]["out"]["status"], b["out"]["status"])
@@ -222,31 +202,47 @@ def test_warp_per_instance_equals_cta_per_instance(handle, N):
         assert np.array_equal(res[0]["active"], b["active"])
 
 
-def test_warp_rollout_equals_cta_rollout(handle):
-    """Closed loop with pushes: the two kernel families stay together tick by tick (1e-9 over 120 ticks)."""
+def test_warp_rollouts_match_tick_by_tick_with_pushes(handle):
+    """Closed loop with pushes: both rollout builds (one and two warps per instance) follow the same loop driven tick by
+    tick from the host -- footstep switch, push on ticks [ct0, ct1), tick, Controller bookkeeping -- for 120 ticks."""
     model = abi.formc_model()
     handle.formc_set_model(model)
     state, walk, inst, plan = synth.formc_batch(64, seed=77, dcm_spread=0.01, k0_cap=300)
     push = synth.push_batch(64, formc=True)
     push["ct0"] = 20; push["ct1"] = 34
     push["ax"] *= 0.3; push["ay"] *= 0.3           # keep most instances inside the 9 cm ZMP box for the whole run
+    T, dt = 120, float(model["dt"][0])
+    bs = []
     try:
-        handle.set_option("formc_kernel", 1)
-        a = handle.formc_rollout(state, walk, inst, plan, 120, push=push)
-        handle.set_option("formc_kernel", 2)
-        bs = []
-        for variant in (1, 2):           # one warp per instance, two warps per instance
+        for variant in (1, 2):
             handle.set_option("formc_variant", variant)
-            bs.append(handle.formc_rollout(state, walk, inst, plan, 120, push=push))
+            bs.append(handle.formc_rollout(state, walk, inst, plan, T, push=push))
     finally:
-        handle.set_option("formc_kernel", 0)
         handle.set_option("formc_variant", 0)
-    ok = (a["status"] & (abi.ST_Z_FAIL | abi.ST_X_FAIL | abi.ST_Y_FAIL)) == 0
+    st, wk = state.copy(), walk.copy()
+    traj = np.zeros((len(st), T, 6)); status = np.zeros(len(st), dtype=np.int32)
+    for t in range(T):
+        for i in range(len(st)):
+            fc = wk["footstep_counter"][i]
+            if fc < inst["n_steps"][i] and wk["sim_time"][i] >= plan[inst["plan_first_row"][i] + fc, 3] - 1:
+                wk["control_iter"][i] = 0; wk["mpc_iter"][i] = 0
+                wk["footstep_counter"][i] += 1; wk["support_foot"][i] = 1 - wk["support_foot"][i]
+        pushed = (t >= push["ct0"]) & (t < push["ct1"])
+        st["com_vel"][pushed, 0] += dt * push["ax"][pushed]
+        st["com_vel"][pushed, 1] += dt * push["ay"][pushed]
+        g = handle.formc_solve_batch(st, wk, inst, plan, want_primal=False, want_active=False)
+        st = g["out"]["next"].copy()
+        status |= g["out"]["status"]
+        traj[:, t, :3] = st["com_pos"]; traj[:, t, 3:] = st["com_vel"]
+        wk["control_iter"] += 1
+        wk["mpc_iter"] = np.floor(wk["control_iter"] * 0.01 / 0.01).astype(np.int32)   # Controller.cpp:504, in doubles
+        wk["sim_time"] += 1
+    ok = (status & (abi.ST_Z_FAIL | abi.ST_X_FAIL | abi.ST_Y_FAIL)) == 0
     assert ok.mean() > 0.5
     for b in bs:
-        assert np.array_equal(a["status"] & 7, b["status"] & 7)
-        assert np.abs(a["traj"][ok] - b["traj"][ok]).max() <= 1e-9
-        assert np.array_equal(a["walk"]["footstep_counter"], b["walk"]["footstep_counter"])
+        assert np.array_equal(b["status"] & 7, status & 7)
+        assert np.abs(b["traj"][ok] - traj[ok]).max() <= 1e-9
+        assert np.array_equal(b["walk"]["footstep_counter"], wk["footstep_counter"])
     assert np.abs(bs[0]["traj"][ok] - bs[1]["traj"][ok]).max() <= 1e-11
 
 
@@ -396,16 +392,11 @@ def test_packed_tick_records_and_resident_instances(handle, variant):
         handle.formc_set_plan(None); handle.formc_set_instances(None)
 
 
-def test_packed_call_needs_the_warp_kernel_family(handle):
-    model = abi.formc_model()
-    handle.formc_set_model(model)
-    state, walk, inst, plan = synth.formc_batch(8, seed=78)
-    handle.set_option("formc_kernel", 1)
-    try:
-        with pytest.raises(Exception):
-            handle.formc_solve_batch_packed(abi.pack_ticks(state, walk), inst, plan)
-    finally:
-        handle.set_option("formc_kernel", 0)
+def test_removed_kernel_options_are_refused(handle):
+    """The options that selected the CTA- and cluster-per-instance tick kernels are unknown names now (ISMPC_ERR_ARG)."""
+    for name, values in (("formc_kernel", (0, 1, 2)), ("formc_cluster_size", (0, 1, 2, 4, 8))):
+        for v in values:
+            assert handle._L.ismpc_set_option(handle._h, name.encode(), v) == -1      # ISMPC_ERR_ARG
 
 
 @pytest.mark.parametrize("N", [37, 101, 512])
@@ -496,9 +487,9 @@ def test_batch_beyond_residency_grid_stride(handle):
         handle.set_option("formc_variant", 0); handle.formc_set_plan(None); handle.formc_set_instances(None)
 
 
-def test_out_of_range_plan_rows_are_flagged_not_read(handle):
+def test_out_of_range_plan_rows_are_flagged_not_read_by_warp_builds(handle):
     """An instance record whose plan rows lie outside the plan table comes back with ISMPC_ST_WINDOW and its state
-    untouched (tick, both kernel builds) or unmoved (rollout); its neighbours are unaffected."""
+    untouched (tick: the pair and the one-warp build) or unmoved (rollout); its neighbours are unaffected."""
     model = abi.formc_model()
     handle.formc_set_model(model)
     state, walk, inst, plan = synth.formc_batch(64, seed=77, k0_cap=300)
@@ -508,16 +499,16 @@ def test_out_of_range_plan_rows_are_flagged_not_read(handle):
     bad["plan_first_row"][10] = -40                        # negative
     bad["n_steps"][20] = 1 << 28                           # absurd length
     ok = np.ones(64, bool); ok[[3, 10, 20]] = False
-    for name, value in (("formc_variant", 0), ("formc_variant", 1), ("formc_kernel", 1)):    # pair, one-warp, CTA kernels
-        handle.set_option(name, value)
+    for variant in (0, 1):            # the automatic choice (pair kernel at this batch size), one warp per instance
+        handle.set_option("formc_variant", variant)
         try:
             g = handle.formc_solve_batch(state, walk, bad, plan)
         finally:
-            handle.set_option(name, 0)
+            handle.set_option("formc_variant", 0)
         for i in (3, 10, 20):
             assert g["out"]["status"][i] == abi.ST_WINDOW
             assert np.array_equal(g["out"]["next"]["com_pos"][i], state["com_pos"][i])
-        if name == "formc_variant" and value == 0:
+        if variant == 0:
             assert g["out"][ok].tobytes() == ref["out"][ok].tobytes()
         else:
             assert np.abs(g["out"]["next"]["com_pos"][ok] - ref["out"]["next"]["com_pos"][ok]).max() < 1e-9

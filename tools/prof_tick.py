@@ -47,8 +47,6 @@ if which == "formcp":
     sys.exit(0)
 if which == "formc":
     h.formc_set_model(abi.formc_model())
-    if os.environ.get("ISMPC_FORMC_KERNEL"):
-        h.set_option("formc_kernel", int(os.environ["ISMPC_FORMC_KERNEL"]))
     if os.environ.get("ISMPC_VARIANT"):
         h.set_option("formc_variant", int(os.environ["ISMPC_VARIANT"]))
     if not os.environ.get("ISMPC_NO_GAIT"):
@@ -98,7 +96,7 @@ if os.environ.get("ISMPC_DBG"):
     ph = (C.c_longlong * 64)()
     binding.lib().ismpc_debug_read_phases(ph)
     v = list(ph)[:24]
-    if which == "formc" and os.environ.get("ISMPC_FORMC_KERNEL", "0") != "1":
+    if which == "formc":
         names = ["midpoints", "riccati", "rows+general", "lambda", "stab_row", "knapsack", "integrate"]
         tot = float(sum(v[:7])) or 1.0
         print("warp kernel, last launch: mean cycles per instance and phase (n=%d)" % n)
@@ -149,9 +147,6 @@ if os.environ.get("ISMPC_DBG"):
         print("last 8 items to finish: (start, dur, iters)", [(int(st_[i]), int(du[i]), int(its[i])) for i in order[-8:]])
         order = np.argsort(du)
         print("longest 8 items: (start, dur, iters)", [(int(st_[i]), int(du[i]), int(its[i])) for i in order[-8:]])
-    nz = [(i, x) for i, x in enumerate(v) if x]
-    print("phase clocks (CTA 0): stamp -> cycles since the previous non-zero stamp:",
-          [(nz[k][0], nz[k][1] - nz[k - 1][1]) for k in range(1, len(nz))], "total", nz[-1][1] - nz[0][1] if nz else 0)
     names = ["eval", "viol_scan", "schur_col", "apply_J", "apply_Jt", "ratio", "step_dir", "x_mu_update", "append", "drop",
              "A:build", "A:pdas_total", "A:selfcheck", "A:it_passA", "A:it_solve", "A:it_passB", "A:it_reguess", "A:epilogue"]
     acc = list(ph)[32:32 + len(names)]

@@ -10,7 +10,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from quadruped_gait_generation_ismpc_b200 import abi, binding, synth  # noqa: E402
 
 h = binding.Handle(0, max_batch=4096)
-# form C: pair kernel (small batch), warp kernels (beyond residency), CTA and cluster families, rollouts, general path
+# form C: pair kernel (small batch), warp kernels (beyond residency), rollouts, general path
 model = abi.formc_model()
 h.formc_set_model(model)
 state, walk, inst, plan = synth.formc_batch(96, seed=3)
@@ -28,12 +28,6 @@ print("formc warp tick/rollout (2048): failed", int((g["out"]["status"] & 7 != 0
 sv, wv, iv, pv = synth.formc_batch(64, seed=5, vary_height=True, z_spread=0.2)      # vertical rows active -> das path
 g = h.formc_solve_batch(sv, wv, iv, pv)
 print("formc general path: z-active instances", int((np.abs(g["active"][:, :100]).sum(axis=1) > 0).sum()))
-for name, val in (("formc_kernel", 1), ("formc_cluster_size", 4)):
-    h.set_option(name, val)
-    g = h.formc_solve_batch(state, walk, inst, plan)
-    r = h.formc_rollout(state[:16], walk[:16], inst[:16], plan, 5)
-h.set_option("formc_cluster_size", 0); h.set_option("formc_kernel", 0)
-print("formc CTA / cluster ok")
 # form A: tick (cold), rollout (warm), forced dual-active-set fallback
 am = abi.forma_model()
 h.forma_set_model(am)
