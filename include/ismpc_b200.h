@@ -516,6 +516,38 @@ int ismpc_qp_hotstart_batch(ismpc_handle* h, int n, const int32_t* mat_index_opt
                             double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
                             int mem, void* stream);
 
+/* Box bounds on the variables, qpOASES' standard form init(H, g, A, lb, ub, lbA, ubA) / hotstart(g, lb, ub, lbA, ubA):
+ *     min 1/2 x'Hx + g'x  s.t.  lb <= x <= ub,  lbA <= A x <= ubA.
+ * ismpc_qp_solve_batch_bounds is ismpc_qp_solve_batch_ws with the box; ismpc_qp_hotstart_batch_bounds is
+ * ismpc_qp_hotstart_batch with the box (the resident sets hold H and the rows of A only and are used unchanged;
+ * mat_index_opt, out-of-range indices and "dense_resident_gemm" behave as in that call).  Unlike the same bound written
+ * as a row of A, a bound adds nothing to the set-up products or to the resident tables.
+ *   lb, ub: n x nV; either may be NULL, which makes every value on that side absent.  |value| >= 1e20 is an absent side.
+ *   nC = 0 is allowed, with A, lbA and ubA NULL (a bounds-only QP, qpOASES' QProblemB).
+ *   A variable with |ub - lb| <= 1e-12 max(1, |lb|) is fixed: an equality, installed with the equality rows before any
+ *   inequality and never dropped.  lb > ub beyond that tolerance, or a bound that contradicts the equality rows, fails the
+ *   problem with ISMPC_ST_QP_FAIL.
+ *   y_opt, ws_opt: n x (nV + nC), bounds first, then the rows of A (qpOASES' getDualSolution / getWorkingSet order).
+ *   y > 0 / ws = -1 at a lower side, y < 0 / ws = +1 at an upper side; a fixed variable reports ws = -1, as an
+ *   equality row does.
+ *   ws_guess: n x (nV + nC) in the same layout, may alias ws_opt; the rules of ismpc_qp_solve_batch_ws apply to the bound
+ *   entries too (entries of fixed variables and of absent sides are ignored, dependent entries start free, the answer is
+ *   the cold call's for any guess).  iters_opt counts the working-set changes of bounds and rows together.
+ *   lb = ub = NULL: the constraint half of y_opt / ws_opt and x, status and iters are the bytes of
+ *   ismpc_qp_solve_batch_ws / ismpc_qp_hotstart_batch on the same inputs; the bound half is zero. */
+int ismpc_qp_solve_batch_bounds(ismpc_handle* h, int n, int nV, int nC,
+                                const double* H, const double* g, const double* A,
+                                const double* lb, const double* ub, const double* lbA, const double* ubA,
+                                const int8_t* ws_guess,
+                                double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
+                                int mem, void* stream);
+
+int ismpc_qp_hotstart_batch_bounds(ismpc_handle* h, int n, const int32_t* mat_index_opt,
+                                   const double* g, const double* lb, const double* ub, const double* lbA, const double* ubA,
+                                   const int8_t* ws_guess,
+                                   double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
+                                   int mem, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -22,7 +22,8 @@ EXPORTS = ["ismpc_version", "ismpc_error_string", "ismpc_create", "ismpc_destroy
            "ismpc_handle_stream", "ismpc_wait", "ismpc_host_alloc", "ismpc_host_free", "ismpc_formc_rollout_ex",
            "ismpc_forma_rollout_ex2", "ismpc_kf_filter_batch_f64", "ismpc_formc_set_instances",
            "ismpc_formc_solve_batch_packed", "ismpc_qp_solve_batch_ws", "ismpc_qp_set_matrices",
-           "ismpc_qp_hotstart_batch", "ismpc_forma_solve_batch_ws"]
+           "ismpc_qp_hotstart_batch", "ismpc_forma_solve_batch_ws", "ismpc_qp_solve_batch_bounds",
+           "ismpc_qp_hotstart_batch_bounds"]
 
 _lib = None
 
@@ -95,6 +96,8 @@ def lib():
     L.ismpc_qp_solve_batch_ws.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 11 + [C.c_int, C.c_void_p]
     L.ismpc_qp_set_matrices.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 3 + [C.c_int]
     L.ismpc_qp_hotstart_batch.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 10 + [C.c_int, C.c_void_p]
+    L.ismpc_qp_solve_batch_bounds.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 13 + [C.c_int, C.c_void_p]
+    L.ismpc_qp_hotstart_batch_bounds.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 12 + [C.c_int, C.c_void_p]
     L.ismpc_handle_stream.restype = C.c_void_p
     L.ismpc_handle_stream.argtypes = [C.c_void_p]
     L.ismpc_wait.argtypes = [C.c_void_p, C.c_void_p]
@@ -439,9 +442,22 @@ class Handle:
         self._check(rc, "ismpc_qp_solve_batch_ws")
 
     # ---- generic dense QP (solveQP seam) ----------------------------------------------------------
-    def qp_solve_batch(self, H, g, A, lbA, ubA, ws_guess=None):
+    def qp_solve_batch_bounds_raw(self, n, nV, nC, H, g, A, lb, ub, lbA, ubA, x, y=None, ws=None, status=None, iters=None,
+                                  mem=abi.MEM_DEVICE, stream=None, ws_guess=None):
+        """Raw ismpc_qp_solve_batch_bounds: every array is a numpy array (host), an integer address (device) or None;
+        y, ws and ws_guess are n x (nV + nC)."""
+        rc = self._L.ismpc_qp_solve_batch_bounds(self._h, n, nV, nC, _ptr(H), _ptr(g), _ptr(A), _ptr(lb), _ptr(ub),
+                                                 _ptr(lbA), _ptr(ubA), _ptr(ws_guess), _ptr(x), _ptr(y), _ptr(ws),
+                                                 _ptr(status), _ptr(iters), mem, C.c_void_p(stream) if stream else None)
+        self._check(rc, "ismpc_qp_solve_batch_bounds")
+
+    def qp_solve_batch(self, H, g, A, lbA, ubA, ws_guess=None, lb=None, ub=None):
         """ws_guess (n x nC int8, <0 lower / >0 upper / 0 free, e.g. the "ws" of an earlier call): hot start from that
-        working set; the results are those of the cold call to rounding, "iters" counts the changes made after it."""
+        working set; the results are those of the cold call to rounding, "iters" counts the changes made after it.
+        lb / ub (n x nV, either may be None = absent): box bounds on x through ismpc_qp_solve_batch_bounds; "y", "ws" and
+        ws_guess are then n x (nV + nC), bounds first.  A, lbA and ubA may be None when there are no rows."""
+        if lb is not None or ub is not None:
+            return self._qp_bounds(False, H, g, A, lb, ub, lbA, ubA, ws_guess, None)
         H = np.ascontiguousarray(H, dtype=np.float64); g = np.ascontiguousarray(g, dtype=np.float64)
         A = np.ascontiguousarray(A, dtype=np.float64)
         lbA = np.ascontiguousarray(lbA, dtype=np.float64); ubA = np.ascontiguousarray(ubA, dtype=np.float64)
@@ -483,9 +499,39 @@ class Handle:
                                                   abi.MEM_HOST), "ismpc_qp_set_matrices")
         return mat_status
 
-    def qp_hotstart_batch(self, g, lbA, ubA, ws_guess=None, mat_index=None):
+    def _qp_bounds(self, resident, H, g, A, lb, ub, lbA, ubA, ws_guess, mat_index):
+        """qp_solve_batch (resident False) or qp_hotstart_batch (resident True) with box bounds."""
+        g = np.ascontiguousarray(g, dtype=np.float64)
+        n, nV = g.shape
+        nC = 0 if lbA is None else np.shape(lbA)[1]
+        f64 = lambda a: None if a is None else np.ascontiguousarray(a, dtype=np.float64)
+        lb, ub, lbA, ubA = f64(lb), f64(ub), f64(lbA), f64(ubA)
+        for name, a, shape in (("lb", lb, (n, nV)), ("ub", ub, (n, nV)), ("lbA", lbA, (n, nC)), ("ubA", ubA, (n, nC))):
+            if a is not None and a.shape != shape:
+                raise ValueError("%s must be %d x %d, got %s" % (name, shape[0], shape[1], a.shape))
+        nR = nV + nC
+        x = np.zeros((n, nV)); y = np.zeros((n, nR)); ws = np.zeros((n, nR), dtype=np.int8)
+        status = np.zeros(n, dtype=np.int32); iters = np.zeros(n, dtype=np.int32)
+        guess = None if ws_guess is None else np.ascontiguousarray(ws_guess, dtype=np.int8)
+        if guess is not None and guess.shape != (n, nR):
+            raise ValueError("ws_guess must be %d x %d, got %s" % (n, nR, guess.shape))
+        if not resident:
+            self.qp_solve_batch_bounds_raw(n, nV, nC, f64(H), g, f64(A) if nC else None, lb, ub, lbA, ubA, x, y, ws,
+                                           status, iters, mem=abi.MEM_HOST, ws_guess=guess)
+        else:
+            idx = None if mat_index is None else np.ascontiguousarray(mat_index, dtype=np.int32)
+            if idx is not None and idx.shape != (n,):
+                raise ValueError("mat_index must have %d entries, got %s" % (n, idx.shape))
+            self.qp_hotstart_batch_bounds_raw(n, g, lb, ub, lbA, ubA, x, y, ws, status, iters, mat_index=idx,
+                                              ws_guess=guess, mem=abi.MEM_HOST)
+        return dict(x=x, y=y, ws=ws, status=status, iters=iters)
+
+    def qp_hotstart_batch(self, g, lbA, ubA, ws_guess=None, mat_index=None, lb=None, ub=None):
         """ismpc_qp_hotstart_batch: n problems against the resident sets, problem p on set mat_index[p] (None: set p, or
-        set 0 when one set is resident).  ws_guess as in qp_solve_batch.  Returns the dict of qp_solve_batch."""
+        set 0 when one set is resident).  ws_guess, lb and ub as in qp_solve_batch (with lb or ub,
+        ismpc_qp_hotstart_batch_bounds).  Returns the dict of qp_solve_batch."""
+        if lb is not None or ub is not None:
+            return self._qp_bounds(True, None, g, None, lb, ub, lbA, ubA, ws_guess, mat_index)
         g = np.ascontiguousarray(g, dtype=np.float64)
         lbA = np.ascontiguousarray(lbA, dtype=np.float64); ubA = np.ascontiguousarray(ubA, dtype=np.float64)
         n, nV = g.shape
@@ -510,6 +556,14 @@ class Handle:
                                              _ptr(x), _ptr(y), _ptr(ws), _ptr(status), _ptr(iters), mem,
                                              C.c_void_p(stream) if stream else None)
         self._check(rc, "ismpc_qp_hotstart_batch")
+
+    def qp_hotstart_batch_bounds_raw(self, n, g, lb, ub, lbA, ubA, x, y=None, ws=None, status=None, iters=None,
+                                     mat_index=None, ws_guess=None, mem=abi.MEM_DEVICE, stream=None):
+        """Raw ismpc_qp_hotstart_batch_bounds: every array is a numpy array (host), an integer address (device) or None."""
+        rc = self._L.ismpc_qp_hotstart_batch_bounds(self._h, n, _ptr(mat_index), _ptr(g), _ptr(lb), _ptr(ub), _ptr(lbA),
+                                                    _ptr(ubA), _ptr(ws_guess), _ptr(x), _ptr(y), _ptr(ws), _ptr(status),
+                                                    _ptr(iters), mem, C.c_void_p(stream) if stream else None)
+        self._check(rc, "ismpc_qp_hotstart_batch_bounds")
 
 
 # ---- all GPUs of one box behind one C ABI (include/ismpc_b200_multigpu.h, lib/libismpc_b200_mg.so) --------------------

@@ -31,9 +31,9 @@ struct DevBuf {
 };
 
 // Host-memory calls stage their buffers in ismpc_handle::stage, taken in the order the call asks for them: a loop of one
-// call keeps each buffer in one role, so a buffer grows once.  The form-A tick and rollouts stage the most (12 arguments;
+// call keeps each buffer in one role, so a buffer grows once.  ismpc_qp_solve_batch_bounds stages the most (13 arguments;
 // NULL ones keep their place).
-constexpr int STAGE_SLOTS = 12;
+constexpr int STAGE_SLOTS = 13;
 
 struct ismpc_handle {
     int device = 0;
@@ -804,26 +804,29 @@ extern "C" int ismpc_kf_filter_batch_f64(ismpc_handle* h, int n, int n_steps, co
 // ---------------------------------------------------------------------------------------------------
 // Generic dense QP (solveQP seam)
 // ---------------------------------------------------------------------------------------------------
-extern "C" int ismpc_qp_solve_batch_ws(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* g,
-                                       const double* A, const double* lbA, const double* ubA, const int8_t* ws_guess,
-                                       double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
-                                       int mem, void* stream)
+// The cold / guessed seam calls, with (bounds) or without the box lbx <= x <= ubx: y, ws and the guess are n x nR, nR =
+// nV + nC with bounds (bounds first), nC without.
+static int qp_solve_common(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* g, const double* A,
+                           bool bounds, const double* lbx, const double* ubx, const double* lbA, const double* ubA,
+                           const int8_t* ws_guess, double* x, double* y_opt, int8_t* ws_opt, int32_t* status,
+                           int32_t* iters_opt, int mem, void* stream)
 {
     if (!h) return ISMPC_ERR_ARG;
     if (n < 0 || n > h->max_batch || nV < 1 || nV > ISMPC_MAX_N || nC < 0 || nC > 2 * ISMPC_MAX_N + 8 || !H || !g ||
         (nC > 0 && (!A || !lbA || !ubA)) || !x || !status)
         return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
-    if (nC == 0) ws_guess = nullptr;           // nothing to guess
+    const int nR = bounds ? nV + nC : nC;
+    if (nR == 0) ws_guess = nullptr;           // nothing to guess
     CK(cudaSetDevice(h->device));
-    if (h->q_work.ensure(qp_dense_work_doubles(n, nV, nC) * sizeof(double))) return ISMPC_ERR_ALLOC;
+    if (h->q_work.ensure(qp_dense_work_doubles(n, nV, nC, bounds) * sizeof(double))) return ISMPC_ERR_ALLOC;
     Staged s(h, mem, stream, false);
-    const size_t szg = (size_t)n * nV, szb = (size_t)n * nC;
+    const size_t szg = (size_t)n * nV, szb = (size_t)n * nC, szr = (size_t)n * nR;
     // both dense-seam calls stage their outputs first and in one order, so that they share the output staging: the
     // rows a failed problem leaves unwritten come back as the previous dense-seam call left them
     double* dx = s.out(x, szg);
-    double* dy = s.out(y_opt, szb);
-    int8_t* dws = s.out(ws_opt, szb);
+    double* dy = s.out(y_opt, szr);
+    int8_t* dws = s.out(ws_opt, szr);
     int32_t* dst = s.out(status, n);
     int32_t* dit = s.out(iters_opt, n);
     const double* dH = s.in(H, szg * nV);
@@ -831,11 +834,31 @@ extern "C" int ismpc_qp_solve_batch_ws(ismpc_handle* h, int n, int nV, int nC, c
     const double* dA = s.in(A, szb * nV);
     const double* dlb = s.in(lbA, szb);
     const double* dub = s.in(ubA, szb);
-    const int8_t* dgs = s.in(ws_guess, szb);       // a buffer of its own: the guess may alias ws_opt
+    const int8_t* dgs = s.in(ws_guess, szr);       // a buffer of its own: the guess may alias ws_opt
+    const double* dlbx = bounds ? s.in(lbx, szg) : nullptr;
+    const double* dubx = bounds ? s.in(ubx, szg) : nullptr;
     if (s.err) return s.err;
-    return s.finish(qp_dense_launch(n, nV, nC, dH, dg, dA, dlb, dub, (const signed char*)dgs, dx, dy, (signed char*)dws, dst,
-                                    dit, (double*)h->q_work.p, h->opt_dense_dmma, s.st),
+    return s.finish(qp_dense_launch(n, nV, nC, dH, dg, dA, dlb, dub, bounds, dlbx, dubx, (const signed char*)dgs, dx, dy,
+                                    (signed char*)dws, dst, dit, (double*)h->q_work.p, h->opt_dense_dmma, s.st),
                     "qp_dense_launch");
+}
+
+extern "C" int ismpc_qp_solve_batch_ws(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* g,
+                                       const double* A, const double* lbA, const double* ubA, const int8_t* ws_guess,
+                                       double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
+                                       int mem, void* stream)
+{
+    return qp_solve_common(h, n, nV, nC, H, g, A, false, nullptr, nullptr, lbA, ubA, ws_guess, x, y_opt, ws_opt, status,
+                           iters_opt, mem, stream);
+}
+
+extern "C" int ismpc_qp_solve_batch_bounds(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* g,
+                                           const double* A, const double* lb, const double* ub, const double* lbA,
+                                           const double* ubA, const int8_t* ws_guess, double* x, double* y_opt,
+                                           int8_t* ws_opt, int32_t* status, int32_t* iters_opt, int mem, void* stream)
+{
+    return qp_solve_common(h, n, nV, nC, H, g, A, true, lb, ub, lbA, ubA, ws_guess, x, y_opt, ws_opt, status, iters_opt,
+                           mem, stream);
 }
 
 extern "C" int ismpc_qp_solve_batch(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* g,
@@ -861,7 +884,7 @@ extern "C" int ismpc_qp_set_matrices(ismpc_handle* h, int n_mat, int nV, int nC,
     const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
     if (h->r_tab.ensure(qp_sets_table_doubles(n_mat, nV, nC) * sizeof(double)) ||
         h->r_stat.ensure((size_t)n_mat * sizeof(int32_t)) ||
-        h->r_work.ensure(qp_sets_work_doubles(0, n_mat, nV, nC) * sizeof(double)))
+        h->r_work.ensure(qp_sets_work_doubles(0, n_mat, nV, nC, false) * sizeof(double)))
         return ISMPC_ERR_ALLOC;
     const cudaMemcpyKind kind = mem == ISMPC_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
     double* tab = (double*)h->r_tab.p;
@@ -877,10 +900,11 @@ extern "C" int ismpc_qp_set_matrices(ismpc_handle* h, int n_mat, int nV, int nC,
     return ISMPC_OK;
 }
 
-extern "C" int ismpc_qp_hotstart_batch(ismpc_handle* h, int n, const int32_t* mat_index_opt, const double* g,
-                                       const double* lbA, const double* ubA, const int8_t* ws_guess, double* x,
-                                       double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt, int mem,
-                                       void* stream)
+// The calls against the resident sets, with (bounds) or without the box; layouts as in qp_solve_common.
+static int qp_hotstart_common(ismpc_handle* h, int n, const int32_t* mat_index_opt, const double* g, bool bounds,
+                              const double* lbx, const double* ubx, const double* lbA, const double* ubA,
+                              const int8_t* ws_guess, double* x, double* y_opt, int8_t* ws_opt, int32_t* status,
+                              int32_t* iters_opt, int mem, void* stream)
 {
     if (!h) return ISMPC_ERR_ARG;
     if (n < 0 || n > h->max_batch || !g || !x || !status || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
@@ -889,28 +913,49 @@ extern "C" int ismpc_qp_hotstart_batch(ismpc_handle* h, int n, const int32_t* ma
     const int nV = h->r_nV, nC = h->r_nC, n_mat = h->r_nmat;
     if ((nC > 0 && (!lbA || !ubA)) || (!mat_index_opt && n_mat > 1 && n > n_mat)) return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
-    if (nC == 0) ws_guess = nullptr;
+    const int nR = bounds ? nV + nC : nC;
+    if (nR == 0) ws_guess = nullptr;
     CK(cudaSetDevice(h->device));
-    if (h->r_work.ensure(qp_sets_work_doubles(n, n_mat, nV, nC) * sizeof(double))) return ISMPC_ERR_ALLOC;
+    if (h->r_work.ensure(qp_sets_work_doubles(n, n_mat, nV, nC, bounds) * sizeof(double))) return ISMPC_ERR_ALLOC;
     Staged s(h, mem, stream, false);
-    const size_t szg = (size_t)n * nV, szb = (size_t)n * nC;
+    const size_t szg = (size_t)n * nV, szb = (size_t)n * nC, szr = (size_t)n * nR;
     // outputs first, as in ismpc_qp_solve_batch_ws; x, y and ws are staged with the caller's bytes, so that a problem
     // the call does not touch (set index out of range) keeps them, as with device buffers
     double* dx = s.inout(x, szg);
-    double* dy = s.inout(y_opt, szb);
-    int8_t* dws = s.inout(ws_opt, szb);
+    double* dy = s.inout(y_opt, szr);
+    int8_t* dws = s.inout(ws_opt, szr);
     int32_t* dst = s.out(status, n);
     int32_t* dit = s.out(iters_opt, n);
     const double* dg = s.in(g, szg);
     const double* dlb = s.in(lbA, szb);
     const double* dub = s.in(ubA, szb);
     const int32_t* didx = s.in(mat_index_opt, n);
-    const int8_t* dgs = s.in(ws_guess, szb);
+    const int8_t* dgs = s.in(ws_guess, szr);
+    const double* dlbx = bounds ? s.in(lbx, szg) : nullptr;
+    const double* dubx = bounds ? s.in(ubx, szg) : nullptr;
     if (s.err) return s.err;
     return s.finish(qp_sets_launch(n, nV, nC, n_mat, (const double*)h->r_tab.p, (const int32_t*)h->r_stat.p, didx, dg, dlb,
-                                   dub, (const signed char*)dgs, dx, dy, (signed char*)dws, dst, dit,
+                                   dub, bounds, dlbx, dubx, (const signed char*)dgs, dx, dy, (signed char*)dws, dst, dit,
                                    (double*)h->r_work.p, h->opt_dense_resident_gemm, h->opt_dense_dmma, s.st),
                     "qp_sets_launch");
+}
+
+extern "C" int ismpc_qp_hotstart_batch(ismpc_handle* h, int n, const int32_t* mat_index_opt, const double* g,
+                                       const double* lbA, const double* ubA, const int8_t* ws_guess, double* x,
+                                       double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt, int mem,
+                                       void* stream)
+{
+    return qp_hotstart_common(h, n, mat_index_opt, g, false, nullptr, nullptr, lbA, ubA, ws_guess, x, y_opt, ws_opt, status,
+                              iters_opt, mem, stream);
+}
+
+extern "C" int ismpc_qp_hotstart_batch_bounds(ismpc_handle* h, int n, const int32_t* mat_index_opt, const double* g,
+                                              const double* lb, const double* ub, const double* lbA, const double* ubA,
+                                              const int8_t* ws_guess, double* x, double* y_opt, int8_t* ws_opt,
+                                              int32_t* status, int32_t* iters_opt, int mem, void* stream)
+{
+    return qp_hotstart_common(h, n, mat_index_opt, g, true, lb, ub, lbA, ubA, ws_guess, x, y_opt, ws_opt, status, iters_opt,
+                              mem, stream);
 }
 
 // ---------------------------------------------------------------------------------------------------

@@ -47,16 +47,17 @@ int feet_export_launch(int n, const ismpc_feet_model_t& m, const ismpc_feet_inst
                        cudaStream_t st);
 
 int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, const double* A, const double* lbA,
-                    const double* ubA, const signed char* ws_guess, double* x, double* y, signed char* ws,
-                    int32_t* status, int32_t* iters, double* work, int use_dmma, cudaStream_t st);
-size_t qp_dense_work_doubles(int n, int nV, int nC);
+                    const double* ubA, bool bounds, const double* lbx, const double* ubx, const signed char* ws_guess,
+                    double* x, double* y, signed char* ws, int32_t* status, int32_t* iters, double* work, int use_dmma,
+                    cudaStream_t st);
+size_t qp_dense_work_doubles(int n, int nV, int nC, bool bounds);
 // the resident matrix family of the dense seam (ismpc_qp_set_matrices / ismpc_qp_hotstart_batch)
 size_t qp_sets_table_doubles(int n_mat, int nV, int nC);
-size_t qp_sets_work_doubles(int n, int n_mat, int nV, int nC);
+size_t qp_sets_work_doubles(int n, int n_mat, int nV, int nC, bool bounds);
 int qp_sets_build(int n_mat, int nV, int nC, double* tab, int32_t* fstat, double* work, int use_dmma, cudaStream_t st);
 int qp_sets_launch(int n, int nV, int nC, int n_mat, const double* tab, const int32_t* fstat, const int32_t* idx,
-                   const double* g, const double* lbA, const double* ubA, const signed char* ws_guess, double* x,
-                   double* y, signed char* ws, int32_t* status, int32_t* iters, double* work, int use_gemm, int use_dmma,
-                   cudaStream_t st);
+                   const double* g, const double* lbA, const double* ubA, bool bounds, const double* lbx,
+                   const double* ubx, const signed char* ws_guess, double* x, double* y, signed char* ws, int32_t* status,
+                   int32_t* iters, double* work, int use_gemm, int use_dmma, cudaStream_t st);
 
 }  // namespace ismpc

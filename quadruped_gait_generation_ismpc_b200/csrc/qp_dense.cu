@@ -21,26 +21,31 @@ struct DenseLayout {          // offsets (in doubles) inside one problem's works
 };
 
 // tables = false: the slice of the resident path (qp_resident_launch), the vectors only -- the tables belong to the resident
-// set, x0 and A x0 to the n x (nV + nC) block its x0 step writes
-__host__ __device__ inline DenseLayout dense_layout(int nV, int nC, bool tables = true)
+// set, x0 and A x0 to the n x (nV + nC) block its x0 step writes.  bounds = true: the working set and the row states span the
+// nV bound rows as well (dense_das_kernel<.., .., true>)
+__host__ __device__ inline DenseLayout dense_layout(int nV, int nC, bool tables = true, bool bounds = false)
 {
     DenseLayout l;
     const size_t vv = tables ? (size_t)nV * nV : 0, cv = tables ? (size_t)nC * nV : 0, cc = tables ? (size_t)nC * nC : 0;
-    l.qmax = (nV + 1 < nC ? nV + 1 : nC); if (l.qmax < 1) l.qmax = 1;
+    const int m = bounds ? nV + nC : nC;
+    l.qmax = (nV + 1 < m ? nV + 1 : m); if (l.qmax < 1) l.qmax = 1;
     size_t o = 0;
     l.Lh = o; o += vv; l.Linv = o; o += vv; l.Hinv = o; o += vv;
     l.D = o; o += cv; l.S = o; o += cc;
     l.x0 = o; o += tables ? nV : 0; l.rv = o; o += tables ? nC : 0; l.az = o; o += nC; l.z = o; o += nV;
     l.Lw = o; o += (size_t)l.qmax * (l.qmax + 1) / 2;
     l.mu = o; o += l.qmax; l.r = o; o += l.qmax; l.y = o; o += l.qmax;
-    l.ints = o; o += (size_t)(l.qmax * sizeof(int) + l.qmax + nC + 15) / 8 + 2;
+    l.ints = o; o += (size_t)(l.qmax * sizeof(int) + l.qmax + m + 15) / 8 + 2;
     l.total = (o + 1) & ~(size_t)1;
     return l;
 }
 
-// n problem slices, then (warm start only) n x nC doubles of A x0, kept while rv moves; outside the slices so that the
-// cold path's layout does not depend on it
-size_t qp_dense_work_doubles(int n, int nV, int nC) { return (dense_layout(nV, nC).total + nC) * (size_t)n + 16; }
+// n problem slices, then (warm start only) n x nC doubles of A x0 (with bounds: n x (nV + nC) of x0 | A x0), kept while rv
+// moves; outside the slices so that the cold path's layout does not depend on it
+size_t qp_dense_work_doubles(int n, int nV, int nC, bool bounds)
+{
+    return (dense_layout(nV, nC, true, bounds).total + nC + (bounds ? nV : 0)) * (size_t)n + 16;
+}
 
 // ---- set-up kernels (batched over problems with blockIdx.z / blockIdx.y) --------------------------------
 __global__ void dense_copy_H(int nV, const double* H, double* work, size_t stride, size_t offL)
@@ -319,6 +324,77 @@ struct DenseWarmProb : DenseProb {
     }
 };
 
+// Box bounds lb <= x <= ub as nV rows e_i' ahead of the rows of A: ids [0, nV) are the bounds, [nV, nV + nC) the rows.
+// No table of their own: [Hinv; D] (HD, one (nV + nC) x nV block in both layouts) is the D-role table of the extended rows,
+// and S_ext = [[Hinv, D'], [D, S]] is read from HD and S.  rv is [x | A x] (x0 and A x0 are adjacent in both layouts), the
+// bound half moved by the step z itself.
+struct DenseBoundsProb : DenseProb {
+    const double *HD, *lbx, *ubx;       // lbx / ubx: this problem's nV bounds, NULL = that side absent
+    const double* z;                    // the step direction step_dir writes (w + l.z)
+    __device__ int m() const { return nV + nC; }
+    __device__ double lo(int i) const { return i < nV ? (lbx ? lbx[i] : -1e20) : lb[i - nV]; }
+    __device__ double hi(int i) const { return i < nV ? (ubx ? ubx[i] : 1e20) : ub[i - nV]; }
+    __device__ double schur(int a, int b) const
+    {
+        if (a < nV) return HD[(size_t)b * nV + a];
+        if (b < nV) return HD[(size_t)a * nV + b];
+        return S[(size_t)(a - nV) * nC + (b - nV)];
+    }
+    // a_c' H^-1 a_id for row c of A: a gather with stride nV when id is a bound
+    __device__ double row_col(int id, int c) const
+    {
+        return id < nV ? HD[(size_t)(nV + c) * nV + id] : S[(size_t)(id - nV) * nC + c];
+    }
+    __device__ void step_dir(int idp, int sgp, const int* wid, const signed char* wsg, const double* r, int q,
+                             double* zo) const
+    {
+        const int lane = lane_id();
+        for (int i = lane; i < nV; i += 32) {
+            double acc = (double)sgp * HD[(size_t)idp * nV + i];
+            for (int k = 0; k < q; ++k) acc -= (double)wsg[k] * r[k] * HD[(size_t)wid[k] * nV + i];
+            zo[i] = acc;
+        }
+        for (int i = lane; i < nC; i += 32) {
+            double acc = (double)sgp * row_col(idp, i);
+            for (int k = 0; k < q; ++k) acc -= (double)wsg[k] * r[k] * row_col(wid[k], i);
+            az[i] = acc;
+        }
+        __syncwarp();
+    }
+    __device__ void on_step(double t) const
+    {
+        const int lane = lane_id();
+        for (int i = lane; i < nV; i += 32) rv[i] += t * z[i];
+        for (int i = lane; i < nC; i += 32) rv[nV + i] += t * az[i];
+        __syncwarp();
+    }
+};
+
+struct DenseBoundsWarmProb : DenseBoundsProb {
+    const double* rv0_;                 // x0 | A x0, kept while rv moves
+    __device__ double rv0(int i) const { return rv0_[i]; }
+    __device__ void combine(const int* wid, const signed char* wsg, const double* mu, int q, double* x) const
+    {
+        const int lane = lane_id();
+        for (int i = lane; i < nV; i += 32) {
+            double acc = rv0_[i];
+            for (int k = 0; k < q; ++k) acc += (double)wsg[k] * mu[k] * HD[(size_t)wid[k] * nV + i];
+            x[i] = acc;
+            rv[i] = acc;
+        }
+        for (int i = lane; i < nC; i += 32) {
+            double acc = rv0_[nV + i];
+            for (int k = 0; k < q; ++k) acc += (double)wsg[k] * mu[k] * row_col(wid[k], i);
+            rv[nV + i] = acc;
+        }
+        __syncwarp();
+    }
+};
+
+template <bool WARM, bool BOUNDS>
+using DenseProbT = std::conditional_t<BOUNDS, std::conditional_t<WARM, DenseBoundsWarmProb, DenseBoundsProb>,
+                                      std::conditional_t<WARM, DenseWarmProb, DenseProb>>;
+
 constexpr int DENSE_R = 64;      // rows of the inverse factor kept in shared memory (16.6 KB per warp)
 constexpr int DENSE_WARPS = 4;   // QPs per CTA
 
@@ -328,10 +404,13 @@ constexpr int DENSE_WARPS = 4;   // QPs per CTA
 // (the seam).  SETS = true: they come from the problem's resident set and sets.xr, the slice (dense_layout(.., false))
 // holds the vectors only, and the status starts from the set's; a problem whose set index is out of range is flagged and
 // nothing else of it is written.  The algorithm is the same, so the same inputs give the same bytes.
-template <bool WARM, bool SETS>
+// BOUNDS = true: the rows are [I; A] with the box lbx <= x <= ubx (n x nV each, NULL = that side absent) as the first nV
+// (DenseBoundsProb); y, ws and ws_guess are n x (nV + nC), bounds first.  A variable whose bounds cross is flagged.
+template <bool WARM, bool SETS, bool BOUNDS>
 __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const double* ubA, double* work,
                                  size_t stride, DenseLayout l, int R, double* x, double* y, signed char* ws,
-                                 int32_t* status, int32_t* iters, const signed char* ws_guess, DenseSets sets)
+                                 int32_t* status, int32_t* iters, const signed char* ws_guess, DenseSets sets,
+                                 const double* lbx, const double* ubx)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int p = blockIdx.x * DENSE_WARPS + warp_id();
@@ -369,22 +448,29 @@ __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const
     } else {
         st = status[p];
     }
-    double* rv = SETS ? x0 + nV : w + l.rv;
+    double* rv = BOUNDS ? x0 : SETS ? x0 + nV : w + l.rv;
+    const int nR = BOUNDS ? nV + nC : nC;       // rows of the working set's row space
     int it = 0;
-    if (st == 0 && nC > 0) {
-        for (int i = lane; i < nC; i += 32) dw.state[i] = 0;
+    if (st == 0 && nR > 0) {
+        for (int i = lane; i < nR; i += 32) dw.state[i] = 0;
         __syncwarp();
         const DenseProb pb0{nV, nC, D, S, lb, ub, rv, w + l.az};
-        std::conditional_t<WARM, DenseWarmProb, DenseProb> pb{pb0};
+        DenseProbT<WARM, BOUNDS> pb{pb0};
+        if constexpr (BOUNDS) {
+            pb.HD = D - (size_t)nV * nV;
+            pb.lbx = lbx ? lbx + (size_t)p * nV : nullptr;
+            pb.ubx = ubx ? ubx + (size_t)p * nV : nullptr;
+            pb.z = w + l.z;
+        }
         if constexpr (WARM) {
-            double* rv0 = work + (size_t)n * stride + (size_t)p * nC;
-            pb.x0 = x0; pb.rv0_ = rv0;
-            for (int i = lane; i < nC; i += 32) rv0[i] = pb.rv[i];
+            double* rv0 = work + (size_t)n * stride + (size_t)p * nR;
+            if constexpr (BOUNDS) pb.rv0_ = rv0; else { pb.x0 = x0; pb.rv0_ = rv0; }
+            for (int i = lane; i < nR; i += 32) rv0[i] = pb.rv[i];
             __syncwarp();
         }
         // equalities first, in row order; never dropped (enableEqualities, qpOASES/Options.cpp:191-218)
-        for (int c = 0; c < nC; ++c) {
-            const double lo = lb[c], hi = ub[c];
+        for (int c = 0; c < nR; ++c) {
+            const double lo = BOUNDS ? pb.lo(c) : lb[c], hi = BOUNDS ? pb.hi(c) : ub[c];
             if (fabs(hi - lo) <= 1e-12 * fmax(1.0, fabs(lo))) {
                 const double val = pb.rv[c];
                 int rc = das_add_equality(pb, dw, xp, w + l.z, c, val, lo);
@@ -394,28 +480,30 @@ __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const
                     if (lane == 0) dw.state[c] = -1;
                 } else if (rc < 0) st |= ISMPC_ST_QP_FAIL;
                 __syncwarp();
+            } else if (BOUNDS && c < nV && lo > hi) {
+                st |= ISMPC_ST_QP_FAIL;                 // crossed bounds: the box is empty
             }
         }
         dw.neq = dw.q;
         int drops = 0;
         if constexpr (WARM) {
-            const signed char* gp = ws_guess + (size_t)p * nC;
+            const signed char* gp = ws_guess + (size_t)p * nR;
             drops = das_warm_install(pb, dw, xp, [&](int i) {
                 const int gs = gp[i];
                 if (gs == 0) return 0;
-                const double lo = lb[i], hi = ub[i];
+                const double lo = BOUNDS ? pb.lo(i) : lb[i], hi = BOUNDS ? pb.hi(i) : ub[i];
                 if (fabs(hi - lo) <= 1e-12 * fmax(1.0, fabs(lo))) return 0;          // equality rows: always active
                 if (fabs(gs < 0 ? lo : hi) >= 1e20) return 0;                         // infinite side (qpOASES INFTY)
                 return gs < 0 ? +1 : -1;
             });
         }
-        int rc = das_solve(pb, dw, xp, pb.rv, w + l.z, 20 * (nV + nC) + 50, &it);
+        int rc = das_solve(pb, dw, xp, pb.rv, w + l.z, 20 * (nV + nR) + 50, &it);
         it += drops;
         if (rc != 0) st |= ISMPC_ST_QP_FAIL;
-        if (y) for (int i = lane; i < nC; i += 32) y[(size_t)p * nC + i] = 0.0;
-        if (ws) for (int i = lane; i < nC; i += 32) ws[(size_t)p * nC + i] = dw.state[i];
+        if (y) for (int i = lane; i < nR; i += 32) y[(size_t)p * nR + i] = 0.0;
+        if (ws) for (int i = lane; i < nR; i += 32) ws[(size_t)p * nR + i] = dw.state[i];
         __syncwarp();
-        if (y) for (int k = lane; k < dw.q; k += 32) y[(size_t)p * nC + dw.wid[k]] = (double)dw.wsg[k] * dw.mu[k];
+        if (y) for (int k = lane; k < dw.q; k += 32) y[(size_t)p * nR + dw.wid[k]] = (double)dw.wsg[k] * dw.mu[k];
     }
     if (lane == 0) { status[p] = st; if (iters) iters[p] = it; }
 }
@@ -438,11 +526,13 @@ void dense_hinv_launch(int n, int nV, double* work, size_t stride, size_t offLin
     dense_hinv<<<gr, b, 0, st>>>(nV, work, stride, offLinv, offHinv);
 }
 
+// bounds = false: lbx / ubx unused (ismpc_qp_solve_batch[_ws]); true: the box rows ahead of A (ismpc_qp_solve_batch_bounds)
 int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, const double* A, const double* lbA,
-                    const double* ubA, const signed char* ws_guess, double* x, double* y, signed char* ws,
-                    int32_t* status, int32_t* iters, double* work, int use_dmma, cudaStream_t st)
+                    const double* ubA, bool bounds, const double* lbx, const double* ubx, const signed char* ws_guess,
+                    double* x, double* y, signed char* ws, int32_t* status, int32_t* iters, double* work, int use_dmma,
+                    cudaStream_t st)
 {
-    const DenseLayout l = dense_layout(nV, nC);
+    const DenseLayout l = dense_layout(nV, nC, true, bounds);
     const size_t stride = l.total;
     const size_t vv = (size_t)nV * nV;
     dense_copy_H<<<dim3((unsigned)((vv + 255) / 256), n), 256, 0, st>>>(nV, H, work, stride, l.Lh);
@@ -460,10 +550,11 @@ int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, con
     dense_x0_rv<<<n, 128, 0, st>>>(nV, nC, g, A, work, stride, l, x);
     const int R = l.qmax < DENSE_R ? l.qmax : DENSE_R;
     const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
-    auto kern = ws_guess ? dense_das_kernel<true, false> : dense_das_kernel<false, false>;
+    auto kern = bounds ? (ws_guess ? dense_das_kernel<true, false, true> : dense_das_kernel<false, false, true>)
+                       : (ws_guess ? dense_das_kernel<true, false, false> : dense_das_kernel<false, false, false>);
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
     kern<<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
-        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess, DenseSets{});
+        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess, DenseSets{}, lbx, ubx);
     return (int)cudaGetLastError();
 }
 
@@ -475,11 +566,11 @@ size_t qp_sets_table_doubles(int n_mat, int nV, int nC)
 }
 
 // set-up: 2 n_mat nV^2 (Lh | Linv, scratch); per call: n slices of vectors, x0 | A x0 (n x (nV + nC)), A x0 kept for the
-// warm start (n x nC)
-size_t qp_sets_work_doubles(int n, int n_mat, int nV, int nC)
+// warm start (n x nC; with bounds x0 | A x0, n x (nV + nC))
+size_t qp_sets_work_doubles(int n, int n_mat, int nV, int nC, bool bounds)
 {
     const size_t setup = 2 * (size_t)n_mat * nV * nV;
-    const size_t call = (dense_layout(nV, nC, false).total + nV + 2 * (size_t)nC) * n;
+    const size_t call = (dense_layout(nV, nC, false, bounds).total + nV + 2 * (size_t)nC + (bounds ? nV : 0)) * n;
     return (setup > call ? setup : call) + 16;
 }
 
@@ -502,31 +593,32 @@ int qp_sets_build(int n_mat, int nV, int nC, double* tab, int32_t* fstat, double
     return (int)cudaGetLastError();
 }
 
-// One call against the resident sets: the x0 step, then dense_das_kernel<WARM, true>.  A single shared set (n_mat = 1,
-// use_gemm) takes x0 | A x0 for the whole batch from one tensor-core product, [X0 | R0] (n x (nV + nC)) = -G [Hinv; D]';
+// One call against the resident sets: the x0 step, then dense_das_kernel<WARM, true, bounds>.  A single shared set (n_mat =
+// 1, use_gemm) takes x0 | A x0 for the whole batch from one tensor-core product, [X0 | R0] (n x (nV + nC)) = -G [Hinv; D]';
 // otherwise the per-problem mat-vecs of the seam.
 int qp_sets_launch(int n, int nV, int nC, int n_mat, const double* tab, const int32_t* fstat, const int32_t* idx,
-                   const double* g, const double* lbA, const double* ubA, const signed char* ws_guess, double* x,
-                   double* y, signed char* ws, int32_t* status, int32_t* iters, double* work, int use_gemm, int use_dmma,
-                   cudaStream_t st)
+                   const double* g, const double* lbA, const double* ubA, bool bounds, const double* lbx,
+                   const double* ubx, const signed char* ws_guess, double* x, double* y, signed char* ws, int32_t* status,
+                   int32_t* iters, double* work, int use_gemm, int use_dmma, cudaStream_t st)
 {
     const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV, cc = (size_t)nC * nC;
-    const DenseLayout l = dense_layout(nV, nC, false);
+    const DenseLayout l = dense_layout(nV, nC, false, bounds);
     const size_t stride = l.total;
     DenseSets sets;
     sets.HD = tab; sets.S = tab + (size_t)n_mat * (vv + cv); sets.A = sets.S + (size_t)n_mat * cc;
     sets.fstat = fstat; sets.idx = idx; sets.n_mat = n_mat;
-    sets.xr = work + (size_t)n * (stride + nC);
+    sets.xr = work + (size_t)n * (stride + nC + (bounds ? nV : 0));
     if (n_mat == 1 && use_gemm)
         dense_gemm_launch(use_dmma, 1, n, nV + nC, nV, g, 0, nV, 1, sets.HD, 0, nV, 1, sets.xr, 0, st, -1.0);
     else
         dense_x0_rv_sets<<<n, 128, 0, st>>>(n, nV, nC, g, sets);
     const int R = l.qmax < DENSE_R ? l.qmax : DENSE_R;
     const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
-    auto kern = ws_guess ? dense_das_kernel<true, true> : dense_das_kernel<false, true>;
+    auto kern = bounds ? (ws_guess ? dense_das_kernel<true, true, true> : dense_das_kernel<false, true, true>)
+                       : (ws_guess ? dense_das_kernel<true, true, false> : dense_das_kernel<false, true, false>);
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
     kern<<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
-        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess, sets);
+        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess, sets, lbx, ubx);
     return (int)cudaGetLastError();
 }
 

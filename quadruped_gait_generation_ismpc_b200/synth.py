@@ -333,3 +333,37 @@ def dense_qp_family(shape, n, n_mat=1, T=1, seed=SEED0 ^ 29):
         raise ValueError("unknown shape %r" % shape)
     g, lb, ub = _drift(Hs, As, idx, g0, lb0, ub0, T, rng)
     return Hs, As, idx, g, lb, ub
+
+
+def dense_split_bounds(H, g, A, lbA, ubA):
+    """The dense QP (H, g, A, lbA, ubA) with its bound rows moved into box bounds, the layout of
+    ismpc_qp_solve_batch_bounds: a row that is a positive multiple s e_j of a unit vector in every problem of the batch
+    becomes lb_j = lbA / s, ub_j = ubA / s (an absent side, |v| >= 1e20, stays as it is), at most one row per variable
+    (the first in row order); the other rows stay in A in their order.  "formc_horizontal": 101 rows -> 1 row + 100
+    bounds; "forma_stacked": the first kinematic row of each axis (and a ZMP row that carries a single variable) moves.
+    Returns a dict: H, g, A (n, nC', nV), lb / ub (n, nV; -1e20 / 1e20 where no row moved), lbA / ubA (n, nC'),
+    row_map (nC,) the index of each original row in the extended row space [bounds (nV) | rows of A (nC')], and
+    row_scale (n, nC) its s (1 for a row that stays): original row r is row_scale[:, r] times row row_map[r] of [I; A],
+    with bounds row_scale times [lb | lbA][row_map[r]], and its multiplier is y[:, row_map[r]] / row_scale[:, r]."""
+    A = np.asarray(A, dtype=np.float64); lbA = np.asarray(lbA, dtype=np.float64); ubA = np.asarray(ubA, dtype=np.float64)
+    n, (nC, nV) = lbA.shape[0], A.shape[1:]            # A may be one set (1, nC, nV) shared by the n problems
+    nz = A != 0
+    j = np.argmax(nz, axis=2)                                          # (n, nC): first nonzero column
+    s = np.take_along_axis(A, j[..., None], axis=2)[..., 0]
+    unit = (nz.sum(axis=2) == 1).all(axis=0) & (j == j[:1]).all(axis=0) & (s > 0).all(axis=0)
+    moved, used = {}, set()
+    for r in np.flatnonzero(unit):
+        v = int(j[0, r])
+        if v not in used:
+            used.add(v); moved[int(r)] = v
+    keep = [r for r in range(nC) if r not in moved]
+    lb = np.full((n, nV), -1e20); ub = np.full((n, nV), 1e20)
+    row_map = np.empty(nC, dtype=np.int64); row_scale = np.ones((n, nC))
+    for r, v in moved.items():
+        sr = s[:, r]
+        lb[:, v] = np.where(np.abs(lbA[:, r]) >= 1e20, lbA[:, r], lbA[:, r] / sr)
+        ub[:, v] = np.where(np.abs(ubA[:, r]) >= 1e20, ubA[:, r], ubA[:, r] / sr)
+        row_map[r] = v; row_scale[:, r] = sr
+    row_map[keep] = nV + np.arange(len(keep))
+    return dict(H=H, g=g, A=A[:, keep, :], lb=lb, ub=ub, lbA=lbA[:, keep], ubA=ubA[:, keep], row_map=row_map,
+                row_scale=row_scale)
