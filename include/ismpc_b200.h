@@ -548,6 +548,35 @@ int ismpc_qp_hotstart_batch_bounds(ismpc_handle* h, int n, const int32_t* mat_in
                                    double* x, double* y_opt, int8_t* ws_opt, int32_t* status, int32_t* iters_opt,
                                    int mem, void* stream);
 
+/* Gradients of the dense seam: the adjoint of ismpc_qp_solve_batch_bounds at its solution.  With the rows [I; A] (bounds
+ * first) and W the entries with ws != 0, the solution satisfies H x + g = A_W' y_W and A_W x = b_W (b the side ws reports).
+ * For an upstream gradient v = dL/dx the call returns (p, q) with
+ *     H p + A_W' q = v,   A_W p = 0,   q = 0 outside W,
+ * from which, for a loss L(x):  dL/dg = -p;  dL/db_i = q_i on the side ws reports (-1 lower, +1 upper; equality rows and
+ * fixed variables report -1), 0 on the other side and off W;  dL/dH = -(p x' + x p') / 2 (H read as symmetric);
+ * dL/dA = y_A p' - q_A x' (the row halves of y and q).
+ * Where strict complementarity fails (a row active with multiplier 0, or inactive with zero slack) the solution map has a
+ * kink; there this is the derivative for the working set the forward reported, one element of the generalized Jacobian
+ * (the convention of OptNet / qpth).
+ *   ws: the forward's ws_opt, n x (nV + nC) (the bounds layout only: a caller without a box calls the bounds calls with
+ *   lb = ub = NULL, which give the bytes of the calls without bounds).  Entries are installed in row order; an entry
+ *   linearly dependent on those before it, or beyond nV independent entries, is skipped and gets q = 0.  No bound is an
+ *   argument: ws holds everything the adjoint needs, since an infinite side never appears in it.
+ *   v: n x nV.  p: n x nV.  q: n x (nV + nC).  status: n int32, 0 or ISMPC_ST_QP_FAIL for a problem whose H is not
+ *   positive definite; such a problem's rows of p and q are left as they were.
+ *   mem: ISMPC_MEM_HOST or ISMPC_MEM_DEVICE. */
+int ismpc_qp_adjoint_batch(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* A,
+                           const int8_t* ws, const double* v, double* p, double* q, int32_t* status,
+                           int mem, void* stream);
+/* The same against the resident sets of ismpc_qp_set_matrices (the adjoint of ismpc_qp_hotstart_batch_bounds);
+ * mat_index_opt as in ismpc_qp_hotstart_batch.  A set index outside [0, n_mat), or a set whose H is not positive definite,
+ * flags that problem ISMPC_ST_QP_FAIL and leaves its rows of p and q as they were.  One set per problem gives the bytes of
+ * ismpc_qp_adjoint_batch; a single shared set with "dense_resident_gemm" = 1 takes H^-1 v from a tensor-core product (the
+ * same answers to rounding).  ISMPC_ERR_MODEL when no sets are resident. */
+int ismpc_qp_hotstart_adjoint_batch(ismpc_handle* h, int n, const int32_t* mat_index_opt,
+                                    const int8_t* ws, const double* v, double* p, double* q, int32_t* status,
+                                    int mem, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -23,7 +23,7 @@ EXPORTS = ["ismpc_version", "ismpc_error_string", "ismpc_create", "ismpc_destroy
            "ismpc_forma_rollout_ex2", "ismpc_kf_filter_batch_f64", "ismpc_formc_set_instances",
            "ismpc_formc_solve_batch_packed", "ismpc_qp_solve_batch_ws", "ismpc_qp_set_matrices",
            "ismpc_qp_hotstart_batch", "ismpc_forma_solve_batch_ws", "ismpc_qp_solve_batch_bounds",
-           "ismpc_qp_hotstart_batch_bounds"]
+           "ismpc_qp_hotstart_batch_bounds", "ismpc_qp_adjoint_batch", "ismpc_qp_hotstart_adjoint_batch"]
 
 _lib = None
 
@@ -98,6 +98,8 @@ def lib():
     L.ismpc_qp_hotstart_batch.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 10 + [C.c_int, C.c_void_p]
     L.ismpc_qp_solve_batch_bounds.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 13 + [C.c_int, C.c_void_p]
     L.ismpc_qp_hotstart_batch_bounds.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 12 + [C.c_int, C.c_void_p]
+    L.ismpc_qp_adjoint_batch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 7 + [C.c_int, C.c_void_p]
+    L.ismpc_qp_hotstart_adjoint_batch.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 6 + [C.c_int, C.c_void_p]
     L.ismpc_handle_stream.restype = C.c_void_p
     L.ismpc_handle_stream.argtypes = [C.c_void_p]
     L.ismpc_wait.argtypes = [C.c_void_p, C.c_void_p]
@@ -564,6 +566,50 @@ class Handle:
                                                     _ptr(ubA), _ptr(ws_guess), _ptr(x), _ptr(y), _ptr(ws), _ptr(status),
                                                     _ptr(iters), mem, C.c_void_p(stream) if stream else None)
         self._check(rc, "ismpc_qp_hotstart_batch_bounds")
+
+    # ---- gradients of the dense seam (the adjoint at a solution of the bounds calls) -----------------------------------
+    def qp_adjoint_batch_raw(self, n, nV, nC, H, A, ws, v, p, q, status, mem=abi.MEM_DEVICE, stream=None):
+        """Raw ismpc_qp_adjoint_batch: every array is a numpy array (host), an integer address (device) or None."""
+        rc = self._L.ismpc_qp_adjoint_batch(self._h, n, nV, nC, _ptr(H), _ptr(A), _ptr(ws), _ptr(v), _ptr(p), _ptr(q),
+                                            _ptr(status), mem, C.c_void_p(stream) if stream else None)
+        self._check(rc, "ismpc_qp_adjoint_batch")
+
+    def qp_hotstart_adjoint_batch_raw(self, n, ws, v, p, q, status, mat_index=None, mem=abi.MEM_DEVICE, stream=None):
+        """Raw ismpc_qp_hotstart_adjoint_batch: every array is a numpy array (host), an integer address (device) or None."""
+        rc = self._L.ismpc_qp_hotstart_adjoint_batch(self._h, n, _ptr(mat_index), _ptr(ws), _ptr(v), _ptr(p), _ptr(q),
+                                                     _ptr(status), mem, C.c_void_p(stream) if stream else None)
+        self._check(rc, "ismpc_qp_hotstart_adjoint_batch")
+
+    def qp_adjoint_batch(self, H, A, ws, v):
+        """ismpc_qp_adjoint_batch: (p, q) with H p + A_W' q = v, A_W p = 0 over the working set ws (n x (nV + nC), the
+        "ws" of qp_solve_batch with lb / ub).  A may be None when there are no rows.  Returns dict(p, q, status)."""
+        H = np.ascontiguousarray(H, dtype=np.float64); v = np.ascontiguousarray(v, dtype=np.float64)
+        n, nV = v.shape
+        A = None if A is None else np.ascontiguousarray(A, dtype=np.float64)
+        nC = 0 if A is None else A.shape[1]
+        return self._qp_adjoint(False, n, nV, nC, H, A, ws, v, None)
+
+    def qp_hotstart_adjoint_batch(self, ws, v, mat_index=None):
+        """ismpc_qp_hotstart_adjoint_batch: qp_adjoint_batch against the resident sets, problem p on set mat_index[p] as in
+        qp_hotstart_batch.  Returns dict(p, q, status)."""
+        v = np.ascontiguousarray(v, dtype=np.float64)
+        n, nV = v.shape
+        nC = np.shape(ws)[1] - nV
+        idx = None if mat_index is None else np.ascontiguousarray(mat_index, dtype=np.int32)
+        if idx is not None and idx.shape != (n,):
+            raise ValueError("mat_index must have %d entries, got %s" % (n, idx.shape))
+        return self._qp_adjoint(True, n, nV, nC, None, None, ws, v, idx)
+
+    def _qp_adjoint(self, resident, n, nV, nC, H, A, ws, v, idx):
+        ws = np.ascontiguousarray(ws, dtype=np.int8)
+        if ws.shape != (n, nV + nC):
+            raise ValueError("ws must be %d x %d, got %s" % (n, nV + nC, ws.shape))
+        p = np.zeros((n, nV)); q = np.zeros((n, nV + nC)); status = np.zeros(n, dtype=np.int32)
+        if resident:
+            self.qp_hotstart_adjoint_batch_raw(n, ws, v, p, q, status, mat_index=idx, mem=abi.MEM_HOST)
+        else:
+            self.qp_adjoint_batch_raw(n, nV, nC, H, A, ws, v, p, q, status, mem=abi.MEM_HOST)
+        return dict(p=p, q=q, status=status)
 
 
 # ---- all GPUs of one box behind one C ABI (include/ismpc_b200_multigpu.h, lib/libismpc_b200_mg.so) --------------------

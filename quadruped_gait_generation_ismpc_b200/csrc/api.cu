@@ -958,6 +958,62 @@ extern "C" int ismpc_qp_hotstart_batch_bounds(ismpc_handle* h, int n, const int3
                               mem, stream);
 }
 
+// The adjoints of the bounds calls: ws and q are n x (nV + nC).  p and q are staged with the caller's bytes, so that a
+// failed problem keeps its rows in both memory modes.
+extern "C" int ismpc_qp_adjoint_batch(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* A,
+                                      const int8_t* ws, const double* v, double* p, double* q, int32_t* status, int mem,
+                                      void* stream)
+{
+    if (!h) return ISMPC_ERR_ARG;
+    if (n < 0 || n > h->max_batch || nV < 1 || nV > ISMPC_MAX_N || nC < 0 || nC > 2 * ISMPC_MAX_N + 8 || !H ||
+        (nC > 0 && !A) || !ws || !v || !p || !q || !status || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
+        return ISMPC_ERR_ARG;
+    if (n == 0) return ISMPC_OK;
+    CK(cudaSetDevice(h->device));
+    if (h->q_work.ensure(qp_dense_adjoint_work_doubles(n, nV, nC) * sizeof(double))) return ISMPC_ERR_ALLOC;
+    Staged s(h, mem, stream, false);
+    const size_t szg = (size_t)n * nV, szr = (size_t)n * (nV + nC);
+    double* dp = s.inout(p, szg);
+    double* dq = s.inout(q, szr);
+    int32_t* dst = s.out(status, n);
+    const double* dH = s.in(H, szg * nV);
+    const double* dA = s.in(A, (size_t)n * nC * nV);
+    const int8_t* dws = s.in(ws, szr);
+    const double* dv = s.in(v, szg);
+    if (s.err) return s.err;
+    return s.finish(qp_dense_adjoint_launch(n, nV, nC, dH, dA, (const signed char*)dws, dv, dp, dq, dst, (double*)h->q_work.p,
+                                            h->opt_dense_dmma, s.st),
+                    "qp_dense_adjoint_launch");
+}
+
+extern "C" int ismpc_qp_hotstart_adjoint_batch(ismpc_handle* h, int n, const int32_t* mat_index_opt, const int8_t* ws,
+                                               const double* v, double* p, double* q, int32_t* status, int mem,
+                                               void* stream)
+{
+    if (!h) return ISMPC_ERR_ARG;
+    if (n < 0 || n > h->max_batch || !ws || !v || !p || !q || !status || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
+        return ISMPC_ERR_ARG;
+    if (h->r_nmat == 0) return ISMPC_ERR_MODEL;
+    const int nV = h->r_nV, nC = h->r_nC, n_mat = h->r_nmat;
+    if (!mat_index_opt && n_mat > 1 && n > n_mat) return ISMPC_ERR_ARG;
+    if (n == 0) return ISMPC_OK;
+    CK(cudaSetDevice(h->device));
+    if (h->r_work.ensure(qp_sets_work_doubles(n, n_mat, nV, nC, true) * sizeof(double))) return ISMPC_ERR_ALLOC;
+    Staged s(h, mem, stream, false);
+    const size_t szg = (size_t)n * nV, szr = (size_t)n * (nV + nC);
+    double* dp = s.inout(p, szg);
+    double* dq = s.inout(q, szr);
+    int32_t* dst = s.out(status, n);
+    const int32_t* didx = s.in(mat_index_opt, n);
+    const int8_t* dws = s.in(ws, szr);
+    const double* dv = s.in(v, szg);
+    if (s.err) return s.err;
+    return s.finish(qp_sets_adjoint_launch(n, nV, nC, n_mat, (const double*)h->r_tab.p, (const int32_t*)h->r_stat.p, didx,
+                                           (const signed char*)dws, dv, dp, dq, dst, (double*)h->r_work.p,
+                                           h->opt_dense_resident_gemm, h->opt_dense_dmma, s.st),
+                    "qp_sets_adjoint_launch");
+}
+
 // ---------------------------------------------------------------------------------------------------
 // FP64 peak micro-benchmark (roofline denominator)
 // ---------------------------------------------------------------------------------------------------

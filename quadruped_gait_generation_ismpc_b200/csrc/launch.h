@@ -59,5 +59,13 @@ int qp_sets_launch(int n, int nV, int nC, int n_mat, const double* tab, const in
                    const double* g, const double* lbA, const double* ubA, bool bounds, const double* lbx,
                    const double* ubx, const signed char* ws_guess, double* x, double* y, signed char* ws, int32_t* status,
                    int32_t* iters, double* work, int use_gemm, int use_dmma, cudaStream_t st);
+// the adjoint of the bounds calls at their solution (ismpc_qp_adjoint_batch / ismpc_qp_hotstart_adjoint_batch); the
+// resident call's workspace is qp_sets_work_doubles(n, n_mat, nV, nC, true)
+size_t qp_dense_adjoint_work_doubles(int n, int nV, int nC);
+int qp_dense_adjoint_launch(int n, int nV, int nC, const double* H, const double* A, const signed char* ws, const double* v,
+                            double* p, double* q, int32_t* status, double* work, int use_dmma, cudaStream_t st);
+int qp_sets_adjoint_launch(int n, int nV, int nC, int n_mat, const double* tab, const int32_t* fstat, const int32_t* idx,
+                           const signed char* ws, const double* v, double* p, double* q, int32_t* status, double* work,
+                           int use_gemm, int use_dmma, cudaStream_t st);
 
 }  // namespace ismpc

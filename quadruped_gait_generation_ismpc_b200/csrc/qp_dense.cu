@@ -105,7 +105,7 @@ __global__ void dense_tri_inverse(int N, double* work, size_t stride, size_t off
 // read of Linv.  CTA = 4 warps, 64 x 64 tile of C, each warp 32 x 32 = 4 x 4 DMMA tiles (32 accumulators per thread);
 // K in chunks of 16 through shared memory, rows padded to 20 doubles so that the 8 x 4 / 4 x 8 fragment loads of a
 // half-warp fall into 16 distinct 8-byte banks.  C is stored as alpha times the sum: the set-up products pass 1 (exact),
-// the resident path's x0 step (qp_resident_launch) passes -1.
+// the resident path's x0 step (qp_resident_launch) passes -1, its adjoint's p0 step (qp_sets_adjoint_launch) +1.
 constexpr int DG_T = 64, DG_KC = 16, DG_LD = 20;
 
 __device__ __forceinline__ void dmma_m8n8k4(double& d0, double& d1, double a, double b)
@@ -526,13 +526,10 @@ void dense_hinv_launch(int n, int nV, double* work, size_t stride, size_t offLin
     dense_hinv<<<gr, b, 0, st>>>(nV, work, stride, offLinv, offHinv);
 }
 
-// bounds = false: lbx / ubx unused (ismpc_qp_solve_batch[_ws]); true: the box rows ahead of A (ismpc_qp_solve_batch_bounds)
-int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, const double* A, const double* lbA,
-                    const double* ubA, bool bounds, const double* lbx, const double* ubx, const signed char* ws_guess,
-                    double* x, double* y, signed char* ws, int32_t* status, int32_t* iters, double* work, int use_dmma,
-                    cudaStream_t st)
+// The seam's per-call set-up: factor H, Hinv, D and S into each problem's slice (layout l), the factor status into status.
+static void dense_setup_launch(int n, int nV, int nC, const double* H, const double* A, const DenseLayout& l, double* work,
+                               int32_t* status, int use_dmma, cudaStream_t st)
 {
-    const DenseLayout l = dense_layout(nV, nC, true, bounds);
     const size_t stride = l.total;
     const size_t vv = (size_t)nV * nV;
     dense_copy_H<<<dim3((unsigned)((vv + 255) / 256), n), 256, 0, st>>>(nV, H, work, stride, l.Lh);
@@ -547,6 +544,17 @@ int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, con
         // S (nC x nC) = A * D'
         dense_gemm_launch(use_dmma, n, nC, nC, nV, A, (size_t)nC * nV, nV, 1, work + l.D, stride, nV, 1, work + l.S, stride, st);
     }
+}
+
+// bounds = false: lbx / ubx unused (ismpc_qp_solve_batch[_ws]); true: the box rows ahead of A (ismpc_qp_solve_batch_bounds)
+int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, const double* A, const double* lbA,
+                    const double* ubA, bool bounds, const double* lbx, const double* ubx, const signed char* ws_guess,
+                    double* x, double* y, signed char* ws, int32_t* status, int32_t* iters, double* work, int use_dmma,
+                    cudaStream_t st)
+{
+    const DenseLayout l = dense_layout(nV, nC, true, bounds);
+    const size_t stride = l.total;
+    dense_setup_launch(n, nV, nC, H, A, l, work, status, use_dmma, st);
     dense_x0_rv<<<n, 128, 0, st>>>(nV, nC, g, A, work, stride, l, x);
     const int R = l.qmax < DENSE_R ? l.qmax : DENSE_R;
     const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
@@ -593,6 +601,17 @@ int qp_sets_build(int n_mat, int nV, int nC, double* tab, int32_t* fstat, double
     return (int)cudaGetLastError();
 }
 
+// The resident tables (tab: [Hinv; D] of every set, then S, then A) as the kernels read them; xr: n x (nV + nC)
+static DenseSets dense_sets(int n_mat, int nV, int nC, const double* tab, const int32_t* fstat, const int32_t* idx, double* xr)
+{
+    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV, cc = (size_t)nC * nC;
+    DenseSets sets;
+    sets.HD = tab; sets.S = tab + (size_t)n_mat * (vv + cv); sets.A = sets.S + (size_t)n_mat * cc;
+    sets.fstat = fstat; sets.idx = idx; sets.n_mat = n_mat;
+    sets.xr = xr;
+    return sets;
+}
+
 // One call against the resident sets: the x0 step, then dense_das_kernel<WARM, true, bounds>.  A single shared set (n_mat =
 // 1, use_gemm) takes x0 | A x0 for the whole batch from one tensor-core product, [X0 | R0] (n x (nV + nC)) = -G [Hinv; D]';
 // otherwise the per-problem mat-vecs of the seam.
@@ -601,13 +620,9 @@ int qp_sets_launch(int n, int nV, int nC, int n_mat, const double* tab, const in
                    const double* ubx, const signed char* ws_guess, double* x, double* y, signed char* ws, int32_t* status,
                    int32_t* iters, double* work, int use_gemm, int use_dmma, cudaStream_t st)
 {
-    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV, cc = (size_t)nC * nC;
     const DenseLayout l = dense_layout(nV, nC, false, bounds);
     const size_t stride = l.total;
-    DenseSets sets;
-    sets.HD = tab; sets.S = tab + (size_t)n_mat * (vv + cv); sets.A = sets.S + (size_t)n_mat * cc;
-    sets.fstat = fstat; sets.idx = idx; sets.n_mat = n_mat;
-    sets.xr = work + (size_t)n * (stride + nC + (bounds ? nV : 0));
+    const DenseSets sets = dense_sets(n_mat, nV, nC, tab, fstat, idx, work + (size_t)n * (stride + nC + (bounds ? nV : 0)));
     if (n_mat == 1 && use_gemm)
         dense_gemm_launch(use_dmma, 1, n, nV + nC, nV, g, 0, nV, 1, sets.HD, 0, nV, 1, sets.xr, 0, st, -1.0);
     else
@@ -620,6 +635,172 @@ int qp_sets_launch(int n, int nV, int nC, int n_mat, const double* tab, const in
     kern<<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
         n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess, sets, lbx, ubx);
     return (int)cudaGetLastError();
+}
+
+// ---- the adjoint of the bounds calls (ismpc_qp_adjoint_batch / ismpc_qp_hotstart_adjoint_batch) --------------------
+// For v = dL/dx at a solution with working set W (rows [I; A], the ws of the forward), (p, q) solves
+//     H p + A_W' q = v,   A_W p = 0,   q = 0 outside W.
+// In the engine's terms this is the warm start's install with g := -v and every right-hand side zero: p0 = Hinv v and
+// r0 = A p0 (the forward's x0 | A x0), every ws entry installed factor-only, mu = J'J (0 - N_W' p0), no drops, then
+// p = p0 + sum_k mu_k sg_k Hinv a_k and q_{id_k} = -sg_k mu_k.
+
+// [p0 | r0] = [Hinv v | A Hinv v], one CTA per problem: the loops of dense_x0_rv / dense_x0_rv_sets in the same order, so
+// that the seam and one set per problem give the same bytes.  SETS = false: Hinv from the problem's slice, A the caller's.
+// A problem whose set index is out of range is skipped here and flagged by dense_adjoint_kernel.
+template <bool SETS>
+__global__ void dense_adjoint_p0(int nV, int nC, const double* v, const double* A, const double* work, size_t stride,
+                                 DenseLayout l, DenseSets sets, double* pr, size_t spr)
+{
+    const size_t p = blockIdx.x;
+    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
+    const double *Hinv, *Ap;
+    if constexpr (SETS) {
+        const int m = sets.set_of((int)p);
+        if (m < 0 || m >= sets.n_mat) return;
+        Hinv = sets.HD + (size_t)m * (vv + cv);
+        Ap = sets.A + (size_t)m * cv;
+    } else {
+        Hinv = work + p * stride + l.Hinv;
+        Ap = A + p * cv;
+    }
+    const double* vp = v + p * nV;
+    double* p0 = pr + p * spr;
+    for (int i = threadIdx.x; i < nV; i += blockDim.x) {
+        double s = 0.0;
+        for (int j = 0; j < nV; ++j) s += Hinv[(size_t)j * nV + i] * vp[j];
+        p0[i] = s;
+    }
+    __syncthreads();
+    for (int c = threadIdx.x; c < nC; c += blockDim.x) {
+        double s = 0.0;
+        for (int j = 0; j < nV; ++j) s += Ap[(size_t)c * nV + j] * p0[j];
+        p0[nV + c] = s;
+    }
+}
+
+// One warp per problem, DENSE_WARPS per CTA; the first R rows of J in shared memory, the rest in the slice (layout l, the
+// bounds layout of dense_das_kernel).  pr: [p0 | r0] of problem p at pr + p * spr.  SETS as in dense_das_kernel: a
+// problem whose set index is out of range, or whose set (or, on the seam, H) is not positive definite, is flagged
+// ISMPC_ST_QP_FAIL and nothing else of it is written.
+template <bool SETS>
+__global__ void dense_adjoint_kernel(int n, int nV, int nC, double* work, size_t stride, DenseLayout l, int R,
+                                     const signed char* ws, const double* pr, size_t spr, double* pout, double* qout,
+                                     int32_t* status, DenseSets sets)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int p = blockIdx.x * DENSE_WARPS + warp_id();
+    if (p >= n) return;
+    const int lane = lane_id();
+    double* w = work + (size_t)p * stride;
+    DasWork dw;
+    dw.Js = reinterpret_cast<double*>(smem_raw) + (size_t)warp_id() * tri(R, 0);
+    dw.Jg = w + l.Lw; dw.R = R;
+    dw.mu = w + l.mu; dw.r = w + l.r; dw.y = w + l.y;
+    dw.wid = reinterpret_cast<int*>(w + l.ints);
+    dw.wsg = reinterpret_cast<signed char*>(dw.wid + l.qmax);
+    dw.state = dw.wsg + l.qmax;
+    dw.q = 0; dw.neq = 0; dw.qmax = l.qmax;
+    const double *HD, *S;
+    int st;
+    if constexpr (SETS) {
+        const int m = sets.set_of(p);
+        if (m < 0 || m >= sets.n_mat) {
+            if (lane == 0) status[p] = ISMPC_ST_QP_FAIL;
+            return;
+        }
+        const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
+        HD = sets.HD + (size_t)m * (vv + cv);
+        S = sets.S + (size_t)m * nC * nC;
+        st = sets.fstat[m];
+    } else {
+        HD = w + l.Hinv;
+        S = w + l.S;
+        st = status[p];
+    }
+    if (st != 0) {
+        if (lane == 0) status[p] = ISMPC_ST_QP_FAIL;
+        return;
+    }
+    const int nR = nV + nC;
+    for (int i = lane; i < nR; i += 32) dw.state[i] = 0;
+    __syncwarp();
+    const DenseProb pb0{nV, nC, HD + (size_t)nV * nV, S, nullptr, nullptr, nullptr, nullptr};
+    DenseBoundsProb pb{pb0};
+    pb.HD = HD;
+    // every entry of ws in row order, factor only; dependent entries and entries beyond nV / qmax are skipped
+    const signed char* wp = ws + (size_t)p * nR;
+    for (int base = 0; base < nR; base += 32) {
+        const int i = base + lane;
+        const int s = i < nR ? wp[i] : 0;
+        unsigned cand = __ballot_sync(ISMPC_FULL_MASK, s != 0);
+        while (cand) {
+            const int b = __ffs(cand) - 1;
+            cand &= cand - 1;
+            const int sgp = __shfl_sync(ISMPC_FULL_MASK, s, b) < 0 ? +1 : -1;
+            if (dw.q >= nV || dw.q >= dw.qmax) break;
+            das_factor_append(pb, dw, base + b, sgp);
+        }
+    }
+    // mu = J'J (0 - N_W' p0): row id of [I; A] at p0 is element id of [p0 | r0]
+    const double* p0 = pr + (size_t)p * spr;
+    for (int k = lane; k < dw.q; k += 32) dw.y[k] = -(double)dw.wsg[k] * p0[dw.wid[k]];
+    __syncwarp();
+    das_apply_J(dw);
+    das_apply_Jt(dw);                           // dw.r = mu
+    double* pp = pout + (size_t)p * nV;
+    for (int i = lane; i < nV; i += 32) {
+        double acc = p0[i];
+        for (int k = 0; k < dw.q; ++k) acc += (double)dw.wsg[k] * dw.r[k] * HD[(size_t)dw.wid[k] * nV + i];
+        pp[i] = acc;
+    }
+    double* qp = qout + (size_t)p * nR;
+    for (int i = lane; i < nR; i += 32) qp[i] = 0.0;
+    __syncwarp();
+    for (int k = lane; k < dw.q; k += 32) qp[dw.wid[k]] = -(double)dw.wsg[k] * dw.r[k];
+    if (lane == 0) status[p] = 0;
+}
+
+template <bool SETS>
+static int dense_adjoint_run(int n, int nV, int nC, double* work, const DenseLayout& l, const signed char* ws,
+                             const double* pr, size_t spr, double* p, double* q, int32_t* status, const DenseSets& sets,
+                             cudaStream_t st)
+{
+    const int R = l.qmax < DENSE_R ? l.qmax : DENSE_R;
+    const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
+    cudaFuncSetAttribute(dense_adjoint_kernel<SETS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
+    dense_adjoint_kernel<SETS><<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
+        n, nV, nC, work, l.total, l, R, ws, pr, spr, p, q, status, sets);
+    return (int)cudaGetLastError();
+}
+
+// The seam: set-up as qp_dense_launch (status = the factor status), [p0 | r0] in the slice's x0 | rv.
+size_t qp_dense_adjoint_work_doubles(int n, int nV, int nC)
+{
+    return dense_layout(nV, nC, true, true).total * (size_t)n + 16;
+}
+
+int qp_dense_adjoint_launch(int n, int nV, int nC, const double* H, const double* A, const signed char* ws, const double* v,
+                            double* p, double* q, int32_t* status, double* work, int use_dmma, cudaStream_t st)
+{
+    const DenseLayout l = dense_layout(nV, nC, true, true);
+    dense_setup_launch(n, nV, nC, H, A, l, work, status, use_dmma, st);
+    dense_adjoint_p0<false><<<n, 128, 0, st>>>(nV, nC, v, A, work, l.total, l, DenseSets{}, work + l.x0, l.total);
+    return dense_adjoint_run<false>(n, nV, nC, work, l, ws, work + l.x0, l.total, p, q, status, DenseSets{}, st);
+}
+
+// Against the resident sets (workspace qp_sets_work_doubles(n, n_mat, nV, nC, true)): [p0 | r0] where the forward keeps
+// x0 | A x0; a single shared set (use_gemm) takes it for the whole batch from one tensor-core product, V [Hinv; D]'.
+int qp_sets_adjoint_launch(int n, int nV, int nC, int n_mat, const double* tab, const int32_t* fstat, const int32_t* idx,
+                           const signed char* ws, const double* v, double* p, double* q, int32_t* status, double* work,
+                           int use_gemm, int use_dmma, cudaStream_t st)
+{
+    const DenseLayout l = dense_layout(nV, nC, false, true);
+    const DenseSets sets = dense_sets(n_mat, nV, nC, tab, fstat, idx, work + (size_t)n * (l.total + nC + nV));
+    if (n_mat == 1 && use_gemm)
+        dense_gemm_launch(use_dmma, 1, n, nV + nC, nV, v, 0, nV, 1, sets.HD, 0, nV, 1, sets.xr, 0, st);
+    else
+        dense_adjoint_p0<true><<<n, 128, 0, st>>>(nV, nC, v, nullptr, nullptr, 0, l, sets, sets.xr, nV + nC);
+    return dense_adjoint_run<true>(n, nV, nC, work, l, ws, sets.xr, nV + nC, p, q, status, sets, st);
 }
 
 }  // namespace ismpc
