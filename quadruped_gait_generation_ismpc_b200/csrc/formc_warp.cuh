@@ -102,9 +102,14 @@ __host__ __device__ inline int formc_warp_epl(int N) { return (N + 31) >> 5; }
 // Feedback-law table of one pattern: FORMC_LAW_W component vectors in the kernel's shared-memory layout
 // [component][e*32 + lane] (sample i = lane*E + e; zero padding), so that ONE bulk copy (TMA) stages a pattern.
 __host__ __device__ inline size_t formc_law_pattern_doubles(int N) { return (size_t)FORMC_LAW_W * formc_warp_epl(N) * 32; }
+// Shared memory of a CTA of the warp kernels: the vectors, the mbarrier and ONE 128-byte record staging area (the packed
+// input record, then the result record).  At N = 100 that is 11 408 bytes: 16 resident CTAs, with the 1 KB the system
+// reserves for each, fit the SM's 196 KB shared-memory configuration (a second staging area made it 200 960 bytes, one
+// configuration step up, with 32 KB less L1 for the 128-register build's spills and the plan rows): 5.13 -> 4.91 us per
+// streamed 1,024-instance tick on a B200.
 __host__ __device__ inline size_t formc_warp_smem_bytes(int N)
 {
-    return (size_t)FORMC_WARP_VECS * formc_warp_epl(N) * 32 * sizeof(double) + 16 + 128 + 128;   // + mbarrier + staging of the result record (store_record_warp) + of the packed input record (load_tick_record)
+    return (size_t)FORMC_WARP_VECS * formc_warp_epl(N) * 32 * sizeof(double) + 16 + 128;
 }
 
 struct FormCWarpShared {     // [e*32 + lane] each
@@ -476,6 +481,7 @@ __device__ __forceinline__ void formc_tick_warp(const FormCWarpShared& sm, const
     double viol = 0.0;
     bool bad = false;
     if (staged) { mbar_wait(sm.bar, bar_parity); bar_parity ^= 1u; }
+    ISMPC_WPHASE(14);
     const bool use_law = __all_sync(ISMPC_FULL_MASK, flat && law != nullptr);
     if (use_law) formc_law_apply(sm, N, E, lane, rq0, z0, zd0, dt, g, mdl.fz_max, bad, viol);
     else {

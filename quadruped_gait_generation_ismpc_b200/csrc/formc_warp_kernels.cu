@@ -152,6 +152,9 @@ formc_tick_warp_kernel(FormCWarpArgs wa)
     const FormCArgs& a = wa.base;
     const int lane = threadIdx.x;
     const int N = a.model.N;
+#ifdef ISMPC_PHASE_TIMING
+    long long wt_ = clock64();
+#endif
     FormCWarpShared sm;
     formc_warp_carve(smem_d, formc_warp_epl(N), sm);
     pdl_launch_dependents();
@@ -162,20 +165,36 @@ formc_tick_warp_kernel(FormCWarpArgs wa)
 #ifdef ISMPC_PHASE_TIMING
     if (lane == 0 && blockIdx.x < 8192) { g_trace[3 * blockIdx.x] = dbg_globaltimer(); g_trace[3 * blockIdx.x + 2] = dbg_smid(); }
 #endif
-    double* stg_out = smem_d + (FORMC_WARP_VECS * formc_warp_epl(N) * 32 + 2);
-    double* stg_in = stg_out + 16;
+    // one 128-byte staging area serves the packed input record (taken into registers right away) and, at the end of the
+    // tick, the result record
+    double* stg = smem_d + (FORMC_WARP_VECS * formc_warp_epl(N) * 32 + 2);
+#ifdef ISMPC_PHASE_TIMING
+    ISMPC_WPHASE(12);
+#endif
     for (int inst = blockIdx.x; inst < a.n; inst += gridDim.x) {
         ismpc_state_t st; ismpc_walk_t wk;
-        if constexpr (PACKED) load_tick_record_issue(a.tick, inst, stg_in, lane);
+        if constexpr (PACKED) load_tick_record_issue(a.tick, inst, stg, lane);
         else { st = a.state[inst]; wk = a.walk[inst]; }
         const ismpc_formc_inst_t in = formc_checked_inst(a.inst[inst], a.plan_rows);
-        if constexpr (PACKED) { __syncwarp(); load_tick_record_take(stg_in, st, wk); __syncwarp(); }
+        if constexpr (PACKED) { __syncwarp(); load_tick_record_take(stg, st, wk); __syncwarp(); }
+#ifdef ISMPC_PHASE_TIMING
+        // phases 12 set-up, 13 records, 15 result store (14: law table, formc_tick_warp).  The store consumes the loaded
+        // records, so the clock read after it waits for their arrival (a load alone does not stall the warp).
+        if (lane == 0) reinterpret_cast<volatile double*>(stg)[0] = st.com_pos[2] + wk.sim_time + in.com_height;
+        ISMPC_WPHASE(13);
+#endif
         ismpc_formc_out_t r;
         formc_tick_warp(sm, a.model, a.T, wa.R, st, wk, in, a.plan, ws, r,
                         a.primal ? a.primal + (size_t)inst * 3 * N : nullptr,
                         a.active ? a.active + (size_t)inst * 3 * N : nullptr, parity);
-        if constexpr (PACKED) store_record_warp(a.out + inst, r, stg_out, lane, 0);
+#ifdef ISMPC_PHASE_TIMING
+        wt_ = clock64();
+#endif
+        if constexpr (PACKED) store_record_warp(a.out + inst, r, stg, lane, 0);
         else if (lane == 0) store_record(a.out + inst, r);
+#ifdef ISMPC_PHASE_TIMING
+        ISMPC_WPHASE(15);
+#endif
     }
 #ifdef ISMPC_PHASE_TIMING
     if (lane == 0 && blockIdx.x < 8192) g_trace[3 * blockIdx.x + 1] = dbg_globaltimer();

@@ -1,5 +1,6 @@
 """A/B of two builds of the library on the same box: the 1,024-instance form-C tick as a 20-node CUDA graph (strictly ordered,
-and as programmatic dependents), L2 flushed before every replay.  usage: python tools/ab_tick.py libA.so [libB.so ...]"""
+and as programmatic dependents), L2 flushed before every replay.  usage: python tools/ab_tick.py libA.so [libB.so ...]
+ISMPC_AB_N sets the instances per tick (default 1,024)."""
 import os
 import statistics
 import subprocess
@@ -17,7 +18,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from quadruped_gait_generation_ismpc_b200 import abi, binding, synth  # noqa: E402
 
 binding.LIB_PATH = os.path.abspath(sys.argv[1])
-n, K = 1024, 20
+n, K = int(os.environ.get("ISMPC_AB_N", "1024")), 20
 dev = torch.device("cuda", 0)
 h = binding.Handle(0, max_batch=n)
 h.formc_set_model(abi.formc_model()); h.formc_prepare_gait(35, 10)

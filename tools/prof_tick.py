@@ -51,19 +51,28 @@ if which == "formc":
         h.set_option("formc_variant", int(os.environ["ISMPC_VARIANT"]))
     if not os.environ.get("ISMPC_NO_GAIT"):
         h.formc_prepare_gait(35, 10)
-    st, wk, ins, pl = synth.formc_batch(n)
-    d = [to_dev(x) for x in (st, wk, ins, pl)]
+    if os.environ.get("ISMPC_PDL"):
+        h.set_option("formc_pdl", int(os.environ["ISMPC_PDL"]))
+    # ISMPC_SLOTS > 1: the launches of a burst read distinct batches and the L2 is flushed before every burst (records
+    # come from HBM, as in bench.py); default: one batch, L2-warm
+    n_slots = int(os.environ.get("ISMPC_SLOTS", "1"))
+    batches = [synth.formc_batch(n, seed=synth.SEED0 + s) for s in range(min(n_slots, 8))]
+    slots = [[to_dev(x) for x in batches[s % len(batches)]] + [batches[s % len(batches)][3].shape[0]] for s in range(n_slots)]
     out = torch.zeros(n * abi.FORMC_OUT.itemsize, dtype=torch.uint8, device=dev)
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev) if n_slots > 1 else None
     for r in range(reps):
         if os.environ.get("ISMPC_DBG") and r == reps - 1:
-            binding.lib().ismpc_debug_reset_phases()
+            torch.cuda.synchronize(); binding.lib().ismpc_debug_reset_phases()
         burst = int(os.environ.get("ISMPC_BURST", "20"))     # launches between the events: hides the host-side launch cost
+        if flush is not None:
+            flush.fill_(r & 0x7f)
         e0.record()
-        for _ in range(burst):
-            h.formc_solve_batch_raw(n, d[0].data_ptr(), d[1].data_ptr(), d[2].data_ptr(), d[3].data_ptr(), pl.shape[0],
+        for b in range(burst):
+            d = slots[(r * burst + b) % n_slots]
+            h.formc_solve_batch_raw(n, d[0].data_ptr(), d[1].data_ptr(), d[2].data_ptr(), d[3].data_ptr(), d[4],
                                     out.data_ptr(), stream=torch.cuda.current_stream().cuda_stream)
         e1.record(); e1.synchronize()
-        print("formc tick n=%d: %.1f us per launch (%d back-to-back)" % (n, e0.elapsed_time(e1) * 1e3 / burst, burst))
+        print("formc tick n=%d: %.2f us per launch (%d back-to-back)" % (n, e0.elapsed_time(e1) * 1e3 / burst, burst))
 else:
     h.forma_set_model(abi.forma_model())
     inst, ft, plan = synth.forma_batch(n, gait="trot")
@@ -98,9 +107,12 @@ if os.environ.get("ISMPC_DBG"):
     v = list(ph)[:24]
     if which == "formc":
         names = ["midpoints", "riccati", "rows+general", "lambda", "stab_row", "knapsack", "integrate"]
-        tot = float(sum(v[:7])) or 1.0
-        print("warp kernel, last launch: mean cycles per instance and phase (n=%d)" % n)
-        for nm, a in zip(names, v[:7]):
+        # warp tick kernel: CTA set-up (entry -> first record request issued), records (request -> usable), law table
+        # (mbar_wait, inside 'riccati' before), result record store
+        knames = [(12, "cta_setup"), (13, "records"), (14, "law_wait"), (15, "store")]
+        tot = float(sum(v[:7]) + sum(v[k] for k, _ in knames)) or 1.0
+        print("warp kernel, last burst: mean cycles per instance and phase (n=%d)" % n)
+        for nm, a in list(zip(names, v[:7])) + [(nm, v[k]) for k, nm in knames]:
             print("  %-12s %9.0f  %5.1f%%" % (nm, a / (n * burst), 100.0 * a / tot))
         print("  total %.0f cycles/instance; newton fallbacks %d, in-warp riccati %d, general vertical %d"
               % (tot / (n * burst), ph[29], ph[30], ph[31]))
@@ -110,9 +122,12 @@ if os.environ.get("ISMPC_DBG"):
         tr = (C.c_longlong * (3 * m))()
         binding.lib().ismpc_debug_read_trace(tr, 3 * m)
         tr = np.array(list(tr)).reshape(m, 3)
+        tr = tr[:int(np.count_nonzero(tr[:, 1]))]          # the CTAs of the grid (fewer than n when a CTA takes several instances)
+        m = len(tr)
         t0 = tr[:, 0].min()
         st_, en_ = tr[:, 0] - t0, tr[:, 1] - t0
         du = en_ - st_
+        print("  %d CTAs, %.2f instances per CTA" % (m, n / m))
         print("  CTA trace of the last launch (ns): start p50 %d p90 %d max %d | duration p50 %d p90 %d p99 %d max %d | end max %d"
               % (np.percentile(st_, 50), np.percentile(st_, 90), st_.max(), np.percentile(du, 50), np.percentile(du, 90),
                  np.percentile(du, 99), du.max(), en_.max()))
