@@ -342,6 +342,46 @@ int ismpc_forma_solve_batch_ws(ismpc_handle* h, int n, const ismpc_forma_inst_t*
                                ismpc_forma_out_t* out, double* primal_opt, int8_t* active_opt,
                                int mem, void* stream);
 
+/* Gradients of one form-A tick with respect to the inputs of its record and the footstep plan: the adjoint of
+ * ismpc_forma_solve_batch[_ws] at its solution.  Per instance and axis, with variables v = [zd(C); xf(F)], W = the
+ * stability row plus the rows the forward reports active, and the upstream gradients u = dL/d(next state of the axis) and
+ * w = dL/dv, the call solves
+ *     H p + A_W' q = w + e_0 B_u(eta)' u,   A_W p = 0,   q = 0 outside W
+ * (the adjoint of ismpc_qp_adjoint_batch on the form-A rows) and applies the chain rule through the QP's build: the cost
+ * targets g_f = -Q_foot plan(fs_counter + 1 + f) (clamped to n_fs as the build does), the stability row's right-hand side
+ * x + xd/eta - xz - ant (state, fs_store and the plan rows the centerline samples of the anticipative tail interpolate,
+ * cl(P) at the absolute index P included), the ZMP bounds -xz -+ w/2 + m_i0 cur_fs, the first kinematic row's bounds
+ * (cur_fs), the state update s+ = A_u s + B_u zd_0, and eta = sqrt(g_eta / height) wherever it enters (stability row
+ * coefficients, right-hand side, A_u, B_u).  The stability row's multiplier, which the forward does not return, is recovered
+ * from the same factor.
+ *   primal, active: the forward's primal_opt / active_opt for these records (n x 2(C+F); active: < 0 lower, > 0 upper).
+ *   Working-set entries are installed in row order (stability row, ZMP rows, kinematic rows); an entry linearly dependent
+ *   on those before it, or beyond C + F independent entries, is skipped and gets q = 0.  Where strict complementarity
+ *   fails the result is the derivative for the working set the forward reported (see ismpc_qp_adjoint_batch).
+ *   v_st (nullable): n x 6, dL/d out.st.  v_primal (nullable): n x 2(C+F), dL/d primal (out.pred_fs are its xf entries:
+ *   add their gradient there).  Both NULL: zero gradients.
+ *   grad: n records, overwritten.  grad_plan (nullable): plan_rows x 2, dL/d fs_plan ACCUMULATED into (+=): each
+ *   (instance, axis) adds its sum for a plan row once, so the bytes are reproducible when no two instances share plan
+ *   rows; rows shared by instances receive the sum of their contributions in an unspecified order.
+ *   grad[i].status: 0, or ISMPC_ST_QP_FAIL for a record outside the tables (flagged and skipped as the forward does: its
+ *   gradients stay zero and no plan row of it is touched) or a singular system.
+ *   Gradients of a forward that failed (ISMPC_ST_QP_FAIL or ISMPC_ST_WINDOW in out.status) are meaningless: the caller
+ *   masks them.  ISMPC_ST_GI_FALLBACK is informational and needs no mask.
+ *   mem: ISMPC_MEM_HOST or ISMPC_MEM_DEVICE.  Every argument is checked before the device is touched; ISMPC_ERR_MODEL
+ *   without ismpc_forma_set_model. */
+typedef struct {
+    double st[6];                   /* dL/d(x, xd, xz, y, yd, yz) of the record */
+    double cur_fs[2], fs_store[2];
+    double height, wx, wy;
+    int32_t status, reserved;       /* 0, or ISMPC_ST_QP_FAIL: record outside the tables / singular system */
+} ismpc_forma_grad_t;
+
+int ismpc_forma_adjoint_batch(ismpc_handle* h, int n, const ismpc_forma_inst_t* inst,
+                              const int32_t* fs_timing, int timing_len, const double* fs_plan, int plan_rows,
+                              const double* primal, const int8_t* active,
+                              const double* v_st, const double* v_primal,
+                              ismpc_forma_grad_t* grad, double* grad_plan, int mem, void* stream);
+
 /* Closed loop of the MATLAB scripts (bang.m:99-563, QP-1 loop): n_ticks ticks on the device with the
  * footstep switch, plan shift and centerline rebuild (bang.m:529-563).  inst is advanced in place;
  * fs_plan is modified in place (per-instance rows are shifted at every switch).

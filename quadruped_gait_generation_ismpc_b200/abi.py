@@ -28,6 +28,8 @@ FORMA_INST = np.dtype([("st", "f8", 6), ("cur_fs", "f8", 2), ("fs_store", "f8", 
                        ("plan_first_row", "i4"), ("n_fs", "i4")], align=True)
 FORMA_OUT = np.dtype([("st", "f8", 6), ("pred_fs", "f8", 2 * MAX_FSTEPS), ("kkt_res", "f8"),
                       ("status", "i4"), ("iters", "i4")], align=True)
+FORMA_GRAD = np.dtype([("st", "f8", 6), ("cur_fs", "f8", 2), ("fs_store", "f8", 2), ("height", "f8"), ("wx", "f8"),
+                       ("wy", "f8"), ("status", "i4"), ("reserved", "i4")], align=True)      # ismpc_forma_grad_t
 PUSH = np.dtype([("fs", "i4"), ("ct0", "i4"), ("ct1", "i4"), ("reserved", "i4"),
                  ("ax", "f8"), ("ay", "f8")], align=True)
 
@@ -47,12 +49,12 @@ KF_STATE64 = np.dtype([("state", "f8", (3, 5)), ("sigma", "f8", (3, 25))], align
 
 SIZES = {"ismpc_state_t": 72, "ismpc_walk_t": 24, "ismpc_formc_model_t": 72, "ismpc_formc_inst_t": 40,
          "ismpc_formc_out_t": 128, "ismpc_formc_tick_t": 128, "ismpc_forma_model_t": 72, "ismpc_forma_inst_t": 136,
-         "ismpc_forma_out_t": 192, "ismpc_push_t": 32, "ismpc_feet_model_t": 56, "ismpc_feet_inst_t": 32, "ismpc_plan_model_t": 48, "ismpc_plan_req_t": 16, "ismpc_kf_model_t": 172, "ismpc_kf_state_t": 360,
+         "ismpc_forma_out_t": 192, "ismpc_forma_grad_t": 112, "ismpc_push_t": 32, "ismpc_feet_model_t": 56, "ismpc_feet_inst_t": 32, "ismpc_plan_model_t": 48, "ismpc_plan_req_t": 16, "ismpc_kf_model_t": 172, "ismpc_kf_state_t": 360,
          "ismpc_kf_sample_t": 48, "ismpc_kf_state64_t": 720}
 DTYPES = {"ismpc_state_t": STATE, "ismpc_walk_t": WALK, "ismpc_formc_model_t": FORMC_MODEL,
           "ismpc_formc_inst_t": FORMC_INST, "ismpc_formc_out_t": FORMC_OUT, "ismpc_formc_tick_t": FORMC_TICK,
           "ismpc_forma_model_t": FORMA_MODEL, "ismpc_forma_inst_t": FORMA_INST,
-          "ismpc_forma_out_t": FORMA_OUT, "ismpc_push_t": PUSH, "ismpc_feet_model_t": FEET_MODEL,
+          "ismpc_forma_out_t": FORMA_OUT, "ismpc_forma_grad_t": FORMA_GRAD, "ismpc_push_t": PUSH, "ismpc_feet_model_t": FEET_MODEL,
           "ismpc_feet_inst_t": FEET_INST, "ismpc_plan_model_t": PLAN_MODEL, "ismpc_plan_req_t": PLAN_REQ,
           "ismpc_kf_model_t": KF_MODEL, "ismpc_kf_state_t": KF_STATE, "ismpc_kf_sample_t": KF_SAMPLE, "ismpc_kf_state64_t": KF_STATE64}
 

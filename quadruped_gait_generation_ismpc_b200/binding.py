@@ -23,7 +23,8 @@ EXPORTS = ["ismpc_version", "ismpc_error_string", "ismpc_create", "ismpc_destroy
            "ismpc_forma_rollout_ex2", "ismpc_kf_filter_batch_f64", "ismpc_formc_set_instances",
            "ismpc_formc_solve_batch_packed", "ismpc_qp_solve_batch_ws", "ismpc_qp_set_matrices",
            "ismpc_qp_hotstart_batch", "ismpc_forma_solve_batch_ws", "ismpc_qp_solve_batch_bounds",
-           "ismpc_qp_hotstart_batch_bounds", "ismpc_qp_adjoint_batch", "ismpc_qp_hotstart_adjoint_batch"]
+           "ismpc_qp_hotstart_batch_bounds", "ismpc_qp_adjoint_batch", "ismpc_qp_hotstart_adjoint_batch",
+           "ismpc_forma_adjoint_batch"]
 
 _lib = None
 
@@ -82,6 +83,7 @@ def lib():
     L.ismpc_forma_set_model.argtypes = [C.c_void_p, C.c_void_p]
     L.ismpc_forma_solve_batch.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
     L.ismpc_forma_solve_batch_ws.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
+    L.ismpc_forma_adjoint_batch.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 6 + [C.c_int, C.c_void_p]
     L.ismpc_forma_rollout.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
     L.ismpc_forma_rollout_ex.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [C.c_int, C.c_void_p]
     L.ismpc_feet_place_rollout.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
@@ -144,6 +146,13 @@ def _ptr(a):
     if isinstance(a, int):
         return C.c_void_p(a)
     return C.c_void_p(a.ctypes.data)
+
+
+def _shaped(a, dtype, shape, name):
+    a = np.ascontiguousarray(a, dtype=dtype)
+    if a.shape != shape:
+        raise ValueError("%s must be %s, got %s" % (name, " x ".join(map(str, shape)), a.shape))
+    return a
 
 
 class Handle:
@@ -335,6 +344,33 @@ class Handle:
                                                 plan_rows, _ptr(ws_guess), ws_shift, _ptr(out), _ptr(primal), _ptr(active),
                                                 mem, st)
         self._check(rc, "ismpc_forma_solve_batch_ws")
+
+    def forma_adjoint_batch_raw(self, n, inst, fs_timing, timing_len, fs_plan, plan_rows, primal, active, grad,
+                                v_st=None, v_primal=None, grad_plan=None, mem=abi.MEM_DEVICE, stream=None):
+        """Raw ismpc_forma_adjoint_batch: every array is a numpy array (host), an integer address (device) or None."""
+        rc = self._L.ismpc_forma_adjoint_batch(self._h, n, _ptr(inst), _ptr(fs_timing), timing_len, _ptr(fs_plan), plan_rows,
+                                               _ptr(primal), _ptr(active), _ptr(v_st), _ptr(v_primal), _ptr(grad),
+                                               _ptr(grad_plan), mem, C.c_void_p(stream) if stream else None)
+        self._check(rc, "ismpc_forma_adjoint_batch")
+
+    def forma_adjoint_batch(self, inst, fs_timing, fs_plan, primal, active, v_st=None, v_primal=None, want_plan=True):
+        """Gradients of a form-A tick (ismpc_forma_adjoint_batch) at the solution the forward returned for these records:
+        primal / active are its "primal" / "active", v_st (n x 6) and v_primal (n x 2(C+F)) the upstream gradients of
+        out["st"] and of the primal (either may be None).  Returns dict(grad = FORMA_GRAD records, plan = dL/d fs_plan
+        (rows x 2) or None without want_plan)."""
+        n = len(inst)
+        nV = 2 * (int(self.forma["C"][0]) + int(self.forma["F"][0]))
+        fs_timing = np.ascontiguousarray(fs_timing, dtype=np.int32)
+        fs_plan = np.ascontiguousarray(fs_plan, dtype=np.float64)
+        f64 = lambda a, shape, name: None if a is None else _shaped(a, np.float64, shape, name)
+        primal = _shaped(primal, np.float64, (n, nV), "primal")
+        active = _shaped(active, np.int8, (n, nV), "active")
+        v_st, v_primal = f64(v_st, (n, 6), "v_st"), f64(v_primal, (n, nV), "v_primal")
+        grad = np.zeros(n, dtype=abi.FORMA_GRAD)
+        plan = np.zeros_like(fs_plan) if want_plan else None
+        self.forma_adjoint_batch_raw(n, np.ascontiguousarray(inst), fs_timing, len(fs_timing), fs_plan, fs_plan.shape[0],
+                                     primal, active, grad, v_st, v_primal, plan, mem=abi.MEM_HOST)
+        return dict(grad=grad, plan=plan)
 
     def forma_rollout(self, inst, fs_timing, fs_plan, n_ticks, push=None, want_traj=True):
         n = len(inst)

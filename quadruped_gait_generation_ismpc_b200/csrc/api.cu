@@ -633,6 +633,40 @@ extern "C" int ismpc_forma_solve_batch(ismpc_handle* h, int n, const ismpc_forma
                                       active_opt, mem, stream);
 }
 
+// The adjoint of a tick.  grad_plan is staged with the caller's bytes (it is accumulated into); grad is overwritten.
+extern "C" int ismpc_forma_adjoint_batch(ismpc_handle* h, int n, const ismpc_forma_inst_t* inst, const int32_t* fs_timing,
+                                         int timing_len, const double* fs_plan, int plan_rows, const double* primal,
+                                         const int8_t* active, const double* v_st, const double* v_primal,
+                                         ismpc_forma_grad_t* grad, double* grad_plan, int mem, void* stream)
+{
+    if (!h) return ISMPC_ERR_ARG;
+    if (n < 0 || n > h->max_batch || !inst || !fs_timing || timing_len <= 0 || !fs_plan || plan_rows <= 0 || !primal ||
+        !active || !grad || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
+        return ISMPC_ERR_ARG;
+    if (!h->forma_ready) return ISMPC_ERR_MODEL;
+    if (n == 0) return ISMPC_OK;
+    CK(cudaSetDevice(h->device));
+    FormALaunchPlan lp;
+    forma_adjoint_plan(h->am, h->sm_count, 2LL * n, &lp);
+    if (h->a_Lwork.ensure((lp.spill_doubles + 2) * sizeof(double))) return ISMPC_ERR_ALLOC;
+    const size_t mb = (size_t)h->max_batch, nV = 2 * (size_t)(h->am.C + h->am.F);
+    Staged s(h, mem, stream, false);
+    FormAAdjArgs a;
+    a.n = n; a.model = h->am; a.timing_len = timing_len; a.plan_rows = plan_rows;
+    a.grad = s.out(grad, n, mb);
+    a.grad_plan = s.inout(grad_plan, (size_t)plan_rows * 2);
+    a.inst = s.in(inst, n, mb);
+    a.fs_timing = s.in(fs_timing, timing_len);
+    a.fs_plan = s.in(fs_plan, (size_t)plan_rows * 2);
+    a.primal = s.in(primal, n * nV, mb * nV);
+    a.active = (const signed char*)s.in(active, n * nV, mb * nV);
+    a.v_st = s.in(v_st, (size_t)n * 6, mb * 6);
+    a.v_primal = s.in(v_primal, n * nV, mb * nV);
+    if (s.err) return s.err;
+    return s.finish(forma_adjoint_launch(a, lp, lp.spill_doubles ? (double*)h->a_Lwork.p : nullptr, s.st),
+                    "forma_adjoint_launch");
+}
+
 extern "C" int ismpc_forma_rollout(ismpc_handle* h, int n, int n_ticks, ismpc_forma_inst_t* inst,
                                    const int32_t* fs_timing, int timing_len, double* fs_plan, int plan_rows,
                                    const ismpc_push_t* push, double* traj_opt, int32_t* status_opt, int mem,

@@ -653,6 +653,62 @@ __device__ __noinline__ int forma_pdas(const FormAShared& sm, const FormAProb& p
 #include "forma_reg.cuh"
 namespace ismpc {
 
+// ---- the build of a tick's QP, shared by the tick and its adjoint ----
+// Stability row coefficients (bang.m:200-207) into sm.a, their prefix sums into sm.PA; returns saa = a'a.
+// e^{-eta dt i} for i = lane + 32 k as exp(-eta dt lane) * exp(-32 eta dt)^k: five exp calls per lane for the whole
+// build instead of thirteen and a pow (products of <= 8 factors: a few 1e-16 relative).  lam = e^{-eta dt},
+// lamC = e^{-eta dt C}, e32 = e^{-32 eta dt}, el = e^{-eta dt lane}.
+__device__ __forceinline__ double forma_stability(const FormAShared& sm, int C, double eta, double dt, double lam,
+                                                  double lamC, double e32, double el)
+{
+    const int lane = lane_id();
+    const double k1 = (1.0 / eta) * (1.0 - lam) / (1.0 - lamC);
+    const double k2 = dt * lamC;
+    double saa = 0.0;
+    {
+        double ei = el;
+        for (int i = lane; i < C; i += 32) {
+            const double ai = k1 * ei - k2;
+            sm.a[i] = ai; sm.PA[i] = ai; saa += ai * ai;
+            ei *= e32;
+        }
+    }
+    saa = warp_sum(saa);
+    __syncwarp();
+    warp_prefix_sum_smem(sm.PA, C);
+    return saa;
+}
+
+// Mapping (bang.m:126-140) into sm.mw / sm.mp and the ZMP bounds (bang.m:147-150) into sm.lo / sm.hi.
+// ftw (lane l): fs_timing entry fsCounter + l (1-based, clamped to the table); zq: the ZMP state; cur: current footstep.
+// pf = number of footstep switches up to tick t (the timing table increases, so the reference's early-exit loop counts
+// the leading run of `t >= ft`); the loops run a uniform number of rounds so that the shuffles are warp-wide
+__device__ __forceinline__ void forma_mapping(const FormAShared& sm, int C, int F, int j, int fs_counter, int n_timing,
+                                              int ds, int ftw, double zq, double w_box, double cur)
+{
+    const int lane = lane_id();
+    const int rounds = (C + 31) >> 5;
+    for (int k = 0; k < rounds; ++k) {
+        const int i = lane + 32 * k;
+        const int t = j + i + 1;                                    // MATLAB j+i with i 1-based
+        int pf = 0; bool run = true;
+        for (int mstep = 1; mstep <= F + 1; ++mstep) {
+            const int fm = __shfl_sync(ISMPC_FULL_MASK, ftw, mstep);
+            run = run && (fs_counter + mstep <= n_timing) && (t >= fm);
+            pf += run ? 1 : 0;
+        }
+        const int fr = __shfl_sync(ISMPC_FULL_MASK, ftw, pf + 1);   // ft[min(fsCounter + pf + 1, n_timing) - 1]
+        if (i < C) {
+            const int rem = fr - t;
+            const double wgt = (rem > ds) ? 1.0 : (double)rem / (double)ds;
+            sm.mw[i] = wgt; sm.mp[i] = (signed char)pf;
+            const double m0 = (pf == 0) ? wgt : 0.0;                // mapping(:,1): weight on the current footstep
+            sm.lo[i] = 1.0 * (-zq - w_box / 2) + m0 * cur;
+            sm.hi[i] = 1.0 * (-zq + w_box / 2) + m0 * cur;
+        }
+    }
+}
+
 // self-check of a solve: equality residual and worst bound violation (sm.x, sm.rv against sm.lo / sm.hi)
 __device__ __forceinline__ void forma_selfcheck(const FormAShared& sm, int C, int n, double& eqv, double& viol)
 {
@@ -776,48 +832,11 @@ __device__ inline int forma_tick_axis(const FormAShared& sm, const ismpc_forma_m
     if (segP > n_fs - 2) { segP = n_fs - 2; rP = step - 1; }
     const double clPa = plan[segP * 2 + axis], clPb = plan[(segP + 1) * 2 + axis];
     // ---- stability row coefficients (bang.m:200-207) ----
-    // e^{-eta dt i} for i = lane + 32 k as exp(-eta dt lane) * exp(-32 eta dt)^k: five exp calls per lane for the whole
-    // build instead of thirteen and a pow (products of <= 8 factors: a few 1e-16 relative)
     const double ed = eta * dt;
     const double lam = exp(-ed), lamC = exp(-ed * (double)C), e32 = exp(-32.0 * ed), el = exp(-ed * (double)lane);
-    const double k1 = (1.0 / eta) * (1.0 - lam) / (1.0 - lamC);
-    const double k2 = dt * lamC;
-    double saa = 0.0;
-    {
-        double ei = el;
-        for (int i = lane; i < C; i += 32) {
-            const double ai = k1 * ei - k2;
-            sm.a[i] = ai; sm.PA[i] = ai; saa += ai * ai;
-            ei *= e32;
-        }
-    }
-    saa = warp_sum(saa);
-    __syncwarp();
-    warp_prefix_sum_smem(sm.PA, C);
+    const double saa = forma_stability(sm, C, eta, dt, lam, lamC, e32, el);
     // ---- mapping (bang.m:126-140) + ZMP bounds (bang.m:147-150) ----
-    // pf = number of footstep switches up to tick t (the timing table increases, so the reference's early-exit loop counts
-    // the leading run of `t >= ft`); the loops run a uniform number of rounds so that the shuffles are warp-wide
-    const double zq = st3[2];
-    const int rounds = (C + 31) >> 5;
-    for (int k = 0; k < rounds; ++k) {
-        const int i = lane + 32 * k;
-        const int t = j + i + 1;                                    // MATLAB j+i with i 1-based
-        int pf = 0; bool run = true;
-        for (int mstep = 1; mstep <= F + 1; ++mstep) {
-            const int fm = __shfl_sync(ISMPC_FULL_MASK, ftw, mstep);
-            run = run && (fs_counter + mstep <= n_timing) && (t >= fm);
-            pf += run ? 1 : 0;
-        }
-        const int fr = __shfl_sync(ISMPC_FULL_MASK, ftw, pf + 1);   // ft[min(fsCounter + pf + 1, n_timing) - 1]
-        if (i < C) {
-            const int rem = fr - t;
-            const double wgt = (rem > ds) ? 1.0 : (double)rem / (double)ds;
-            sm.mw[i] = wgt; sm.mp[i] = (signed char)pf;
-            const double m0 = (pf == 0) ? wgt : 0.0;                // mapping(:,1): weight on the current footstep
-            sm.lo[i] = 1.0 * (-zq - w_box / 2) + m0 * cur;
-            sm.hi[i] = 1.0 * (-zq + w_box / 2) + m0 * cur;
-        }
-    }
+    forma_mapping(sm, C, F, j, fs_counter, n_timing, ds, ftw, st3[2], w_box, cur);
     // ---- kinematic bounds (bang.m:163-190) ----
     for (int f = lane; f < F; f += 32) {
         double bnd = (axis == 0) ? ((fs_counter == 1 && f == 0) ? mdl.disp_forw_dummy : mdl.disp_forw)

@@ -334,4 +334,249 @@ int forma_rollout_launch(const FormAArgs& a_in, const FormALaunchPlan& p, ismpc_
     return (int)cudaGetLastError();
 }
 
+// ---- the adjoint of a tick (ismpc_forma_adjoint_batch) ------------------------------------------------------------------
+// Centerline sample cl(t) = wa * plan[seg] + wb * plan[seg + 1] -- the weights forma_centerline applies.
+__device__ __forceinline__ void forma_cl_weights(int n_fs, int step, int ds, int first_ramp, int t, int& seg, double& wa,
+                                                 double& wb)
+{
+    seg = (t - 1) / step;
+    int r = (t - 1) - seg * step;
+    if (seg > n_fs - 2) { seg = n_fs - 2; r = step - 1; }
+    wa = 1.0; wb = 0.0;
+    if (seg == 0 && !first_ramp) return;
+    if (r < step - ds) return;
+    const int k = r - (step - ds);
+    if (ds == 1 || k == ds - 1) { wa = 0.0; wb = 1.0; return; }
+    wb = (double)k / (double)(ds - 1); wa = 1.0 - wb;
+}
+
+__device__ __forceinline__ int forma_cl_seg(int n_fs, int step, int t)
+{
+    const int seg = (t - 1) / step;
+    return seg > n_fs - 2 ? n_fs - 2 : seg;
+}
+
+// One warp per (instance, axis), persistent: warp s of the grid takes items s, s + (warps in the grid), ...  Per item:
+// the tick's build (forma_stability, forma_mapping) into the FormAProb the forward solved, the working set installed
+// factor only in row order (stability row first), then with p0 = H^-1 (w + e_0 B_u' u):
+//     mu = J'J (0 - N_W' p0),  p = p0 + sum_k mu_k sg_k H^-1 a_k,  q_{id_k} = -sg_k mu_k,
+// the stability row's multiplier y_s = [S^-1 N_W' (x + H^-1 g)]_0 from the same factor, and the routing through the build.
+// Shared memory per warp: the tick's carve (no CTA header); sm.x = p0 then p, sm.z = step, sm.rv = row values,
+// sm.lo = x + H^-1 g, sm.hi = q per row.
+__global__ void __launch_bounds__(FORMA_MAX_THREADS, 8) forma_adjoint_kernel(FormAAdjArgs a, int R, int warps_per_cta,
+                                                                          double* Jspill)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int warp = warp_id(), lane = lane_id();
+    const int C = a.model.C, F = a.model.F, P = a.model.P, n = C + F;
+    const double dt = a.model.dt, qz_inv = 1.0 / a.model.q_zdot, qf_inv = 1.0 / a.model.q_foot, Qf = a.model.q_foot;
+    const size_t slot = (size_t)blockIdx.x * warps_per_cta + warp;
+    FormAShared sm;
+    forma_carve(smem_raw + forma_warp_smem_bytes(C, F, R) * warp, C, F, R,
+                Jspill ? Jspill + slot * forma_spill_doubles(C, F, R) : nullptr, sm);
+    const long long stride = (long long)gridDim.x * warps_per_cta;
+    for (long long item = (long long)slot; item < 2LL * a.n; item += stride) {
+        const int inst = (int)(item >> 1), axis = (int)(item & 1);
+        const ismpc_forma_inst_t in = a.inst[inst];
+        ismpc_forma_grad_t* gr = a.grad + inst;
+        if (!forma_inst_in_range(in, a.fs_timing, a.plan_rows, a.timing_len)) {        // never read outside the caller's tables
+            if (lane == 0) atomicOr(&gr->status, (int)ISMPC_ST_QP_FAIL);
+            continue;
+        }
+        const double* plan = a.fs_plan + (size_t)in.plan_first_row * 2;
+        const int32_t* ft = a.fs_timing + in.timing_first;
+        const int j = in.j, fsc = in.fs_counter, ds = in.ds, n_fs = in.n_fs, ramp = in.cl_first_ramp;
+        const int step = ft[1] - ft[0];
+        const double eta = sqrt(a.model.g_eta / in.height);
+        const double s0 = in.st[axis * 3 + 0], s1 = in.st[axis * 3 + 1], s2 = in.st[axis * 3 + 2];
+        const double cur = in.cur_fs[axis], store = in.fs_store[axis];
+        int idxw = fsc + lane; if (idxw > in.n_timing) idxw = in.n_timing;
+        const int ftw = ft[idxw - 1];
+        // ---- the forward's build ----
+        const double ed = eta * dt;
+        const double lam = exp(-ed), lamC = exp(-ed * (double)C), e32 = exp(-32.0 * ed), el = exp(-ed * (double)lane);
+        const double saa = forma_stability(sm, C, eta, dt, lam, lamC, e32, el);
+        forma_mapping(sm, C, F, j, fsc, in.n_timing, ds, ftw, s2, axis == 0 ? in.wx : in.wy, cur);
+        const double* xg = a.primal + ((size_t)inst * 2 + axis) * n;
+        const signed char* act = a.active + (size_t)inst * 2 * n;
+        // ---- upstream: u = dL/ds+, w = dL/dv; p0 = H^-1 (w + e_0 B_u' u); sm.lo = x + H^-1 g ----
+        double u0 = 0.0, u1 = 0.0, u2 = 0.0;
+        if (a.v_st) { const double* vs = a.v_st + (size_t)inst * 6 + axis * 3; u0 = vs[0]; u1 = vs[1]; u2 = vs[2]; }
+        const double ex = exp(ed), exi = 1.0 / ex;
+        const double ch = 0.5 * (ex + exi), sh = 0.5 * (ex - exi);    // as forma_integrate
+        const double bu = (dt - sh / eta) * u0 + (1.0 - ch) * u1 + dt * u2;
+        const double* vp = a.v_primal ? a.v_primal + ((size_t)inst * 2 + axis) * n : nullptr;
+        for (int i = lane; i < n; i += 32) {
+            const double vt = (vp ? vp[i] : 0.0) + (i == 0 ? bu : 0.0);
+            sm.x[i] = vt * (i < C ? qz_inv : qf_inv);
+            double t = xg[i];
+            if (i >= C) { int row = fsc + 1 + (i - C); if (row > n_fs) row = n_fs; t -= plan[(row - 1) * 2 + axis]; }
+            sm.lo[i] = t;
+            sm.hi[i] = 0.0;
+        }
+        __syncwarp();
+        FormAProb pb{C, F, dt, qz_inv, qf_inv, saa, sm.a, sm.PA, sm.mw, sm.lo, sm.hi, sm.mp, sm.scr};
+        // ---- W in row order, factor only: the stability row (id n, equality), then the reported rows ----
+        DasWork w = sm.das;
+        w.q = 0; w.neq = 0;
+        const double spp = das_schur_col(pb, w, n, +1);
+        if (!(spp > 0.0) || !isfinite(spp)) {
+            if (lane == 0) atomicOr(&gr->status, (int)ISMPC_ST_QP_FAIL);
+            continue;
+        }
+        das_append(w, n, +1, spp, 0.0);
+        w.neq = 1;
+        for (int base = 0; base < n; base += 32) {
+            const int i = base + lane;
+            int s = 0;
+            if (i < C) s = act[axis * C + i];
+            else if (i < n) s = act[2 * C + axis * F + (i - C)];
+            unsigned cand = __ballot_sync(ISMPC_FULL_MASK, s != 0);
+            while (cand) {
+                const int b = __ffs(cand) - 1;
+                cand &= cand - 1;
+                const int sgp = __shfl_sync(ISMPC_FULL_MASK, s, b) < 0 ? +1 : -1;
+                if (w.q >= n) break;
+                das_factor_append(pb, w, base + b, sgp);
+            }
+        }
+        // ---- y_s: entry 0 of S^-1 N_W' (x + H^-1 g) ----
+        auto row_values = [&](const double* v) {      // sm.rv = the rows at v; returns the stability row's value
+            pb.eval(v, sm.rv);
+            double sv = 0.0;
+            for (int i = lane; i < C; i += 32) sv += sm.a[i] * v[i];
+            return warp_sum(sv);
+        };
+        double sv = row_values(sm.lo);
+        for (int k = lane; k < w.q; k += 32) { const int id = w.wid[k]; w.y[k] = (double)w.wsg[k] * (id == n ? sv : sm.rv[id]); }
+        __syncwarp();
+        das_apply_J(w);
+        das_apply_Jt(w);
+        const double y_s = w.r[0];
+        __syncwarp();
+        // ---- mu, p, q ----
+        sv = row_values(sm.x);
+        for (int k = lane; k < w.q; k += 32) { const int id = w.wid[k]; w.y[k] = -(double)w.wsg[k] * (id == n ? sv : sm.rv[id]); }
+        __syncwarp();
+        das_apply_J(w);
+        das_apply_Jt(w);                                                   // w.r = mu
+        pb.step_dir(n, 0, w.wid, w.wsg, w.r, w.q, sm.z);                   // sm.z = -sum_k mu_k sg_k H^-1 a_k
+        for (int i = lane; i < n; i += 32) sm.x[i] -= sm.z[i];
+        for (int k = lane; k < w.q; k += 32) if (w.wid[k] < n) sm.hi[w.wid[k]] = -(double)w.wsg[k] * w.r[k];
+        const double q_s = -w.r[0];
+        __syncwarp();
+        // ---- routing through the build ----
+        const double k1 = (1.0 / eta) * (1.0 - lam) / (1.0 - lamC);
+        const double k1p = k1 * (dt * lam / (1.0 - lam) - 1.0 / eta - dt * (double)C * lamC / (1.0 - lamC));
+        double g_xz = 0.0, g_w = 0.0, g_cur = 0.0, g_eta = 0.0;
+        {
+            double ei = el;
+            for (int i = lane; i < C; i += 32) {
+                const double qi = sm.hi[i];
+                const int s = act[axis * C + i];
+                g_xz -= qi;
+                if (s != 0) g_w += (s < 0 ? -0.5 : 0.5) * qi;
+                if (sm.mp[i] == 0) g_cur += sm.mw[i] * qi;
+                const double dai = (k1p - k1 * dt * (double)i) * ei + dt * dt * (double)C * lamC;   // da_i / d eta
+                g_eta += (y_s * sm.x[i] - q_s * xg[i]) * dai;
+                ei *= e32;
+            }
+        }
+        // anticipative tail: d ant / d fs_store and d ant / d eta
+        double sE = 0.0, sdE = 0.0;
+        for (int i = C + 1 + lane; i <= P; i += 32) {
+            const double ei = exp(-ed * (double)i), E = ei * (1.0 - lam), dE = -dt * (double)i * E + ei * dt * lam;
+            sE += E;
+            sdE += dE * (forma_centerline(plan, n_fs, axis, step, ds, ramp, j + i) - store);
+        }
+        g_xz = warp_sum(g_xz); g_w = warp_sum(g_w); g_cur = warp_sum(g_cur); g_eta = warp_sum(g_eta);
+        sE = warp_sum(sE); sdE = warp_sum(sdE);
+        const double eP = exp(-ed * (double)P);
+        const double dant_deta = sdE - dt * (double)P * eP * (forma_centerline(plan, n_fs, axis, step, ds, ramp, P) - store);
+        const double zd0 = xg[0];
+        g_eta += q_s * (-s1 / (eta * eta) - dant_deta);
+        {   // d(A_u s + B_u zd0)/d eta
+            const double dA01 = dt * ch / eta - sh / (eta * eta), dA10 = sh + eta * dt * ch;
+            g_eta += u0 * (dt * sh * s0 + dA01 * s1 - dt * sh * s2 - dA01 * zd0);
+            g_eta += u1 * (dA10 * s0 + dt * sh * s1 - dA10 * s2 - dt * sh * zd0);
+        }
+        // ---- plan rows: targets, the tail's centerline samples and cl(P), one sum per row in a fixed order ----
+        if (a.grad_plan) {
+            const int g_lo = fsc < n_fs - 1 ? fsc : n_fs - 1, g_hi = fsc + F - 1 < n_fs - 1 ? fsc + F - 1 : n_fs - 1;
+            const int t_lo = forma_cl_seg(n_fs, step, j + C + 1), t_hi = forma_cl_seg(n_fs, step, j + P) + 1;
+            int segP; double waP, wbP;
+            forma_cl_weights(n_fs, step, ds, ramp, P, segP, waP, wbP);
+            const bool tail = P > C;
+            int r_lo = g_lo < segP ? g_lo : segP, r_hi = g_hi > segP + 1 ? g_hi : segP + 1;
+            if (tail) { r_lo = r_lo < t_lo ? r_lo : t_lo; r_hi = r_hi > t_hi ? r_hi : t_hi; }
+            double* gp = a.grad_plan + (size_t)in.plan_first_row * 2 + axis;
+            for (int r = r_lo; r <= r_hi; ++r) {
+                const bool in_tail = tail && r >= t_lo && r <= t_hi;
+                if (!(r >= g_lo && r <= g_hi) && !in_tail && r != segP && r != segP + 1) continue;
+                double c = 0.0;
+                if (in_tail) {     // samples t = j + i with seg(t) in {r - 1, r}
+                    int a0 = (r - 1) * step + 1, a1 = r >= n_fs - 2 ? j + P : (r + 1) * step;
+                    if (a0 < j + C + 1) a0 = j + C + 1;
+                    if (a1 > j + P) a1 = j + P;
+                    for (int t = a0 + lane; t <= a1; t += 32) {
+                        int seg; double wa, wb;
+                        forma_cl_weights(n_fs, step, ds, ramp, t, seg, wa, wb);
+                        const double E = exp(-ed * (double)(t - j)) * (1.0 - lam);
+                        c += E * ((seg == r ? wa : 0.0) + (seg + 1 == r ? wb : 0.0));
+                    }
+                    c = warp_sum(c);
+                }
+                c += eP * ((segP == r ? waP : 0.0) + (segP + 1 == r ? wbP : 0.0));
+                double val = -q_s * c;                                       // d beq / d ant = -1
+                for (int f = 0; f < F; ++f) {
+                    const int row = fsc + f < n_fs - 1 ? fsc + f : n_fs - 1;
+                    if (row == r) val += Qf * sm.x[C + f];                   // g_f = -Q_foot plan row
+                }
+                if (lane == 0) atomicAdd(gp + (size_t)r * 2, val);
+            }
+        }
+        if (lane == 0) {
+            gr->st[axis * 3 + 0] = q_s + ch * u0 + eta * sh * u1;
+            gr->st[axis * 3 + 1] = q_s / eta + (sh / eta) * u0 + ch * u1;
+            gr->st[axis * 3 + 2] = -q_s + g_xz + (1.0 - ch) * u0 - eta * sh * u1 + u2;
+            gr->cur_fs[axis] = g_cur + sm.hi[C];                             // ZMP bounds, first kinematic row
+            gr->fs_store[axis] = q_s * (sE + eP);                            // beq = ... - ant, ant linear in -fs_store
+            if (axis == 0) gr->wx = g_w; else gr->wy = g_w;
+            atomicAdd(&gr->height, g_eta * (-eta / (2.0 * in.height)));
+        }
+        __syncwarp();
+    }
+}
+
+void forma_adjoint_plan(const ismpc_forma_model_t& m, int sm_count, long long items, FormALaunchPlan* p)
+{
+    const int C = m.C, F = m.F, q = C + F + 1;
+    const size_t lim = 227 * 1024;
+    const int wpc = FORMA_MAX_THREADS / 32;
+    // rows of the working set's inverse factor in shared memory, the rest in the spill slices.  With 32 rows a warp takes
+    // 14.8 KB at C = 100, F = 3, so 7 CTAs (14 warps) fit an SM by their sizes: the 2,048 items of a 1,024-instance batch
+    // start in one wave on 148 SMs
+    int R = q < 32 ? q : 32;
+    while (R > 1 && forma_warp_smem_bytes(C, F, R) * wpc > lim) --R;
+    p->R = R; p->warps_per_cta = wpc; p->kernel = 0; p->use_pdas = 0; p->warm_start = 0;
+    p->smem = forma_warp_smem_bytes(C, F, R) * wpc;
+    int b = 0;
+    cudaFuncSetAttribute(forma_adjoint_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
+    const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, forma_adjoint_kernel, 32 * wpc, p->smem);
+    const long long per_sm = (e == cudaSuccess && b > 0) ? b : 1;
+    const long long ctas = (items + wpc - 1) / wpc, resident = per_sm * sm_count;
+    p->grid = (int)(ctas < resident ? ctas : resident);
+    if (p->grid < 1) p->grid = 1;
+    p->spill_doubles = forma_spill_doubles(C, F, R) * (size_t)p->grid * wpc;
+}
+
+int forma_adjoint_launch(const FormAAdjArgs& a, const FormALaunchPlan& p, double* Jspill, cudaStream_t st)
+{
+    cudaError_t e = cudaFuncSetAttribute(forma_adjoint_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
+    if (e != cudaSuccess) return (int)e;
+    cudaMemsetAsync(a.grad, 0, (size_t)a.n * sizeof(ismpc_forma_grad_t), st);
+    forma_adjoint_kernel<<<p.grid, 32 * p.warps_per_cta, p.smem, st>>>(a, p.R, p.warps_per_cta, Jspill);
+    return (int)cudaGetLastError();
+}
+
 }  // namespace ismpc

@@ -33,6 +33,25 @@ int forma_tick_launch(const FormAArgs& a, const FormALaunchPlan& p, const signed
 int forma_rollout_launch(const FormAArgs& a, const FormALaunchPlan& p, ismpc_forma_inst_t* inst_io,
                          double* fs_plan_io, const ismpc_push_t* push, int n_ticks, double* traj, double* pred,
                          int32_t* status, int32_t* trace, cudaStream_t st);
+// the adjoint of a tick (ismpc_forma_adjoint_batch): plan of its launch (R, warps_per_cta, grid, smem, spill_doubles),
+// then the launch with a spill workspace of p.spill_doubles
+struct FormAAdjArgs {
+    int n;
+    ismpc_forma_model_t model;
+    const ismpc_forma_inst_t* inst;
+    const int32_t* fs_timing;
+    int timing_len;
+    const double* fs_plan;
+    int plan_rows;
+    const double* primal;
+    const signed char* active;
+    const double* v_st;             // nullable
+    const double* v_primal;         // nullable
+    ismpc_forma_grad_t* grad;
+    double* grad_plan;              // nullable
+};
+void forma_adjoint_plan(const ismpc_forma_model_t& m, int sm_count, long long items, FormALaunchPlan* p);
+int forma_adjoint_launch(const FormAAdjArgs& a, const FormALaunchPlan& p, double* Jspill, cudaStream_t st);
 int plan_generate_launch(int n, const ismpc_plan_model_t& m, const ismpc_plan_req_t* req, double* foot_plan, double* center,
                          int rows, cudaStream_t st);
 int kf_filter_launch(int n, int n_steps, const ismpc_kf_model_t& m, ismpc_kf_state_t* state, const ismpc_kf_sample_t* samples,
