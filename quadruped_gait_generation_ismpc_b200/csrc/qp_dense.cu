@@ -403,7 +403,9 @@ constexpr int DENSE_WARPS = 4;   // QPs per CTA
 // SETS = false: the tables (D, S) and x0 / A x0 sit in the problem's workspace slice, status[p] holds the factor status
 // (the seam).  SETS = true: they come from the problem's resident set and sets.xr, the slice (dense_layout(.., false))
 // holds the vectors only, and the status starts from the set's; a problem whose set index is out of range is flagged and
-// nothing else of it is written.  The algorithm is the same, so the same inputs give the same bytes.
+// nothing else of it is written.  The algorithm is the same, so the same inputs give the same bytes.  The seam keeps its
+// own SETS = false builds: run as n per-problem sets, its bounds calls are slower on the SETS = true builds (B200, 1,024
+// QPs of nV = 206 with a box: cold 1.36 -> 1.61 s, 20 hot-started ticks 6.6 -> 10.5 s; profiles/r11_dense_seam_as_sets.json).
 // BOUNDS = true: the rows are [I; A] with the box lbx <= x <= ubx (n x nV each, NULL = that side absent) as the first nV
 // (DenseBoundsProb); y, ws and ws_guess are n x (nV + nC), bounds first.  A variable whose bounds cross is flagged.
 template <bool WARM, bool SETS, bool BOUNDS>
@@ -506,24 +508,6 @@ __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const
         if (y) for (int k = lane; k < dw.q; k += 32) y[(size_t)p * nR + dw.wid[k]] = (double)dw.wsg[k] * dw.mu[k];
     }
     if (lane == 0) { status[p] = st; if (iters) iters[p] = it; }
-}
-
-__global__ void dense_hinv(int N, double* work, size_t stride, size_t offLinv, size_t offHinv)
-{
-    const double* Linv = work + (size_t)blockIdx.z * stride + offLinv;
-    double* Hinv = work + (size_t)blockIdx.z * stride + offHinv;
-    const int i = blockIdx.y * blockDim.y + threadIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= N || j >= N) return;
-    const int k0 = i > j ? i : j;
-    double s = 0.0;
-    for (int k = k0; k < N; ++k) s += Linv[(size_t)k * N + i] * Linv[(size_t)k * N + j];
-    Hinv[(size_t)i * N + j] = s;
-}
-
-void dense_hinv_launch(int n, int nV, double* work, size_t stride, size_t offLinv, size_t offHinv, cudaStream_t st)
-{
-    dim3 b(16, 16), gr((nV + 15) / 16, (nV + 15) / 16, n);
-    dense_hinv<<<gr, b, 0, st>>>(nV, work, stride, offLinv, offHinv);
 }
 
 // The seam's per-call set-up: factor H, Hinv, D and S into each problem's slice (layout l), the factor status into status.
