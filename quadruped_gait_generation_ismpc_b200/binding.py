@@ -155,6 +155,24 @@ def _shaped(a, dtype, shape, name):
     return a
 
 
+def _mat_index(mat_index, n):
+    """mat_index of a call against the resident dense sets as the C calls take it (None stays None)."""
+    idx = None if mat_index is None else np.ascontiguousarray(mat_index, dtype=np.int32)
+    if idx is not None and idx.shape != (n,):
+        raise ValueError("mat_index must have %d entries, got %s" % (n, idx.shape))
+    return idx
+
+
+def _qp_outputs(n, nV, nR, ws_guess):
+    """The outputs of a dense QP call with nR rows per problem (dict of x, y, ws, status, iters) and ws_guess as the C
+    calls take it (None stays None)."""
+    guess = None if ws_guess is None else np.ascontiguousarray(ws_guess, dtype=np.int8)
+    if guess is not None and guess.shape != (n, nR):
+        raise ValueError("ws_guess must be %d x %d, got %s" % (n, nR, guess.shape))
+    return dict(x=np.zeros((n, nV)), y=np.zeros((n, nR)), ws=np.zeros((n, nR), dtype=np.int8),
+                status=np.zeros(n, dtype=np.int32), iters=np.zeros(n, dtype=np.int32)), guess
+
+
 class Handle:
     """One handle per GPU (include/ismpc_b200.h: ismpc_create / ismpc_destroy)."""
 
@@ -501,21 +519,9 @@ class Handle:
         lbA = np.ascontiguousarray(lbA, dtype=np.float64); ubA = np.ascontiguousarray(ubA, dtype=np.float64)
         n, nV = H.shape[0], H.shape[1]
         nC = A.shape[1]
-        x = np.zeros((n, nV)); y = np.zeros((n, nC)); ws = np.zeros((n, nC), dtype=np.int8)
-        status = np.zeros(n, dtype=np.int32); iters = np.zeros(n, dtype=np.int32)
-        if ws_guess is None:
-            rc = self._L.ismpc_qp_solve_batch(self._h, n, nV, nC, _ptr(H), _ptr(g), _ptr(A), _ptr(lbA), _ptr(ubA),
-                                              _ptr(x), _ptr(y), _ptr(ws), _ptr(status), _ptr(iters), abi.MEM_HOST, None)
-            self._check(rc, "ismpc_qp_solve_batch")
-            return dict(x=x, y=y, ws=ws, status=status, iters=iters)
-        guess = np.ascontiguousarray(ws_guess, dtype=np.int8)
-        if guess.shape != (n, nC):
-            raise ValueError("ws_guess must be %d x %d, got %s" % (n, nC, guess.shape))
-        rc = self._L.ismpc_qp_solve_batch_ws(self._h, n, nV, nC, _ptr(H), _ptr(g), _ptr(A), _ptr(lbA), _ptr(ubA),
-                                             _ptr(guess), _ptr(x), _ptr(y), _ptr(ws), _ptr(status), _ptr(iters),
-                                             abi.MEM_HOST, None)
-        self._check(rc, "ismpc_qp_solve_batch_ws")
-        return dict(x=x, y=y, ws=ws, status=status, iters=iters)
+        out, guess = _qp_outputs(n, nV, nC, ws_guess)
+        self.qp_solve_batch_raw(n, nV, nC, H, g, A, lbA, ubA, **out, mem=abi.MEM_HOST, ws_guess=guess)
+        return out
 
     # ---- resident matrices of the dense seam (factor once, solve many right-hand sides) -----------------------
     def qp_set_matrices(self, H, A):
@@ -547,22 +553,14 @@ class Handle:
         for name, a, shape in (("lb", lb, (n, nV)), ("ub", ub, (n, nV)), ("lbA", lbA, (n, nC)), ("ubA", ubA, (n, nC))):
             if a is not None and a.shape != shape:
                 raise ValueError("%s must be %d x %d, got %s" % (name, shape[0], shape[1], a.shape))
-        nR = nV + nC
-        x = np.zeros((n, nV)); y = np.zeros((n, nR)); ws = np.zeros((n, nR), dtype=np.int8)
-        status = np.zeros(n, dtype=np.int32); iters = np.zeros(n, dtype=np.int32)
-        guess = None if ws_guess is None else np.ascontiguousarray(ws_guess, dtype=np.int8)
-        if guess is not None and guess.shape != (n, nR):
-            raise ValueError("ws_guess must be %d x %d, got %s" % (n, nR, guess.shape))
+        out, guess = _qp_outputs(n, nV, nV + nC, ws_guess)
         if not resident:
-            self.qp_solve_batch_bounds_raw(n, nV, nC, f64(H), g, f64(A) if nC else None, lb, ub, lbA, ubA, x, y, ws,
-                                           status, iters, mem=abi.MEM_HOST, ws_guess=guess)
+            self.qp_solve_batch_bounds_raw(n, nV, nC, f64(H), g, f64(A) if nC else None, lb, ub, lbA, ubA, **out,
+                                           mem=abi.MEM_HOST, ws_guess=guess)
         else:
-            idx = None if mat_index is None else np.ascontiguousarray(mat_index, dtype=np.int32)
-            if idx is not None and idx.shape != (n,):
-                raise ValueError("mat_index must have %d entries, got %s" % (n, idx.shape))
-            self.qp_hotstart_batch_bounds_raw(n, g, lb, ub, lbA, ubA, x, y, ws, status, iters, mat_index=idx,
+            self.qp_hotstart_batch_bounds_raw(n, g, lb, ub, lbA, ubA, **out, mat_index=_mat_index(mat_index, n),
                                               ws_guess=guess, mem=abi.MEM_HOST)
-        return dict(x=x, y=y, ws=ws, status=status, iters=iters)
+        return out
 
     def qp_hotstart_batch(self, g, lbA, ubA, ws_guess=None, mat_index=None, lb=None, ub=None):
         """ismpc_qp_hotstart_batch: n problems against the resident sets, problem p on set mat_index[p] (None: set p, or
@@ -574,18 +572,10 @@ class Handle:
         lbA = np.ascontiguousarray(lbA, dtype=np.float64); ubA = np.ascontiguousarray(ubA, dtype=np.float64)
         n, nV = g.shape
         nC = lbA.shape[1]
-        x = np.zeros((n, nV)); y = np.zeros((n, nC)); ws = np.zeros((n, nC), dtype=np.int8)
-        status = np.zeros(n, dtype=np.int32); iters = np.zeros(n, dtype=np.int32)
-        guess = None if ws_guess is None else np.ascontiguousarray(ws_guess, dtype=np.int8)
-        if guess is not None and guess.shape != (n, nC):
-            raise ValueError("ws_guess must be %d x %d, got %s" % (n, nC, guess.shape))
-        idx = None if mat_index is None else np.ascontiguousarray(mat_index, dtype=np.int32)
-        if idx is not None and idx.shape != (n,):
-            raise ValueError("mat_index must have %d entries, got %s" % (n, idx.shape))
-        rc = self._L.ismpc_qp_hotstart_batch(self._h, n, _ptr(idx), _ptr(g), _ptr(lbA), _ptr(ubA), _ptr(guess), _ptr(x),
-                                             _ptr(y), _ptr(ws), _ptr(status), _ptr(iters), abi.MEM_HOST, None)
-        self._check(rc, "ismpc_qp_hotstart_batch")
-        return dict(x=x, y=y, ws=ws, status=status, iters=iters)
+        out, guess = _qp_outputs(n, nV, nC, ws_guess)
+        self.qp_hotstart_batch_raw(n, g, lbA, ubA, **out, mat_index=_mat_index(mat_index, n), ws_guess=guess,
+                                   mem=abi.MEM_HOST)
+        return out
 
     def qp_hotstart_batch_raw(self, n, g, lbA, ubA, x, y=None, ws=None, status=None, iters=None, mat_index=None,
                               ws_guess=None, mem=abi.MEM_DEVICE, stream=None):
@@ -631,10 +621,7 @@ class Handle:
         v = np.ascontiguousarray(v, dtype=np.float64)
         n, nV = v.shape
         nC = np.shape(ws)[1] - nV
-        idx = None if mat_index is None else np.ascontiguousarray(mat_index, dtype=np.int32)
-        if idx is not None and idx.shape != (n,):
-            raise ValueError("mat_index must have %d entries, got %s" % (n, idx.shape))
-        return self._qp_adjoint(True, n, nV, nC, None, None, ws, v, idx)
+        return self._qp_adjoint(True, n, nV, nC, None, None, ws, v, _mat_index(mat_index, n))
 
     def _qp_adjoint(self, resident, n, nV, nC, H, A, ws, v, idx):
         ws = np.ascontiguousarray(ws, dtype=np.int8)

@@ -838,6 +838,18 @@ extern "C" int ismpc_kf_filter_batch_f64(ismpc_handle* h, int n, int n_steps, co
 // ---------------------------------------------------------------------------------------------------
 // Generic dense QP (solveQP seam)
 // ---------------------------------------------------------------------------------------------------
+// The shapes the dense seam takes: nV variables, nC rows of A.
+static bool qp_shape_ok(int nV, int nC) { return nV >= 1 && nV <= ISMPC_MAX_N && nC >= 0 && nC <= 2 * ISMPC_MAX_N + 8; }
+
+// The resident sets a call of n problems solves against: ISMPC_ERR_MODEL without sets; ISMPC_ERR_ARG without an index
+// when there are fewer sets than problems (and more than one set).
+static int qp_sets_check(const ismpc_handle* h, int n, const int32_t* mat_index_opt)
+{
+    if (h->r_nmat == 0) return ISMPC_ERR_MODEL;
+    if (!mat_index_opt && h->r_nmat > 1 && n > h->r_nmat) return ISMPC_ERR_ARG;
+    return ISMPC_OK;
+}
+
 // The cold / guessed seam calls, with (bounds) or without the box lbx <= x <= ubx: y, ws and the guess are n x nR, nR =
 // nV + nC with bounds (bounds first), nC without.
 static int qp_solve_common(ismpc_handle* h, int n, int nV, int nC, const double* H, const double* g, const double* A,
@@ -846,8 +858,7 @@ static int qp_solve_common(ismpc_handle* h, int n, int nV, int nC, const double*
                            int32_t* iters_opt, int mem, void* stream)
 {
     if (!h) return ISMPC_ERR_ARG;
-    if (n < 0 || n > h->max_batch || nV < 1 || nV > ISMPC_MAX_N || nC < 0 || nC > 2 * ISMPC_MAX_N + 8 || !H || !g ||
-        (nC > 0 && (!A || !lbA || !ubA)) || !x || !status)
+    if (n < 0 || n > h->max_batch || !qp_shape_ok(nV, nC) || !H || !g || (nC > 0 && (!A || !lbA || !ubA)) || !x || !status)
         return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
     const int nR = bounds ? nV + nC : nC;
@@ -912,7 +923,7 @@ extern "C" int ismpc_qp_set_matrices(ismpc_handle* h, int n_mat, int nV, int nC,
     if (n_mat < 0 || n_mat > h->max_batch || n_mat > 65535 || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
         return ISMPC_ERR_ARG;
     if (n_mat == 0) { h->r_nmat = 0; return ISMPC_OK; }
-    if (nV < 1 || nV > ISMPC_MAX_N || nC < 0 || nC > 2 * ISMPC_MAX_N + 8 || !H || (nC > 0 && !A)) return ISMPC_ERR_ARG;
+    if (!qp_shape_ok(nV, nC) || !H || (nC > 0 && !A)) return ISMPC_ERR_ARG;
     CK(cudaSetDevice(h->device));
     h->r_nmat = 0;                             // until the new sets are built
     const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
@@ -943,9 +954,9 @@ static int qp_hotstart_common(ismpc_handle* h, int n, const int32_t* mat_index_o
     if (!h) return ISMPC_ERR_ARG;
     if (n < 0 || n > h->max_batch || !g || !x || !status || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
         return ISMPC_ERR_ARG;
-    if (h->r_nmat == 0) return ISMPC_ERR_MODEL;
+    if (int rc = qp_sets_check(h, n, mat_index_opt)) return rc;
     const int nV = h->r_nV, nC = h->r_nC, n_mat = h->r_nmat;
-    if ((nC > 0 && (!lbA || !ubA)) || (!mat_index_opt && n_mat > 1 && n > n_mat)) return ISMPC_ERR_ARG;
+    if (nC > 0 && (!lbA || !ubA)) return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
     const int nR = bounds ? nV + nC : nC;
     if (nR == 0) ws_guess = nullptr;
@@ -999,8 +1010,8 @@ extern "C" int ismpc_qp_adjoint_batch(ismpc_handle* h, int n, int nV, int nC, co
                                       void* stream)
 {
     if (!h) return ISMPC_ERR_ARG;
-    if (n < 0 || n > h->max_batch || nV < 1 || nV > ISMPC_MAX_N || nC < 0 || nC > 2 * ISMPC_MAX_N + 8 || !H ||
-        (nC > 0 && !A) || !ws || !v || !p || !q || !status || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
+    if (n < 0 || n > h->max_batch || !qp_shape_ok(nV, nC) || !H || (nC > 0 && !A) || !ws || !v || !p || !q || !status ||
+        (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
         return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
@@ -1027,9 +1038,8 @@ extern "C" int ismpc_qp_hotstart_adjoint_batch(ismpc_handle* h, int n, const int
     if (!h) return ISMPC_ERR_ARG;
     if (n < 0 || n > h->max_batch || !ws || !v || !p || !q || !status || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
         return ISMPC_ERR_ARG;
-    if (h->r_nmat == 0) return ISMPC_ERR_MODEL;
+    if (int rc = qp_sets_check(h, n, mat_index_opt)) return rc;
     const int nV = h->r_nV, nC = h->r_nC, n_mat = h->r_nmat;
-    if (!mat_index_opt && n_mat > 1 && n > n_mat) return ISMPC_ERR_ARG;
     if (n == 0) return ISMPC_OK;
     CK(cudaSetDevice(h->device));
     if (h->r_work.ensure(qp_sets_work_doubles(n, n_mat, nV, nC, true) * sizeof(double))) return ISMPC_ERR_ALLOC;

@@ -40,11 +40,28 @@ __host__ __device__ inline DenseLayout dense_layout(int nV, int nC, bool tables 
     return l;
 }
 
-// n problem slices, then (warm start only) n x nC doubles of A x0 (with bounds: n x (nV + nC) of x0 | A x0), kept while rv
-// moves; outside the slices so that the cold path's layout does not depend on it
+// The workspace of one call, offsets in doubles: n problem slices (layout l), then the warm start's row values kept while rv
+// moves (n x nR: A x0, with bounds x0 | A x0), then, without tables, xr: x0 | A x0 of each problem (n x (nV + nC); with
+// tables they sit in the slice).  The kept rows are outside the slices so that the cold path's layout does not depend on
+// them.  dense_das_kernel finds them at work + n * stride by itself, so kept must stay n * l.total.
+struct DenseCallWork {
+    DenseLayout l;
+    size_t kept, xr, total;
+};
+
+static DenseCallWork dense_call_work(int n, int nV, int nC, bool bounds, bool tables)
+{
+    DenseCallWork c;
+    c.l = dense_layout(nV, nC, tables, bounds);
+    c.kept = (size_t)n * c.l.total;
+    c.xr = c.kept + (size_t)n * (nC + (bounds ? nV : 0));
+    c.total = c.xr + (tables ? 0 : (size_t)n * (nV + nC));
+    return c;
+}
+
 size_t qp_dense_work_doubles(int n, int nV, int nC, bool bounds)
 {
-    return (dense_layout(nV, nC, true, bounds).total + nC + (bounds ? nV : 0)) * (size_t)n + 16;
+    return dense_call_work(n, nV, nC, bounds, true).total + 16;
 }
 
 // ---- set-up kernels (batched over problems with blockIdx.z / blockIdx.y) --------------------------------
@@ -206,33 +223,11 @@ static void dense_gemm_launch(int use_dmma, int n, int M, int Nc, int K, const d
         dense_gemm_nt_cc<<<dim3((Nc + 15) / 16, (M + 15) / 16, n), dim3(16, 16), 0, st>>>(M, Nc, K, X, sx, sxr, sxk, Y, sy, syr, syk, C, sc, alpha);
 }
 
-// x0 = -Hinv g ; rv0 = A x0 ; one CTA per problem
-__global__ void dense_x0_rv(int nV, int nC, const double* g, const double* A, double* work, size_t stride,
-                            DenseLayout l, double* x_out)
-{
-    const size_t p = blockIdx.x;
-    double* w = work + p * stride;
-    const double* Hinv = w + l.Hinv;
-    const double* gp = g + p * nV;
-    for (int i = threadIdx.x; i < nV; i += blockDim.x) {
-        double s = 0.0;
-        for (int j = 0; j < nV; ++j) s += Hinv[(size_t)j * nV + i] * gp[j];
-        w[l.x0 + i] = -s;
-        x_out[p * nV + i] = -s;
-    }
-    __syncthreads();
-    const double* Ap = A + p * (size_t)nC * nV;
-    for (int c = threadIdx.x; c < nC; c += blockDim.x) {
-        double s = 0.0;
-        for (int j = 0; j < nV; ++j) s += Ap[(size_t)c * nV + j] * w[l.x0 + j];
-        w[l.rv + c] = s;
-    }
-}
-
 // ---- the resident matrix family (ismpc_qp_set_matrices / ismpc_qp_hotstart_batch) --------------------------
 // n_mat sets of one shape, built once by the set-up kernels above: per set [Hinv; D] as one (nV + nC) x nV row-major
 // block (HD, stride nV^2 + nC nV), S (stride nC^2), a copy of A (stride nC nV) and the factor status.  Problem p of a call
-// solves against set idx[p] (idx = NULL: set p, or set 0 when n_mat = 1).
+// solves against set idx[p] (idx = NULL: set p, or set 0 when n_mat = 1).  The shape is not stored: the struct is a
+// parameter of dense_das_kernel, whose builds are pinned by their SASS.
 struct DenseSets {
     const double *HD, *S, *A;
     const int32_t* fstat;       // n_mat: dense_cholesky's status of each set
@@ -240,31 +235,51 @@ struct DenseSets {
     int n_mat;
     double* xr;                 // n x (nV + nC): x0 | A x0 of each problem (written by the x0 step, rv moves in place)
     __host__ __device__ int set_of(int p) const { return idx ? idx[p] : (n_mat == 1 ? 0 : p); }
+    __host__ __device__ bool valid(int m) const { return m >= 0 && m < n_mat; }
+    // set m's [Hinv; D], S and A
+    __host__ __device__ const double* hd(int m, int nV, int nC) const { return HD + (size_t)m * ((size_t)nV * nV + (size_t)nC * nV); }
+    __host__ __device__ const double* s(int m, int nC) const { return S + (size_t)m * nC * nC; }
+    __host__ __device__ const double* a(int m, int nV, int nC) const { return A + (size_t)m * nC * nV; }
 };
 
-// x0 = -Hinv g ; rv0 = A x0 from the problem's set, one CTA per problem: the loops of dense_x0_rv in the same order, so
-// that x0 and A x0 (and with them every later decision) are bit-identical to the seam's.  A problem whose index is out of
-// range is skipped here and flagged by dense_das_kernel.
-__global__ void dense_x0_rv_sets(int n, int nV, int nC, const double* g, DenseSets sets)
+// The x0 step, one CTA per problem: out = alpha [Hinv v | A Hinv v] (alpha = -1, v = g: x0 | A x0 of the solve; alpha = 1,
+// v = dL/dx: p0 | r0 of the adjoint), the row half computed from the stored alpha Hinv v.  Every call uses these loops in
+// this order, so that the seam and one set per problem give the same bytes.  SETS = false: Hinv and out (x0 | rv) in the
+// problem's slice (stride slice), A the caller's, and x (or NULL) also receives the first half; SETS = true: Hinv and A
+// from the problem's set, out in sets.xr (dense_das_kernel copies x0 to x), and a problem whose set index is out of range
+// is skipped here (the warp kernels flag it).  Without x the first half is stored to out twice: a NULL test inside the
+// loop makes the compiler version the loops (half again as many instructions).
+template <bool SETS>
+__global__ void dense_x0_step(int nV, int nC, const double* v, double alpha, const double* Hinv, double* out, size_t slice,
+                              const double* A, DenseSets sets, double* x)
 {
     const size_t p = blockIdx.x;
-    const int m = sets.set_of((int)p);
-    if (m < 0 || m >= sets.n_mat) return;
-    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
-    const double* Hinv = sets.HD + (size_t)m * (vv + cv);
-    const double* gp = g + p * nV;
-    double* x0 = sets.xr + p * (nV + nC);
+    const double* Ap;
+    double* o;
+    if constexpr (SETS) {
+        const int m = sets.set_of((int)p);
+        if (!sets.valid(m)) return;
+        Hinv = sets.hd(m, nV, nC);
+        Ap = sets.a(m, nV, nC);
+        o = sets.xr + p * (nV + nC);
+    } else {
+        Hinv += p * slice;
+        Ap = A + p * (size_t)nC * nV;
+        o = out + p * slice;
+    }
+    const double* vp = v + p * nV;
+    double* xo = SETS || !x ? o : x + p * nV;
     for (int i = threadIdx.x; i < nV; i += blockDim.x) {
         double s = 0.0;
-        for (int j = 0; j < nV; ++j) s += Hinv[(size_t)j * nV + i] * gp[j];
-        x0[i] = -s;
+        for (int j = 0; j < nV; ++j) s += Hinv[(size_t)j * nV + i] * vp[j];
+        o[i] = alpha * s;
+        xo[i] = alpha * s;
     }
     __syncthreads();
-    const double* Ap = sets.A + (size_t)m * cv;
     for (int c = threadIdx.x; c < nC; c += blockDim.x) {
         double s = 0.0;
-        for (int j = 0; j < nV; ++j) s += Ap[(size_t)c * nV + j] * x0[j];
-        x0[nV + c] = s;
+        for (int j = 0; j < nV; ++j) s += Ap[(size_t)c * nV + j] * o[j];
+        o[nV + c] = s;
     }
 }
 
@@ -408,6 +423,9 @@ constexpr int DENSE_WARPS = 4;   // QPs per CTA
 // QPs of nV = 206 with a box: cold 1.36 -> 1.61 s, 20 hot-started ticks 6.6 -> 10.5 s; profiles/r11_dense_seam_as_sets.json).
 // BOUNDS = true: the rows are [I; A] with the box lbx <= x <= ubx (n x nV each, NULL = that side absent) as the first nV
 // (DenseBoundsProb); y, ws and ws_guess are n x (nV + nC), bounds first.  A variable whose bounds cross is flagged.
+// The set lookup below is an inline copy of DenseSets::valid / hd / s, and the kept rows' work + n * stride is
+// DenseCallWork::kept: routing either through the shared code changes the SASS of all eight builds, which
+// tests/golden/dense_das_sass_all.json pins.
 template <bool WARM, bool SETS, bool BOUNDS>
 __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const double* ubA, double* work,
                                  size_t stride, DenseLayout l, int R, double* x, double* y, signed char* ws,
@@ -510,24 +528,45 @@ __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const
     if (lane == 0) { status[p] = st; if (iters) iters[p] = it; }
 }
 
-// The seam's per-call set-up: factor H, Hinv, D and S into each problem's slice (layout l), the factor status into status.
+// Factor n matrices H (already at work + offL, stride sw) into L there and Linv at work + offLinv, then [Hinv; D] (HD, D at
+// HD + nV^2, stride shd) and S (stride ss) from A (stride nC nV); the factor status into status.
+static void dense_factor(int n, int nV, int nC, const double* A, double* work, size_t sw, size_t offL, size_t offLinv,
+                         double* HD, size_t shd, double* S, size_t ss, int32_t* status, int use_dmma, cudaStream_t st)
+{
+    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
+    dense_cholesky<<<n, 256, 0, st>>>(nV, work, sw, offL, status);
+    dense_tri_inverse<<<dim3((nV + 63) / 64, n), 64, 0, st>>>(nV, work, sw, offL, offLinv);
+    // Hinv = Linv' Linv: element (i, k) of the left operand is Linv[k][i] (strides 1, nV); the triangular zeros are
+    // multiplied through (2x the flops of the triangular sum, at several times its speed)
+    dense_gemm_launch(use_dmma, n, nV, nV, nV, work + offLinv, sw, 1, nV, work + offLinv, sw, 1, nV, HD, shd, st);
+    if (nC > 0) {
+        // D (nC x nV) = A (nC x nV) * Hinv' (Hinv symmetric, row-major over k)
+        dense_gemm_launch(use_dmma, n, nC, nV, nV, A, cv, nV, 1, HD, shd, nV, 1, HD + vv, shd, st);
+        // S (nC x nC) = A * D'
+        dense_gemm_launch(use_dmma, n, nC, nC, nV, A, cv, nV, 1, HD + vv, shd, nV, 1, S, ss, st);
+    }
+}
+
+// The seam's per-call set-up: H copied into each problem's slice (layout l; Hinv and D are adjacent there, as in a set),
+// factored there.
 static void dense_setup_launch(int n, int nV, int nC, const double* H, const double* A, const DenseLayout& l, double* work,
                                int32_t* status, int use_dmma, cudaStream_t st)
 {
-    const size_t stride = l.total;
     const size_t vv = (size_t)nV * nV;
-    dense_copy_H<<<dim3((unsigned)((vv + 255) / 256), n), 256, 0, st>>>(nV, H, work, stride, l.Lh);
-    dense_cholesky<<<n, 256, 0, st>>>(nV, work, stride, l.Lh, status);
-    dense_tri_inverse<<<dim3((nV + 63) / 64, n), 64, 0, st>>>(nV, work, stride, l.Lh, l.Linv);
-    // Hinv = Linv' Linv: element (i, k) of the left operand is Linv[k][i] (strides 1, nV); the triangular zeros are
-    // multiplied through (2x the flops of the triangular sum, at several times its speed)
-    dense_gemm_launch(use_dmma, n, nV, nV, nV, work + l.Linv, stride, 1, nV, work + l.Linv, stride, 1, nV, work + l.Hinv, stride, st);
-    if (nC > 0) {
-        // D (nC x nV) = A (nC x nV) * Hinv' (Hinv symmetric, row-major over k)
-        dense_gemm_launch(use_dmma, n, nC, nV, nV, A, (size_t)nC * nV, nV, 1, work + l.Hinv, stride, nV, 1, work + l.D, stride, st);
-        // S (nC x nC) = A * D'
-        dense_gemm_launch(use_dmma, n, nC, nC, nV, A, (size_t)nC * nV, nV, 1, work + l.D, stride, nV, 1, work + l.S, stride, st);
-    }
+    dense_copy_H<<<dim3((unsigned)((vv + 255) / 256), n), 256, 0, st>>>(nV, H, work, l.total, l.Lh);
+    dense_factor(n, nV, nC, A, work, l.total, l.Lh, l.Linv, work + l.Hinv, l.total, work + l.S, l.total, status, use_dmma, st);
+}
+
+// One warp per problem, DENSE_WARPS per CTA; the first R rows of the working set's inverse factor in shared memory.
+static int dense_warp_rows(const DenseLayout& l) { return l.qmax < DENSE_R ? l.qmax : DENSE_R; }
+
+template <typename... P, typename... Args>
+static int dense_warp_launch(void (*kern)(P...), int n, int R, cudaStream_t st, Args... args)
+{
+    const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
+    kern<<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(args...);
+    return (int)cudaGetLastError();
 }
 
 // bounds = false: lbx / ubx unused (ismpc_qp_solve_batch[_ws]); true: the box rows ahead of A (ismpc_qp_solve_batch_bounds)
@@ -536,18 +575,14 @@ int qp_dense_launch(int n, int nV, int nC, const double* H, const double* g, con
                     double* x, double* y, signed char* ws, int32_t* status, int32_t* iters, double* work, int use_dmma,
                     cudaStream_t st)
 {
-    const DenseLayout l = dense_layout(nV, nC, true, bounds);
-    const size_t stride = l.total;
+    const DenseLayout l = dense_call_work(n, nV, nC, bounds, true).l;
     dense_setup_launch(n, nV, nC, H, A, l, work, status, use_dmma, st);
-    dense_x0_rv<<<n, 128, 0, st>>>(nV, nC, g, A, work, stride, l, x);
-    const int R = l.qmax < DENSE_R ? l.qmax : DENSE_R;
-    const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
+    dense_x0_step<false><<<n, 128, 0, st>>>(nV, nC, g, -1.0, work + l.Hinv, work + l.x0, l.total, A, DenseSets{}, x);
     auto kern = bounds ? (ws_guess ? dense_das_kernel<true, false, true> : dense_das_kernel<false, false, true>)
                        : (ws_guess ? dense_das_kernel<true, false, false> : dense_das_kernel<false, false, false>);
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
-    kern<<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
-        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess, DenseSets{}, lbx, ubx);
-    return (int)cudaGetLastError();
+    const int R = dense_warp_rows(l);
+    return dense_warp_launch(kern, n, R, st, n, nV, nC, lbA, ubA, work, l.total, l, R, x, y, ws, status, iters, ws_guess,
+                             DenseSets{}, lbx, ubx);
 }
 
 // ---- resident matrix family ------------------------------------------------------------------------------
@@ -557,12 +592,11 @@ size_t qp_sets_table_doubles(int n_mat, int nV, int nC)
     return (size_t)n_mat * (vv + cv + cc + cv);
 }
 
-// set-up: 2 n_mat nV^2 (Lh | Linv, scratch); per call: n slices of vectors, x0 | A x0 (n x (nV + nC)), A x0 kept for the
-// warm start (n x nC; with bounds x0 | A x0, n x (nV + nC))
+// set-up: 2 n_mat nV^2 (Lh | Linv, scratch); per call: dense_call_work without tables
 size_t qp_sets_work_doubles(int n, int n_mat, int nV, int nC, bool bounds)
 {
     const size_t setup = 2 * (size_t)n_mat * nV * nV;
-    const size_t call = (dense_layout(nV, nC, false, bounds).total + nV + 2 * (size_t)nC + (bounds ? nV : 0)) * n;
+    const size_t call = dense_call_work(n, nV, nC, bounds, false).total;
     return (setup > call ? setup : call) + 16;
 }
 
@@ -570,18 +604,10 @@ size_t qp_sets_work_doubles(int n, int n_mat, int nV, int nC, bool bounds)
 // device) is already copied into the Lh scratch (work, stride nV^2), A into the set's copy.
 int qp_sets_build(int n_mat, int nV, int nC, double* tab, int32_t* fstat, double* work, int use_dmma, cudaStream_t st)
 {
-    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV, cc = (size_t)nC * nC;
-    double* HD = tab;
-    double* S = HD + (size_t)n_mat * (vv + cv);
-    const double* A = S + (size_t)n_mat * cc;
-    const size_t offLinv = (size_t)n_mat * vv;
-    dense_cholesky<<<n_mat, 256, 0, st>>>(nV, work, vv, 0, fstat);
-    dense_tri_inverse<<<dim3((nV + 63) / 64, n_mat), 64, 0, st>>>(nV, work, vv, 0, offLinv);
-    dense_gemm_launch(use_dmma, n_mat, nV, nV, nV, work + offLinv, vv, 1, nV, work + offLinv, vv, 1, nV, HD, vv + cv, st);
-    if (nC > 0) {
-        dense_gemm_launch(use_dmma, n_mat, nC, nV, nV, A, cv, nV, 1, HD, vv + cv, nV, 1, HD + vv, vv + cv, st);
-        dense_gemm_launch(use_dmma, n_mat, nC, nC, nV, A, cv, nV, 1, HD + vv, vv + cv, nV, 1, S, cc, st);
-    }
+    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
+    double* S = tab + (size_t)n_mat * (vv + cv);
+    dense_factor(n_mat, nV, nC, S + (size_t)n_mat * nC * nC, work, vv, 0, (size_t)n_mat * vv, tab, vv + cv, S, (size_t)nC * nC,
+                 fstat, use_dmma, st);
     return (int)cudaGetLastError();
 }
 
@@ -604,21 +630,17 @@ int qp_sets_launch(int n, int nV, int nC, int n_mat, const double* tab, const in
                    const double* ubx, const signed char* ws_guess, double* x, double* y, signed char* ws, int32_t* status,
                    int32_t* iters, double* work, int use_gemm, int use_dmma, cudaStream_t st)
 {
-    const DenseLayout l = dense_layout(nV, nC, false, bounds);
-    const size_t stride = l.total;
-    const DenseSets sets = dense_sets(n_mat, nV, nC, tab, fstat, idx, work + (size_t)n * (stride + nC + (bounds ? nV : 0)));
+    const DenseCallWork cw = dense_call_work(n, nV, nC, bounds, false);
+    const DenseSets sets = dense_sets(n_mat, nV, nC, tab, fstat, idx, work + cw.xr);
     if (n_mat == 1 && use_gemm)
-        dense_gemm_launch(use_dmma, 1, n, nV + nC, nV, g, 0, nV, 1, sets.HD, 0, nV, 1, sets.xr, 0, st, -1.0);
+        dense_gemm_launch(use_dmma, 1, n, nV + nC, nV, g, 0, nV, 1, sets.hd(0, nV, nC), 0, nV, 1, sets.xr, 0, st, -1.0);
     else
-        dense_x0_rv_sets<<<n, 128, 0, st>>>(n, nV, nC, g, sets);
-    const int R = l.qmax < DENSE_R ? l.qmax : DENSE_R;
-    const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
+        dense_x0_step<true><<<n, 128, 0, st>>>(nV, nC, g, -1.0, nullptr, nullptr, 0, nullptr, sets, nullptr);
     auto kern = bounds ? (ws_guess ? dense_das_kernel<true, true, true> : dense_das_kernel<false, true, true>)
                        : (ws_guess ? dense_das_kernel<true, true, false> : dense_das_kernel<false, true, false>);
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
-    kern<<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
-        n, nV, nC, lbA, ubA, work, stride, l, R, x, y, ws, status, iters, ws_guess, sets, lbx, ubx);
-    return (int)cudaGetLastError();
+    const int R = dense_warp_rows(cw.l);
+    return dense_warp_launch(kern, n, R, st, n, nV, nC, lbA, ubA, work, cw.l.total, cw.l, R, x, y, ws, status, iters, ws_guess,
+                             sets, lbx, ubx);
 }
 
 // ---- the adjoint of the bounds calls (ismpc_qp_adjoint_batch / ismpc_qp_hotstart_adjoint_batch) --------------------
@@ -627,40 +649,6 @@ int qp_sets_launch(int n, int nV, int nC, int n_mat, const double* tab, const in
 // In the engine's terms this is the warm start's install with g := -v and every right-hand side zero: p0 = Hinv v and
 // r0 = A p0 (the forward's x0 | A x0), every ws entry installed factor-only, mu = J'J (0 - N_W' p0), no drops, then
 // p = p0 + sum_k mu_k sg_k Hinv a_k and q_{id_k} = -sg_k mu_k.
-
-// [p0 | r0] = [Hinv v | A Hinv v], one CTA per problem: the loops of dense_x0_rv / dense_x0_rv_sets in the same order, so
-// that the seam and one set per problem give the same bytes.  SETS = false: Hinv from the problem's slice, A the caller's.
-// A problem whose set index is out of range is skipped here and flagged by dense_adjoint_kernel.
-template <bool SETS>
-__global__ void dense_adjoint_p0(int nV, int nC, const double* v, const double* A, const double* work, size_t stride,
-                                 DenseLayout l, DenseSets sets, double* pr, size_t spr)
-{
-    const size_t p = blockIdx.x;
-    const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
-    const double *Hinv, *Ap;
-    if constexpr (SETS) {
-        const int m = sets.set_of((int)p);
-        if (m < 0 || m >= sets.n_mat) return;
-        Hinv = sets.HD + (size_t)m * (vv + cv);
-        Ap = sets.A + (size_t)m * cv;
-    } else {
-        Hinv = work + p * stride + l.Hinv;
-        Ap = A + p * cv;
-    }
-    const double* vp = v + p * nV;
-    double* p0 = pr + p * spr;
-    for (int i = threadIdx.x; i < nV; i += blockDim.x) {
-        double s = 0.0;
-        for (int j = 0; j < nV; ++j) s += Hinv[(size_t)j * nV + i] * vp[j];
-        p0[i] = s;
-    }
-    __syncthreads();
-    for (int c = threadIdx.x; c < nC; c += blockDim.x) {
-        double s = 0.0;
-        for (int j = 0; j < nV; ++j) s += Ap[(size_t)c * nV + j] * p0[j];
-        p0[nV + c] = s;
-    }
-}
 
 // One warp per problem, DENSE_WARPS per CTA; the first R rows of J in shared memory, the rest in the slice (layout l, the
 // bounds layout of dense_das_kernel).  pr: [p0 | r0] of problem p at pr + p * spr.  SETS as in dense_das_kernel: a
@@ -688,13 +676,12 @@ __global__ void dense_adjoint_kernel(int n, int nV, int nC, double* work, size_t
     int st;
     if constexpr (SETS) {
         const int m = sets.set_of(p);
-        if (m < 0 || m >= sets.n_mat) {
+        if (!sets.valid(m)) {
             if (lane == 0) status[p] = ISMPC_ST_QP_FAIL;
             return;
         }
-        const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
-        HD = sets.HD + (size_t)m * (vv + cv);
-        S = sets.S + (size_t)m * nC * nC;
+        HD = sets.hd(m, nV, nC);
+        S = sets.s(m, nC);
         st = sets.fstat[m];
     } else {
         HD = w + l.Hinv;
@@ -744,32 +731,21 @@ __global__ void dense_adjoint_kernel(int n, int nV, int nC, double* work, size_t
     if (lane == 0) status[p] = 0;
 }
 
-template <bool SETS>
-static int dense_adjoint_run(int n, int nV, int nC, double* work, const DenseLayout& l, const signed char* ws,
-                             const double* pr, size_t spr, double* p, double* q, int32_t* status, const DenseSets& sets,
-                             cudaStream_t st)
-{
-    const int R = l.qmax < DENSE_R ? l.qmax : DENSE_R;
-    const size_t sbytes = (size_t)tri(R, 0) * sizeof(double) * DENSE_WARPS;
-    cudaFuncSetAttribute(dense_adjoint_kernel<SETS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
-    dense_adjoint_kernel<SETS><<<(n + DENSE_WARPS - 1) / DENSE_WARPS, 32 * DENSE_WARPS, sbytes, st>>>(
-        n, nV, nC, work, l.total, l, R, ws, pr, spr, p, q, status, sets);
-    return (int)cudaGetLastError();
-}
-
-// The seam: set-up as qp_dense_launch (status = the factor status), [p0 | r0] in the slice's x0 | rv.
+// The seam: set-up as qp_dense_launch (status = the factor status), [p0 | r0] in the slice's x0 | rv; no kept rows.
 size_t qp_dense_adjoint_work_doubles(int n, int nV, int nC)
 {
-    return dense_layout(nV, nC, true, true).total * (size_t)n + 16;
+    return dense_call_work(n, nV, nC, true, true).kept + 16;
 }
 
 int qp_dense_adjoint_launch(int n, int nV, int nC, const double* H, const double* A, const signed char* ws, const double* v,
                             double* p, double* q, int32_t* status, double* work, int use_dmma, cudaStream_t st)
 {
-    const DenseLayout l = dense_layout(nV, nC, true, true);
+    const DenseLayout l = dense_call_work(n, nV, nC, true, true).l;
     dense_setup_launch(n, nV, nC, H, A, l, work, status, use_dmma, st);
-    dense_adjoint_p0<false><<<n, 128, 0, st>>>(nV, nC, v, A, work, l.total, l, DenseSets{}, work + l.x0, l.total);
-    return dense_adjoint_run<false>(n, nV, nC, work, l, ws, work + l.x0, l.total, p, q, status, DenseSets{}, st);
+    dense_x0_step<false><<<n, 128, 0, st>>>(nV, nC, v, 1.0, work + l.Hinv, work + l.x0, l.total, A, DenseSets{}, nullptr);
+    const int R = dense_warp_rows(l);
+    return dense_warp_launch(dense_adjoint_kernel<false>, n, R, st, n, nV, nC, work, l.total, l, R, ws, work + l.x0, l.total,
+                             p, q, status, DenseSets{});
 }
 
 // Against the resident sets (workspace qp_sets_work_doubles(n, n_mat, nV, nC, true)): [p0 | r0] where the forward keeps
@@ -778,13 +754,15 @@ int qp_sets_adjoint_launch(int n, int nV, int nC, int n_mat, const double* tab, 
                            const signed char* ws, const double* v, double* p, double* q, int32_t* status, double* work,
                            int use_gemm, int use_dmma, cudaStream_t st)
 {
-    const DenseLayout l = dense_layout(nV, nC, false, true);
-    const DenseSets sets = dense_sets(n_mat, nV, nC, tab, fstat, idx, work + (size_t)n * (l.total + nC + nV));
+    const DenseCallWork cw = dense_call_work(n, nV, nC, true, false);
+    const DenseSets sets = dense_sets(n_mat, nV, nC, tab, fstat, idx, work + cw.xr);
     if (n_mat == 1 && use_gemm)
-        dense_gemm_launch(use_dmma, 1, n, nV + nC, nV, v, 0, nV, 1, sets.HD, 0, nV, 1, sets.xr, 0, st);
+        dense_gemm_launch(use_dmma, 1, n, nV + nC, nV, v, 0, nV, 1, sets.hd(0, nV, nC), 0, nV, 1, sets.xr, 0, st);
     else
-        dense_adjoint_p0<true><<<n, 128, 0, st>>>(nV, nC, v, nullptr, nullptr, 0, l, sets, sets.xr, nV + nC);
-    return dense_adjoint_run<true>(n, nV, nC, work, l, ws, sets.xr, nV + nC, p, q, status, sets, st);
+        dense_x0_step<true><<<n, 128, 0, st>>>(nV, nC, v, 1.0, nullptr, nullptr, 0, nullptr, sets, nullptr);
+    const int R = dense_warp_rows(cw.l);
+    return dense_warp_launch(dense_adjoint_kernel<true>, n, R, st, n, nV, nC, work, cw.l.total, cw.l, R, ws, sets.xr, nV + nC,
+                             p, q, status, sets);
 }
 
 }  // namespace ismpc

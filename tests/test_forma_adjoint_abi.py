@@ -1,21 +1,14 @@
 """ismpc_forma_adjoint_batch (gradients of the formulation-A tick) without a GPU: argument checks before the device is
 touched in both memory modes, ISMPC_ERR_MODEL without a model, and the kernels -- forma_adjoint_kernel compiles for sm_100a
 without spills, and every existing form-A kernel keeps the SASS it had before the tick's build was shared with it."""
-import hashlib
-import json
-import os
 import re
-import shutil
-import subprocess
 
 import numpy as np
-import pytest
 
+import sass_golden
 from quadruped_gait_generation_ismpc_b200 import abi, binding
 
 ISMPC_ERR_ARG, ISMPC_ERR_MODEL = -1, -3      # include/ismpc_b200.h
-HERE = os.path.dirname(os.path.abspath(__file__))
-CSRC = os.path.join(os.path.dirname(HERE), "quadruped_gait_generation_ismpc_b200", "csrc")
 
 
 def test_adjoint_rejects_bad_arguments_without_touching_outputs():
@@ -54,39 +47,17 @@ def test_adjoint_rejects_bad_arguments_without_touching_outputs():
     assert (grad["height"] == 5.0).all() and (gp == 5.0).all()
 
 
-def _sass(cuobjdump, obj):
-    out = subprocess.run([cuobjdump, "-sass", obj], capture_output=True, text=True, check=True).stdout
-    res, cur = {}, None
-    for line in out.splitlines():
-        m = re.match(r"\s*Function : (\S+)", line)
-        if m:
-            cur = m.group(1); res[cur] = []
-        elif cur and line.strip() and not line.strip().startswith("."):
-            res[cur].append(line.strip())
-    return res
-
-
 def test_adjoint_kernel_compiles_without_spills_and_every_forma_kernel_keeps_its_sass(tmp_path):
     """Compiles forma_kernels.cu with the library's flags.  forma_adjoint_kernel exists and spills nothing; the SASS of
     every tick, rollout and fold kernel, symbol names kept, hashes to what it was before the adjoint existed
     (tests/golden/forma_sass.json, recorded with the nvcc named there; another nvcc may schedule differently)."""
-    nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-    if not os.path.exists(nvcc):
-        pytest.skip("no nvcc")
-    golden = json.load(open(os.path.join(HERE, "golden", "forma_sass.json")))
-    obj = str(tmp_path / "forma_kernels.o")
-    r = subprocess.run([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler",
-                        "-fPIC", "--fmad=true", "-Xptxas", "-v", "-c", os.path.join(CSRC, "forma_kernels.cu"), "-o", obj],
-                       capture_output=True, text=True, check=True)
-    log = r.stderr.split("Compiling entry function")
+    gold = sass_golden.golden("forma_sass.json")
+    funcs, stderr = sass_golden.compile_sass("forma_kernels.cu", tmp_path, ["-Xptxas", "-v"])
+    log = stderr.split("Compiling entry function")
     adj = [blk for blk in log if "forma_adjoint_kernel" in blk.splitlines()[0]]
     assert len(adj) == 1
     assert re.search(r"\b0 bytes spill stores, 0 bytes spill loads", adj[0]), adj[0]
-    funcs = _sass(os.path.join(os.path.dirname(nvcc), "cuobjdump"), obj)
-    assert sorted(k for k in funcs if "forma_adjoint_kernel" not in k) == sorted(golden["kernels"])
-    version = re.search(r"release \S+, V(\S+)", subprocess.run([nvcc, "--version"], capture_output=True,
-                                                                text=True).stdout).group(1)
-    if version != golden["nvcc"]:
-        pytest.skip("SASS recorded with nvcc %s, this is %s" % (golden["nvcc"], version))
-    for name, digest in golden["kernels"].items():
-        assert hashlib.sha256("\n".join(funcs[name]).encode()).hexdigest() == digest, name
+    assert sorted(k for k in funcs if "forma_adjoint_kernel" not in k) == sorted(gold["kernels"])
+    sass_golden.skip_unless_recorded_nvcc(gold)
+    for name, digest in gold["kernels"].items():
+        assert sass_golden.digest(funcs[name]) == digest, name

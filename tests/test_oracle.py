@@ -365,9 +365,7 @@ def test_horizontal_qp_is_a_knapsack_problem():
 def test_portable_solver_on_infeasible_qps():
     """The portable dual active set reports infeasible QPs as such (never a buffer overrun, never ret = 0 with a point that
     violates its rows) and agrees with qpOASES' return code where oracle/_ref is present."""
-    import sys, os
-    sys.path.insert(0, os.path.dirname(__file__))
-    from test_qp_dense_gpu import _infeasible_batch
+    from dense_cases import _infeasible_batch
     H, g, A, lb, ub = _infeasible_batch()
     p = O.qp_batch(H, g, A, lb, ub, solver=O.SOLVER_PORT)
     assert (p["ret"][0::2] != 0).all() and (p["ret"][1::2] == 0).all(), p["ret"]

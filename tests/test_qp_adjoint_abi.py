@@ -2,22 +2,18 @@
 before the device is touched, qp_torch.route_gradients against the chain rule through a numpy KKT solve, and the kernels --
 dense_adjoint_kernel compiles for sm_100a and every dense_das_kernel build keeps the SASS it had before the adjoint
 existed."""
-import hashlib
-import json
 import os
 import re
-import shutil
-import subprocess
 
 import numpy as np
-import pytest
 import torch
 
+import sass_golden
 from quadruped_gait_generation_ismpc_b200 import abi, binding, qp_torch
+from dense_cases import _kkt_adjoint, _planted
 
 ISMPC_ERR_ARG = -1      # include/ismpc_b200.h
 HERE = os.path.dirname(os.path.abspath(__file__))
-CSRC = os.path.join(os.path.dirname(HERE), "quadruped_gait_generation_ismpc_b200", "csrc")
 
 
 def test_adjoint_entry_points_reject_bad_arguments_without_touching_outputs():
@@ -65,39 +61,6 @@ def test_adjoint_entry_points_reject_bad_arguments_without_touching_outputs():
     assert (p == 5.0).all() and (q == 5.0).all() and (st == 9).all()
 
 
-def _planted(rng, n, nV, nC):
-    """QP data with a planted solution: x, a working set over [I; A] (lower, upper and equality entries) with multipliers of
-    the right sign, g = A_W' y_W - H x, and bounds tight on W and slack off it."""
-    M = rng.normal(size=(n, nV, nV))
-    H = M @ M.transpose(0, 2, 1) / nV + np.eye(nV)
-    A = rng.normal(size=(n, nC, nV))
-    x = rng.normal(size=(n, nV))
-    ws = rng.choice([-1, 0, 0, 1], size=(n, nV + nC)).astype(np.int8)
-    ws[:, nV // 2:nV] = 0; ws[:, nV + nC // 2:] = 0              # keep |W| < nV
-    y = np.where(ws < 0, 1.0, np.where(ws > 0, -1.0, 0.0)) * rng.uniform(0.5, 2.0, ws.shape)
-    ws[:, nV] = -1                                                # an equality row: free-signed multiplier
-    y[:, nV] = rng.normal(size=n)
-    Ae = np.concatenate([np.broadcast_to(np.eye(nV), (n, nV, nV)), A], axis=1)
-    g = np.einsum("nji,nj->ni", Ae, y) - np.einsum("nij,nj->ni", H, x)
-    r = np.einsum("nij,nj->ni", Ae, x)
-    lo = np.where(ws < 0, r, r - rng.uniform(0.5, 1.0, r.shape)); hi = np.where(ws > 0, r, r + rng.uniform(0.5, 1.0, r.shape))
-    hi[:, nV] = lo[:, nV]
-    return H, g, A, Ae, x, y, ws, lo, hi
-
-
-def _kkt_adjoint(H, Ae, ws, v):
-    """(p, q) of H p + A_W' q = v, A_W p = 0 by one dense KKT solve per problem."""
-    n, nV = v.shape
-    p = np.zeros((n, nV)); q = np.zeros(ws.shape)
-    for k in range(n):
-        W = np.flatnonzero(ws[k])
-        AW = Ae[k, W]
-        K = np.block([[H[k], AW.T], [AW, np.zeros((len(W), len(W)))]])
-        s = np.linalg.solve(K, np.concatenate([v[k], np.zeros(len(W))]))
-        p[k] = s[:nV]; q[k, W] = s[nV:]
-    return p, q
-
-
 def test_route_gradients_is_the_chain_rule_through_the_kkt_system():
     """d(v'x) along a random direction of each input, from the linearised KKT system of the planted working set, equals
     <route_gradients(..)[input], direction>."""
@@ -140,39 +103,18 @@ def test_route_gradients_is_the_chain_rule_through_the_kkt_system():
             assert abs(got - want) <= 1e-10 * max(1.0, abs(want)), (k, name, got, want)
 
 
-def _sass(cuobjdump, obj):
-    out = subprocess.run([cuobjdump, "-sass", obj], capture_output=True, text=True, check=True).stdout
-    res, cur = {}, None
-    for line in out.splitlines():
-        m = re.match(r"\s*Function : (\S+)", line)
-        if m:
-            cur = m.group(1); res[cur] = []
-        elif cur and line.strip() and not line.strip().startswith("."):
-            res[cur].append(line.strip())
-    return res
-
-
 def test_adjoint_kernel_compiles_and_every_active_set_build_keeps_its_sass(tmp_path):
     """Compiles qp_dense.cu with the library's flags.  dense_adjoint_kernel<SETS> exists for both SETS; the SASS of all
     eight dense_das_kernel<WARM, SETS, BOUNDS> builds, symbol names stripped, hashes to what it was before the adjoint
     existed (tests/golden/dense_das_sass_all.json, recorded with the nvcc named there; another nvcc may schedule
     differently)."""
-    nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-    if not os.path.exists(nvcc):
-        pytest.skip("no nvcc")
-    golden = json.load(open(os.path.join(HERE, "golden", "dense_das_sass_all.json")))
-    obj = str(tmp_path / "qp_dense.o")
-    subprocess.run([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler",
-                    "-fPIC", "--fmad=true", "-c", os.path.join(CSRC, "qp_dense.cu"), "-o", obj], check=True)
-    funcs = _sass(os.path.join(os.path.dirname(nvcc), "cuobjdump"), obj)
+    gold = sass_golden.golden("dense_das_sass_all.json")
+    funcs, _ = sass_golden.compile_sass("qp_dense.cu", tmp_path)
     adj = sorted(re.search(r"dense_adjoint_kernelILb(\d)EEE", k).group(1) for k in funcs if "dense_adjoint_kernel" in k)
     assert adj == ["0", "1"]
     kern = {"WARM=%s,SETS=%s,BOUNDS=%s" % re.search(r"dense_das_kernelILb(\d)ELb(\d)ELb(\d)EEE", k).groups():
-            hashlib.sha256("\n".join(v).encode()).hexdigest() for k, v in funcs.items() if "dense_das_kernel" in k}
-    assert sorted(kern) == sorted(golden["kernels"])
-    version = re.search(r"release \S+, V(\S+)", subprocess.run([nvcc, "--version"], capture_output=True,
-                                                                text=True).stdout).group(1)
-    if version != golden["nvcc"]:
-        pytest.skip("SASS recorded with nvcc %s, this is %s" % (golden["nvcc"], version))
-    for name, digest in golden["kernels"].items():
+            sass_golden.digest(v) for k, v in funcs.items() if "dense_das_kernel" in k}
+    assert sorted(kern) == sorted(gold["kernels"])
+    sass_golden.skip_unless_recorded_nvcc(gold)
+    for name, digest in gold["kernels"].items():
         assert kern[name] == digest, name

@@ -6,8 +6,7 @@ import pytest
 import torch
 
 from quadruped_gait_generation_ismpc_b200 import abi, qp_torch, synth
-from test_qp_adjoint_abi import _planted
-from test_qp_bounds_gpu import _box_qps, _forma_box
+from dense_cases import _box_qps, _forma_box, _planted
 
 pytestmark = pytest.mark.gpu
 FAIL = 64                                  # ISMPC_ST_QP_FAIL

@@ -7,7 +7,7 @@ import torch
 
 from oracle import oracle as O
 from quadruped_gait_generation_ismpc_b200 import qp_torch
-from test_qp_adjoint_abi import _kkt_adjoint, _planted
+from dense_cases import _kkt_adjoint, _planted
 
 
 def _solve(H, g, A, lb, ub, lbA, ubA):

@@ -1,21 +1,12 @@
 """ismpc_qp_solve_batch_bounds / ismpc_qp_hotstart_batch_bounds (box bounds in the dense QP seam): argument checks before
-the device is touched, synth.dense_split_bounds, and the kernels -- the bounds instantiations compile for sm_100a and the
-instantiations without bounds compile to the SASS they had before bounds existed."""
-import hashlib
-import json
-import os
-import re
-import shutil
-import subprocess
-
+the device is touched, and synth.dense_split_bounds.  The SASS of every dense_das_kernel build is pinned by
+test_qp_adjoint_abi."""
 import numpy as np
 import pytest
 
 from quadruped_gait_generation_ismpc_b200 import abi, binding, synth
 
 ISMPC_ERR_ARG = -1      # include/ismpc_b200.h
-HERE = os.path.dirname(os.path.abspath(__file__))
-CSRC = os.path.join(os.path.dirname(HERE), "quadruped_gait_generation_ismpc_b200", "csrc")
 
 
 def test_bounds_entry_points_reject_bad_arguments_without_touching_outputs():
@@ -66,40 +57,3 @@ def test_split_bounds_restacks_to_the_original(shape):
         np.testing.assert_allclose(back, orig, rtol=1e-15, atol=0)
     unmoved = np.setdiff1d(np.arange(nV), d["row_map"])
     assert (d["lb"][:, unmoved] == -1e20).all() and (d["ub"][:, unmoved] == 1e20).all()
-
-
-def _sass(cuobjdump, obj):
-    out = subprocess.run([cuobjdump, "-sass", obj], capture_output=True, text=True, check=True).stdout
-    res, cur = {}, None
-    for line in out.splitlines():
-        m = re.match(r"\s*Function : (\S+)", line)
-        if m:
-            cur = m.group(1); res[cur] = []
-        elif cur and line.strip() and not line.strip().startswith("."):
-            res[cur].append(line.strip())
-    return res
-
-
-def test_kernels_compile_and_the_instantiations_without_bounds_keep_their_sass(tmp_path):
-    """Compiles qp_dense.cu with the library's flags.  The SASS of dense_das_kernel<WARM, SETS, false>, symbol names
-    stripped, must hash to what dense_das_kernel<WARM, SETS> compiled to before the BOUNDS flag existed
-    (tests/golden/dense_das_sass.json, recorded with the nvcc named there; another nvcc may schedule differently)."""
-    nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-    if not os.path.exists(nvcc):
-        pytest.skip("no nvcc")
-    golden = json.load(open(os.path.join(HERE, "golden", "dense_das_sass.json")))
-    obj = str(tmp_path / "qp_dense.o")
-    subprocess.run([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler",
-                    "-fPIC", "--fmad=true", "-c", os.path.join(CSRC, "qp_dense.cu"), "-o", obj], check=True)
-    funcs = _sass(os.path.join(os.path.dirname(nvcc), "cuobjdump"), obj)
-    kern = {re.search(r"dense_das_kernelILb(\d)ELb(\d)ELb(\d)EEE", k).groups(): v
-            for k, v in funcs.items() if "dense_das_kernel" in k}
-    assert sorted(kern) == [(w, s, b) for w in "01" for s in "01" for b in "01"]
-    version = re.search(r"release \S+, V(\S+)", subprocess.run([nvcc, "--version"], capture_output=True,
-                                                                text=True).stdout).group(1)
-    if version != golden["nvcc"]:
-        pytest.skip("SASS recorded with nvcc %s, this is %s" % (golden["nvcc"], version))
-    for w in "01":
-        for s in "01":
-            digest = hashlib.sha256("\n".join(kern[(w, s, "0")]).encode()).hexdigest()
-            assert digest == golden["kernels"]["WARM=%s,SETS=%s" % (w, s)], (w, s)

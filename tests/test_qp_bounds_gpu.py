@@ -7,30 +7,9 @@ import pytest
 
 from quadruped_gait_generation_ismpc_b200 import abi, synth
 from oracle import oracle as O
-from test_qp_warm_gpu import _same_as_cold, _oracle_parity, _forma_midgait, _forma_dense
+from dense_cases import _box_qps, _forma_box, _forma_dense, _forma_midgait, _oracle_parity, _same_as_cold
 
 pytestmark = pytest.mark.gpu
-
-
-def _box_qps(seed, n, nV, nC):
-    """Dense QPs around a feasible point x0: rows as in the hot-start tests (two equalities, one-sided rows) when nC > 0,
-    and a box mixing finite, lower-only, upper-only, absent and fixed sides."""
-    rng = np.random.default_rng(seed)
-    M = rng.normal(size=(n, nV, nV))
-    H = M @ M.transpose(0, 2, 1) / nV + np.eye(nV)
-    g = 3.0 * rng.normal(size=(n, nV)); A = rng.normal(size=(n, nC, nV))
-    x0 = rng.normal(size=(n, nV))
-    ax = np.einsum("nij,nj->ni", A, x0)
-    lbA = ax - rng.uniform(0.05, 1.0, size=(n, nC)); ubA = ax + rng.uniform(0.05, 1.0, size=(n, nC))
-    if nC >= 8:
-        lbA[:, :2] = ubA[:, :2] = ax[:, :2]
-        lbA[:, 2:5] = -1e20; ubA[:, 5:8] = 1e20
-    lb = x0 - rng.uniform(0.02, 0.5, size=(n, nV)); ub = x0 + rng.uniform(0.02, 0.5, size=(n, nV))
-    kind = rng.integers(0, 5, size=(n, nV))          # 0, 1 finite, 2 lower only, 3 upper only, 4 absent
-    lb[kind == 3] = -1e20; ub[kind == 2] = 1e20
-    lb[kind == 4] = -1e20; ub[kind == 4] = 1e20
-    lb[:, nV // 2] = ub[:, nV // 2] = x0[:, nV // 2]  # one fixed variable per problem
-    return H, g, A, lb, ub, lbA, ubA
 
 
 def _stack(H, g, A, lb, ub, lbA, ubA):
@@ -66,15 +45,6 @@ def _split(shape, n):
     H, g, A, lbA, ubA = synth.dense_qp_batch(shape, n)
     d = synth.dense_split_bounds(H, g, A, lbA, ubA)
     return d["H"], d["g"], d["A"], d["lb"], d["ub"], d["lbA"], d["ubA"]
-
-
-def _forma_box(handle, n):
-    """forma_stacked with a box on every variable, feasible and binding: around the rows' minimiser for a perturbed g."""
-    H, g, A, lbA, ubA = synth.dense_qp_batch("forma_stacked", n)
-    rng = np.random.default_rng(11)
-    xf = handle.qp_solve_batch(H, g + rng.normal(0.0, 0.5, g.shape), A, lbA, ubA)["x"]
-    w = rng.uniform(0.002, 0.05, size=xf.shape)
-    return H, g, A, xf - w, xf + w[:, ::-1], lbA, ubA
 
 
 def _workloads(handle):

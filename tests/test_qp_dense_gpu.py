@@ -7,6 +7,7 @@ import pytest
 from quadruped_gait_generation_ismpc_b200 import abi, synth
 from oracle import oracle as O
 from parity import PRIMAL_TOL, primal_rel_err, active_set_mismatch
+from dense_cases import _infeasible_batch
 
 pytestmark = pytest.mark.gpu
 
@@ -135,25 +136,6 @@ def test_unconstrained_and_infeasible(handle):
     r2 = handle.qp_solve_batch(H, g, A, lb2, ub2)
     assert (r2["status"] == 0).all()
     np.testing.assert_allclose(r2["x"], -np.linalg.solve(H, g[..., None])[..., 0], rtol=1e-9, atol=1e-10)
-
-
-def _infeasible_batch(seed=17, n=32, nV=14, nC=24):
-    """Strictly convex QPs of which every second one is infeasible: two parallel rows with disjoint intervals, and for
-    a few a whole cone of rows that pushes the working set to nV rows before the contradiction shows."""
-    rng = np.random.default_rng(seed)
-    M = rng.normal(size=(n, nV, nV))
-    H = M @ M.transpose(0, 2, 1) / nV + np.eye(nV)
-    g = rng.normal(size=(n, nV)); A = rng.normal(size=(n, nC, nV))
-    x0 = rng.normal(size=(n, nV))
-    ax = np.einsum("nij,nj->ni", A, x0)
-    lb = ax - rng.uniform(0.1, 1.0, size=(n, nC)); ub = ax + rng.uniform(0.1, 1.0, size=(n, nC))
-    for i in range(0, n, 2):
-        A[i, -1] = A[i, 3]
-        lb[i, -1] = ub[i, 3] + 0.5; ub[i, -1] = ub[i, 3] + 1.0          # row 3 and the last row cannot both hold
-        if i % 4 == 0:                                                   # tight box on every variable first
-            A[i, :nV] = np.eye(nV); lb[i, :nV] = x0[i] - 1e-3; ub[i, :nV] = x0[i] + 1e-3
-            A[i, -1] = 1.0; lb[i, -1] = x0[i].sum() + 1.0; ub[i, -1] = x0[i].sum() + 2.0
-    return H, g, A, lb, ub
 
 
 def test_infeasible_dense_qps_are_flagged_like_qpoases(handle):

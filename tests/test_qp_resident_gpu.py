@@ -8,7 +8,7 @@ from quadruped_gait_generation_ismpc_b200 import abi, synth
 from quadruped_gait_generation_ismpc_b200.binding import IsmpcError
 from oracle import oracle as O
 from parity import PRIMAL_TOL, primal_rel_err
-from test_qp_warm_gpu import _forma_dense, _forma_midgait, _infeasible_batch, _oracle_parity, _random_qps, _same_as_cold
+from dense_cases import _forma_dense, _forma_midgait, _infeasible_batch, _oracle_parity, _random_qps, _same_as_cold
 
 pytestmark = pytest.mark.gpu
 
