@@ -508,7 +508,12 @@ int ismpc_kf_filter_batch_f64(ismpc_handle* h, int n, int n_steps, const ismpc_k
  * min 1/2 x'Hx + g'x  s.t. lbA <= A x <= ubA.  H: n x nV x nV, g: n x nV, A: n x nC x nV (row-major),
  * lbA/ubA: n x nC.  x: n x nV.  y_opt (nullable): n x nC constraint duals (qpOASES sign);
  * ws_opt (nullable): n x nC int8 working set; status: n int32 (0 ok, ISMPC_ST_QP_FAIL otherwise);
- * iters_opt (nullable): n int32. */
+ * iters_opt (nullable): n int32.
+ * Accepted shapes, for every call of the dense seam (the resident sets and the adjoints too): 1 <= nV <= ISMPC_MAX_N and
+ * 0 <= nC <= 2 ISMPC_MAX_N + 8; anything else is ISMPC_ERR_ARG.  Batch sizes: 0 <= n <= the handle's max_batch, and
+ * 0 <= n_mat <= max_batch for ismpc_qp_set_matrices; batches past 65,535 problems are factored in slices of 65,535 with
+ * the bytes of the same problems solved in smaller calls.  The working set holds up to nV independent rows (a vertex
+ * of the feasible set is a valid solution). */
 int ismpc_qp_solve_batch(ismpc_handle* h, int n, int nV, int nC,
                          const double* H, const double* g, const double* A,
                          const double* lbA, const double* ubA,

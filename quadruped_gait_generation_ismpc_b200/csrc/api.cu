@@ -920,7 +920,7 @@ extern "C" int ismpc_qp_set_matrices(ismpc_handle* h, int n_mat, int nV, int nC,
                                      int32_t* mat_status_opt, int mem)
 {
     if (!h) return ISMPC_ERR_ARG;
-    if (n_mat < 0 || n_mat > h->max_batch || n_mat > 65535 || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
+    if (n_mat < 0 || n_mat > h->max_batch || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
         return ISMPC_ERR_ARG;
     if (n_mat == 0) { h->r_nmat = 0; return ISMPC_OK; }
     if (!qp_shape_ok(nV, nC) || !H || (nC > 0 && !A)) return ISMPC_ERR_ARG;

@@ -529,31 +529,45 @@ __global__ void dense_das_kernel(int n, int nV, int nC, const double* lbA, const
 }
 
 // Factor n matrices H (already at work + offL, stride sw) into L there and Linv at work + offLinv, then [Hinv; D] (HD, D at
-// HD + nV^2, stride shd) and S (stride ss) from A (stride nC nV); the factor status into status.
+// HD + nV^2, stride shd) and S (stride ss) from A (stride nC nV); the factor status into status.  The triangular inverse and
+// the products put the problem on grid y / z, which stops at DENSE_GRID_YZ: a larger batch runs in slices of that many
+// problems from offset base pointers (each problem's bytes do not depend on the slice it is in).
+constexpr int DENSE_GRID_YZ = 65535;
+
 static void dense_factor(int n, int nV, int nC, const double* A, double* work, size_t sw, size_t offL, size_t offLinv,
                          double* HD, size_t shd, double* S, size_t ss, int32_t* status, int use_dmma, cudaStream_t st)
 {
     const size_t vv = (size_t)nV * nV, cv = (size_t)nC * nV;
     dense_cholesky<<<n, 256, 0, st>>>(nV, work, sw, offL, status);
-    dense_tri_inverse<<<dim3((nV + 63) / 64, n), 64, 0, st>>>(nV, work, sw, offL, offLinv);
-    // Hinv = Linv' Linv: element (i, k) of the left operand is Linv[k][i] (strides 1, nV); the triangular zeros are
-    // multiplied through (2x the flops of the triangular sum, at several times its speed)
-    dense_gemm_launch(use_dmma, n, nV, nV, nV, work + offLinv, sw, 1, nV, work + offLinv, sw, 1, nV, HD, shd, st);
-    if (nC > 0) {
-        // D (nC x nV) = A (nC x nV) * Hinv' (Hinv symmetric, row-major over k)
-        dense_gemm_launch(use_dmma, n, nC, nV, nV, A, cv, nV, 1, HD, shd, nV, 1, HD + vv, shd, st);
-        // S (nC x nC) = A * D'
-        dense_gemm_launch(use_dmma, n, nC, nC, nV, A, cv, nV, 1, HD + vv, shd, nV, 1, S, ss, st);
+    for (int p0 = 0; p0 < n; p0 += DENSE_GRID_YZ) {
+        const int k = n - p0 < DENSE_GRID_YZ ? n - p0 : DENSE_GRID_YZ;
+        double* wk = work + (size_t)p0 * sw;
+        double* hd = HD + (size_t)p0 * shd;
+        const double* Ak = A + (size_t)p0 * cv;
+        dense_tri_inverse<<<dim3((nV + 63) / 64, k), 64, 0, st>>>(nV, wk, sw, offL, offLinv);
+        // Hinv = Linv' Linv: element (i, k) of the left operand is Linv[k][i] (strides 1, nV); the triangular zeros are
+        // multiplied through (2x the flops of the triangular sum, at several times its speed)
+        dense_gemm_launch(use_dmma, k, nV, nV, nV, wk + offLinv, sw, 1, nV, wk + offLinv, sw, 1, nV, hd, shd, st);
+        if (nC > 0) {
+            // D (nC x nV) = A (nC x nV) * Hinv' (Hinv symmetric, row-major over k)
+            dense_gemm_launch(use_dmma, k, nC, nV, nV, Ak, cv, nV, 1, hd, shd, nV, 1, hd + vv, shd, st);
+            // S (nC x nC) = A * D'
+            dense_gemm_launch(use_dmma, k, nC, nC, nV, Ak, cv, nV, 1, hd + vv, shd, nV, 1, S + (size_t)p0 * ss, ss, st);
+        }
     }
 }
 
 // The seam's per-call set-up: H copied into each problem's slice (layout l; Hinv and D are adjacent there, as in a set),
-// factored there.
+// factored there; both in slices of at most DENSE_GRID_YZ problems, as dense_factor.
 static void dense_setup_launch(int n, int nV, int nC, const double* H, const double* A, const DenseLayout& l, double* work,
                                int32_t* status, int use_dmma, cudaStream_t st)
 {
     const size_t vv = (size_t)nV * nV;
-    dense_copy_H<<<dim3((unsigned)((vv + 255) / 256), n), 256, 0, st>>>(nV, H, work, l.total, l.Lh);
+    for (int p0 = 0; p0 < n; p0 += DENSE_GRID_YZ) {
+        const int k = n - p0 < DENSE_GRID_YZ ? n - p0 : DENSE_GRID_YZ;
+        dense_copy_H<<<dim3((unsigned)((vv + 255) / 256), k), 256, 0, st>>>(nV, H + (size_t)p0 * vv, work + (size_t)p0 * l.total,
+                                                                           l.total, l.Lh);
+    }
     dense_factor(n, nV, nC, A, work, l.total, l.Lh, l.Linv, work + l.Hinv, l.total, work + l.S, l.total, status, use_dmma, st);
 }
 
