@@ -274,6 +274,49 @@ typedef struct {
  * of this handle is in flight. */
 int ismpc_formc_set_instances(ismpc_handle* h, const ismpc_formc_inst_t* inst, int n, int mem);
 
+/* Gradients of one form-C tick with respect to the inputs of its record and the footstep plan: the adjoint of
+ * ismpc_formc_solve_batch at the solution that call returned for the same records (state, walk, inst and plan_xyzt
+ * passed explicitly; resident instances and plans are not used by this call).  No QP is re-solved: the forward's
+ * intermediates are rebuilt from the records and primal / active, and the chain runs backwards through the integration
+ * (lambda_0, x, y state, u_0, f_0), the x and y QPs (closed form on the reported saturation sets: free rows
+ * u = mid + nu a, saturated rows u = mid +- rho), their right-hand sides (state, the anticipative tails, eta), the
+ * stability row a = C_sc A_{N-1}...A_{i+1} B_i (eta through C_sc = [1, 1/eta], lambda through A_i, B_i), lambda_k =
+ * f_k / (m z_pos_k) with z_pos = S_bar f + base (z0, zd0), and the vertical QP: H_z p + A_W' q = f_bar, A_W p = 0 with
+ * W = the flight-phase equalities and the S_bar rows the forward reported active, dL/dF_z = -p, F_z affine in z0, zd0,
+ * com_height and the window's mid_z.  eta = sqrt(g / com_height) collects every eta term into com_height.
+ *   primal, active: the forward's primal_opt / active_opt for these records (n x 3N).  Where strict complementarity
+ *   fails the result is the derivative for the working set the forward reported, as in ismpc_qp_adjoint_batch and
+ *   ismpc_forma_adjoint_batch.  Vertical working-set entries dependent on those before them are skipped (q = 0).
+ *   v_next (nullable): n x 9, dL/d out.next (com_pos, com_vel, zmp_pos; zmp_pos is carried through, its gradient is the
+ *   identity).  v_primal (nullable): n x 3N, dL/d primal; out.zmp_in and out.fz0 are primal entries [N], [2N] and [0]:
+ *   add their gradient there.  out.lambda0 and out.kkt_res are not differentiated.  Both NULL: zero gradients.
+ *   grad: n records, overwritten.  grad_plan (nullable): plan_rows x 4 in the plan_xyzt layout, dL/d plan ACCUMULATED
+ *   into (+=) in columns x, y, z (column t is never written); each instance adds its sum for a plan row once, so the
+ *   bytes are reproducible when no two instances share plan rows; rows shared by instances receive the sum of their
+ *   contributions in an unspecified order.
+ *   grad[i].status: 0; ISMPC_ST_WINDOW for a record the forward skips (window beyond the plan, plan rows outside the
+ *   table): zero gradients, no plan row touched; ISMPC_ST_Z_FAIL when the reported vertical working set does not fit the
+ *   factor (48 entries): zero gradients.
+ *   Gradients of a forward whose out.status has a bit of ST_FAIL_MASK (Z / X / Y fail, window) or ISMPC_ST_NAN_GUARD are
+ *   meaningless, and such a record's intermediates may be NaN and reach its plan rows: leave it out of the call
+ *   (formc_torch does).  ISMPC_ST_XY_SKIPPED is a regular case (u = 0, no horizontal gradients).
+ *   mem: ISMPC_MEM_HOST or ISMPC_MEM_DEVICE.  Every argument is checked before the device is touched; ISMPC_ERR_MODEL
+ *   without ismpc_formc_set_model. */
+typedef struct {
+    ismpc_state_t state;        /* dL/d(com_pos, com_vel, zmp_pos) of the record */
+    double com_height, box_w, box_w_init;
+    int32_t status, reserved;   /* 0, ISMPC_ST_WINDOW (record skipped as the forward skips it), or
+                                   ISMPC_ST_Z_FAIL (reported vertical working set does not fit FORMC_QMAX) */
+} ismpc_formc_grad_t;           /* 104 bytes */
+
+int ismpc_formc_adjoint_batch(ismpc_handle* h, int n,
+                              const ismpc_state_t* state, const ismpc_walk_t* walk, const ismpc_formc_inst_t* inst,
+                              const double* plan_xyzt, int plan_rows,
+                              const double* primal, const int8_t* active,
+                              const double* v_next, const double* v_primal,
+                              ismpc_formc_grad_t* grad, double* grad_plan,
+                              int mem, void* stream);
+
 /* ismpc_formc_solve_batch with the per-tick arguments packed: tick[i] = {state, walk} of instance i (128-byte records;
  * the array must be 16-byte aligned).  inst / plan_xyzt may be NULL (= the resident ones), results are bit-identical to
  * ismpc_formc_solve_batch on the same values.

@@ -24,7 +24,7 @@ EXPORTS = ["ismpc_version", "ismpc_error_string", "ismpc_create", "ismpc_destroy
            "ismpc_formc_solve_batch_packed", "ismpc_qp_solve_batch_ws", "ismpc_qp_set_matrices",
            "ismpc_qp_hotstart_batch", "ismpc_forma_solve_batch_ws", "ismpc_qp_solve_batch_bounds",
            "ismpc_qp_hotstart_batch_bounds", "ismpc_qp_adjoint_batch", "ismpc_qp_hotstart_adjoint_batch",
-           "ismpc_forma_adjoint_batch"]
+           "ismpc_forma_adjoint_batch", "ismpc_formc_adjoint_batch"]
 
 _lib = None
 
@@ -75,6 +75,7 @@ def lib():
     L.ismpc_formc_set_plan.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
     L.ismpc_formc_set_model.argtypes = [C.c_void_p, C.c_void_p]
     L.ismpc_formc_solve_batch.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
+    L.ismpc_formc_adjoint_batch.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 6 + [C.c_int, C.c_void_p]
     L.ismpc_formc_set_instances.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
     L.ismpc_formc_solve_batch_packed.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
     L.ismpc_formc_rollout.argtypes = [C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
@@ -267,6 +268,32 @@ class Handle:
                                              _ptr(out), _ptr(primal), _ptr(active), mem,
                                              C.c_void_p(stream) if stream else None)
         self._check(rc, "ismpc_formc_solve_batch")
+
+    def formc_adjoint_batch_raw(self, n, state, walk, inst, plan, plan_rows, primal, active, grad, v_next=None,
+                                v_primal=None, grad_plan=None, mem=abi.MEM_DEVICE, stream=None):
+        """Raw ismpc_formc_adjoint_batch: every array is a numpy array (host), an integer address (device) or None."""
+        rc = self._L.ismpc_formc_adjoint_batch(self._h, n, _ptr(state), _ptr(walk), _ptr(inst), _ptr(plan), plan_rows,
+                                               _ptr(primal), _ptr(active), _ptr(v_next), _ptr(v_primal), _ptr(grad),
+                                               _ptr(grad_plan), mem, C.c_void_p(stream) if stream else None)
+        self._check(rc, "ismpc_formc_adjoint_batch")
+
+    def formc_adjoint_batch(self, state, walk, inst, plan, primal, active, v_next=None, v_primal=None, want_plan=True):
+        """Gradients of a form-C tick (ismpc_formc_adjoint_batch) at the solution the forward returned for these records:
+        primal / active are its "primal" / "active", v_next (n x 9: com_pos, com_vel, zmp_pos of out["next"]) and
+        v_primal (n x 3N) the upstream gradients (either may be None).  Returns dict(grad = FORMC_GRAD records,
+        plan = dL/d plan (rows x 4, column t zero) or None without want_plan)."""
+        n = len(state)
+        N = int(self.formc["N"][0])
+        plan = np.ascontiguousarray(plan, dtype=np.float64)
+        f64 = lambda a, shape, name: None if a is None else _shaped(a, np.float64, shape, name)
+        primal = _shaped(primal, np.float64, (n, 3 * N), "primal")
+        active = _shaped(active, np.int8, (n, 3 * N), "active")
+        v_next, v_primal = f64(v_next, (n, 9), "v_next"), f64(v_primal, (n, 3 * N), "v_primal")
+        grad = np.zeros(n, dtype=abi.FORMC_GRAD)
+        gplan = np.zeros_like(plan) if want_plan else None
+        self.formc_adjoint_batch_raw(n, np.ascontiguousarray(state), np.ascontiguousarray(walk), np.ascontiguousarray(inst),
+                                     plan, plan.shape[0], primal, active, grad, v_next, v_primal, gplan, mem=abi.MEM_HOST)
+        return dict(grad=grad, plan=gplan)
 
     def formc_set_instances(self, inst, mem=abi.MEM_HOST, n=None):
         """Per-instance constants resident in the handle (inst=None forgets them); afterwards inst=None in the tick calls."""

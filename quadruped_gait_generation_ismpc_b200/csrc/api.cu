@@ -50,6 +50,8 @@ struct ismpc_handle {
     ismpc_formc_model_t cm{};
     DevBuf c_tables, c_work, c_info;
     DevBuf c_ric_none, c_ric_gait, c_law_none, c_law_gait, c_ws, c_plan, c_inst;
+    DevBuf c_adj_ws;               // per-warp workspace of ismpc_formc_adjoint_batch (its own: a tick may run on another stream)
+    int adj_res = 0;               // resident CTAs of the adjoint kernel for the current model, 0 = not queried
     int inst_res_n = 0;            // instance records resident in c_inst (ismpc_formc_set_instances), 0 = none
     int opt_host_zero_copy = 1;    // packed host-memory ticks: the kernel reads / writes the caller's pinned buffers itself
     int plan_res_rows = 0;         // rows of the resident footstep-plan table (ismpc_formc_set_plan), 0 = none
@@ -322,7 +324,7 @@ extern "C" int ismpc_formc_set_model(ismpc_handle* h, const ismpc_formc_model_t*
     if (rc) return fail_cuda(h, (cudaError_t)rc, "formc_law_launch");
     CK(cudaStreamSynchronize(0));
     h->cm = *m;
-    h->ric_S = h->ric_F = 0; h->w_res[0] = 0;
+    h->ric_S = h->ric_F = 0; h->w_res[0] = 0; h->adj_res = 0;
     h->formc_ready = true;
     return ISMPC_OK;
 }
@@ -468,6 +470,49 @@ extern "C" int ismpc_formc_solve_batch(ismpc_handle* h, int n, const ismpc_state
     a.active = (signed char*)s.out(active_opt, n * N3, mb * N3);
     if (s.err) return s.err;
     return s.finish(formc_launch_tick(h, a, n, s.st), "formc_tick_launch");
+}
+
+// The adjoint of a tick.  grad_plan is staged with the caller's bytes (it is accumulated into); grad is overwritten.
+extern "C" int ismpc_formc_adjoint_batch(ismpc_handle* h, int n, const ismpc_state_t* state, const ismpc_walk_t* walk,
+                                         const ismpc_formc_inst_t* inst, const double* plan_xyzt, int plan_rows,
+                                         const double* primal, const int8_t* active, const double* v_next,
+                                         const double* v_primal, ismpc_formc_grad_t* grad, double* grad_plan, int mem,
+                                         void* stream)
+{
+    if (!h) return ISMPC_ERR_ARG;
+    if (n < 0 || n > h->max_batch || !state || !walk || !inst || !plan_xyzt || plan_rows <= 0 || !primal || !active ||
+        !grad || (mem != ISMPC_MEM_HOST && mem != ISMPC_MEM_DEVICE))
+        return ISMPC_ERR_ARG;
+    if (!h->formc_ready) return ISMPC_ERR_MODEL;
+    if (n == 0) return ISMPC_OK;
+    CK(cudaSetDevice(h->device));
+    const int N = h->cm.N;
+    if (h->adj_res <= 0) {
+        const int r = formc_adjoint_resident(N, h->sm_count);
+        if (r <= 0) return fail_cuda(h, (cudaError_t)(-r), "formc_adjoint_resident");
+        h->adj_res = r;
+    }
+    const int grid = n < h->adj_res ? n : h->adj_res;
+    const size_t stride = formc_adjoint_ws_stride(N);
+    if (h->c_adj_ws.ensure((size_t)grid * stride * sizeof(double))) return ISMPC_ERR_ALLOC;
+    const size_t mb = (size_t)h->max_batch, N3 = 3 * (size_t)N, NN = (size_t)N * N;
+    Staged s(h, mem, stream, false);
+    FormCAdjArgs a;
+    const double* T = (const double*)h->c_tables.p;
+    a.n = n; a.model = h->cm; a.Hinv = T; a.G = T + NN; a.M = T + 2 * NN;
+    a.plan_rows = plan_rows; a.ws = (double*)h->c_adj_ws.p; a.ws_stride = stride;
+    a.grad = s.out(grad, n, mb);
+    a.grad_plan = s.inout(grad_plan, (size_t)plan_rows * 4);
+    a.state = s.in(state, n, mb);
+    a.walk = s.in(walk, n, mb);
+    a.inst = s.in(inst, n, mb);
+    a.plan = s.in(plan_xyzt, (size_t)plan_rows * 4);
+    a.primal = s.in(primal, n * N3, mb * N3);
+    a.active = (const signed char*)s.in(active, n * N3, mb * N3);
+    a.v_next = s.in(v_next, (size_t)n * 9, mb * 9);
+    a.v_primal = s.in(v_primal, n * N3, mb * N3);
+    if (s.err) return s.err;
+    return s.finish(formc_adjoint_launch(a, grid, s.st), "formc_adjoint_launch");
 }
 
 extern "C" int ismpc_formc_set_instances(ismpc_handle* h, const ismpc_formc_inst_t* inst, int n, int mem)

@@ -52,6 +52,30 @@ struct FormAAdjArgs {
 };
 void forma_adjoint_plan(const ismpc_forma_model_t& m, int sm_count, long long items, FormALaunchPlan* p);
 int forma_adjoint_launch(const FormAAdjArgs& a, const FormALaunchPlan& p, double* Jspill, cudaStream_t st);
+// the adjoint of a form-C tick (ismpc_formc_adjoint_batch, formc_adjoint_kernels.cu): one warp per instance, persistent
+struct FormCAdjArgs {
+    int n;
+    ismpc_formc_model_t model;
+    const double* Hinv;             // H_z^-1, S_bar H_z^-1, S_bar H_z^-1 S_bar' of the model (FormCTables order)
+    const double* G;
+    const double* M;
+    const ismpc_state_t* state;
+    const ismpc_walk_t* walk;
+    const ismpc_formc_inst_t* inst;
+    const double* plan;
+    int plan_rows;
+    const double* primal;
+    const signed char* active;
+    const double* v_next;           // nullable, n x 9
+    const double* v_primal;         // nullable, n x 3N
+    ismpc_formc_grad_t* grad;
+    double* grad_plan;              // nullable, plan_rows x 4
+    double* ws;                     // grid x formc_adjoint_ws_stride(N) doubles
+    size_t ws_stride;
+};
+size_t formc_adjoint_ws_stride(int N);
+int formc_adjoint_resident(int N, int sm_count);        // resident CTAs (> 0), or minus a cudaError_t
+int formc_adjoint_launch(const FormCAdjArgs& a, int grid, cudaStream_t st);
 int plan_generate_launch(int n, const ismpc_plan_model_t& m, const ismpc_plan_req_t* req, double* foot_plan, double* center,
                          int rows, cudaStream_t st);
 int kf_filter_launch(int n, int n_steps, const ismpc_kf_model_t& m, ismpc_kf_state_t* state, const ismpc_kf_sample_t* samples,

@@ -2,6 +2,7 @@
 #include "api.cu"
 #include "formc_kernels.cu"
 #include "formc_warp_kernels.cu"
+#include "formc_adjoint_kernels.cu"
 #include "forma_kernels.cu"
 #include "qp_dense.cu"
 #include "feet_kernels.cu"

@@ -3,6 +3,7 @@
 formc_batch  -- config 2: independent trot instances for MPCSolver::solve (formulation C)
 forma_batch  -- configs 2/3: trot / walk instances for the canonical ISMPC (formulation A) at the
                 start-of-gait state (tick j = 1); mid-gait states are produced by rolling these forward
+formc_next_walk -- the next tick's formulation-C walk records (the Controller's bookkeeping between ticks)
 forma_next_records -- the next tick's formulation-A records from a tick's results (a caller-driven closed loop)
 """
 import numpy as np
@@ -83,6 +84,26 @@ def formc_batch(n, seed=SEED0 ^ 2, N=100, n_steps=40, S=35, F_ds=10, vary_height
         inst["S"][i] = S; inst["F_ds"][i] = F_ds
         inst["plan_first_row"][i] = i * n_steps; inst["n_steps"][i] = n_steps
     return state, walk, inst, plan
+
+
+def formc_next_walk(walk, inst, plan, model=None):
+    """The walk records of the next form-C tick, as the Controller keeps them (Controller.cpp:297-302, 503-504) and as
+    ismpc_formc_rollout advances them: control_iter += 1, mpc_iter = floor(control_iter * dtc / dt) with dt and dtc of
+    `model` (abi.formc_model(); None: the defaults, dtc = dt), sim_time += 1, then the footstep switch -- once sim_time
+    reaches the next footstep's time minus one tick (plan column t), control_iter and mpc_iter restart at 0,
+    footstep_counter advances and the support foot changes.  Returns a new array."""
+    m = abi.formc_model() if model is None else model
+    dt, dtc = float(np.ravel(m["dt"])[0]), float(np.ravel(m["dtc"])[0])
+    wk = walk.copy()
+    wk["control_iter"] += 1
+    wk["mpc_iter"] = np.floor(wk["control_iter"] * dtc / dt).astype(np.int32)
+    wk["sim_time"] += 1
+    for i in range(len(wk)):
+        fc = int(wk["footstep_counter"][i])
+        if fc < inst["n_steps"][i] and wk["sim_time"][i] >= plan[int(inst["plan_first_row"][i]) + fc, 3] - 1:
+            wk["control_iter"][i] = 0; wk["mpc_iter"][i] = 0
+            wk["footstep_counter"][i] += 1; wk["support_foot"][i] = 1 - wk["support_foot"][i]
+    return wk
 
 
 def forma_batch(n, seed=SEED0 ^ 3, gait="trot", C=100, step=50, ds=20, sim_ticks=2000, vary=False,
